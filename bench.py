@@ -12,6 +12,12 @@ n = 2048, d = 8 (S = 256 hyper-parameter vectors per GPU per step), is reported 
 
 `--impl reference` times the CPU restatement of the reference path (oracle/, numpy + OpenBLAS with all host
 threads) on a bounded sample of the same workload; Julia is not installed, so the reference itself cannot run.
+
+`--dump-outputs DIR` writes, after the timed steps, what each timed path returned to its caller in its last step as
+DIR/<name>.npy (float64; argmax indices are stored as float64, exact below 2^53): the (best value, index) pair of the
+resident, pinned and pageable EI scoring passes, the S log-likelihoods, and the log-likelihoods and (S, d + 2)
+gradients of the value + gradient pass.  Every input is seeded, so two builds run with the same arguments can be
+compared output for output.  Under torchrun every rank writes its own files, suffixed _rank<r>.
 """
 import argparse
 import json
@@ -25,6 +31,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it (it may be read-only)
 
 N_TRAIN, X_DIM, KERNEL_ID = 2048, 8, 2
 M_PER_GPU = 1 << 21
@@ -105,9 +112,18 @@ def use_all_host_threads():
 
 
 def cpu_score_once(post, Xs, best):
+    """-> (best value, index), the pair the GPU path returns."""
     from oracle import boss_oracle as O
     acq, _, _ = O.ei_acquisition([[post]], Xs, [1.0], best, None)
-    return O.julia_argmax_fast(acq)
+    bi = O.julia_argmax_fast(acq)
+    return float(acq[bi]), bi
+
+
+def dump_outputs(out_dir, outputs, suffix=""):
+    """Each output as out_dir/<name><suffix>.npy in float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def cpu_baseline(budget_s=12.0):
@@ -158,8 +174,10 @@ def run_reference(args):
         cpu_score_once(post, Xs[:, :2048], best)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cpu_score_once(post, Xs, best)
+        res = cpu_score_once(post, Xs, best)
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"ei_best_value": [res[0]], "ei_best_index": [res[1]]})
     val = CPU_SAMPLE_M / dt
     # mode A beside it: what BOSS.jl's maximizers actually do - one candidate per call (grid.jl:52-53)
     t1 = time.perf_counter(); k = 0
@@ -342,8 +360,11 @@ def run_gpu(args):
             ms = float(t.item())
         return ms / steps, launches, out
 
+    suffix = f"_rank{rank}" if world > 1 else ""
     if args.only == "loglik":          # profiling aid: only the batched log-likelihood step
         ms_ll, launches_ll, _ = timed(step_loglik, args.steps, args.warmup)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"loglik": t_ll.cpu().numpy()}, suffix)
         if rank == 0:
             print(json.dumps({"only": "loglik", "ms_per_step": ms_ll, "evals_per_s": S * world / (ms_ll * 1e-3),
                               "gpu_launches": int(launches_ll)}), file=args.out, flush=True)
@@ -361,8 +382,15 @@ def run_gpu(args):
     ms_ll_serial, _, _ = timed(step_loglik, 2, 3)
     chol_ms, chol_cnt = _lib.last_kernel_ms(2)
     _lib.set_timing(False)
+    ll_out = t_ll.cpu().numpy()                                               # step_loglik_grad overwrites t_ll
     ms_llg, launches_llg, _ = timed(step_loglik_grad, max(2, args.steps // 2), 3)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {
+            "ei_best_value": [res[0]], "ei_best_index": [res[1]],
+            "ei_e2e_best_value": [res_e2e[0]], "ei_e2e_best_index": [res_e2e[1]],
+            "ei_e2e_pageable_best_value": [res_e2e_pg[0]], "ei_e2e_pageable_best_index": [res_e2e_pg[1]],
+            "loglik": ll_out, "loglik_grad_value": t_ll.cpu().numpy(), "loglik_grad": t_gr.cpu().numpy()}, suffix)
     # one candidate per call -- the access pattern of the reference's stock maximizers (acq(x) inside NLopt / Optim,
     # grid.jl:52-53): host-pointer C-ABI calls, wall time per call (H2D of the point, all kernels, D2H of the result)
     x1 = np.ascontiguousarray(Xs_pageable[:, :1])
@@ -490,7 +518,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the C3/C4/C5 per-config numbers (N=1 only)")
     ap.add_argument("--only", default="all", choices=["all", "loglik"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     with StdoutToStderr() as real_stdout:
         args.out = real_stdout
