@@ -80,6 +80,7 @@ EXPORTS = {
     "boss_dbg_kernel_fn": (C.c_int, [C.c_int, _vp, C.c_int, _vp]),
     "boss_dbg_check_redzones": (C.c_int64, [_i64p]),
     "boss_dbg_redzone_selftest": (C.c_int64, []),
+    "boss_dbg_screen_stats": (C.c_int, [_i64p]),
 }
 for _name, (_res, _args) in EXPORTS.items():
     _f = getattr(lib, _name)          # AttributeError here = header and library disagree
@@ -534,3 +535,11 @@ def dbg_check_redzones():
     n = C.c_int64(0)
     bad = lib.boss_dbg_check_redzones(C.byref(n))
     return int(bad), int(n.value)
+
+
+def dbg_screen_stats():
+    """Argmax screening of the last scoring call on the current device: (state, candidates bounded, survivors);
+    state 0 = not screened, 1 = screened, 2 = fell back to the full path after the first chunk."""
+    out = (C.c_int64 * 3)()
+    _check(lib.boss_dbg_screen_stats(out), "boss_dbg_screen_stats")
+    return int(out[0]), int(out[1]), int(out[2])

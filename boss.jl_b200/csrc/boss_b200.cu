@@ -134,6 +134,8 @@ struct Ctx {
   DevBuf ks, muv, sumsq, xs_stage, pm_stage, cm_stage, acq_stage, mu_stage, var_stage, st_stage, grad_stage;
   DevBuf blk_val, blk_idx, small, chol_L, chol_Winv, chol_misc, tt, vt, ut, dmu, dvar, pmg_stage;
   DevBuf part_mu, part_ss, part_gm, part_gv, cov_p, cov_stage, chol_W, chol_WT, ll_vec, ll_part, ms_buf;   // split-invariant partial sums (score.cuh / grad.cuh)
+  DevBuf scr_misc, scr_pool;         // argmax screening: bounds, counts, seed batch / survivor pool (score_core)
+  int64_t scr_stats[3] = {0, 0, 0};  // last scoring call: screened (1) or fell back (2), candidates bounded, pool size
   // event pool for per-kernel-class timing
   cudaEvent_t ev_a[EV_POOL], ev_b[EV_POOL];
   int ev_class[EV_POOL];
@@ -1137,6 +1139,60 @@ struct Stager {
   }
 };
 
+// Argmax screening (DESIGN.md 2.9) runs for calls of at least this many candidates (BOSS_SCREEN_MIN_M overrides, read
+// per call): below it the bounds, the seed batch and the two waits of the first chunk are a visible share of the call.
+constexpr long long SCREEN_MIN_M = 65536;
+constexpr size_t SCREEN_POOL_BYTES = (size_t)1 << 30;   // pool for every candidate of the call; larger calls are not screened
+constexpr double SCREEN_MIN_T = 0x1p-960;   // below it the EI evaluations lose relative precision (DESIGN.md 2.9)
+long long screen_min_m() {
+  const char *e = getenv("BOSS_SCREEN_MIN_M");
+  return e ? atoll(e) : SCREEN_MIN_M;
+}
+
+// device buffers of a screened call: the bounds of one chunk, per-256 survivor counts, the pool size (two slots),
+// the seed selection (two ping-pong rounds), the seed batch and the survivor pool
+struct ScreenBufs {
+  double *bound = nullptr, *seed_x = nullptr, *seed_pm = nullptr, *pool_x = nullptr, *pool_pm = nullptr;
+  int *cnt = nullptr, *ti[2] = {};
+  unsigned long long *tk[2] = {};
+  long long *base = nullptr, *pool_idx = nullptr;
+  unsigned char *seed_cm = nullptr, *pool_cm = nullptr;
+  int setup(long long M, int CH, int d, int y_dim, bool pm, bool cm) {
+    size_t tot = 0;
+    auto take = [&tot](size_t bytes) {
+      const size_t o = tot;
+      tot += (bytes + 255) / 256 * 256;
+      return o;
+    };
+    const size_t ntk = (size_t)(CH + TOPK_IN - 1) / TOPK_IN * SEED_N;
+    const size_t o_bound = take((size_t)CH * 8), o_cnt = take((size_t)(CH + 255) / 256 * 4), o_base = take(16);
+    const size_t o_tk0 = take(ntk * 8), o_tk1 = take(ntk * 8), o_ti0 = take(ntk * 4), o_ti1 = take(ntk * 4);
+    const size_t o_sx = take((size_t)SEED_N * d * 8), o_spm = take((size_t)SEED_N * y_dim * 8), o_scm = take(SEED_N);
+    CUDA_TRY(C().scr_misc.ensure(tot));
+    unsigned char *b = C().scr_misc.as<unsigned char>();
+    bound = reinterpret_cast<double *>(b + o_bound);
+    cnt = reinterpret_cast<int *>(b + o_cnt);
+    base = reinterpret_cast<long long *>(b + o_base);
+    tk[0] = reinterpret_cast<unsigned long long *>(b + o_tk0);
+    tk[1] = reinterpret_cast<unsigned long long *>(b + o_tk1);
+    ti[0] = reinterpret_cast<int *>(b + o_ti0);
+    ti[1] = reinterpret_cast<int *>(b + o_ti1);
+    seed_x = reinterpret_cast<double *>(b + o_sx);
+    seed_pm = reinterpret_cast<double *>(b + o_spm);
+    seed_cm = b + o_scm;
+    tot = 0;
+    const size_t o_px = take((size_t)M * d * 8), o_pidx = take((size_t)M * 8);
+    const size_t o_ppm = pm ? take((size_t)M * y_dim * 8) : 0, o_pcm = cm ? take((size_t)M) : 0;
+    CUDA_TRY(C().scr_pool.ensure(tot));
+    b = C().scr_pool.as<unsigned char>();
+    pool_x = reinterpret_cast<double *>(b + o_px);
+    pool_idx = reinterpret_cast<long long *>(b + o_pidx);
+    pool_pm = pm ? reinterpret_cast<double *>(b + o_ppm) : nullptr;
+    pool_cm = cm ? b + o_pcm : nullptr;
+    return 0;
+  }
+};
+
 int score_core(ScoreArgs &a) {
   const int nsl = a.y_dim * a.n_samples;
   if (nsl < 1 || a.y_dim > MAX_YDIM) return fail(BOSS_ERR_ARG, "score: y_dim must be in 1..16");
@@ -1223,6 +1279,128 @@ int score_core(ScoreArgs &a) {
     CUDA_TRY(cudaStreamSynchronize(C().stream));
     mixp.eps = C().tt.as<double>();
   }
+
+  // ---- argmax screening (DESIGN.md 2.9): a call that wants only the argmax of the closed-form EI over many
+  // candidates bounds every candidate from its mean alone and scores exactly only those that can still win ----
+  if (!a.internal) C().scr_stats[0] = C().scr_stats[1] = C().scr_stats[2] = 0;
+  const size_t pool_row = (size_t)d * 8 + (a.prior_mean ? (size_t)a.y_dim * 8 : 0) + 8 + (a.cons_mask ? 1 : 0);
+  bool screen = a.want_argmax && a.best && !a.internal && !a.acq && !a.grad && !a.mu_out && !a.var_out && !a.status_out &&
+                !a.mix && a.M >= screen_min_m() && (size_t)a.M * pool_row <= SCREEN_POOL_BYTES &&
+                getenv("BOSS_NO_SCREEN") == nullptr;
+  ScreenBufs sc;
+  double thr = -INFINITY;   // survivors: bound >= thr or NaN
+  if (screen) {
+    int rc = sc.setup(a.M, CH, d, a.y_dim, a.prior_mean != nullptr, a.cons_mask != nullptr);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemsetAsync(sc.base, 0, 16, C().stream));
+  }
+  // one chunk of a screened call: the means of every slice (xcov without K*^T), the bounds, the survivors appended to
+  // the pool.  The first chunk also sets the threshold from the seed batch and ends screening (the chunk is then scored
+  // on the full path from the same staged inputs) when the bound does not separate: T not positive, or more than a
+  // quarter of the chunk surviving.
+  auto screen_chunk = [&](AcqParams ap, const double *xs_dev, long long in_off, int cidx) -> int {
+    const long long m0 = ap.m0;
+    const int ch = ap.chunk, ncb = (ch + 127) / 128, nb = (ch + 255) / 256;
+    for (int q = 0; q < nsl; ++q) {
+      const boss_gp *h = sl[q];
+      XcovParams xp{};
+      xp.Xs = xs_dev;
+      xp.M = a.M;
+      xp.m0 = m0;
+      xp.in_off = in_off;
+      xp.d = d;
+      xp.n = h->n;
+      xp.n_pad = h->n_pad;
+      xp.ktiles = h->ktiles;
+      xp.Xt = h->Xt;
+      xp.invl = h->invl;
+      xp.disc_bits = h->disc;
+      xp.alpha = h->alpha;
+      xp.a2 = h->a2;
+      xp.Ks = C().ks.as<double>();
+      xp.mu_part = C().part_mu.as<double>();
+      xp.ld = CH;
+      const int nks = std::max(1, std::min(h->nblk, (16 * 148 + ncb - 1) / ncb));
+      {
+        Timed t(1);
+        launch_xcov_mean(h->kernel_id, h->dp, xp, dim3(ncb, nks), C().stream);
+      }
+      reduce_rows_kernel<<<(ncb * 128 + 255) / 256, 256, 0, C().stream>>>(C().part_mu.as<double>(), 2 * h->nblk, (size_t)CH,
+                                                                        C().muv.as<double>() + (size_t)q * CH, ncb * 128);
+    }
+    AcqParams bp = ap;   // EI at the prior variance, PoF = 1, no guards -> sc.bound[c]
+    bp.sumsq = nullptr;
+    bp.has_ymax = 0;
+    bp.lb = bp.ub = nullptr;
+    bp.cons_mask = nullptr;
+    bp.acq = sc.bound;
+    bp.out_off = m0;
+    bp.blk_val = nullptr;
+    bp.blk_idx = nullptr;
+    acq_kernel<<<nb, 256, 0, C().stream>>>(bp);
+    C().launches += 2 * nsl + 1;
+    const size_t c0 = (size_t)(m0 - ap.in_off);   // the chunk's first candidate in the input arrays
+    const double *xs_c = ap.Xs + c0 * d;
+    const double *pm_c = ap.prior_mean ? ap.prior_mean + c0 * a.y_dim : nullptr;
+    const unsigned char *cm_c = ap.cons_mask ? ap.cons_mask + c0 : nullptr;
+    if (cidx == 0) {
+      // seed: the exact scores of the SEED_N highest bounds; the best of them is a lower bound of the maximum
+      int n = ch, par = 0;
+      const unsigned long long *kin = nullptr;
+      const int *iin = nullptr;
+      do {
+        const int nbk = (n + TOPK_IN - 1) / TOPK_IN;
+        seed_topk_kernel<<<nbk, 1024, 0, C().stream>>>(kin ? nullptr : sc.bound, kin, iin, n, sc.tk[par], sc.ti[par]);
+        ++C().launches;
+        kin = sc.tk[par];
+        iin = sc.ti[par];
+        par ^= 1;
+        n = nbk * SEED_N;
+      } while (n > SEED_N);
+      const int ns = std::min(SEED_N, ch);
+      seed_gather_kernel<<<1, SEED_N, 0, C().stream>>>(iin, ns, xs_c, pm_c, cm_c, d, a.y_dim, sc.seed_x, sc.seed_pm, sc.seed_cm);
+      ++C().launches;
+      ScoreArgs s = a;
+      s.Xs = sc.seed_x;
+      s.M = ns;
+      s.prior_mean = pm_c ? sc.seed_pm : nullptr;
+      s.cons_mask = cm_c ? sc.seed_cm : nullptr;
+      s.gen = nullptr;
+      s.dev = true;
+      s.internal = true;
+      double T = 0.0;
+      int64_t ti = -1;
+      s.best_val = &T;
+      s.best_idx = &ti;
+      int rc = score_core(s);
+      if (rc) return rc;
+      // the seed call used this call's small block (a^2, bounds, running winner): restore it for the rest of the call
+      CUDA_TRY(cudaMemcpyAsync(small, hs.data(), sm_n * 8, cudaMemcpyHostToDevice, C().stream));
+      C().scr_stats[1] = ch;
+      if (!(T >= SCREEN_MIN_T)) {
+        C().scr_stats[0] = 2;
+        screen = false;
+        return 0;
+      }
+      thr = T * (1.0 - 0x1p-30);
+    }
+    screen_count_kernel<<<nb, 256, 0, C().stream>>>(sc.bound, ch, thr, sc.cnt);
+    CompactParams cpar{sc.bound, ch, thr, sc.cnt, m0, xs_c, pm_c, cm_c, d, a.y_dim, sc.base, cidx & 1,
+                     sc.pool_x, sc.pool_pm, sc.pool_cm, sc.pool_idx};
+    screen_compact_kernel<<<nb, 256, 0, C().stream>>>(cpar);
+    C().launches += 2;
+    if (cidx == 0) {
+      long long surv = 0;
+      CUDA_TRY(cudaMemcpyAsync(&surv, sc.base + 1, 8, cudaMemcpyDeviceToHost, C().stream));
+      CUDA_TRY(cudaStreamSynchronize(C().stream));
+      C().scr_stats[2] = surv;
+      if (4 * surv > ch) {
+        C().scr_stats[0] = 2;
+        screen = false;
+      }
+    }
+    return 0;
+  };
 
   // ---- host staging plan (two slots): byte offsets of every array inside a slot ----
   const bool host = !a.dev;
@@ -1387,7 +1565,11 @@ int score_core(ScoreArgs &a) {
     ap.blk_val = a.want_argmax ? C().blk_val.as<double>() : nullptr;
     ap.blk_idx = a.want_argmax ? C().blk_idx.as<long long>() : nullptr;
     ap.mix = mixp;
-    for (int q = 0; q < nsl; ++q) {
+    if (screen) {
+      int rc = screen_chunk(ap, xs_dev, in_off, cidx);
+      if (rc) return rc;
+    }
+    for (int q = 0; q < nsl && !screen; ++q) {
       const boss_gp *h = sl[q];
       // Small candidate batches (multi-start optimiser iterations, single-point calls) cannot fill 148 SMs
       // with one CTA per 128 candidates: deal the training chunks / W row blocks of a candidate block to
@@ -1525,7 +1707,7 @@ int score_core(ScoreArgs &a) {
         C().launches += 3;
       }
     }
-    if (!fused_chunk) {
+    if (!fused_chunk && !screen) {
       const int nb = (ch + 255) / 256;
       acq_kernel<<<nb, 256, 0, C().stream>>>(ap);
       ++C().launches;
@@ -1560,6 +1742,41 @@ int score_core(ScoreArgs &a) {
     }
   }
   CUDA_TRY(cudaGetLastError());
+  if (screen) {
+    // the pool (survivors in ascending order) through the ordinary path; its first-maximal winner maps back to the
+    // call's index
+    long long npool = 0;
+    CUDA_TRY(cudaMemcpyAsync(&npool, sc.base + (cidx & 1), 8, cudaMemcpyDeviceToHost, C().stream));
+    CUDA_TRY(cudaStreamSynchronize(C().stream));
+    if (host) CUDA_TRY(cudaStreamSynchronize(cp));
+    C().scr_stats[0] = 1;
+    C().scr_stats[1] = a.M;
+    C().scr_stats[2] = npool;
+    if (npool < 1) return fail(BOSS_ERR_STATE, "score: argmax screening kept no candidate");   // the seed's winner always survives
+    ScoreArgs s = a;
+    s.Xs = sc.pool_x;
+    s.M = npool;
+    s.prior_mean = sc.pool_pm;
+    s.cons_mask = sc.pool_cm;
+    s.gen = nullptr;
+    s.dev = true;
+    s.internal = true;
+    double bv = 0.0;
+    int64_t bi = -1;
+    s.best_val = &bv;
+    s.best_idx = &bi;
+    int rc = score_core(s);
+    if (rc) return rc;
+    long long idx = -1;
+    if (bi >= 0) {
+      CUDA_TRY(cudaMemcpyAsync(&idx, sc.pool_idx + bi, 8, cudaMemcpyDeviceToHost, C().stream));
+      CUDA_TRY(cudaStreamSynchronize(C().stream));
+    }
+    a.any_fail = s.any_fail;
+    if (a.best_val) *a.best_val = bv;
+    if (a.best_idx) *a.best_idx = idx;
+    return 0;
+  }
   if (a.internal && !a.want_argmax && !C().timing) {   // a round of the multi-start driver: it synchronises itself
     a.any_fail = 0;
     return 0;
@@ -2778,6 +2995,14 @@ int boss_dbg_factors(const boss_gp *gp, double *L, double *W, double *alpha) {
       for (int c = 0; c < n; ++c) W[(size_t)r * n + c] = buf[p_index(r, c, gp->ktiles)];
   }
   if (alpha) CUDA_TRY(cudaMemcpy(alpha, gp->alpha, (size_t)n * 8, cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+// Argmax screening of the last scoring call on the current device (DESIGN.md 2.9): out[0] = 0 not screened, 1 screened,
+// 2 fell back to the full path after the first chunk; out[1] = candidates bounded; out[2] = candidates that survived.
+int boss_dbg_screen_stats(int64_t *out) {
+  REQUIRE_INIT();
+  for (int i = 0; i < 3; ++i) out[i] = C().scr_stats[i];
   return 0;
 }
 

@@ -145,7 +145,8 @@ __device__ __forceinline__ double acq_candidate(const AcqParams &p, const int c,
         const size_t row = (size_t)(s * p.y_dim + i) * p.chunk_ld + c;
         double mu = p.mu[row];
         if (p.prior_mean) mu = p.prior_mean[(size_t)(m - p.in_off) * p.y_dim + i] + mu;
-        double var = p.a2[s * p.y_dim + i] - p.sumsq[row] + VAR_JITTER;
+        // sumsq == null: the prior variance a^2 + 1e-18, an upper bound of the posterior one (argmax screening)
+        double var = p.a2[s * p.y_dim + i] - (p.sumsq ? p.sumsq[row] : 0.0) + VAR_JITTER;
         const bool ok = clip_var(var);
         if (!ok) failed = true;
         if (p.mu_out) p.mu_out[m - p.out_off] = mu;
@@ -278,6 +279,128 @@ __global__ void argmax_final_kernel(const double *blk_val, const long long *blk_
       *bidx = si[0];
     }
   }
+}
+
+// ---------------------------------------------------------------------------------------------
+// argmax screening (DESIGN.md 2.9).  acq_kernel with sumsq == null and PoF / guards off writes, per candidate, the
+// EI at the prior standard deviation: an upper bound of its acquisition.  A candidate whose bound is below the exact
+// score of some candidate (the best of a small seed batch) cannot be the argmax; the others are compacted, in
+// ascending order, into a pool that the ordinary chunk loop scores.
+// ---------------------------------------------------------------------------------------------
+constexpr int SEED_N = 128;     // seed candidates: the highest bounds of the first chunk
+constexpr int TOPK_IN = 2048;   // elements one CTA of seed_topk_kernel sorts
+
+// larger bound -> larger key; NaN lowest (a NaN bound is kept by the compaction anyway, it is not worth a seed slot)
+__device__ __forceinline__ unsigned long long bound_key(double b) {
+  if (b != b) return 0ull;
+  const unsigned long long u = (unsigned long long)__double_as_longlong(b);
+  return (u >> 63) ? ~u : (u | 0x8000000000000000ull);
+}
+
+// The SEED_N best of each TOPK_IN inputs (key descending, then index ascending) in that order; the inputs are the
+// bounds of a chunk (bounds != null, index = position) or the (key, index) output of an earlier round.
+__global__ void __launch_bounds__(1024) seed_topk_kernel(const double *bounds, const unsigned long long *kin,
+                                                         const int *iin, int n, unsigned long long *kout, int *iout) {
+  __shared__ unsigned long long sk[TOPK_IN];
+  __shared__ int si[TOPK_IN];
+  const int tid = threadIdx.x, base = blockIdx.x * TOPK_IN;
+  for (int e = tid; e < TOPK_IN; e += 1024) {
+    const int g = base + e;
+    unsigned long long k = 0ull;
+    int i = 0x7fffffff;   // padding sorts last
+    if (g < n) {
+      k = bounds ? bound_key(bounds[g]) : kin[g];
+      i = bounds ? g : iin[g];
+    }
+    sk[e] = k;
+    si[e] = i;
+  }
+  for (int k = 2; k <= TOPK_IN; k <<= 1)   // bitonic sort, one compare-exchange per thread and step
+    for (int j = k >> 1; j > 0; j >>= 1) {
+      __syncthreads();
+      const int a = ((tid & ~(j - 1)) << 1) | (tid & (j - 1)), b = a | j;
+      const bool b_first = sk[b] > sk[a] || (sk[b] == sk[a] && si[b] < si[a]);
+      if (b_first == ((a & k) == 0)) {
+        const unsigned long long tk = sk[a];
+        sk[a] = sk[b];
+        sk[b] = tk;
+        const int ti = si[a];
+        si[a] = si[b];
+        si[b] = ti;
+      }
+    }
+  __syncthreads();
+  if (tid < SEED_N) {
+    kout[blockIdx.x * SEED_N + tid] = sk[tid];
+    iout[blockIdx.x * SEED_N + tid] = si[tid];
+  }
+}
+
+// row s of the seed batch = candidate sel[s] of the chunk (xs / pm / cm point at the chunk's first candidate)
+__global__ void seed_gather_kernel(const int *sel, int ns, const double *xs, const double *pm, const unsigned char *cm,
+                                   int d, int y_dim, double *sx, double *spm, unsigned char *scm) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= ns) return;
+  const size_t c = (size_t)sel[s];
+  for (int j = 0; j < d; ++j) sx[(size_t)s * d + j] = xs[c * d + j];
+  if (pm)
+    for (int i = 0; i < y_dim; ++i) spm[(size_t)s * y_dim + i] = pm[c * y_dim + i];
+  if (cm) scm[s] = cm[c];
+}
+
+// a candidate stays unless its bound is below thr = T (1 - 2^-30); a NaN bound stays
+__device__ __forceinline__ bool screen_keep(const double *bound, int c, int ch, double thr) {
+  return c < ch && !(bound[c] < thr);
+}
+
+__global__ void __launch_bounds__(256) screen_count_kernel(const double *bound, int ch, double thr, int *cnt) {
+  const int k = __syncthreads_count(screen_keep(bound, blockIdx.x * 256 + threadIdx.x, ch, thr));
+  if (threadIdx.x == 0) cnt[blockIdx.x] = k;
+}
+
+struct CompactParams {
+  const double *bound;
+  int ch;
+  double thr;
+  const int *cnt;                // survivors per 256 candidates (screen_count_kernel)
+  long long m0;                  // index (within the call) of the chunk's first candidate
+  const double *xs, *pm;         // the chunk's first candidate (pm may be null)
+  const unsigned char *cm;       // or null
+  int d, y_dim;
+  long long *base;               // pool size before this chunk in base[par]; the last CTA writes the size after it to base[par ^ 1]
+  int par;
+  double *px, *ppm;              // pool: candidates, prior means,
+  unsigned char *pcm;            //       constraint-mask entries,
+  long long *pidx;               //       index within the call
+};
+
+// ordered compaction: survivors keep their relative order, so the pool's first-maximal argmax is the call's
+__global__ void __launch_bounds__(256) screen_compact_kernel(CompactParams p) {
+  __shared__ long long s_off;
+  __shared__ int s_warp[8];
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5, b = blockIdx.x;
+  if (w == 0) {
+    long long s = 0;
+    for (int j = lane; j < b; j += 32) s += p.cnt[j];
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if (lane == 0) {
+      s_off = p.base[p.par] + s;
+      if (b == (int)gridDim.x - 1) p.base[p.par ^ 1] = s_off + p.cnt[b];
+    }
+  }
+  const int c = b * 256 + tid;
+  const bool keep = screen_keep(p.bound, c, p.ch, p.thr);
+  const unsigned bal = __ballot_sync(0xffffffffu, keep);
+  if (lane == 0) s_warp[w] = __popc(bal);
+  __syncthreads();
+  if (!keep) return;
+  long long o = s_off + __popc(bal & ((1u << lane) - 1u));
+  for (int q = 0; q < w; ++q) o += s_warp[q];
+  for (int j = 0; j < p.d; ++j) p.px[o * p.d + j] = p.xs[(size_t)c * p.d + j];
+  if (p.pm)
+    for (int i = 0; i < p.y_dim; ++i) p.ppm[o * p.y_dim + i] = p.pm[(size_t)c * p.y_dim + i];
+  if (p.cm) p.pcm[o] = p.cm[c];
+  p.pidx[o] = p.m0 + c;
 }
 
 // ---------------------------------------------------------------------------------------------

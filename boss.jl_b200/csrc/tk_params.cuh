@@ -91,6 +91,7 @@ struct SmallLoglikParams {
 bool launch_build_k(int kid, int dp, const BuildKParams &p, dim3 grid, cudaStream_t st);
 bool launch_loglik_grad_tile(int kid, int dp, const LlGradParams &p, dim3 grid, cudaStream_t st);
 bool launch_xcov(int kid, int dp, const XcovParams &p, dim3 grid, cudaStream_t st);
+bool launch_xcov_mean(int kid, int dp, const XcovParams &p, dim3 grid, cudaStream_t st);   // mu partials only (p.Ks unused)
 bool launch_cov_finish(int kid, int dp, const CovFinishParams &p, dim3 grid, cudaStream_t st);
 bool launch_grad(int kid, int dp, const GradParams &p, dim3 grid, cudaStream_t st);
 bool launch_loglik_small(int kid, int dp, const SmallLoglikParams &p, int nblocks, cudaStream_t st);

@@ -8,7 +8,8 @@ namespace boss {
 
 // grid = (candidate blocks, splits over the 128-point training chunks).  Every chunk's contribution to
 // mu is written as its own partial (fixed summation order downstream), so results do not depend on the split.
-template <int KID, int DP>
+// STORE_KS = false: the mean partials only (argmax screening needs mu, not K*^T); same partials, same bits.
+template <int KID, int DP, bool STORE_KS = true>
 __global__ void __launch_bounds__(256) xcov_kernel(XcovParams p) {
   __shared__ double xt[XCOV_KC * DP];
   __shared__ double al[XCOV_KC];
@@ -48,6 +49,7 @@ __global__ void __launch_bounds__(256) xcov_kernel(XcovParams p) {
       }
 #pragma unroll
       for (int kk = 0; kk < 8; ++kk) mu_acc = fma(v[kk], al[mcol * 8 + kk], mu_acc);
+      if (!STORE_KS) continue;
       const int kg = k0 + mcol * 8;  // global training index of v[0]
       double *dst = rowbase + (size_t)(kg >> 4) * TILE_ELEMS + (((kg >> 3) & 1) << 6);
 #pragma unroll
@@ -157,6 +159,11 @@ __global__ void __launch_bounds__(256) grad_kernel(GradParams p) {
 
 bool launch_xcov(int kid, int dp, const XcovParams &p, dim3 grid, cudaStream_t st) {
 #define CALL(K, D) xcov_kernel<K, D><<<grid, 256, 0, st>>>(p)
+  BOSS_DISPATCH_KID_DP(CALL, kid, dp)
+#undef CALL
+}
+bool launch_xcov_mean(int kid, int dp, const XcovParams &p, dim3 grid, cudaStream_t st) {
+#define CALL(K, D) xcov_kernel<K, D, false><<<grid, 256, 0, st>>>(p)
   BOSS_DISPATCH_KID_DP(CALL, kid, dp)
 #undef CALL
 }

@@ -280,6 +280,9 @@ int boss_dbg_factors(const boss_gp *gp, double *L, double *W, double *alpha);   
  * it recommends instead. */
 int64_t boss_dbg_check_redzones(int64_t *n_allocs);
 int64_t boss_dbg_redzone_selftest(void);   /* negative control: writes 2 guard bytes on purpose, returns how many the scan found */
+/* argmax screening of the last scoring call on the current device: out[0] = 0 not screened, 1 screened, 2 fell back
+ * to the full path after the first chunk; out[1] = candidates bounded; out[2] = candidates that survived the bound */
+int boss_dbg_screen_stats(int64_t *out);
 
 #ifdef __cplusplus
 }
