@@ -51,6 +51,10 @@ EXPORTS = {
                                 _dp, _i64p]),
     "boss_ei_score_dev": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                     _vp, _dp, _i64p, _vp]),
+    "boss_ei_score_topk": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int64,
+                                     _vp, _vp]),
+    "boss_ei_score_topk_dev": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                         C.c_int64, _vp, _vp, _vp]),
     "boss_ei_score_grid": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp, C.c_int64, C.c_int64, _vp, _vp, _vp, _vp,
                                      _vp, _vp, _vp, _vp, _dp, _i64p, _vp]),
     "boss_ei_score_uniform": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_int64, C.c_int64, _vp, _vp, _vp,
@@ -271,6 +275,48 @@ def ei_score(slices, y_dim, n_samples, Xs, coefs, best, y_max, lb=None, ub=None,
     _check(lib.boss_ei_score(arr, y_dim, n_samples, _ptr(Xc), M, _ptr(pm), _ptr(co), _ptr(b), _ptr(ym), _ptr(lbv),
                              _ptr(ubv), _ptr(cm), _ptr(acq), None, C.byref(bv), C.byref(bi)), "boss_ei_score")
     return acq, bv.value, bi.value
+
+
+def ei_score_topk(slices, y_dim, n_samples, Xs, coefs, best, y_max, k, lb=None, ub=None, cons_mask=None,
+                  prior_mean_s=None):
+    """The k best candidates of ei_score's scores, selected on the device (include/boss_b200.h, boss_ei_score_topk).
+    -> top_val (k,), top_idx (k,) int64: descending under Julia's isless (NaN first), ties to the lower index."""
+    Xc = _cols(Xs)
+    M, d = Xc.shape
+    assert len(slices) == y_dim * n_samples
+    arr = _slice_array(slices)
+    co = _f64(coefs, (y_dim,))
+    b = None if best is None else np.array([best], dtype=np.float64)
+    ym = None if y_max is None else _f64(y_max, (y_dim,))
+    lbv = None if lb is None else _f64(lb, (d,))
+    ubv = None if ub is None else _f64(ub, (d,))
+    cm = None if cons_mask is None else np.ascontiguousarray(cons_mask, dtype=np.uint8)
+    pm = None if prior_mean_s is None else np.ascontiguousarray(np.asarray(prior_mean_s, dtype=np.float64).T)
+    k = int(k)
+    tv = np.empty(max(k, 0))
+    ti = np.empty(max(k, 0), dtype=np.int64)
+    _check(lib.boss_ei_score_topk(arr, y_dim, n_samples, _ptr(Xc), M, _ptr(pm), _ptr(co), _ptr(b), _ptr(ym), _ptr(lbv),
+                                  _ptr(ubv), _ptr(cm), k, _ptr(tv), _ptr(ti)), "boss_ei_score_topk")
+    return tv, ti
+
+
+def ei_score_topk_dev(slices, y_dim, n_samples, Xs_ptr, M, coefs, best, y_max, k, lb=None, ub=None, prior_mean_ptr=None,
+                      cons_mask_ptr=None, stream=None):
+    """Device-pointer variant of ei_score_topk (arguments as ei_score_dev).  -> top_val (k,), top_idx (k,) on the host."""
+    arr = _slice_array(slices)
+    co = _f64(coefs, (y_dim,))
+    b = None if best is None else np.array([best], dtype=np.float64)
+    ym = None if y_max is None else _f64(y_max, (y_dim,))
+    lbv = None if lb is None else _f64(lb)
+    ubv = None if ub is None else _f64(ub)
+    k = int(k)
+    tv = np.empty(max(k, 0))
+    ti = np.empty(max(k, 0), dtype=np.int64)
+    _check(lib.boss_ei_score_topk_dev(arr, y_dim, n_samples, _vp(Xs_ptr), int(M),
+                                      _vp(prior_mean_ptr) if prior_mean_ptr else None, _ptr(co), _ptr(b), _ptr(ym),
+                                      _ptr(lbv), _ptr(ubv), _vp(cons_mask_ptr) if cons_mask_ptr else None, k, _ptr(tv),
+                                      _ptr(ti), _vp(stream) if stream else None), "boss_ei_score_topk_dev")
+    return tv, ti
 
 
 FIT_AFFINE, FIT_QUADRATIC, FIT_MAX, FIT_MIN = 1, 2, 3, 4
@@ -538,7 +584,7 @@ def dbg_check_redzones():
 
 
 def dbg_screen_stats():
-    """Argmax screening of the last scoring call on the current device: (state, candidates bounded, survivors);
+    """Argmax / top-k screening of the last scoring call on the current device: (state, candidates bounded, survivors);
     state 0 = not screened, 1 = screened, 2 = fell back to the full path after the first chunk."""
     out = (C.c_int64 * 3)()
     _check(lib.boss_dbg_screen_stats(out), "boss_dbg_screen_stats")

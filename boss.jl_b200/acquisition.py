@@ -38,6 +38,16 @@ def julia_argmax(v):
     return int(cand[0])
 
 
+def julia_sortperm_rev(v):
+    """Julia's stable sortperm(v; rev=true): descending under isless (NaN first, +0.0 before -0.0), ties to the lower
+    index.  The order of boss_ei_score_topk; its first element is julia_argmax(v)."""
+    v = np.asarray(v, dtype=np.float64)
+    u = np.ascontiguousarray(v).view(np.uint64)
+    key = np.where((u >> np.uint64(63)) != 0, ~u, u | np.uint64(1 << 63))
+    key = np.where(np.isnan(v), np.uint64(0xFFFFFFFFFFFFFFFF), key)
+    return np.argsort(~key, kind="stable")
+
+
 def sample_eps(y_dim: int, count: int, rng=None):
     """sample_ϵs (expected_improvement.jl:118): y_dim x count standard normal draws."""
     rng = np.random.default_rng() if rng is None else rng
@@ -184,6 +194,19 @@ class Acquisition:
         _, bv, bi = _lib.ei_score(self.slices, self.y_dim, len(self.posts), X, self.coefs, self.best, self.y_max,
                                   lb, ub, cm, self._prior_mean(X), want_acq=False)
         return int(bi), float(bv)
+
+    def topk(self, X, k):
+        """-> (indices (k,), values (k,)) of the k best columns of X in julia_sortperm_rev order.  LinFitness selects on
+        the device (boss_ei_score_topk); a NonlinFitness scores every column and sorts on the host."""
+        X = np.asarray(X, dtype=np.float64)
+        if self.nonlin:
+            acq = self._mc_acq(X)
+            top = julia_sortperm_rev(acq)[:k]
+            return top, acq[top]
+        lb, ub, cm = self._guards(X)
+        vals, idx = _lib.ei_score_topk(self.slices, self.y_dim, len(self.posts), X, self.coefs, self.best, self.y_max, k,
+                                       lb, ub, cm, self._prior_mean(X))
+        return idx, vals
 
     def value_and_grad(self, X):
         """-> acq (M,), grad (d, M).  Prior-mean gradients are not propagated for closure means."""

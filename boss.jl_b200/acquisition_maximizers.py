@@ -89,6 +89,14 @@ def _rand_in_domain(am: SamplingAM, domain: Domain):
     return None
 
 
+def _draw_samples(am: SamplingAM, domain: Domain):
+    """sampling.jl:37-48: `samples` rejection-sampled points (d x M); the ones that failed are dropped."""
+    xs = [x for x in (_rand_in_domain(am, domain) for _ in range(am.samples)) if x is not None]
+    if not xs:
+        raise RuntimeError("SamplingAM: No samples were successfully drawn!")
+    return np.stack(xs, axis=1)
+
+
 def batched_lbfgs_maximize(value_and_grad, starts, lb, ub, iters=60, history=8, discrete=None, publish_active=None):
     """Maximise f over the box [lb, ub] from every column of `starts` simultaneously (projected L-BFGS with Armijo
     backtracking).  value_and_grad(X: d x S) -> (f: S, g: d x S).  Returns X (d x S), f (S).
@@ -198,17 +206,15 @@ def maximize_acquisition(am, problem: BossProblem, options: BossOptions = BossOp
         idx, val = acq.argmax(pts)
         return pts[:, idx].copy(), val
     if isinstance(am, SamplingAM):
-        xs = [x for x in (_rand_in_domain(am, dom) for _ in range(am.samples)) if x is not None]
-        if not xs:
-            raise RuntimeError("SamplingAM: No samples were successfully drawn!")
-        X = np.stack(xs, axis=1)
+        X = _draw_samples(am, dom)
         if return_all:
             return X, acq(X)
         idx, val = acq.argmax(X)
         return X[:, idx].copy(), val
     if isinstance(am, SampleOptAM):
-        X, vals = maximize_acquisition(am.sampler, problem, options, return_all=True, acq=acq)
-        top = np.argsort(-vals, kind="stable")[: am.multistart]
+        # the `multistart` best samples, selected on the device (Acquisition.topk: isless order, NaN first)
+        X = _draw_samples(am.sampler, dom)
+        top, _ = acq.topk(X, min(am.multistart, X.shape[1]))
         return maximize_acquisition(OptimizationAM(X[:, top], am.iters), problem, options, acq=acq)
     if isinstance(am, OptimizationAM):
         lb, ub = dom.bounds

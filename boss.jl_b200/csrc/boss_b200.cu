@@ -30,6 +30,7 @@
 #include "score_narrow.cuh"
 #include "append.cuh"
 #include "multistart.cuh"
+#include "topk.cuh"
 
 using namespace boss;
 
@@ -135,6 +136,7 @@ struct Ctx {
   DevBuf blk_val, blk_idx, small, chol_L, chol_Winv, chol_misc, tt, vt, ut, dmu, dvar, pmg_stage;
   DevBuf part_mu, part_ss, part_gm, part_gv, cov_p, cov_stage, chol_W, chol_WT, ll_vec, ll_part, ms_buf;   // split-invariant partial sums (score.cuh / grad.cuh)
   DevBuf scr_misc, scr_pool;         // argmax screening: bounds, counts, seed batch / survivor pool (score_core)
+  DevBuf topk;                       // top-k calls: running set, chunk scores, selection state, sorted result
   int64_t scr_stats[3] = {0, 0, 0};  // last scoring call: screened (1) or fell back (2), candidates bounded, pool size
   // event pool for per-kernel-class timing
   cudaEvent_t ev_a[EV_POOL], ev_b[EV_POOL];
@@ -351,6 +353,7 @@ int set_kernel_attrs() {
   CUDA_TRY(cudaFuncSetAttribute(trtri_acc_rl_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
   CUDA_TRY(cudaFuncSetAttribute(trtri_row_rl_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
   CUDA_TRY(cudaFuncSetAttribute(score_trmm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
+  CUDA_TRY(cudaFuncSetAttribute(topk_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TOPK_SORT_SMEM));
   CUDA_TRY(cudaFuncSetAttribute(wtv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
   CUDA_TRY(cudaFuncSetAttribute(score_narrow_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, NW_SMEM_BYTES));
   CUDA_TRY(cudaFuncSetAttribute(score_narrow_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, NW_SMEM_BYTES));
@@ -1075,6 +1078,10 @@ struct ScoreArgs {
   void *caller_stream = nullptr;  // dev == true: the stream the caller produced its device arrays on (NULL = legacy default stream)
   bool internal = false;          // dev == true from inside the library (arrays were produced on the library stream)
   const MixParams *mix = nullptr; // MC-EI for NonlinFitness expression sets (score.cuh); null = LinFitness closed form
+  long long topk = 0;             // > 0: the topk best (value, index) pairs in isless order go to top_val / top_idx (host)
+  double *top_val = nullptr;
+  int64_t *top_idx = nullptr;
+  const long long *topk_map = nullptr;   // device, or null: returned indices are topk_map[i] (the screened pool's origins)
 };
 
 // Julia's isless order on (value, index): NaN maximal, -0.0 < +0.0, ties -> lowest index (host twin of acq_better)
@@ -1157,7 +1164,7 @@ struct ScreenBufs {
   unsigned long long *tk[2] = {};
   long long *base = nullptr, *pool_idx = nullptr;
   unsigned char *seed_cm = nullptr, *pool_cm = nullptr;
-  int setup(long long M, int CH, int d, int y_dim, bool pm, bool cm) {
+  int setup(long long M, int CH, int d, int y_dim, bool pm, bool cm, int ns_max) {
     size_t tot = 0;
     auto take = [&tot](size_t bytes) {
       const size_t o = tot;
@@ -1167,7 +1174,7 @@ struct ScreenBufs {
     const size_t ntk = (size_t)(CH + TOPK_IN - 1) / TOPK_IN * SEED_N;
     const size_t o_bound = take((size_t)CH * 8), o_cnt = take((size_t)(CH + 255) / 256 * 4), o_base = take(16);
     const size_t o_tk0 = take(ntk * 8), o_tk1 = take(ntk * 8), o_ti0 = take(ntk * 4), o_ti1 = take(ntk * 4);
-    const size_t o_sx = take((size_t)SEED_N * d * 8), o_spm = take((size_t)SEED_N * y_dim * 8), o_scm = take(SEED_N);
+    const size_t o_sx = take((size_t)ns_max * d * 8), o_spm = take((size_t)ns_max * y_dim * 8), o_scm = take(ns_max);
     CUDA_TRY(C().scr_misc.ensure(tot));
     unsigned char *b = C().scr_misc.as<unsigned char>();
     bound = reinterpret_cast<double *>(b + o_bound);
@@ -1189,6 +1196,65 @@ struct ScreenBufs {
     pool_idx = reinterpret_cast<long long *>(b + o_pidx);
     pool_pm = pm ? reinterpret_cast<double *>(b + o_ppm) : nullptr;
     pool_cm = cm ? b + o_pcm : nullptr;
+    return 0;
+  }
+};
+
+// seed batch of a screened top-k call: the S_k highest bounds of the first chunk, S_k = 2k rounded up to 128, at least
+// SEED_N and at most the chunk (DESIGN.md 2.10)
+int topk_seed_n(long long k, int ch) {
+  return (int)std::min<long long>(ch, std::max<long long>(SEED_N, (2 * k + 127) / 128 * 128));
+}
+
+// device buffers of a top-k call (topk.cuh): two running sets of `cap` pairs, the chunk's scores, the selection state
+// and per-256 counts, the sorted result.  Sized by the outermost call; the nested seed and pool calls fit inside.
+struct TopkBufs {
+  double *run_val[2] = {}, *scores = nullptr, *out_val = nullptr;
+  long long *run_idx[2] = {}, *out_idx = nullptr;
+  SelectState *st = nullptr;
+  int2 *cnt = nullptr;
+  int setup(int cap, int CH, long long k) {
+    size_t tot = 0;
+    auto take = [&tot](size_t bytes) {
+      const size_t o = tot;
+      tot += (bytes + 255) / 256 * 256;
+      return o;
+    };
+    const size_t o_rv0 = take((size_t)cap * 8), o_rv1 = take((size_t)cap * 8), o_ri0 = take((size_t)cap * 8),
+                 o_ri1 = take((size_t)cap * 8), o_sc = take((size_t)CH * 8), o_st = take(sizeof(SelectState)),
+                 o_cnt = take(((size_t)cap + CH + 255) / 256 * sizeof(int2)), o_ov = take((size_t)k * 8),
+                 o_oi = take((size_t)k * 8);
+    CUDA_TRY(C().topk.ensure(tot));
+    unsigned char *b = C().topk.as<unsigned char>();
+    run_val[0] = reinterpret_cast<double *>(b + o_rv0);
+    run_val[1] = reinterpret_cast<double *>(b + o_rv1);
+    run_idx[0] = reinterpret_cast<long long *>(b + o_ri0);
+    run_idx[1] = reinterpret_cast<long long *>(b + o_ri1);
+    scores = reinterpret_cast<double *>(b + o_sc);
+    st = reinterpret_cast<SelectState *>(b + o_st);
+    cnt = reinterpret_cast<int2 *>(b + o_cnt);
+    out_val = reinterpret_cast<double *>(b + o_ov);
+    out_idx = reinterpret_cast<long long *>(b + o_oi);
+    return 0;
+  }
+  // the `target` best of (in's running set, in's new values) -> out, in ascending index order (topk.cuh)
+  int select(const SelectIn &in, int target, double *out_val_, long long *out_idx_) {
+    const int N = in.r + in.n;
+    if (N < 1 || target < 1) return 0;
+    select_init_kernel<<<1, 256, 0, C().stream>>>(st, target >= N ? N : target);
+    ++C().launches;
+    if (target < N) {
+      const int gh = std::min((N + 255) / 256, 8 * 148);
+      for (int shift = 56; shift >= 0; shift -= 8) {
+        select_hist_kernel<<<gh, 256, 0, C().stream>>>(in, st, shift);
+        select_scan_kernel<<<1, 256, 0, C().stream>>>(st, shift);
+      }
+      C().launches += 16;
+    }
+    const int nb = (N + 255) / 256;
+    select_count_kernel<<<nb, 256, 0, C().stream>>>(in, st, cnt);
+    select_compact_kernel<<<nb, 256, 0, C().stream>>>(in, st, cnt, out_val_, out_idx_);
+    C().launches += 2;
     return 0;
   }
 };
@@ -1284,15 +1350,26 @@ int score_core(ScoreArgs &a) {
   // candidates bounds every candidate from its mean alone and scores exactly only those that can still win ----
   if (!a.internal) C().scr_stats[0] = C().scr_stats[1] = C().scr_stats[2] = 0;
   const size_t pool_row = (size_t)d * 8 + (a.prior_mean ? (size_t)a.y_dim * 8 : 0) + 8 + (a.cons_mask ? 1 : 0);
-  bool screen = a.want_argmax && a.best && !a.internal && !a.acq && !a.grad && !a.mu_out && !a.var_out && !a.status_out &&
-                !a.mix && a.M >= screen_min_m() && (size_t)a.M * pool_row <= SCREEN_POOL_BYTES &&
-                getenv("BOSS_NO_SCREEN") == nullptr;
+  // (top-k calls, DESIGN.md 2.10: the same bound against the k-th best score of a larger seed batch)
+  const int ch0 = (int)std::min<long long>(CH, a.M);   // the first chunk, which the seed batch is drawn from
+  bool screen = (a.want_argmax || a.topk) && a.best && !a.internal && !a.acq && !a.grad && !a.mu_out && !a.var_out &&
+                !a.status_out && !a.mix && a.M >= screen_min_m() && (size_t)a.M * pool_row <= SCREEN_POOL_BYTES &&
+                a.topk <= ch0 && getenv("BOSS_NO_SCREEN") == nullptr;
   ScreenBufs sc;
   double thr = -INFINITY;   // survivors: bound >= thr or NaN
   if (screen) {
-    int rc = sc.setup(a.M, CH, d, a.y_dim, a.prior_mean != nullptr, a.cons_mask != nullptr);
+    int rc = sc.setup(a.M, CH, d, a.y_dim, a.prior_mean != nullptr, a.cons_mask != nullptr,
+                      a.topk ? topk_seed_n(a.topk, ch0) : SEED_N);
     if (rc) return rc;
     CUDA_TRY(cudaMemsetAsync(sc.base, 0, 16, C().stream));
+  }
+  // top-k: the running set (tk_r pairs in tb.run_*[tk_par]) absorbs every scored chunk
+  TopkBufs tb;
+  int tk_r = 0, tk_par = 0;
+  if (a.topk) {
+    const int cap = (int)std::max<long long>(a.topk, topk_seed_n(a.topk, ch0));
+    int rc = tb.setup(cap, CH, a.topk);
+    if (rc) return rc;
   }
   // one chunk of a screened call: the means of every slice (xcov without K*^T), the bounds, the survivors appended to
   // the pool.  The first chunk also sets the threshold from the seed batch and ends screening (the chunk is then scored
@@ -1343,7 +1420,41 @@ int score_core(ScoreArgs &a) {
     const double *xs_c = ap.Xs + c0 * d;
     const double *pm_c = ap.prior_mean ? ap.prior_mean + c0 * a.y_dim : nullptr;
     const unsigned char *cm_c = ap.cons_mask ? ap.cons_mask + c0 : nullptr;
-    if (cidx == 0) {
+    if (cidx == 0 && a.topk) {
+      // seed: the exact scores of the S_k highest bounds (NaN bounds last); the k-th best of them is a lower bound of
+      // the k-th best score of the call
+      const int ns = topk_seed_n(a.topk, ch);
+      SelectIn in{nullptr, nullptr, 0, sc.bound, 0, ch, 1};
+      int rc = tb.select(in, ns, tb.run_val[0], tb.run_idx[0]);
+      if (rc) return rc;
+      seed_gather_kernel<<<(ns + 255) / 256, 256, 0, C().stream>>>(tb.run_idx[0], ns, xs_c, pm_c, cm_c, d, a.y_dim,
+                                                                    sc.seed_x, sc.seed_pm, sc.seed_cm);
+      ++C().launches;
+      ScoreArgs s = a;
+      s.Xs = sc.seed_x;
+      s.M = ns;
+      s.prior_mean = pm_c ? sc.seed_pm : nullptr;
+      s.cons_mask = cm_c ? sc.seed_cm : nullptr;
+      s.gen = nullptr;
+      s.dev = true;
+      s.internal = true;
+      std::vector<double> sv((size_t)a.topk);
+      std::vector<int64_t> si((size_t)a.topk);
+      s.top_val = sv.data();
+      s.top_idx = si.data();
+      s.topk_map = nullptr;
+      rc = score_core(s);
+      if (rc) return rc;
+      CUDA_TRY(cudaMemcpyAsync(small, hs.data(), sm_n * 8, cudaMemcpyHostToDevice, C().stream));
+      C().scr_stats[1] = ch;
+      const double T = sv[(size_t)a.topk - 1];
+      if (!(T >= SCREEN_MIN_T)) {
+        C().scr_stats[0] = 2;
+        screen = false;
+        return 0;
+      }
+      thr = T * (1.0 - 0x1p-30);
+    } else if (cidx == 0) {
       // seed: the exact scores of the SEED_N highest bounds; the best of them is a lower bound of the maximum
       int n = ch, par = 0;
       const unsigned long long *kin = nullptr;
@@ -1565,6 +1676,10 @@ int score_core(ScoreArgs &a) {
     ap.blk_val = a.want_argmax ? C().blk_val.as<double>() : nullptr;
     ap.blk_idx = a.want_argmax ? C().blk_idx.as<long long>() : nullptr;
     ap.mix = mixp;
+    if (a.topk) {   // the chunk's scores stay on the device, for the running top-k set
+      ap.acq = tb.scores;
+      ap.out_off = m0;
+    }
     if (screen) {
       int rc = screen_chunk(ap, xs_dev, in_off, cidx);
       if (rc) return rc;
@@ -1716,6 +1831,14 @@ int score_core(ScoreArgs &a) {
         ++C().launches;
       }
     }
+    if (a.topk && !screen) {   // the best min(k, seen) of (running set, this chunk)
+      const int tgt = (int)std::min<long long>(a.topk, (long long)tk_r + ch);
+      SelectIn in{tb.run_val[tk_par], tb.run_idx[tk_par], tk_r, tb.scores, m0, ch, 0};
+      int rc = tb.select(in, tgt, tb.run_val[tk_par ^ 1], tb.run_idx[tk_par ^ 1]);
+      if (rc) return rc;
+      tk_par ^= 1;
+      tk_r = tgt;
+    }
     if (a.grad) {
       AcqGradParams gp2{ap, C().dmu.as<double>(), C().dvar.as<double>(), pmg_dev, grad_dev};
       acq_grad_kernel<<<(ch + 127) / 128, 128, 0, C().stream>>>(gp2);
@@ -1753,6 +1876,7 @@ int score_core(ScoreArgs &a) {
     C().scr_stats[1] = a.M;
     C().scr_stats[2] = npool;
     if (npool < 1) return fail(BOSS_ERR_STATE, "score: argmax screening kept no candidate");   // the seed's winner always survives
+    if (npool < a.topk) return fail(BOSS_ERR_STATE, "score: top-k screening kept fewer than k candidates");   // the seed's k best survive
     ScoreArgs s = a;
     s.Xs = sc.pool_x;
     s.M = npool;
@@ -1765,16 +1889,36 @@ int score_core(ScoreArgs &a) {
     int64_t bi = -1;
     s.best_val = &bv;
     s.best_idx = &bi;
+    s.topk_map = sc.pool_idx;   // top-k: the pool's k best come back with their indices in this call
     int rc = score_core(s);
     if (rc) return rc;
+    a.any_fail = s.any_fail;
+    if (a.topk) return 0;
     long long idx = -1;
     if (bi >= 0) {
       CUDA_TRY(cudaMemcpyAsync(&idx, sc.pool_idx + bi, 8, cudaMemcpyDeviceToHost, C().stream));
       CUDA_TRY(cudaStreamSynchronize(C().stream));
     }
-    a.any_fail = s.any_fail;
     if (a.best_val) *a.best_val = bv;
     if (a.best_idx) *a.best_idx = idx;
+    return 0;
+  }
+  if (a.topk) {
+    // the running set, sorted in one CTA, to the caller: k pairs, no M-sized output and no host sort
+    if (tk_r != a.topk) return fail(BOSS_ERR_STATE, "score: top-k set incomplete");
+    int P = 2;
+    while (P < tk_r) P <<= 1;
+    topk_sort_kernel<<<1, 1024, (size_t)P * 12, C().stream>>>(tb.run_val[tk_par], tb.run_idx[tk_par], tk_r, P, a.topk_map,
+                                                             tb.out_val, tb.out_idx);
+    ++C().launches;
+    int af = 0;
+    CUDA_TRY(cudaMemcpyAsync(a.top_val, tb.out_val, (size_t)tk_r * 8, cudaMemcpyDeviceToHost, C().stream));
+    CUDA_TRY(cudaMemcpyAsync(a.top_idx, tb.out_idx, (size_t)tk_r * 8, cudaMemcpyDeviceToHost, C().stream));
+    CUDA_TRY(cudaMemcpyAsync(&af, d_anyfail, 4, cudaMemcpyDeviceToHost, C().stream));
+    CUDA_TRY(cudaStreamSynchronize(C().stream));
+    if (host) CUDA_TRY(cudaStreamSynchronize(cp));
+    timing_end();
+    a.any_fail = af;
     return 0;
   }
   if (a.internal && !a.want_argmax && !C().timing) {   // a round of the multi-start driver: it synchronises itself
@@ -1840,6 +1984,8 @@ int score_dispatch(ScoreArgs &a) {
   std::vector<double> bv(nd, 0.0);
   std::vector<int64_t> bi(nd, -1);
   std::vector<long long> first(nd, 0);
+  std::vector<std::vector<double>> tv(nd);   // top-k: each device's block top min(k, count), merged below
+  std::vector<std::vector<int64_t>> ti(nd);
   int rc = for_each_device(nd, [&](int k, Ctx *) {
     ScoreArgs &s = sub[k];
     const long long off = std::min<long long>(a.M, (long long)k * per), cnt = std::min<long long>(per, a.M - off);
@@ -1863,6 +2009,13 @@ int score_dispatch(ScoreArgs &a) {
     if (a.status_out) s.status_out = a.status_out + off;
     s.best_val = &bv[k];
     s.best_idx = &bi[k];
+    if (a.topk) {
+      s.topk = std::min<long long>(a.topk, cnt);
+      tv[k].resize((size_t)s.topk);
+      ti[k].resize((size_t)s.topk);
+      s.top_val = tv[k].data();
+      s.top_idx = ti[k].data();
+    }
     return score_core(s);
   });
   if (rc) return rc;
@@ -1883,6 +2036,18 @@ int score_dispatch(ScoreArgs &a) {
   if (a.want_argmax) {
     if (a.best_val) *a.best_val = best_v;
     if (a.best_idx) *a.best_idx = best_i;
+  }
+  if (a.topk) {   // the k best of the devices' lists in the same order: the set the single-device call selects
+    std::vector<std::pair<double, long long>> all;
+    for (int k = 0; k < nd; ++k)
+      for (size_t e = 0; e < tv[k].size(); ++e) all.emplace_back(tv[k][e], first[k] + ti[k][e]);
+    std::sort(all.begin(), all.end(), [](const std::pair<double, long long> &x, const std::pair<double, long long> &y) {
+      return acq_better_host(x.first, x.second, y.first, y.second);
+    });
+    for (long long e = 0; e < a.topk; ++e) {
+      a.top_val[e] = all[(size_t)e].first;
+      a.top_idx[e] = all[(size_t)e].second;
+    }
   }
   return 0;
 }
@@ -1979,6 +2144,54 @@ int boss_ei_score_dev(const boss_gp *const *slices, int y_dim, int n_samples, co
                       double *acq_dev, double *grad_dev, double *best_val, int64_t *best_idx, void *stream) {
   return ei_score_impl(slices, y_dim, n_samples, Xs_dev, M, prior_mean_s_dev, fit_coefs, best, y_max, lb, ub,
                        cons_mask_dev, acq_dev, grad_dev, best_val, best_idx, true, nullptr, stream);
+}
+
+// The k best candidates of boss_ei_score's scores (header: order, limits); screened like the argmax when `best` is set
+// (DESIGN.md 2.10), otherwise the full path keeps a running top-k set on the device.
+static int ei_score_topk_impl(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
+                              const double *prior_mean_s, const double *fit_coefs, const double *best,
+                              const double *y_max, const double *lb, const double *ub, const uint8_t *cons_mask,
+                              int64_t k, double *top_val, int64_t *top_idx, bool dev, void *stream) {
+  if (!slices || y_dim < 1 || n_samples < 1 || !Xs || M < 1 || !fit_coefs || !top_val || !top_idx)
+    return fail(BOSS_ERR_ARG, "boss_ei_score_topk: bad arguments");
+  if (k < 1 || k > M || k > TOPK_MAX) return fail(BOSS_ERR_ARG, "boss_ei_score_topk: k must be in 1..min(M, 8192)");
+  if ((lb == nullptr) != (ub == nullptr)) return fail(BOSS_ERR_ARG, "boss_ei_score_topk: lb and ub must be given together");
+  ScoreArgs a{};
+  a.slices = slices;
+  a.y_dim = y_dim;
+  a.n_samples = n_samples;
+  a.Xs = Xs;
+  a.M = M;
+  a.prior_mean = prior_mean_s;
+  a.coefs = fit_coefs;
+  a.best = best;
+  a.y_max = y_max;
+  a.lb = lb;
+  a.ub = ub;
+  a.cons_mask = cons_mask;
+  a.dev = dev;
+  a.caller_stream = stream;
+  a.want_argmax = false;
+  a.topk = k;
+  a.top_val = top_val;
+  a.top_idx = top_idx;
+  return score_dispatch(a);
+}
+
+int boss_ei_score_topk(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
+                       const double *prior_mean_s, const double *fit_coefs, const double *best, const double *y_max,
+                       const double *lb, const double *ub, const uint8_t *cons_mask, int64_t k, double *top_val,
+                       int64_t *top_idx) {
+  return ei_score_topk_impl(slices, y_dim, n_samples, Xs, M, prior_mean_s, fit_coefs, best, y_max, lb, ub, cons_mask, k,
+                            top_val, top_idx, false, nullptr);
+}
+
+int boss_ei_score_topk_dev(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs_dev, int64_t M,
+                           const double *prior_mean_s_dev, const double *fit_coefs, const double *best,
+                           const double *y_max, const double *lb, const double *ub, const uint8_t *cons_mask_dev,
+                           int64_t k, double *top_val, int64_t *top_idx, void *stream) {
+  return ei_score_topk_impl(slices, y_dim, n_samples, Xs_dev, M, prior_mean_s_dev, fit_coefs, best, y_max, lb, ub,
+                            cons_mask_dev, k, top_val, top_idx, true, stream);
 }
 
 // Monte-Carlo EI of a NonlinFitness from the small expression set of MixParams (score.cuh), on the device:

@@ -337,7 +337,8 @@ __global__ void __launch_bounds__(1024) seed_topk_kernel(const double *bounds, c
 }
 
 // row s of the seed batch = candidate sel[s] of the chunk (xs / pm / cm point at the chunk's first candidate)
-__global__ void seed_gather_kernel(const int *sel, int ns, const double *xs, const double *pm, const unsigned char *cm,
+template <typename I>
+__global__ void seed_gather_kernel(const I *sel, int ns, const double *xs, const double *pm, const unsigned char *cm,
                                    int d, int y_dim, double *sx, double *spm, unsigned char *scm) {
   const int s = blockIdx.x * blockDim.x + threadIdx.x;
   if (s >= ns) return;

@@ -151,6 +151,25 @@ int boss_ei_score_dev(const boss_gp *const *slices, int y_dim, int n_samples, co
                       const double *y_max, const double *lb, const double *ub, const uint8_t *cons_mask_dev,
                       double *acq_dev, double *grad_dev, double *best_val, int64_t *best_idx, void *stream);
 
+/* The k best candidates of the same scores (SampleOptAM's starts, src/acquisition_maximizers/sample_opt.jl:41-52),
+ * selected on the device: no M-sized output, no host sort.  Arguments as boss_ei_score; top_val / top_idx are HOST
+ * arrays of k (also in the _dev variant, whose other array arguments are device pointers).
+ *   k        1 <= k <= min(M, 8192), BOSS_ERR_ARG otherwise (BOSS.jl's order[1:multistart] throws for multistart > samples)
+ *   order    the scores in descending order under Julia's isless: NaN largest (all NaNs rank equal), -0.0 below +0.0,
+ *            ties to the lower index -- Julia's stable sortperm(vals; rev=true), truncated to k.  This is the order of
+ *            best_val / best_idx too: top_val[0], top_idx[0] equal boss_ei_score's pair bit for bit.
+ *   indices  0-based, into Xs; with boss_init_multi the result is bit-identical to the single-device call.
+ * With `best` set and at least 64 Ki candidates the call scores exactly only candidates whose EI upper bound can still
+ * reach the k best (DESIGN.md 2.10); the result is the same either way.  MC-EI (boss_mcei_score) has no top-k. */
+int boss_ei_score_topk(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
+                       const double *prior_mean_s, const double *fit_coefs, const double *best, const double *y_max,
+                       const double *lb, const double *ub, const uint8_t *cons_mask, int64_t k, double *top_val,
+                       int64_t *top_idx);
+int boss_ei_score_topk_dev(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs_dev, int64_t M,
+                           const double *prior_mean_s_dev, const double *fit_coefs, const double *best,
+                           const double *y_max, const double *lb, const double *ub, const uint8_t *cons_mask_dev,
+                           int64_t k, double *top_val, int64_t *top_idx, void *stream);
+
 /* Same scoring with the candidates GENERATED ON THE DEVICE -- the batch never exists in host memory
  * (16 Mi x 8 candidates = 1 GiB in BASELINE config C2).  Indices are global; a shard [first, first + M) of the
  * index range reproduces exactly the points of the unsharded call, so multi-GPU sharding is by index block.
@@ -280,7 +299,7 @@ int boss_dbg_factors(const boss_gp *gp, double *L, double *W, double *alpha);   
  * it recommends instead. */
 int64_t boss_dbg_check_redzones(int64_t *n_allocs);
 int64_t boss_dbg_redzone_selftest(void);   /* negative control: writes 2 guard bytes on purpose, returns how many the scan found */
-/* argmax screening of the last scoring call on the current device: out[0] = 0 not screened, 1 screened, 2 fell back
+/* argmax / top-k screening of the last scoring call on the current device: out[0] = 0 not screened, 1 screened, 2 fell back
  * to the full path after the first chunk; out[1] = candidates bounded; out[2] = candidates that survived the bound */
 int boss_dbg_screen_stats(int64_t *out);
 

@@ -254,6 +254,29 @@ function score(acq::B200Acquisition, X::AbstractMatrix{<:Real}; want_acq::Bool=t
     end
     return out, bv[], Int(bi[]) + 1
 end
+"The k best columns of X: (values, 1-based indices) in descending isless order (NaN first), ties to the lower index --
+`sortperm(vals; rev=true)[1:k]`.  LinFitness selects on the device (boss_ei_score_topk); MC-EI sorts on the host."
+function score_topk(acq::B200Acquisition, X::AbstractMatrix{<:Real}, k::Integer)
+    Xs = Matrix{Float64}(X)
+    M = size(Xs, 2)
+    1 <= k <= M || throw(BoundsError(1:M, k))                     # as order[1:multistart] in sample_opt.jl
+    f = acq.fitness
+    if !(f isa LinFitness)
+        vals = score(acq, Xs)[1]
+        order = sortperm(vals; rev=true)[1:k]
+        return vals[order], order
+    end
+    pm = prior_means(acq, Xs); cm = cons_mask(acq, Xs)
+    best = isnothing(acq.best) ? nothing : [acq.best]
+    coefs = Vector{Float64}(f.coefs)
+    tv = Vector{Float64}(undef, k); ti = Vector{Int64}(undef, k)
+    GC.@preserve Xs pm cm best coefs check(ccall((:boss_ei_score_topk, LIB), Cint,
+        (Ptr{Ptr{Cvoid}}, Cint, Cint, Ptr{Cdouble}, Int64, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble},
+         Ptr{Cdouble}, Ptr{Cdouble}, Ptr{UInt8}, Int64, Ptr{Cdouble}, Ptr{Int64}),
+        acq.handles, acq.ydim, length(acq.posts), Xs, M, cptr(pm), coefs, cptr(best), cptr(acq.y_max), cptr(acq.lb),
+        cptr(acq.ub), cptr(cm), k, tv, ti))
+    return tv, ti .+ 1
+end
 (acq::B200Acquisition)(X::AbstractMatrix{<:Real}) = score(acq, X)[1]
 (acq::B200Acquisition)(x::AbstractVector{<:Real}) = score(acq, hcat(x))[1][1]
 
@@ -354,9 +377,10 @@ function maximize_b200(am::OptimizationAM, problem, options, acq; starts=BOSS.ge
 end
 # SampleOptAM (sample_opt.jl:41-52)
 function maximize_b200(am::SampleOptAM, problem, options, acq)
-    X, vals = maximize_b200(am.sampler, problem, options, acq; return_all=true)
-    order = reverse(sortperm(vals))
-    starts = X[:, order[1:am.optimizer.multistart]]
+    X = draw_samples(am.sampler, problem)
+    size(X, 2) == 0 && error("SamplingAM: No samples were successfully drawn!")
+    _, order = score_topk(acq, X, am.optimizer.multistart)      # the best samples in sortperm(vals; rev=true) order
+    starts = X[:, order]
     return maximize_b200(am.optimizer, problem, options, acq; starts)
 end
 # SequentialBatchAM (batch.jl:26-38): ONE fit, then an O(n^2) factor-cache append per speculative point -- the
