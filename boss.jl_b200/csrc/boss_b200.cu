@@ -132,10 +132,10 @@ struct Ctx {
   bool timing = false;
   bool attrs_done = false;
   // workspaces
-  DevBuf ks, muv, sumsq, xs_stage, pm_stage, cm_stage, acq_stage, mu_stage, var_stage, st_stage, grad_stage;
-  DevBuf blk_val, blk_idx, small, chol_L, chol_Winv, chol_misc, tt, vt, ut, dmu, dvar, pmg_stage;
+  DevBuf ks, muv, sumsq, xs_stage, pm_stage, acq_stage, mu_stage;
+  DevBuf blk_val, blk_idx, small, chol_L, chol_Winv, chol_misc, tt, vt, ut, dmu, dvar;
   DevBuf part_mu, part_ss, part_gm, part_gv, cov_p, cov_stage, chol_W, chol_WT, ll_vec, ll_part, ms_buf;   // split-invariant partial sums (score.cuh / grad.cuh)
-  DevBuf scr_misc, scr_pool;         // argmax screening: bounds, counts, seed batch / survivor pool (score_core)
+  DevBuf scr_misc, scr_pool;         // argmax screening: bounds, counts, seed batch / survivor pool (Screen)
   DevBuf topk;                       // top-k calls: running set, chunk scores, selection state, sorted result
   int64_t scr_stats[3] = {0, 0, 0};  // last scoring call: screened (1) or fell back (2), candidates bounded, pool size
   // event pool for per-kernel-class timing
@@ -155,7 +155,7 @@ struct Ctx {
   cudaStream_t ll_stream[LL_GROUPS] = {};
   cudaEvent_t ll_fork = nullptr, ll_join[LL_GROUPS] = {};
   std::set<boss_gp *> live;          // handles whose buffers live on this device (boss_shutdown invalidates them)
-  void *pinned = nullptr;            // pinned bounce buffer for pageable host candidates (see stage_h2d)
+  void *pinned = nullptr;            // pinned slots for chunks of host arrays (see HostStaging)
   size_t pinned_cap = 0;
   cudaEvent_t pin_ev[2] = {nullptr, nullptr};
 };
@@ -574,11 +574,10 @@ void shutdown_device(Ctx *cx) {   // g_reg_mu held
     h->dev = -1;
   }
   cx->live.clear();
-  for (DevBuf *b : {&cx->ks, &cx->muv, &cx->sumsq, &cx->xs_stage, &cx->pm_stage, &cx->cm_stage, &cx->acq_stage,
-                    &cx->mu_stage, &cx->var_stage, &cx->st_stage, &cx->grad_stage, &cx->blk_val, &cx->blk_idx, &cx->small,
-                    &cx->chol_L, &cx->chol_Winv, &cx->chol_misc, &cx->tt, &cx->vt, &cx->ut, &cx->dmu, &cx->dvar,
-                    &cx->pmg_stage, &cx->part_mu, &cx->part_ss, &cx->part_gm, &cx->part_gv, &cx->cov_p, &cx->cov_stage,
-                    &cx->chol_W, &cx->chol_WT, &cx->ll_vec, &cx->ll_part, &cx->ms_buf})
+  for (DevBuf *b : {&cx->ks, &cx->muv, &cx->sumsq, &cx->xs_stage, &cx->pm_stage, &cx->acq_stage, &cx->mu_stage,
+                    &cx->blk_val, &cx->blk_idx, &cx->small, &cx->chol_L, &cx->chol_Winv, &cx->chol_misc, &cx->tt, &cx->vt,
+                    &cx->ut, &cx->dmu, &cx->dvar, &cx->part_mu, &cx->part_ss, &cx->part_gm, &cx->part_gv, &cx->cov_p,
+                    &cx->cov_stage, &cx->chol_W, &cx->chol_WT, &cx->ll_vec, &cx->ll_part, &cx->ms_buf})
     b->release();
   pool_release_all();
   if (cx->pinned) cudaFreeHost(cx->pinned);
@@ -1118,18 +1117,86 @@ bool is_pinned_host(const void *p) {
   return at.type == cudaMemoryTypeHost;
 }
 
+// offset of the next `bytes` in a buffer carved in 256-byte aligned pieces, `tot` bytes so far
+size_t take(size_t &tot, size_t bytes) {
+  const size_t o = tot;
+  tot += (bytes + 255) / 256 * 256;
+  return o;
+}
+
+// the one place an XcovParams is filled: slice h against the candidates xs (candidate m in column m - in_off), the
+// partials of the chunk that starts at m0 with leading dimension ld
+XcovParams xcov_params(const boss_gp *h, const double *xs, long long M, long long m0, long long in_off, int d, int ld) {
+  XcovParams xp{};
+  xp.Xs = xs;
+  xp.M = M;
+  xp.m0 = m0;
+  xp.in_off = in_off;
+  xp.d = d;
+  xp.n = h->n;
+  xp.n_pad = h->n_pad;
+  xp.ktiles = h->ktiles;
+  xp.Xt = h->Xt;
+  xp.invl = h->invl;
+  xp.disc_bits = h->disc;
+  xp.alpha = h->alpha;
+  xp.a2 = h->a2;
+  xp.Ks = C().ks.as<double>();
+  xp.mu_part = C().part_mu.as<double>();
+  xp.ld = ld;
+  return xp;
+}
+
+// device arrays of one chunk: candidate m of the call is at position m - off of each
+struct ChunkIO {
+  const double *xs = nullptr, *pm = nullptr, *pmg = nullptr;
+  const unsigned char *cm = nullptr;
+  double *acq = nullptr, *mu = nullptr, *var = nullptr, *grad = nullptr;
+  int *st = nullptr;
+  long long off = 0;
+};
+
 // Host <-> device staging of a chunked call with HOST arrays.  The caller's arrays are ordinary pageable memory in
 // the drop-in case (a Julia Matrix{Float64}); a cudaMemcpyAsync from pageable memory first drains the stream and then
 // copies synchronously, so the GPU would idle during every chunk's transfer.  Instead each chunk's inputs go through
 // one of two pinned slots (host memcpy -> DMA on a copy stream) into one of two device slots while the previous chunk
 // computes, and the outputs of chunk c are copied out of their pinned slot while chunk c+1 runs.
-struct Stager {
-  size_t in_bytes = 0, out_bytes = 0;   // per slot
-  unsigned char *pin_in[2] = {}, *pin_out[2] = {};
-  int ensure(size_t in_b, size_t out_b) {
-    in_bytes = (in_b + 255) / 256 * 256;
-    out_bytes = (out_b + 255) / 256 * 256;
-    const size_t need = 2 * (in_bytes + out_bytes) + 256;
+struct HostStaging {
+  const ScoreArgs *a = nullptr;   // null: the call has no host arrays
+  int d = 0, CH = 0;
+  bool has_pmg = false;
+  bool xs_direct = false;   // the caller's candidate matrix is pinned already: DMA straight from it
+  // byte offsets of every array inside a slot
+  size_t in_xs = 0, in_pm = 0, in_cm = 0, in_pmg = 0, in_total = 0;
+  size_t out_acq = 0, out_mu = 0, out_var = 0, out_st = 0, out_gr = 0, out_total = 0;
+  unsigned char *pin_in[2] = {}, *pin_out[2] = {}, *dev_in[2] = {}, *dev_out[2] = {};
+  cudaStream_t cp = C().ll_stream[LL_GROUPS - 1];   // copy stream (the last log-likelihood group stream is idle here)
+  cudaEvent_t ev_in[2] = {C().ll_join[LL_GROUPS - 1], C().ll_join[LL_GROUPS - 2]};     // H2D of the slot done
+  cudaEvent_t ev_free[2] = {C().ll_join[LL_GROUPS - 3], C().ll_join[LL_GROUPS - 4]};   // compute done with the device slot
+  cudaEvent_t ev_out[2] = {C().pin_ev[0], C().pin_ev[1]};                              // outputs of the slot are in pinned memory
+  bool in_used[2] = {false, false}, free_rec[2] = {false, false};
+  long long prev_m0 = -1;      // the chunk whose outputs wait in their pinned slot
+  int prev_ch = 0, prev_slot = 0;
+
+  int plan(const ScoreArgs &args, int ch_cap, int dim) {
+    a = &args;
+    CH = ch_cap;
+    d = dim;
+    has_pmg = a->grad && a->prior_mean_grad;
+    xs_direct = !a->gen && is_pinned_host(a->Xs);
+    in_xs = take(in_total, (size_t)CH * d * 8);   // device slot always holds the candidates
+    if (a->prior_mean) in_pm = take(in_total, (size_t)CH * a->y_dim * 8);
+    if (a->cons_mask) in_cm = take(in_total, (size_t)CH);
+    if (has_pmg) in_pmg = take(in_total, (size_t)CH * d * a->y_dim * 8);
+    if (a->acq) out_acq = take(out_total, (size_t)CH * 8);
+    if (a->mu_out) out_mu = take(out_total, (size_t)CH * 8);
+    if (a->var_out) out_var = take(out_total, (size_t)CH * 8);
+    if (a->status_out) out_st = take(out_total, (size_t)CH * 4);
+    if (a->grad) out_gr = take(out_total, (size_t)CH * d * 8);
+    const size_t out_slot = std::max<size_t>(out_total, 256);
+    CUDA_TRY(C().xs_stage.ensure(2 * in_total));    // both device input slots
+    CUDA_TRY(C().acq_stage.ensure(2 * out_slot));   // both device output slots
+    const size_t need = 2 * (in_total + out_total) + 256;   // both pinned input and output slots
     if (need > C().pinned_cap) {
       if (C().pinned) cudaFreeHost(C().pinned);
       C().pinned = nullptr;
@@ -1137,68 +1204,381 @@ struct Stager {
       CUDA_TRY(cudaHostAlloc(&C().pinned, need + need / 4, cudaHostAllocDefault));
       C().pinned_cap = need + need / 4;
     }
-    unsigned char *b = reinterpret_cast<unsigned char *>(C().pinned);
-    pin_in[0] = b;
-    pin_in[1] = b + in_bytes;
-    pin_out[0] = b + 2 * in_bytes;
-    pin_out[1] = b + 2 * in_bytes + out_bytes;
+    unsigned char *pin = reinterpret_cast<unsigned char *>(C().pinned);
+    pin_in[0] = pin;
+    pin_in[1] = pin + in_total;
+    pin_out[0] = pin + 2 * in_total;
+    pin_out[1] = pin + 2 * in_total + out_total;
+    dev_in[0] = C().xs_stage.as<unsigned char>();
+    dev_in[1] = dev_in[0] + in_total;
+    dev_out[0] = C().acq_stage.as<unsigned char>();
+    dev_out[1] = dev_out[0] + out_slot;
     return 0;
   }
-};
 
-// Argmax screening (DESIGN.md 2.9) runs for calls of at least this many candidates (BOSS_SCREEN_MIN_M overrides, read
-// per call): below it the bounds, the seed batch and the two waits of the first chunk are a visible share of the call.
-constexpr long long SCREEN_MIN_M = 65536;
-constexpr size_t SCREEN_POOL_BYTES = (size_t)1 << 30;   // pool for every candidate of the call; larger calls are not screened
-constexpr double SCREEN_MIN_T = 0x1p-960;   // below it the EI evaluations lose relative precision (DESIGN.md 2.9)
-long long screen_min_m() {
-  const char *e = getenv("BOSS_SCREEN_MIN_M");
-  return e ? atoll(e) : SCREEN_MIN_M;
-}
+  // device arrays of chunk [m0, m0 + ch) in `slot`: its inputs were staged while the previous chunk was being launched
+  // (the first chunk's are staged here), generated candidates are written into the slot now
+  int chunk_inputs(long long m0, int ch, int slot, ChunkIO &io) {
+    if (m0 == 0) {
+      CUDA_TRY(cudaEventRecord(ev_free[0], C().stream));   // nothing enqueued before this point reads the slots
+      int rc = stage_in(0, ch, 0);
+      if (rc) return rc;
+    }
+    CUDA_TRY(cudaStreamWaitEvent(C().stream, ev_in[slot], 0));
+    io.xs = reinterpret_cast<const double *>(dev_in[slot] + in_xs);
+    if (a->gen) {
+      gen_candidates_kernel<<<(ch * d + 255) / 256, 256, 0, C().stream>>>(*a->gen, m0, ch, const_cast<double *>(io.xs));
+      ++C().launches;
+    }
+    if (a->prior_mean) io.pm = reinterpret_cast<const double *>(dev_in[slot] + in_pm);
+    if (a->cons_mask) io.cm = dev_in[slot] + in_cm;
+    if (has_pmg) io.pmg = reinterpret_cast<const double *>(dev_in[slot] + in_pmg);
+    io.off = m0;   // the slot arrays start at the chunk's first candidate
+    if (a->acq) io.acq = reinterpret_cast<double *>(dev_out[slot] + out_acq);
+    if (a->mu_out) io.mu = reinterpret_cast<double *>(dev_out[slot] + out_mu);
+    if (a->var_out) io.var = reinterpret_cast<double *>(dev_out[slot] + out_var);
+    if (a->status_out) io.st = reinterpret_cast<int *>(dev_out[slot] + out_st);
+    if (a->grad) io.grad = reinterpret_cast<double *>(dev_out[slot] + out_gr);
+    return 0;
+  }
 
-// device buffers of a screened call: the bounds of one chunk, per-256 survivor counts, the pool size (two slots),
-// the seed selection (two ping-pong rounds), the seed batch and the survivor pool
-struct ScreenBufs {
-  double *bound = nullptr, *seed_x = nullptr, *seed_pm = nullptr, *pool_x = nullptr, *pool_pm = nullptr;
-  int *cnt = nullptr, *ti[2] = {};
-  unsigned long long *tk[2] = {};
-  long long *base = nullptr, *pool_idx = nullptr;
-  unsigned char *seed_cm = nullptr, *pool_cm = nullptr;
-  int setup(long long M, int CH, int d, int y_dim, bool pm, bool cm, int ns_max) {
-    size_t tot = 0;
-    auto take = [&tot](size_t bytes) {
-      const size_t o = tot;
-      tot += (bytes + 255) / 256 * 256;
-      return o;
+  // after the chunk's kernels have been enqueued: its outputs go to their pinned slot, and while the chunk runs the next
+  // chunk's inputs are staged and the previous chunk's outputs are handed to the caller
+  int end_chunk(long long m0, int ch, int slot) {
+    CUDA_TRY(cudaEventRecord(ev_free[slot], C().stream));   // the kernels above were the last readers of the input slot
+    free_rec[slot] = true;
+    if (out_total) {
+      CUDA_TRY(cudaMemcpyAsync(pin_out[slot], dev_out[slot], out_total, cudaMemcpyDeviceToHost, C().stream));
+      CUDA_TRY(cudaEventRecord(ev_out[slot], C().stream));
+    }
+    if (m0 + CH < a->M) {
+      int rc = stage_in(m0 + CH, (int)std::min<long long>(CH, a->M - m0 - CH), slot ^ 1);
+      if (rc) return rc;
+    }
+    if (prev_m0 >= 0) {
+      int rc = drain_out(prev_m0, prev_ch, prev_slot);
+      if (rc) return rc;
+    }
+    prev_m0 = m0;
+    prev_ch = ch;
+    prev_slot = slot;
+    return 0;
+  }
+
+  // once the stream has drained: the copy stream is idle and the last chunk's outputs (their event has completed by
+  // then) go to the caller.  Nothing to do for device arrays.
+  int drain_last() {
+    if (!a) return 0;
+    CUDA_TRY(cudaStreamSynchronize(cp));
+    return prev_m0 >= 0 ? drain_out(prev_m0, prev_ch, prev_slot) : 0;
+  }
+
+ private:
+  // inputs of chunk [m0, m0 + ch) -> device slot; returns after the copies have been ENQUEUED on the copy stream
+  int stage_in(long long m0, int ch, int slot) {
+    if (in_used[slot]) CUDA_TRY(cudaEventSynchronize(ev_in[slot]));   // the pinned slot's previous DMA has completed
+    if (free_rec[slot]) CUDA_TRY(cudaStreamWaitEvent(cp, ev_free[slot], 0));   // kernels of chunk c-2 are done with the device slot
+    unsigned char *pin = pin_in[slot], *dv = dev_in[slot];
+    auto put = [&](size_t off, const void *src, size_t bytes) {   // host array -> pinned slot -> device slot
+      std::memcpy(pin + off, src, bytes);
+      return cudaMemcpyAsync(dv + off, pin + off, bytes, cudaMemcpyHostToDevice, cp);
     };
-    const size_t ntk = (size_t)(CH + TOPK_IN - 1) / TOPK_IN * SEED_N;
-    const size_t o_bound = take((size_t)CH * 8), o_cnt = take((size_t)(CH + 255) / 256 * 4), o_base = take(16);
-    const size_t o_tk0 = take(ntk * 8), o_tk1 = take(ntk * 8), o_ti0 = take(ntk * 4), o_ti1 = take(ntk * 4);
-    const size_t o_sx = take((size_t)ns_max * d * 8), o_spm = take((size_t)ns_max * y_dim * 8), o_scm = take(ns_max);
-    CUDA_TRY(C().scr_misc.ensure(tot));
-    unsigned char *b = C().scr_misc.as<unsigned char>();
-    bound = reinterpret_cast<double *>(b + o_bound);
-    cnt = reinterpret_cast<int *>(b + o_cnt);
-    base = reinterpret_cast<long long *>(b + o_base);
-    tk[0] = reinterpret_cast<unsigned long long *>(b + o_tk0);
-    tk[1] = reinterpret_cast<unsigned long long *>(b + o_tk1);
-    ti[0] = reinterpret_cast<int *>(b + o_ti0);
-    ti[1] = reinterpret_cast<int *>(b + o_ti1);
-    seed_x = reinterpret_cast<double *>(b + o_sx);
-    seed_pm = reinterpret_cast<double *>(b + o_spm);
-    seed_cm = b + o_scm;
-    tot = 0;
-    const size_t o_px = take((size_t)M * d * 8), o_pidx = take((size_t)M * 8);
-    const size_t o_ppm = pm ? take((size_t)M * y_dim * 8) : 0, o_pcm = cm ? take((size_t)M) : 0;
-    CUDA_TRY(C().scr_pool.ensure(tot));
-    b = C().scr_pool.as<unsigned char>();
-    pool_x = reinterpret_cast<double *>(b + o_px);
-    pool_idx = reinterpret_cast<long long *>(b + o_pidx);
-    pool_pm = pm ? reinterpret_cast<double *>(b + o_ppm) : nullptr;
-    pool_cm = cm ? b + o_pcm : nullptr;
+    if (!a->gen) {
+      const double *src = a->Xs + (size_t)m0 * d;
+      if (xs_direct)
+        CUDA_TRY(cudaMemcpyAsync(dv + in_xs, src, (size_t)ch * d * 8, cudaMemcpyHostToDevice, cp));
+      else
+        CUDA_TRY(put(in_xs, src, (size_t)ch * d * 8));
+    }
+    if (a->prior_mean) CUDA_TRY(put(in_pm, a->prior_mean + (size_t)m0 * a->y_dim, (size_t)ch * a->y_dim * 8));
+    if (a->cons_mask) CUDA_TRY(put(in_cm, a->cons_mask + m0, (size_t)ch));
+    if (has_pmg) CUDA_TRY(put(in_pmg, a->prior_mean_grad + (size_t)m0 * d * a->y_dim, (size_t)ch * d * a->y_dim * 8));
+    CUDA_TRY(cudaEventRecord(ev_in[slot], cp));
+    in_used[slot] = true;
+    return 0;
+  }
+  // outputs of chunk [m0, m0 + ch): pinned slot -> the caller's arrays (after the chunk's D2H has completed)
+  int drain_out(long long m0, int ch, int slot) {
+    if (out_total == 0) return 0;
+    CUDA_TRY(cudaEventSynchronize(ev_out[slot]));
+    const unsigned char *pin = pin_out[slot];
+    if (a->acq) std::memcpy(a->acq + m0, pin + out_acq, (size_t)ch * 8);
+    if (a->mu_out) std::memcpy(a->mu_out + m0, pin + out_mu, (size_t)ch * 8);
+    if (a->var_out) std::memcpy(a->var_out + m0, pin + out_var, (size_t)ch * 8);
+    if (a->status_out) std::memcpy(a->status_out + m0, pin + out_st, (size_t)ch * 4);
+    if (a->grad) std::memcpy(a->grad + (size_t)m0 * d, pin + out_gr, (size_t)ch * d * 8);
     return 0;
   }
 };
+
+// What every stage of one scoring call reads: its arguments, the slices' replicas on this device, the chunk capacity
+// and the small block of per-call device scalars.
+struct ScoreCall {
+  ScoreArgs &a;
+  std::vector<const boss_gp *> sl;
+  int nsl = 0, d = 0, CH = 0;
+  bool have_vt = false;
+  // small: a2[nsl] | lb[d] | ub[d] | best(1) | bidx(1 as int64) | any_fail(int) | finished-CTA counter (fused epilogue)
+  std::vector<double> hs;   // host image of the small block
+  double *small = nullptr, *d_best = nullptr;
+  long long *d_bidx = nullptr;
+  int *d_anyfail = nullptr;
+  unsigned int *d_counter = nullptr;
+  MixParams mixp{};
+
+  explicit ScoreCall(ScoreArgs &args) : a(args) {}
+
+  // the replicas of the slices on this context's device
+  int bind() {
+    nsl = a.y_dim * a.n_samples;
+    if (nsl < 1 || a.y_dim > MAX_YDIM) return fail(BOSS_ERR_ARG, "score: y_dim must be in 1..16");
+    sl.resize(nsl);
+    for (int q = 0; q < nsl; ++q) {
+      if (!a.slices[q]) return fail(BOSS_ERR_ARG, "score: NULL slice handle");
+      sl[q] = replica_on(a.slices[q], C().device);
+      if (!sl[q]) return fail(BOSS_ERR_STATE, "score: a slice handle has no replica on this device (or was invalidated by boss_shutdown)");
+      if (sl[q]->d != sl[0]->d) return fail(BOSS_ERR_ARG, "score: slices disagree on x_dim");
+    }
+    d = sl[0]->d;
+    return 0;
+  }
+
+  // chunk size, workspaces, the small block and the MC-EI eps matrix on the device
+  int setup() {
+    int max_npad = 0;
+    for (int q = 0; q < nsl; ++q) max_npad = std::max(max_npad, sl[q]->n_pad);
+    // chunk size: K*^T scratch budget 4 GiB, at most 4 waves of 148 CTAs
+    long long ncb_max = (4ll << 30) / (1024ll * max_npad);
+    ncb_max = std::min<long long>(ncb_max, 592);
+    if (ncb_max >= 148) ncb_max = ncb_max / 148 * 148;
+    if (ncb_max < 1) return fail(BOSS_ERR_ARG, "score: n too large for the scratch budget");
+    if (a.grad) ncb_max = std::max<long long>(1, std::min<long long>(ncb_max, ncb_max >= 296 ? 296 : ncb_max));
+    const long long need_cb = (a.M + 127) / 128;
+    const int ncb_cap = (int)std::min<long long>(ncb_max, need_cb);
+    CH = ncb_cap * 128;
+
+    CUDA_TRY(C().ks.ensure((size_t)CH * max_npad * 8));
+    CUDA_TRY(C().muv.ensure((size_t)nsl * CH * 8));
+    CUDA_TRY(C().sumsq.ensure((size_t)nsl * CH * 8));
+    const int max_nblk = max_npad / TM;
+    CUDA_TRY(C().part_mu.ensure((size_t)2 * max_nblk * CH * 8));
+    CUDA_TRY(C().part_ss.ensure((size_t)2 * max_nblk * CH * 8));
+    // batches up to 8192 candidates keep V^T even without gradients: the quarter-row kernels (10 % faster than the
+    // row-split wide kernels up to there) reduce the variance from the stored tile
+    have_vt = a.grad || CH <= 8192;
+    if (have_vt && !a.grad) CUDA_TRY(C().vt.ensure((size_t)CH * max_npad * 8));
+    if (a.grad) {
+      if (d > 32) return fail(BOSS_ERR_ARG, "score: gradients need x_dim <= 32");
+      CUDA_TRY(C().vt.ensure((size_t)CH * max_npad * 8));
+      CUDA_TRY(C().ut.ensure((size_t)CH * max_npad * 8));
+      CUDA_TRY(C().dmu.ensure((size_t)nsl * d * CH * 8));
+      CUDA_TRY(C().dvar.ensure((size_t)nsl * d * CH * 8));
+      CUDA_TRY(C().part_gm.ensure((size_t)2 * max_nblk * d * CH * 8));
+      CUDA_TRY(C().part_gv.ensure((size_t)2 * max_nblk * d * CH * 8));
+    }
+    const int nblk_acq_max = (CH + 127) / 128;     // block winners: per 256 candidates (acq_kernel) or per 128 (fused epilogue)
+    CUDA_TRY(C().blk_val.ensure((size_t)nblk_acq_max * 8));
+    CUDA_TRY(C().blk_idx.ensure((size_t)nblk_acq_max * 8));
+    const size_t sm_n = (size_t)nsl + 2 * d + 5;
+    CUDA_TRY(C().small.ensure(sm_n * 8));
+    small = C().small.as<double>();
+    hs.assign(sm_n, 0.0);
+    for (int q = 0; q < nsl; ++q) hs[q] = sl[q]->a2;
+    if (a.lb && a.ub) {
+      for (int i = 0; i < d; ++i) {
+        hs[nsl + i] = a.lb[i];
+        hs[nsl + d + i] = a.ub[i];
+      }
+    }
+    long long neg1 = -1;
+    std::memcpy(&hs[nsl + 2 * d + 1], &neg1, 8);
+    int rc = upload_small();
+    if (rc) return rc;
+    d_best = small + nsl + 2 * d;
+    d_bidx = reinterpret_cast<long long *>(small + nsl + 2 * d + 1);
+    d_anyfail = reinterpret_cast<int *>(small + nsl + 2 * d + 2);
+    d_counter = reinterpret_cast<unsigned int *>(small + nsl + 2 * d + 3);
+    if (a.mix) {   // MC-EI: the eps matrix (y_dim x n_eps) goes to the device once per call
+      mixp = *a.mix;
+      const size_t eb = (size_t)a.y_dim * mixp.n_eps * 8;
+      CUDA_TRY(C().tt.ensure(eb));
+      CUDA_TRY(cudaMemcpyAsync(C().tt.p, mixp.eps_host, eb, cudaMemcpyHostToDevice, C().stream));
+      CUDA_TRY(cudaStreamSynchronize(C().stream));
+      mixp.eps = C().tt.as<double>();
+    }
+    return 0;
+  }
+
+  // hs is pageable: the runtime has copied these few bytes to its staging memory when the call returns (CUDA's
+  // documented behaviour for pageable-to-device cudaMemcpyAsync), and hs lives until the end of the call: no stream
+  // round trip is needed here
+  int upload_small() const {
+    CUDA_TRY(cudaMemcpyAsync(small, hs.data(), hs.size() * 8, cudaMemcpyHostToDevice, C().stream));
+    return 0;
+  }
+
+  AcqParams acq_params(long long m0, int ch, const ChunkIO &io) const {
+    AcqParams ap{};
+    ap.y_dim = a.y_dim;
+    ap.n_samples = a.n_samples;
+    ap.d = d;
+    ap.M = a.M;
+    ap.m0 = m0;
+    ap.in_off = io.off;
+    ap.out_off = io.off;
+    ap.chunk = ch;
+    ap.chunk_ld = CH;
+    ap.mu = C().muv.as<double>();
+    ap.sumsq = C().sumsq.as<double>();
+    ap.a2 = small;
+    ap.prior_mean = io.pm;
+    for (int i = 0; i < a.y_dim; ++i) {
+      ap.coefs[i] = a.coefs ? a.coefs[i] : (i == 0 ? 1.0 : 0.0);
+      ap.y_max[i] = a.y_max ? a.y_max[i] : INFINITY;
+    }
+    ap.has_best = a.best != nullptr;
+    ap.best = a.best ? *a.best : 0.0;
+    ap.has_ymax = a.y_max != nullptr;
+    ap.Xs = io.xs;
+    ap.lb = (a.lb && a.ub) ? small + nsl : nullptr;
+    ap.ub = (a.lb && a.ub) ? small + nsl + d : nullptr;
+    ap.cons_mask = io.cm;
+    ap.acq = io.acq;
+    ap.mu_out = io.mu;
+    ap.var_out = io.var;
+    ap.status_out = io.st;
+    ap.any_fail = d_anyfail;
+    ap.blk_val = a.want_argmax ? C().blk_val.as<double>() : nullptr;
+    ap.blk_idx = a.want_argmax ? C().blk_idx.as<long long>() : nullptr;
+    ap.mix = mixp;
+    return ap;
+  }
+};
+
+// Slice q of one chunk on the full path: mean partials and K*^T (xcov), the triangular product, the reductions and,
+// with gradients, the gradient launches.  Returns whether the scoring kernel finished the chunk itself (fused epilogue).
+bool score_slice(const ScoreCall &c, int q, const AcqParams &ap, const ChunkIO &io) {
+  const ScoreArgs &a = c.a;
+  const boss_gp *h = c.sl[q];
+  const int CH = c.CH, d = c.d, ch = ap.chunk, ncb = (ch + 127) / 128;
+  // Small candidate batches (multi-start optimiser iterations, single-point calls) cannot fill 148 SMs
+  // with one CTA per 128 candidates: deal the training chunks / W row blocks of a candidate block to
+  // several CTAs.  Partial sums are kept per chunk / per row block, so results do not depend on the split.
+  const int want = (16 * 148 + ncb - 1) / ncb;   // >= 16 CTAs per SM in flight over the launch (4 waves of 4)
+  const int nks = std::max(1, std::min(h->nblk, want));            // xcov / grad: splits over training chunks
+  double cost_w = 0.0, cost_n = 0.0;
+  const int nsp = pick_row_splits(ncb, h->nblk, &cost_w);          // trmm / wtv: zig-zag row-block splits
+  // Small batches: 32-candidate CTAs (score_narrow.cuh) do a quarter of the tensor work per stage of W; worth it
+  // when the wide launch cannot fill the GPU (cost = waves x longest per-CTA share, in block-steps; a narrow stage
+  // takes ~0.3 of a wide one).  Same bits either way.
+  const int ncb32 = (ch + NW_NB - 1) / NW_NB;
+  const int nsp32 = pick_row_splits(ncb32, h->nblk, &cost_n);
+  bool narrow = 0.32 * cost_n < cost_w && getenv("BOSS_NO_NARROW") == nullptr;
+  // Tiny batches: quarter-row-block CTAs (4 nblk per 32 candidates, 4 to an SM).  Cost in the same unit: the
+  // longest CTA's latency-bound walk over 8 nblk short stages, or the launch's tensor work spread over the SMs.
+  const double cost_q = std::max(NQ_COST_CHAIN * h->nblk, NQ_COST_WORK * ncb32 * (h->nblk * (h->nblk + 1) / 2)) + NQ_COST_FIXED;
+  bool quarter = c.have_vt && cost_q < std::min(cost_w, narrow ? 0.32 * cost_n : cost_w) && h->nblk >= 2;
+  if (const char *e = getenv("BOSS_SCORE_PATH")) {   // A/B switch: wide | narrow | quarter
+    if (!strcmp(e, "wide")) narrow = quarter = false;
+    if (!strcmp(e, "narrow")) narrow = true, quarter = false;
+    if (!strcmp(e, "quarter") && c.have_vt) quarter = true;
+  }
+  if (quarter) narrow = false;
+  const int cnt = ncb * 128;
+  {
+    Timed t(1);
+    launch_xcov(h->kernel_id, h->dp, xcov_params(h, io.xs, a.M, ap.m0, io.off, d, CH), dim3(ncb, nks), C().stream);
+  }
+  // One CTA per candidate block walks all of W (large batches) and this is the chunk's last slice: the scoring
+  // kernel finishes the candidates itself (fused epilogue) -- no reduce / acquisition / argmax launches.
+  const bool fuse = nsp == 1 && !narrow && !quarter && q == c.nsl - 1 && getenv("BOSS_UNFUSED_SCORE") == nullptr;
+  if (!fuse && !quarter)
+    reduce_rows_kernel<<<(cnt + 255) / 256, 256, 0, C().stream>>>(C().part_mu.as<double>(), 2 * h->nblk, (size_t)CH,
+                                                               C().muv.as<double>() + (size_t)q * CH, cnt);
+  ScoreParams sp{};
+  sp.W = h->W;
+  sp.Ks = C().ks.as<double>();
+  sp.nblk = h->nblk;
+  sp.ktiles = h->ktiles;
+  sp.ss_part = C().part_ss.as<double>();
+  sp.ld = CH;
+  sp.VT = a.grad ? C().vt.as<double>() : nullptr;
+  if (fuse) {
+    sp.fused = 1;
+    sp.ap = ap;
+    sp.mu_part = C().part_mu.as<double>();
+    sp.P = 2 * h->nblk;
+    sp.mu_row = C().muv.as<double>() + (size_t)q * CH;
+    sp.ss_row = C().sumsq.as<double>() + (size_t)q * CH;
+    sp.best = c.d_best;
+    sp.bidx = c.d_bidx;
+    sp.counter = c.d_counter;
+  }
+  if (quarter) {
+    NarrowParams np{h->W, C().ks.as<double>(), h->nblk, h->ktiles, nullptr, CH, C().vt.as<double>()};
+    Timed t(0);
+    score_quarter_kernel<0, 4, 1><<<dim3(ncb32, 4 * h->nblk), NQ_THREADS, NQ_SMEM_BYTES, C().stream>>>(np);
+    quarter_sumsq_kernel<<<dim3(ncb32, h->nblk), 256, 0, C().stream>>>(C().vt.as<double>(), h->ktiles,
+                                                                     C().part_ss.as<double>(), CH);
+  } else if (narrow) {
+    NarrowParams np{h->W, C().ks.as<double>(), h->nblk, h->ktiles, C().part_ss.as<double>(), CH,
+                    a.grad ? C().vt.as<double>() : nullptr};
+    Timed t(0);
+    score_narrow_kernel<0><<<dim3(ncb32, nsp32), 256, NW_SMEM_BYTES, C().stream>>>(np);
+  } else {
+    Timed t(0);
+    score_trmm_kernel<<<dim3(ncb, nsp), GEMM_THREADS, GEMM_SMEM_BYTES, C().stream>>>(sp);
+  }
+  if (quarter)   // mu partials (xcov) and sums of squares (quarter_sumsq) of this slice in one launch
+    reduce_rows_pair_kernel<<<dim3((cnt + 255) / 256, 2), 256, 0, C().stream>>>(
+        C().part_mu.as<double>(), C().part_ss.as<double>(), 2 * h->nblk, (size_t)CH, C().muv.as<double>() + (size_t)q * CH,
+        C().sumsq.as<double>() + (size_t)q * CH, cnt);
+  else if (!fuse)
+    reduce_rows2_kernel<<<(cnt + 255) / 256, 256, 0, C().stream>>>(C().part_ss.as<double>(), 2 * h->nblk, (size_t)CH,
+                                                                C().sumsq.as<double>() + (size_t)q * CH, cnt);
+  C().launches += fuse ? 2 : 4;
+  if (a.grad) {
+    WtvParams wp{h->WT, C().vt.as<double>(), C().ut.as<double>(), h->nblk, h->ktiles};
+    NarrowParams np{h->WT, C().vt.as<double>(), h->nblk, h->ktiles, nullptr, CH, C().ut.as<double>()};
+    if (quarter) {
+      Timed t(0);
+      score_quarter_kernel<1, 4, 1><<<dim3(ncb32, 4 * h->nblk), NQ_THREADS, NQ_SMEM_BYTES, C().stream>>>(np);
+    } else if (narrow) {
+      Timed t(0);
+      score_narrow_kernel<1><<<dim3(ncb32, nsp32), 256, NW_SMEM_BYTES, C().stream>>>(np);
+    } else {
+      Timed t(0);
+      wtv_kernel<<<dim3(ncb, nsp), GEMM_THREADS, GEMM_SMEM_BYTES, C().stream>>>(wp);
+    }
+    GradParams gq{};
+    gq.Xs = io.xs;
+    gq.M = a.M;
+    gq.m0 = ap.m0;
+    gq.in_off = io.off;
+    gq.d = d;
+    gq.n = h->n;
+    gq.n_pad = h->n_pad;
+    gq.ktiles = h->ktiles;
+    gq.chunk_ld = CH;
+    gq.Xt = h->Xt;
+    gq.invl = h->invl;
+    gq.alpha = h->alpha;
+    gq.disc_bits = h->disc;
+    gq.a2 = h->a2;
+    gq.UT = C().ut.as<double>();
+    gq.gm_part = C().part_gm.as<double>();
+    gq.gv_part = C().part_gv.as<double>();
+    {
+      Timed t(1);
+      launch_grad(h->kernel_id, h->dp, gq, dim3(ncb, nks), C().stream);
+    }
+    GradReduceParams gr{C().part_gm.as<double>(), C().part_gv.as<double>(), 2 * h->nblk, d, CH, cnt, h->invl, h->disc,
+                        C().dmu.as<double>() + (size_t)q * d * CH, C().dvar.as<double>() + (size_t)q * d * CH};
+    grad_reduce_kernel<<<dim3((cnt + 255) / 256, d), 256, 0, C().stream>>>(gr);
+    C().launches += 3;
+  }
+  return fuse;
+}
 
 // seed batch of a screened top-k call: the S_k highest bounds of the first chunk, S_k = 2k rounded up to 128, at least
 // SEED_N and at most the chunk (DESIGN.md 2.10)
@@ -1207,23 +1587,23 @@ int topk_seed_n(long long k, int ch) {
 }
 
 // device buffers of a top-k call (topk.cuh): two running sets of `cap` pairs, the chunk's scores, the selection state
-// and per-256 counts, the sorted result.  Sized by the outermost call; the nested seed and pool calls fit inside.
+// and per-256 counts, the sorted result.  Sized by the outermost call; score_subset checks that the nested seed and pool
+// calls fit inside.
 struct TopkBufs {
   double *run_val[2] = {}, *scores = nullptr, *out_val = nullptr;
   long long *run_idx[2] = {}, *out_idx = nullptr;
   SelectState *st = nullptr;
   int2 *cnt = nullptr;
-  int setup(int cap, int CH, long long k) {
+  long long k = 0;
+  int r = 0, par = 0;   // the running set: r pairs in run_*[par]
+  int setup(long long k_, int CH, int ch0) {
+    k = k_;
+    const int cap = (int)std::max<long long>(k, topk_seed_n(k, ch0));
     size_t tot = 0;
-    auto take = [&tot](size_t bytes) {
-      const size_t o = tot;
-      tot += (bytes + 255) / 256 * 256;
-      return o;
-    };
-    const size_t o_rv0 = take((size_t)cap * 8), o_rv1 = take((size_t)cap * 8), o_ri0 = take((size_t)cap * 8),
-                 o_ri1 = take((size_t)cap * 8), o_sc = take((size_t)CH * 8), o_st = take(sizeof(SelectState)),
-                 o_cnt = take(((size_t)cap + CH + 255) / 256 * sizeof(int2)), o_ov = take((size_t)k * 8),
-                 o_oi = take((size_t)k * 8);
+    const size_t o_rv0 = take(tot, (size_t)cap * 8), o_rv1 = take(tot, (size_t)cap * 8), o_ri0 = take(tot, (size_t)cap * 8),
+                 o_ri1 = take(tot, (size_t)cap * 8), o_sc = take(tot, (size_t)CH * 8), o_st = take(tot, sizeof(SelectState)),
+                 o_cnt = take(tot, ((size_t)cap + CH + 255) / 256 * sizeof(int2)), o_ov = take(tot, (size_t)k * 8),
+                 o_oi = take(tot, (size_t)k * 8);
     CUDA_TRY(C().topk.ensure(tot));
     unsigned char *b = C().topk.as<unsigned char>();
     run_val[0] = reinterpret_cast<double *>(b + o_rv0);
@@ -1257,692 +1637,378 @@ struct TopkBufs {
     C().launches += 2;
     return 0;
   }
+  // the running set becomes the best min(k, seen) of (running set, the chunk's scores)
+  int absorb(long long m0, int ch) {
+    const int tgt = (int)std::min<long long>(k, (long long)r + ch);
+    SelectIn in{run_val[par], run_idx[par], r, scores, m0, ch, 0};
+    int rc = select(in, tgt, run_val[par ^ 1], run_idx[par ^ 1]);
+    if (rc) return rc;
+    par ^= 1;
+    r = tgt;
+    return 0;
+  }
+  // the running set, sorted in one CTA, to the caller: k pairs (indices through `map` unless null), no M-sized output
+  // and no host sort.  The copies are enqueued; the caller synchronises.
+  int finish(const long long *map, double *top_val, int64_t *top_idx) {
+    if (r != k) return fail(BOSS_ERR_STATE, "score: top-k set incomplete");
+    int P = 2;
+    while (P < r) P <<= 1;
+    topk_sort_kernel<<<1, 1024, (size_t)P * 12, C().stream>>>(run_val[par], run_idx[par], r, P, map, out_val, out_idx);
+    ++C().launches;
+    CUDA_TRY(cudaMemcpyAsync(top_val, out_val, (size_t)r * 8, cudaMemcpyDeviceToHost, C().stream));
+    CUDA_TRY(cudaMemcpyAsync(top_idx, out_idx, (size_t)r * 8, cudaMemcpyDeviceToHost, C().stream));
+    return 0;
+  }
+};
+
+int score_core(ScoreArgs &a);
+
+// what a nested call returns besides the top-k pairs
+struct SubsetResult {
+  double best_val = 0.0;
+  int64_t best_idx = -1;
+  int any_fail = 0;
+};
+
+// Every nested call of a screened call: scores M candidates that the library wrote to device memory on its stream (the
+// seed batch or the survivor pool) with the model and acquisition of c's call, top-k pairs to top_val / top_idx with
+// indices through topk_map.  The nested call rewrites the small block, so restore_small puts c's back when the outer
+// call goes on using it.  The outer call holds raw pointers into the small block, the top-k buffers and the screening
+// buffers: a nested call that grew one of them would leave those pointers dangling, so that is an error.
+int score_subset(const ScoreCall &c, const double *x, const double *pm, const unsigned char *cm, long long M,
+                 double *top_val, int64_t *top_idx, const long long *topk_map, bool restore_small, SubsetResult &r) {
+  const size_t held[4] = {C().small.cap, C().topk.cap, C().scr_misc.cap, C().scr_pool.cap};
+  ScoreArgs s = c.a;
+  s.Xs = x;
+  s.M = M;
+  s.prior_mean = pm;
+  s.cons_mask = cm;
+  s.gen = nullptr;
+  s.dev = true;
+  s.internal = true;
+  s.best_val = &r.best_val;
+  s.best_idx = &r.best_idx;
+  s.top_val = top_val;
+  s.top_idx = top_idx;
+  s.topk_map = topk_map;
+  int rc = score_core(s);
+  if (rc) return rc;
+  if (held[0] != C().small.cap || held[1] != C().topk.cap || held[2] != C().scr_misc.cap || held[3] != C().scr_pool.cap)
+    return fail(BOSS_ERR_STATE, "score: a nested scoring call grew a buffer of the outer call");
+  r.any_fail = s.any_fail;
+  return restore_small ? c.upload_small() : 0;
+}
+
+// Argmax screening (DESIGN.md 2.9) runs for calls of at least this many candidates (BOSS_SCREEN_MIN_M overrides, read
+// per call): below it the bounds, the seed batch and the two waits of the first chunk are a visible share of the call.
+constexpr long long SCREEN_MIN_M = 65536;
+constexpr size_t SCREEN_POOL_BYTES = (size_t)1 << 30;   // pool for every candidate of the call; larger calls are not screened
+constexpr double SCREEN_MIN_T = 0x1p-960;   // below it the EI evaluations lose relative precision (DESIGN.md 2.9)
+long long screen_min_m() {
+  const char *e = getenv("BOSS_SCREEN_MIN_M");
+  return e ? atoll(e) : SCREEN_MIN_M;
+}
+
+// Argmax screening (DESIGN.md 2.9): a call that wants only the argmax of the closed-form EI over many candidates bounds
+// every candidate from its mean alone and scores exactly only those that can still win.  Top-k calls (DESIGN.md 2.10)
+// use the same bound against the k-th best score of a larger seed batch.
+struct Screen {
+  enum State { OFF, SCREENING, FELL_BACK } state = OFF;   // scr_stats[0]: 1 once a screened call finished, 2 fell back
+  double thr = -INFINITY;   // survivors: bound >= thr or NaN
+  // device buffers: the bounds of one chunk, per-256 survivor counts, the pool size (two slots), the seed selection
+  // (two ping-pong rounds), the seed batch and the survivor pool
+  double *bound = nullptr, *seed_x = nullptr, *seed_pm = nullptr, *pool_x = nullptr, *pool_pm = nullptr;
+  int *cnt = nullptr, *ti[2] = {};
+  unsigned long long *tk[2] = {};
+  long long *base = nullptr, *pool_idx = nullptr;
+  unsigned char *seed_cm = nullptr, *pool_cm = nullptr;
+
+  bool on() const { return state == SCREENING; }
+
+  // ch0: the first chunk, which the seed batch is drawn from
+  static bool eligible(const ScoreArgs &a, int ch0, int d) {
+    const size_t pool_row = (size_t)d * 8 + (a.prior_mean ? (size_t)a.y_dim * 8 : 0) + 8 + (a.cons_mask ? 1 : 0);
+    return (a.want_argmax || a.topk) && a.best && !a.internal && !a.acq && !a.grad && !a.mu_out && !a.var_out &&
+           !a.status_out && !a.mix && a.M >= screen_min_m() && (size_t)a.M * pool_row <= SCREEN_POOL_BYTES &&
+           a.topk <= ch0 && getenv("BOSS_NO_SCREEN") == nullptr;
+  }
+
+  int begin(const ScoreCall &c, int ch0) {
+    const ScoreArgs &a = c.a;
+    const long long M = a.M;
+    const int CH = c.CH, d = c.d, y_dim = a.y_dim, ns_max = a.topk ? topk_seed_n(a.topk, ch0) : SEED_N;
+    const bool pm = a.prior_mean != nullptr, cm = a.cons_mask != nullptr;
+    size_t tot = 0;
+    const size_t ntk = (size_t)(CH + TOPK_IN - 1) / TOPK_IN * SEED_N;
+    const size_t o_bound = take(tot, (size_t)CH * 8), o_cnt = take(tot, (size_t)(CH + 255) / 256 * 4), o_base = take(tot, 16);
+    const size_t o_tk0 = take(tot, ntk * 8), o_tk1 = take(tot, ntk * 8), o_ti0 = take(tot, ntk * 4), o_ti1 = take(tot, ntk * 4);
+    const size_t o_sx = take(tot, (size_t)ns_max * d * 8), o_spm = take(tot, (size_t)ns_max * y_dim * 8), o_scm = take(tot, ns_max);
+    CUDA_TRY(C().scr_misc.ensure(tot));
+    unsigned char *b = C().scr_misc.as<unsigned char>();
+    bound = reinterpret_cast<double *>(b + o_bound);
+    cnt = reinterpret_cast<int *>(b + o_cnt);
+    base = reinterpret_cast<long long *>(b + o_base);
+    tk[0] = reinterpret_cast<unsigned long long *>(b + o_tk0);
+    tk[1] = reinterpret_cast<unsigned long long *>(b + o_tk1);
+    ti[0] = reinterpret_cast<int *>(b + o_ti0);
+    ti[1] = reinterpret_cast<int *>(b + o_ti1);
+    seed_x = reinterpret_cast<double *>(b + o_sx);
+    seed_pm = reinterpret_cast<double *>(b + o_spm);
+    seed_cm = b + o_scm;
+    tot = 0;
+    const size_t o_px = take(tot, (size_t)M * d * 8), o_pidx = take(tot, (size_t)M * 8);
+    const size_t o_ppm = pm ? take(tot, (size_t)M * y_dim * 8) : 0, o_pcm = cm ? take(tot, (size_t)M) : 0;
+    CUDA_TRY(C().scr_pool.ensure(tot));
+    b = C().scr_pool.as<unsigned char>();
+    pool_x = reinterpret_cast<double *>(b + o_px);
+    pool_idx = reinterpret_cast<long long *>(b + o_pidx);
+    pool_pm = pm ? reinterpret_cast<double *>(b + o_ppm) : nullptr;
+    pool_cm = cm ? b + o_pcm : nullptr;
+    CUDA_TRY(cudaMemsetAsync(base, 0, 16, C().stream));
+    state = SCREENING;
+    return 0;
+  }
+
+  // One chunk: the means of every slice (xcov without K*^T), the bounds, the survivors appended to the pool.  The first
+  // chunk also sets the threshold from the seed batch and ends screening (the chunk is then scored on the full path
+  // from the same staged inputs) when the bound does not separate: T not positive, or more than a quarter of the chunk
+  // surviving.
+  int chunk(const ScoreCall &c, const AcqParams &ap, const ChunkIO &io, int cidx, TopkBufs &tb) {
+    const ScoreArgs &a = c.a;
+    const long long m0 = ap.m0;
+    const int ch = ap.chunk, ncb = (ch + 127) / 128, nb = (ch + 255) / 256;
+    for (int q = 0; q < c.nsl; ++q) {
+      const boss_gp *h = c.sl[q];
+      const int nks = std::max(1, std::min(h->nblk, (16 * 148 + ncb - 1) / ncb));
+      {
+        Timed t(1);
+        launch_xcov_mean(h->kernel_id, h->dp, xcov_params(h, io.xs, a.M, m0, io.off, c.d, c.CH), dim3(ncb, nks),
+                         C().stream);
+      }
+      reduce_rows_kernel<<<(ncb * 128 + 255) / 256, 256, 0, C().stream>>>(C().part_mu.as<double>(), 2 * h->nblk, (size_t)c.CH,
+                                                                        C().muv.as<double>() + (size_t)q * c.CH, ncb * 128);
+    }
+    AcqParams bp = ap;   // EI at the prior variance, PoF = 1, no guards -> bound[c]
+    bp.sumsq = nullptr;
+    bp.has_ymax = 0;
+    bp.lb = bp.ub = nullptr;
+    bp.cons_mask = nullptr;
+    bp.acq = bound;
+    bp.out_off = m0;
+    bp.blk_val = nullptr;
+    bp.blk_idx = nullptr;
+    acq_kernel<<<nb, 256, 0, C().stream>>>(bp);
+    C().launches += 2 * c.nsl + 1;
+    const size_t c0 = (size_t)(m0 - ap.in_off);   // the chunk's first candidate in the input arrays
+    const double *xs_c = ap.Xs + c0 * c.d;
+    const double *pm_c = ap.prior_mean ? ap.prior_mean + c0 * a.y_dim : nullptr;
+    const unsigned char *cm_c = ap.cons_mask ? ap.cons_mask + c0 : nullptr;
+    if (cidx == 0) {
+      int rc = seed(c, ch, xs_c, pm_c, cm_c, tb);
+      if (rc || !on()) return rc;
+    }
+    screen_count_kernel<<<nb, 256, 0, C().stream>>>(bound, ch, thr, cnt);
+    CompactParams cpar{bound, ch, thr, cnt, m0, xs_c, pm_c, cm_c, c.d, a.y_dim, base, cidx & 1,
+                       pool_x, pool_pm, pool_cm, pool_idx};
+    screen_compact_kernel<<<nb, 256, 0, C().stream>>>(cpar);
+    C().launches += 2;
+    if (cidx == 0) {
+      long long surv = 0;
+      CUDA_TRY(cudaMemcpyAsync(&surv, base + 1, 8, cudaMemcpyDeviceToHost, C().stream));
+      CUDA_TRY(cudaStreamSynchronize(C().stream));
+      C().scr_stats[2] = surv;
+      if (4 * surv > ch) fall_back();
+    }
+    return 0;
+  }
+
+  // After the last chunk: the pool (survivors in ascending order) through the ordinary path; its first-maximal winner
+  // (or its k best) map back to the call's indices.
+  int finish(const ScoreCall &c, int nchunks, HostStaging &stg) {
+    ScoreArgs &a = c.a;
+    long long npool = 0;
+    CUDA_TRY(cudaMemcpyAsync(&npool, base + (nchunks & 1), 8, cudaMemcpyDeviceToHost, C().stream));
+    CUDA_TRY(cudaStreamSynchronize(C().stream));
+    int rc = stg.drain_last();
+    if (rc) return rc;
+    C().scr_stats[0] = 1;
+    C().scr_stats[1] = a.M;
+    C().scr_stats[2] = npool;
+    if (npool < 1) return fail(BOSS_ERR_STATE, "score: argmax screening kept no candidate");   // the seed's winner always survives
+    if (npool < a.topk) return fail(BOSS_ERR_STATE, "score: top-k screening kept fewer than k candidates");   // the seed's k best survive
+    SubsetResult r;
+    rc = score_subset(c, pool_x, pool_pm, pool_cm, npool, a.top_val, a.top_idx, pool_idx, false, r);
+    if (rc) return rc;
+    a.any_fail = r.any_fail;
+    if (a.topk) return 0;
+    long long idx = -1;
+    if (r.best_idx >= 0) {
+      CUDA_TRY(cudaMemcpyAsync(&idx, pool_idx + r.best_idx, 8, cudaMemcpyDeviceToHost, C().stream));
+      CUDA_TRY(cudaStreamSynchronize(C().stream));
+    }
+    if (a.best_val) *a.best_val = r.best_val;
+    if (a.best_idx) *a.best_idx = idx;
+    return 0;
+  }
+
+ private:
+  void fall_back() {
+    C().scr_stats[0] = 2;
+    state = FELL_BACK;
+  }
+
+  // The seed batch of the first chunk: the exact scores of its highest bounds.  Their best (argmax) or k-th best
+  // (top-k) score T is a lower bound of the call's best or k-th best score; bounds below T (1 - 2^-30) cannot reach it.
+  int seed(const ScoreCall &c, int ch, const double *xs_c, const double *pm_c, const unsigned char *cm_c, TopkBufs &tb) {
+    const ScoreArgs &a = c.a;
+    int ns;
+    if (a.topk) {   // the S_k highest bounds (NaN bounds last), selected into the top-k buffers
+      ns = topk_seed_n(a.topk, ch);
+      SelectIn in{nullptr, nullptr, 0, bound, 0, ch, 1};
+      int rc = tb.select(in, ns, tb.run_val[0], tb.run_idx[0]);
+      if (rc) return rc;
+      seed_gather_kernel<<<(ns + 255) / 256, 256, 0, C().stream>>>(tb.run_idx[0], ns, xs_c, pm_c, cm_c, c.d, a.y_dim,
+                                                                    seed_x, seed_pm, seed_cm);
+    } else {        // the SEED_N highest bounds: bitonic rounds over TOPK_IN-element blocks
+      int n = ch, par = 0;
+      const unsigned long long *kin = nullptr;
+      const int *iin = nullptr;
+      do {
+        const int nbk = (n + TOPK_IN - 1) / TOPK_IN;
+        seed_topk_kernel<<<nbk, 1024, 0, C().stream>>>(kin ? nullptr : bound, kin, iin, n, tk[par], ti[par]);
+        ++C().launches;
+        kin = tk[par];
+        iin = ti[par];
+        par ^= 1;
+        n = nbk * SEED_N;
+      } while (n > SEED_N);
+      ns = std::min(SEED_N, ch);
+      seed_gather_kernel<<<1, SEED_N, 0, C().stream>>>(iin, ns, xs_c, pm_c, cm_c, c.d, a.y_dim, seed_x, seed_pm, seed_cm);
+    }
+    ++C().launches;
+    std::vector<double> sv((size_t)a.topk);
+    std::vector<int64_t> si((size_t)a.topk);
+    SubsetResult r;
+    int rc = score_subset(c, seed_x, pm_c ? seed_pm : nullptr, cm_c ? seed_cm : nullptr, ns, sv.data(), si.data(),
+                          nullptr, true, r);
+    if (rc) return rc;
+    C().scr_stats[1] = ch;
+    const double T = a.topk ? sv[(size_t)a.topk - 1] : r.best_val;
+    if (!(T >= SCREEN_MIN_T)) {
+      fall_back();
+      return 0;
+    }
+    thr = T * (1.0 - 0x1p-30);
+    return 0;
+  }
 };
 
 int score_core(ScoreArgs &a) {
-  const int nsl = a.y_dim * a.n_samples;
-  if (nsl < 1 || a.y_dim > MAX_YDIM) return fail(BOSS_ERR_ARG, "score: y_dim must be in 1..16");
-  // the replicas of the slices on this context's device
-  std::vector<const boss_gp *> sl(nsl);
-  for (int q = 0; q < nsl; ++q) {
-    if (!a.slices[q]) return fail(BOSS_ERR_ARG, "score: NULL slice handle");
-    sl[q] = replica_on(a.slices[q], C().device);
-    if (!sl[q]) return fail(BOSS_ERR_STATE, "score: a slice handle has no replica on this device (or was invalidated by boss_shutdown)");
-    if (sl[q]->d != sl[0]->d) return fail(BOSS_ERR_ARG, "score: slices disagree on x_dim");
-  }
-  const int d = sl[0]->d;
-  int max_npad = 0;
-  for (int q = 0; q < nsl; ++q) max_npad = std::max(max_npad, sl[q]->n_pad);
+  ScoreCall c(a);
+  int rc = c.bind();
+  if (rc) return rc;
   a.any_fail = 0;
   if (a.M <= 0) {
     if (a.best_idx) *a.best_idx = -1;
     return 0;
   }
   if (a.dev && !a.internal) {
-    int rc = wait_for_caller(a.caller_stream);
+    rc = wait_for_caller(a.caller_stream);
     if (rc) return rc;
   }
-  // chunk size: K*^T scratch budget 4 GiB, at most 4 waves of 148 CTAs
-  long long ncb_max = (4ll << 30) / (1024ll * max_npad);
-  ncb_max = std::min<long long>(ncb_max, 592);
-  if (ncb_max >= 148) ncb_max = ncb_max / 148 * 148;
-  if (ncb_max < 1) return fail(BOSS_ERR_ARG, "score: n too large for the scratch budget");
-  if (a.grad) ncb_max = std::max<long long>(1, std::min<long long>(ncb_max, ncb_max >= 296 ? 296 : ncb_max));
-  const long long need_cb = (a.M + 127) / 128;
-  const int ncb_cap = (int)std::min<long long>(ncb_max, need_cb);
-  const int CH = ncb_cap * 128;
-
-  CUDA_TRY(C().ks.ensure((size_t)CH * max_npad * 8));
-  CUDA_TRY(C().muv.ensure((size_t)nsl * CH * 8));
-  CUDA_TRY(C().sumsq.ensure((size_t)nsl * CH * 8));
-  const int max_nblk = max_npad / TM;
-  CUDA_TRY(C().part_mu.ensure((size_t)2 * max_nblk * CH * 8));
-  CUDA_TRY(C().part_ss.ensure((size_t)2 * max_nblk * CH * 8));
-  // batches up to 8192 candidates keep V^T even without gradients: the quarter-row kernels (10 % faster than the
-  // row-split wide kernels up to there) reduce the variance from the stored tile
-  const bool have_vt = a.grad || CH <= 8192;
-  if (have_vt && !a.grad) CUDA_TRY(C().vt.ensure((size_t)CH * max_npad * 8));
-  if (a.grad) {
-    if (d > 32) return fail(BOSS_ERR_ARG, "score: gradients need x_dim <= 32");
-    CUDA_TRY(C().vt.ensure((size_t)CH * max_npad * 8));
-    CUDA_TRY(C().ut.ensure((size_t)CH * max_npad * 8));
-    CUDA_TRY(C().dmu.ensure((size_t)nsl * d * CH * 8));
-    CUDA_TRY(C().dvar.ensure((size_t)nsl * d * CH * 8));
-    CUDA_TRY(C().part_gm.ensure((size_t)2 * max_nblk * d * CH * 8));
-    CUDA_TRY(C().part_gv.ensure((size_t)2 * max_nblk * d * CH * 8));
-  }
-  const int nblk_acq_max = (CH + 127) / 128;     // block winners: per 256 candidates (acq_kernel) or per 128 (fused epilogue)
-  CUDA_TRY(C().blk_val.ensure((size_t)nblk_acq_max * 8));
-  CUDA_TRY(C().blk_idx.ensure((size_t)nblk_acq_max * 8));
-  // small: a2[nsl] | lb[d] | ub[d] | best(1) | bidx(1 as int64) | any_fail(int) | finished-CTA counter (fused epilogue)
-  const size_t sm_n = (size_t)nsl + 2 * d + 5;
-  CUDA_TRY(C().small.ensure(sm_n * 8));
-  double *small = C().small.as<double>();
-  std::vector<double> hs(sm_n, 0.0);
-  for (int q = 0; q < nsl; ++q) hs[q] = sl[q]->a2;
-  if (a.lb && a.ub) {
-    for (int i = 0; i < d; ++i) {
-      hs[nsl + i] = a.lb[i];
-      hs[nsl + d + i] = a.ub[i];
-    }
-  }
-  long long neg1 = -1;
-  std::memcpy(&hs[nsl + 2 * d + 1], &neg1, 8);
-  CUDA_TRY(cudaMemcpyAsync(small, hs.data(), sm_n * 8, cudaMemcpyHostToDevice, C().stream));
-  // hs is pageable: the runtime has copied these few bytes to its staging memory when the call returns (CUDA's
-  // documented behaviour for pageable-to-device cudaMemcpyAsync), and hs lives until the end of this function: no
-  // stream round trip is needed here
-  double *d_best = small + nsl + 2 * d;
-  long long *d_bidx = reinterpret_cast<long long *>(small + nsl + 2 * d + 1);
-  int *d_anyfail = reinterpret_cast<int *>(small + nsl + 2 * d + 2);
-  unsigned int *d_counter = reinterpret_cast<unsigned int *>(small + nsl + 2 * d + 3);
-  MixParams mixp{};
-  if (a.mix) {   // MC-EI: the eps matrix (y_dim x n_eps) goes to the device once per call
-    mixp = *a.mix;
-    const size_t eb = (size_t)a.y_dim * mixp.n_eps * 8;
-    CUDA_TRY(C().tt.ensure(eb));
-    CUDA_TRY(cudaMemcpyAsync(C().tt.p, mixp.eps_host, eb, cudaMemcpyHostToDevice, C().stream));
-    CUDA_TRY(cudaStreamSynchronize(C().stream));
-    mixp.eps = C().tt.as<double>();
-  }
-
-  // ---- argmax screening (DESIGN.md 2.9): a call that wants only the argmax of the closed-form EI over many
-  // candidates bounds every candidate from its mean alone and scores exactly only those that can still win ----
+  rc = c.setup();
+  if (rc) return rc;
   if (!a.internal) C().scr_stats[0] = C().scr_stats[1] = C().scr_stats[2] = 0;
-  const size_t pool_row = (size_t)d * 8 + (a.prior_mean ? (size_t)a.y_dim * 8 : 0) + 8 + (a.cons_mask ? 1 : 0);
-  // (top-k calls, DESIGN.md 2.10: the same bound against the k-th best score of a larger seed batch)
-  const int ch0 = (int)std::min<long long>(CH, a.M);   // the first chunk, which the seed batch is drawn from
-  bool screen = (a.want_argmax || a.topk) && a.best && !a.internal && !a.acq && !a.grad && !a.mu_out && !a.var_out &&
-                !a.status_out && !a.mix && a.M >= screen_min_m() && (size_t)a.M * pool_row <= SCREEN_POOL_BYTES &&
-                a.topk <= ch0 && getenv("BOSS_NO_SCREEN") == nullptr;
-  ScreenBufs sc;
-  double thr = -INFINITY;   // survivors: bound >= thr or NaN
-  if (screen) {
-    int rc = sc.setup(a.M, CH, d, a.y_dim, a.prior_mean != nullptr, a.cons_mask != nullptr,
-                      a.topk ? topk_seed_n(a.topk, ch0) : SEED_N);
+  const int ch0 = (int)std::min<long long>(c.CH, a.M);   // the first chunk
+  Screen scr;
+  if (Screen::eligible(a, ch0, c.d)) {
+    rc = scr.begin(c, ch0);
     if (rc) return rc;
-    CUDA_TRY(cudaMemsetAsync(sc.base, 0, 16, C().stream));
   }
-  // top-k: the running set (tk_r pairs in tb.run_*[tk_par]) absorbs every scored chunk
-  TopkBufs tb;
-  int tk_r = 0, tk_par = 0;
+  TopkBufs tb;   // top-k: the running set absorbs every scored chunk
   if (a.topk) {
-    const int cap = (int)std::max<long long>(a.topk, topk_seed_n(a.topk, ch0));
-    int rc = tb.setup(cap, CH, a.topk);
+    rc = tb.setup(a.topk, c.CH, ch0);
     if (rc) return rc;
   }
-  // one chunk of a screened call: the means of every slice (xcov without K*^T), the bounds, the survivors appended to
-  // the pool.  The first chunk also sets the threshold from the seed batch and ends screening (the chunk is then scored
-  // on the full path from the same staged inputs) when the bound does not separate: T not positive, or more than a
-  // quarter of the chunk surviving.
-  auto screen_chunk = [&](AcqParams ap, const double *xs_dev, long long in_off, int cidx) -> int {
-    const long long m0 = ap.m0;
-    const int ch = ap.chunk, ncb = (ch + 127) / 128, nb = (ch + 255) / 256;
-    for (int q = 0; q < nsl; ++q) {
-      const boss_gp *h = sl[q];
-      XcovParams xp{};
-      xp.Xs = xs_dev;
-      xp.M = a.M;
-      xp.m0 = m0;
-      xp.in_off = in_off;
-      xp.d = d;
-      xp.n = h->n;
-      xp.n_pad = h->n_pad;
-      xp.ktiles = h->ktiles;
-      xp.Xt = h->Xt;
-      xp.invl = h->invl;
-      xp.disc_bits = h->disc;
-      xp.alpha = h->alpha;
-      xp.a2 = h->a2;
-      xp.Ks = C().ks.as<double>();
-      xp.mu_part = C().part_mu.as<double>();
-      xp.ld = CH;
-      const int nks = std::max(1, std::min(h->nblk, (16 * 148 + ncb - 1) / ncb));
-      {
-        Timed t(1);
-        launch_xcov_mean(h->kernel_id, h->dp, xp, dim3(ncb, nks), C().stream);
-      }
-      reduce_rows_kernel<<<(ncb * 128 + 255) / 256, 256, 0, C().stream>>>(C().part_mu.as<double>(), 2 * h->nblk, (size_t)CH,
-                                                                        C().muv.as<double>() + (size_t)q * CH, ncb * 128);
-    }
-    AcqParams bp = ap;   // EI at the prior variance, PoF = 1, no guards -> sc.bound[c]
-    bp.sumsq = nullptr;
-    bp.has_ymax = 0;
-    bp.lb = bp.ub = nullptr;
-    bp.cons_mask = nullptr;
-    bp.acq = sc.bound;
-    bp.out_off = m0;
-    bp.blk_val = nullptr;
-    bp.blk_idx = nullptr;
-    acq_kernel<<<nb, 256, 0, C().stream>>>(bp);
-    C().launches += 2 * nsl + 1;
-    const size_t c0 = (size_t)(m0 - ap.in_off);   // the chunk's first candidate in the input arrays
-    const double *xs_c = ap.Xs + c0 * d;
-    const double *pm_c = ap.prior_mean ? ap.prior_mean + c0 * a.y_dim : nullptr;
-    const unsigned char *cm_c = ap.cons_mask ? ap.cons_mask + c0 : nullptr;
-    if (cidx == 0 && a.topk) {
-      // seed: the exact scores of the S_k highest bounds (NaN bounds last); the k-th best of them is a lower bound of
-      // the k-th best score of the call
-      const int ns = topk_seed_n(a.topk, ch);
-      SelectIn in{nullptr, nullptr, 0, sc.bound, 0, ch, 1};
-      int rc = tb.select(in, ns, tb.run_val[0], tb.run_idx[0]);
-      if (rc) return rc;
-      seed_gather_kernel<<<(ns + 255) / 256, 256, 0, C().stream>>>(tb.run_idx[0], ns, xs_c, pm_c, cm_c, d, a.y_dim,
-                                                                    sc.seed_x, sc.seed_pm, sc.seed_cm);
-      ++C().launches;
-      ScoreArgs s = a;
-      s.Xs = sc.seed_x;
-      s.M = ns;
-      s.prior_mean = pm_c ? sc.seed_pm : nullptr;
-      s.cons_mask = cm_c ? sc.seed_cm : nullptr;
-      s.gen = nullptr;
-      s.dev = true;
-      s.internal = true;
-      std::vector<double> sv((size_t)a.topk);
-      std::vector<int64_t> si((size_t)a.topk);
-      s.top_val = sv.data();
-      s.top_idx = si.data();
-      s.topk_map = nullptr;
-      rc = score_core(s);
-      if (rc) return rc;
-      CUDA_TRY(cudaMemcpyAsync(small, hs.data(), sm_n * 8, cudaMemcpyHostToDevice, C().stream));
-      C().scr_stats[1] = ch;
-      const double T = sv[(size_t)a.topk - 1];
-      if (!(T >= SCREEN_MIN_T)) {
-        C().scr_stats[0] = 2;
-        screen = false;
-        return 0;
-      }
-      thr = T * (1.0 - 0x1p-30);
-    } else if (cidx == 0) {
-      // seed: the exact scores of the SEED_N highest bounds; the best of them is a lower bound of the maximum
-      int n = ch, par = 0;
-      const unsigned long long *kin = nullptr;
-      const int *iin = nullptr;
-      do {
-        const int nbk = (n + TOPK_IN - 1) / TOPK_IN;
-        seed_topk_kernel<<<nbk, 1024, 0, C().stream>>>(kin ? nullptr : sc.bound, kin, iin, n, sc.tk[par], sc.ti[par]);
-        ++C().launches;
-        kin = sc.tk[par];
-        iin = sc.ti[par];
-        par ^= 1;
-        n = nbk * SEED_N;
-      } while (n > SEED_N);
-      const int ns = std::min(SEED_N, ch);
-      seed_gather_kernel<<<1, SEED_N, 0, C().stream>>>(iin, ns, xs_c, pm_c, cm_c, d, a.y_dim, sc.seed_x, sc.seed_pm, sc.seed_cm);
-      ++C().launches;
-      ScoreArgs s = a;
-      s.Xs = sc.seed_x;
-      s.M = ns;
-      s.prior_mean = pm_c ? sc.seed_pm : nullptr;
-      s.cons_mask = cm_c ? sc.seed_cm : nullptr;
-      s.gen = nullptr;
-      s.dev = true;
-      s.internal = true;
-      double T = 0.0;
-      int64_t ti = -1;
-      s.best_val = &T;
-      s.best_idx = &ti;
-      int rc = score_core(s);
-      if (rc) return rc;
-      // the seed call used this call's small block (a^2, bounds, running winner): restore it for the rest of the call
-      CUDA_TRY(cudaMemcpyAsync(small, hs.data(), sm_n * 8, cudaMemcpyHostToDevice, C().stream));
-      C().scr_stats[1] = ch;
-      if (!(T >= SCREEN_MIN_T)) {
-        C().scr_stats[0] = 2;
-        screen = false;
-        return 0;
-      }
-      thr = T * (1.0 - 0x1p-30);
-    }
-    screen_count_kernel<<<nb, 256, 0, C().stream>>>(sc.bound, ch, thr, sc.cnt);
-    CompactParams cpar{sc.bound, ch, thr, sc.cnt, m0, xs_c, pm_c, cm_c, d, a.y_dim, sc.base, cidx & 1,
-                     sc.pool_x, sc.pool_pm, sc.pool_cm, sc.pool_idx};
-    screen_compact_kernel<<<nb, 256, 0, C().stream>>>(cpar);
-    C().launches += 2;
-    if (cidx == 0) {
-      long long surv = 0;
-      CUDA_TRY(cudaMemcpyAsync(&surv, sc.base + 1, 8, cudaMemcpyDeviceToHost, C().stream));
-      CUDA_TRY(cudaStreamSynchronize(C().stream));
-      C().scr_stats[2] = surv;
-      if (4 * surv > ch) {
-        C().scr_stats[0] = 2;
-        screen = false;
-      }
-    }
-    return 0;
-  };
-
-  // ---- host staging plan (two slots): byte offsets of every array inside a slot ----
-  const bool host = !a.dev;
-  const bool has_pmg = a.grad && a.prior_mean_grad;
-  size_t in_off_xs = 0, in_off_pm = 0, in_off_cm = 0, in_off_pmg = 0, in_total = 0;
-  size_t out_off_acq = 0, out_off_mu = 0, out_off_var = 0, out_off_st = 0, out_off_gr = 0, out_total = 0;
-  Stager stg;
-  bool xs_direct = false;   // the caller's candidate matrix is pinned already: DMA straight from it
-  if (host) {
-    auto take = [](size_t &tot, size_t bytes) {
-      const size_t o = tot;
-      tot += (bytes + 255) / 256 * 256;
-      return o;
-    };
-    xs_direct = !a.gen && is_pinned_host(a.Xs);
-    in_off_xs = take(in_total, (size_t)CH * d * 8);   // device slot always holds the candidates
-    if (a.prior_mean) in_off_pm = take(in_total, (size_t)CH * a.y_dim * 8);
-    if (a.cons_mask) in_off_cm = take(in_total, (size_t)CH);
-    if (has_pmg) in_off_pmg = take(in_total, (size_t)CH * d * a.y_dim * 8);
-    if (a.acq) out_off_acq = take(out_total, (size_t)CH * 8);
-    if (a.mu_out) out_off_mu = take(out_total, (size_t)CH * 8);
-    if (a.var_out) out_off_var = take(out_total, (size_t)CH * 8);
-    if (a.status_out) out_off_st = take(out_total, (size_t)CH * 4);
-    if (a.grad) out_off_gr = take(out_total, (size_t)CH * d * 8);
-    CUDA_TRY(C().xs_stage.ensure(2 * in_total));     // both device input slots
-    CUDA_TRY(C().acq_stage.ensure(2 * std::max<size_t>(out_total, 256)));   // both device output slots
-    int rc = stg.ensure(in_total, out_total);
+  HostStaging stg;
+  if (!a.dev) {
+    rc = stg.plan(a, c.CH, c.d);
     if (rc) return rc;
   }
-  unsigned char *dev_in[2] = {C().xs_stage.as<unsigned char>(), C().xs_stage.as<unsigned char>() + in_total};
-  unsigned char *dev_out[2] = {C().acq_stage.as<unsigned char>(), C().acq_stage.as<unsigned char>() + std::max<size_t>(out_total, 256)};
-  cudaStream_t cp = C().ll_stream[LL_GROUPS - 1];   // copy stream (the last log-likelihood group stream is idle here)
-  cudaEvent_t ev_in[2] = {C().ll_join[LL_GROUPS - 1], C().ll_join[LL_GROUPS - 2]};     // H2D of the slot done
-  cudaEvent_t ev_free[2] = {C().ll_join[LL_GROUPS - 3], C().ll_join[LL_GROUPS - 4]};   // compute done with the device slot
-  cudaEvent_t ev_out[2] = {C().pin_ev[0], C().pin_ev[1]};                              // outputs of the slot are in pinned memory
-  bool in_used[2] = {false, false}, free_rec[2] = {false, false};
-
-  // inputs of chunk [m0, m0 + ch) -> device slot; returns after the copies have been ENQUEUED on the copy stream
-  auto stage_in = [&](long long m0, int ch, int slot) -> int {
-    if (in_used[slot]) CUDA_TRY(cudaEventSynchronize(ev_in[slot]));   // the pinned slot's previous DMA has completed
-    if (free_rec[slot]) CUDA_TRY(cudaStreamWaitEvent(cp, ev_free[slot], 0));   // kernels of chunk c-2 are done with the device slot
-    unsigned char *pin = stg.pin_in[slot], *dv = dev_in[slot];
-    if (!a.gen) {
-      const double *src = a.Xs + (size_t)m0 * d;
-      if (xs_direct) {
-        CUDA_TRY(cudaMemcpyAsync(dv + in_off_xs, src, (size_t)ch * d * 8, cudaMemcpyHostToDevice, cp));
-      } else {
-        std::memcpy(pin + in_off_xs, src, (size_t)ch * d * 8);
-        CUDA_TRY(cudaMemcpyAsync(dv + in_off_xs, pin + in_off_xs, (size_t)ch * d * 8, cudaMemcpyHostToDevice, cp));
-      }
-    }
-    if (a.prior_mean) {
-      std::memcpy(pin + in_off_pm, a.prior_mean + (size_t)m0 * a.y_dim, (size_t)ch * a.y_dim * 8);
-      CUDA_TRY(cudaMemcpyAsync(dv + in_off_pm, pin + in_off_pm, (size_t)ch * a.y_dim * 8, cudaMemcpyHostToDevice, cp));
-    }
-    if (a.cons_mask) {
-      std::memcpy(pin + in_off_cm, a.cons_mask + m0, (size_t)ch);
-      CUDA_TRY(cudaMemcpyAsync(dv + in_off_cm, pin + in_off_cm, (size_t)ch, cudaMemcpyHostToDevice, cp));
-    }
-    if (has_pmg) {
-      std::memcpy(pin + in_off_pmg, a.prior_mean_grad + (size_t)m0 * d * a.y_dim, (size_t)ch * d * a.y_dim * 8);
-      CUDA_TRY(cudaMemcpyAsync(dv + in_off_pmg, pin + in_off_pmg, (size_t)ch * d * a.y_dim * 8, cudaMemcpyHostToDevice, cp));
-    }
-    CUDA_TRY(cudaEventRecord(ev_in[slot], cp));
-    in_used[slot] = true;
-    return 0;
-  };
-  // outputs of chunk [m0, m0 + ch): pinned slot -> the caller's arrays (after the chunk's D2H has completed)
-  auto drain_out = [&](long long m0, int ch, int slot) -> int {
-    if (out_total == 0) return 0;
-    CUDA_TRY(cudaEventSynchronize(ev_out[slot]));
-    const unsigned char *pin = stg.pin_out[slot];
-    if (a.acq) std::memcpy(a.acq + m0, pin + out_off_acq, (size_t)ch * 8);
-    if (a.mu_out) std::memcpy(a.mu_out + m0, pin + out_off_mu, (size_t)ch * 8);
-    if (a.var_out) std::memcpy(a.var_out + m0, pin + out_off_var, (size_t)ch * 8);
-    if (a.status_out) std::memcpy(a.status_out + m0, pin + out_off_st, (size_t)ch * 4);
-    if (a.grad) std::memcpy(a.grad + (size_t)m0 * d, pin + out_off_gr, (size_t)ch * d * 8);
-    return 0;
-  };
 
   timing_begin();
-  if (host) {
-    CUDA_TRY(cudaEventRecord(ev_free[0], C().stream));   // nothing enqueued before this point reads the slots
-    int rc = stage_in(0, (int)std::min<long long>(CH, a.M), 0);
-    if (rc) return rc;
-  }
-  long long prev_m0 = -1;
-  int prev_ch = 0, cidx = 0;
-  for (long long m0 = 0; m0 < a.M; m0 += CH, ++cidx) {
-    const int ch = (int)std::min<long long>(CH, a.M - m0);
-    const int ncb = (ch + 127) / 128;
+  int cidx = 0;
+  for (long long m0 = 0; m0 < a.M; m0 += c.CH, ++cidx) {
+    const int ch = (int)std::min<long long>(c.CH, a.M - m0);
     const int slot = cidx & 1;
-    const double *xs_dev;
-    const double *pm_dev = nullptr;
-    const unsigned char *cm_dev = nullptr;
-    long long in_off, out_off;
-    double *acq_dev = nullptr, *mu_dev = nullptr, *var_dev = nullptr, *grad_dev = nullptr;
-    const double *pmg_dev = nullptr;
-    int *st_dev = nullptr;
+    ChunkIO io;
     if (a.dev) {
-      xs_dev = a.Xs;
-      pm_dev = a.prior_mean;
-      cm_dev = a.cons_mask;
-      in_off = 0;
-      out_off = 0;
-      acq_dev = a.acq;
-      mu_dev = a.mu_out;
-      var_dev = a.var_out;
-      st_dev = a.status_out;
-      grad_dev = a.grad;
-      pmg_dev = a.prior_mean_grad;
+      io = {a.Xs, a.prior_mean, a.prior_mean_grad, a.cons_mask, a.acq, a.mu_out, a.var_out, a.grad, a.status_out, 0};
     } else {
-      // this chunk's inputs were staged while the previous chunk was being launched; the next chunk's go now
-      CUDA_TRY(cudaStreamWaitEvent(C().stream, ev_in[slot], 0));
-      xs_dev = reinterpret_cast<const double *>(dev_in[slot] + in_off_xs);
-      if (a.gen) {
-        gen_candidates_kernel<<<(ch * d + 255) / 256, 256, 0, C().stream>>>(*a.gen, m0, ch, const_cast<double *>(xs_dev));
-        ++C().launches;
-      }
-      if (a.prior_mean) pm_dev = reinterpret_cast<const double *>(dev_in[slot] + in_off_pm);
-      if (a.cons_mask) cm_dev = dev_in[slot] + in_off_cm;
-      if (has_pmg) pmg_dev = reinterpret_cast<const double *>(dev_in[slot] + in_off_pmg);
-      in_off = m0;
-      out_off = m0;
-      if (a.acq) acq_dev = reinterpret_cast<double *>(dev_out[slot] + out_off_acq);
-      if (a.mu_out) mu_dev = reinterpret_cast<double *>(dev_out[slot] + out_off_mu);
-      if (a.var_out) var_dev = reinterpret_cast<double *>(dev_out[slot] + out_off_var);
-      if (a.status_out) st_dev = reinterpret_cast<int *>(dev_out[slot] + out_off_st);
-      if (a.grad) grad_dev = reinterpret_cast<double *>(dev_out[slot] + out_off_gr);
+      rc = stg.chunk_inputs(m0, ch, slot, io);
+      if (rc) return rc;
     }
-    bool fused_chunk = false;
-    AcqParams ap{};
-    ap.y_dim = a.y_dim;
-    ap.n_samples = a.n_samples;
-    ap.d = d;
-    ap.M = a.M;
-    ap.m0 = m0;
-    ap.in_off = host ? m0 : in_off;     // host mode: the slot arrays start at the chunk's first candidate
-    ap.out_off = host ? m0 : out_off;
-    ap.chunk = ch;
-    ap.chunk_ld = CH;
-    ap.mu = C().muv.as<double>();
-    ap.sumsq = C().sumsq.as<double>();
-    ap.a2 = small;
-    ap.prior_mean = pm_dev;
-    for (int i = 0; i < a.y_dim; ++i) {
-      ap.coefs[i] = a.coefs ? a.coefs[i] : (i == 0 ? 1.0 : 0.0);
-      ap.y_max[i] = a.y_max ? a.y_max[i] : INFINITY;
-    }
-    ap.has_best = a.best != nullptr;
-    ap.best = a.best ? *a.best : 0.0;
-    ap.has_ymax = a.y_max != nullptr;
-    ap.Xs = xs_dev;
-    ap.lb = (a.lb && a.ub) ? small + nsl : nullptr;
-    ap.ub = (a.lb && a.ub) ? small + nsl + d : nullptr;
-    ap.cons_mask = cm_dev;
-    ap.acq = acq_dev;
-    ap.mu_out = mu_dev;
-    ap.var_out = var_dev;
-    ap.status_out = st_dev;
-    ap.any_fail = d_anyfail;
-    ap.blk_val = a.want_argmax ? C().blk_val.as<double>() : nullptr;
-    ap.blk_idx = a.want_argmax ? C().blk_idx.as<long long>() : nullptr;
-    ap.mix = mixp;
+    AcqParams ap = c.acq_params(m0, ch, io);
     if (a.topk) {   // the chunk's scores stay on the device, for the running top-k set
       ap.acq = tb.scores;
       ap.out_off = m0;
     }
-    if (screen) {
-      int rc = screen_chunk(ap, xs_dev, in_off, cidx);
+    if (scr.on()) {
+      rc = scr.chunk(c, ap, io, cidx, tb);
       if (rc) return rc;
     }
-    for (int q = 0; q < nsl && !screen; ++q) {
-      const boss_gp *h = sl[q];
-      // Small candidate batches (multi-start optimiser iterations, single-point calls) cannot fill 148 SMs
-      // with one CTA per 128 candidates: deal the training chunks / W row blocks of a candidate block to
-      // several CTAs.  Partial sums are kept per chunk / per row block, so results do not depend on the split.
-      const int want = (16 * 148 + ncb - 1) / ncb;   // >= 16 CTAs per SM in flight over the launch (4 waves of 4)
-      const int nks = std::max(1, std::min(h->nblk, want));            // xcov / grad: splits over training chunks
-      double cost_w = 0.0, cost_n = 0.0;
-      const int nsp = pick_row_splits(ncb, h->nblk, &cost_w);          // trmm / wtv: zig-zag row-block splits
-      // Small batches: 32-candidate CTAs (score_narrow.cuh) do a quarter of the tensor work per stage of W; worth it
-      // when the wide launch cannot fill the GPU (cost = waves x longest per-CTA share, in block-steps; a narrow stage
-      // takes ~0.3 of a wide one).  Same bits either way.
-      const int ncb32 = (ch + NW_NB - 1) / NW_NB;
-      const int nsp32 = pick_row_splits(ncb32, h->nblk, &cost_n);
-      bool narrow = 0.32 * cost_n < cost_w && getenv("BOSS_NO_NARROW") == nullptr;
-      // Tiny batches: quarter-row-block CTAs (4 nblk per 32 candidates, 4 to an SM).  Cost in the same unit: the
-      // longest CTA's latency-bound walk over 8 nblk short stages, or the launch's tensor work spread over the SMs.
-      const double cost_q = std::max(NQ_COST_CHAIN * h->nblk, NQ_COST_WORK * ncb32 * (h->nblk * (h->nblk + 1) / 2)) + NQ_COST_FIXED;
-      bool quarter = have_vt && cost_q < std::min(cost_w, narrow ? 0.32 * cost_n : cost_w) && h->nblk >= 2;
-      if (const char *e = getenv("BOSS_SCORE_PATH")) {   // A/B switch: wide | narrow | quarter
-        if (!strcmp(e, "wide")) narrow = quarter = false;
-        if (!strcmp(e, "narrow")) narrow = true, quarter = false;
-        if (!strcmp(e, "quarter") && have_vt) quarter = true;
-      }
-      if (quarter) narrow = false;
-      const int cnt = ncb * 128;
-      XcovParams xp{};
-      xp.Xs = xs_dev;
-      xp.M = a.M;
-      xp.m0 = m0;
-      xp.in_off = in_off;
-      xp.d = d;
-      xp.n = h->n;
-      xp.n_pad = h->n_pad;
-      xp.ktiles = h->ktiles;
-      xp.Xt = h->Xt;
-      xp.invl = h->invl;
-      xp.disc_bits = h->disc;
-      xp.alpha = h->alpha;
-      xp.a2 = h->a2;
-      xp.Ks = C().ks.as<double>();
-      xp.mu_part = C().part_mu.as<double>();
-      xp.ld = CH;
-      {
-        Timed t(1);
-        launch_xcov(h->kernel_id, h->dp, xp, dim3(ncb, nks), C().stream);
-      }
-      // One CTA per candidate block walks all of W (large batches) and this is the chunk's last slice: the scoring
-      // kernel finishes the candidates itself (fused epilogue) -- no reduce / acquisition / argmax launches.
-      const bool fuse = nsp == 1 && !narrow && !quarter && q == nsl - 1 && getenv("BOSS_UNFUSED_SCORE") == nullptr;
-      fused_chunk = fuse;
-      if (!fuse && !quarter)
-        reduce_rows_kernel<<<(cnt + 255) / 256, 256, 0, C().stream>>>(C().part_mu.as<double>(), 2 * h->nblk, (size_t)CH,
-                                                                   C().muv.as<double>() + (size_t)q * CH, cnt);
-      ScoreParams sp{};
-      sp.W = h->W;
-      sp.Ks = C().ks.as<double>();
-      sp.nblk = h->nblk;
-      sp.ktiles = h->ktiles;
-      sp.ss_part = C().part_ss.as<double>();
-      sp.ld = CH;
-      sp.VT = a.grad ? C().vt.as<double>() : nullptr;
-      if (fuse) {
-        sp.fused = 1;
-        sp.ap = ap;
-        sp.mu_part = C().part_mu.as<double>();
-        sp.P = 2 * h->nblk;
-        sp.mu_row = C().muv.as<double>() + (size_t)q * CH;
-        sp.ss_row = C().sumsq.as<double>() + (size_t)q * CH;
-        sp.best = d_best;
-        sp.bidx = d_bidx;
-        sp.counter = d_counter;
-      }
-      if (quarter) {
-        NarrowParams np{h->W, C().ks.as<double>(), h->nblk, h->ktiles, nullptr, CH, C().vt.as<double>()};
-        Timed t(0);
-        score_quarter_kernel<0, 4, 1><<<dim3(ncb32, 4 * h->nblk), NQ_THREADS, NQ_SMEM_BYTES, C().stream>>>(np);
-        quarter_sumsq_kernel<<<dim3(ncb32, h->nblk), 256, 0, C().stream>>>(C().vt.as<double>(), h->ktiles,
-                                                                         C().part_ss.as<double>(), CH);
-      } else if (narrow) {
-        NarrowParams np{h->W, C().ks.as<double>(), h->nblk, h->ktiles, C().part_ss.as<double>(), CH,
-                        a.grad ? C().vt.as<double>() : nullptr};
-        Timed t(0);
-        score_narrow_kernel<0><<<dim3(ncb32, nsp32), 256, NW_SMEM_BYTES, C().stream>>>(np);
-      } else {
-        Timed t(0);
-        score_trmm_kernel<<<dim3(ncb, nsp), GEMM_THREADS, GEMM_SMEM_BYTES, C().stream>>>(sp);
-      }
-      if (quarter)   // mu partials (xcov) and sums of squares (quarter_sumsq) of this slice in one launch
-        reduce_rows_pair_kernel<<<dim3((cnt + 255) / 256, 2), 256, 0, C().stream>>>(
-            C().part_mu.as<double>(), C().part_ss.as<double>(), 2 * h->nblk, (size_t)CH, C().muv.as<double>() + (size_t)q * CH,
-            C().sumsq.as<double>() + (size_t)q * CH, cnt);
-      else if (!fuse)
-        reduce_rows2_kernel<<<(cnt + 255) / 256, 256, 0, C().stream>>>(C().part_ss.as<double>(), 2 * h->nblk, (size_t)CH,
-                                                                    C().sumsq.as<double>() + (size_t)q * CH, cnt);
-      C().launches += fuse ? 2 : 4;
-      if (a.grad) {
-        WtvParams wp{h->WT, C().vt.as<double>(), C().ut.as<double>(), h->nblk, h->ktiles};
-        if (quarter) {
-          NarrowParams np{h->WT, C().vt.as<double>(), h->nblk, h->ktiles, nullptr, CH, C().ut.as<double>()};
-          Timed t(0);
-          score_quarter_kernel<1, 4, 1><<<dim3(ncb32, 4 * h->nblk), NQ_THREADS, NQ_SMEM_BYTES, C().stream>>>(np);
-        } else if (narrow) {
-          NarrowParams np{h->WT, C().vt.as<double>(), h->nblk, h->ktiles, nullptr, CH, C().ut.as<double>()};
-          Timed t(0);
-          score_narrow_kernel<1><<<dim3(ncb32, nsp32), 256, NW_SMEM_BYTES, C().stream>>>(np);
-        } else {
-          Timed t(0);
-          wtv_kernel<<<dim3(ncb, nsp), GEMM_THREADS, GEMM_SMEM_BYTES, C().stream>>>(wp);
-        }
-        GradParams gq{};
-        gq.Xs = xs_dev;
-        gq.M = a.M;
-        gq.m0 = m0;
-        gq.in_off = in_off;
-        gq.d = d;
-        gq.n = h->n;
-        gq.n_pad = h->n_pad;
-        gq.ktiles = h->ktiles;
-        gq.chunk_ld = CH;
-        gq.Xt = h->Xt;
-        gq.invl = h->invl;
-        gq.alpha = h->alpha;
-        gq.disc_bits = h->disc;
-        gq.a2 = h->a2;
-        gq.UT = C().ut.as<double>();
-        gq.gm_part = C().part_gm.as<double>();
-        gq.gv_part = C().part_gv.as<double>();
-        {
-          Timed t(1);
-          launch_grad(h->kernel_id, h->dp, gq, dim3(ncb, nks), C().stream);
-        }
-        GradReduceParams gr{C().part_gm.as<double>(), C().part_gv.as<double>(), 2 * h->nblk, d, CH, cnt, h->invl, h->disc,
-                            C().dmu.as<double>() + (size_t)q * d * CH, C().dvar.as<double>() + (size_t)q * d * CH};
-        grad_reduce_kernel<<<dim3((cnt + 255) / 256, d), 256, 0, C().stream>>>(gr);
-        C().launches += 3;
-      }
-    }
-    if (!fused_chunk && !screen) {
-      const int nb = (ch + 255) / 256;
-      acq_kernel<<<nb, 256, 0, C().stream>>>(ap);
-      ++C().launches;
-      if (a.want_argmax) {
-        argmax_final_kernel<<<1, 256, 0, C().stream>>>(C().blk_val.as<double>(), C().blk_idx.as<long long>(), nb, d_best, d_bidx);
+    if (!scr.on()) {   // the full path (screening did not take the chunk)
+      bool fused = false;
+      for (int q = 0; q < c.nsl; ++q) fused = score_slice(c, q, ap, io);
+      if (!fused) {
+        const int nb = (ch + 255) / 256;
+        acq_kernel<<<nb, 256, 0, C().stream>>>(ap);
         ++C().launches;
+        if (a.want_argmax) {
+          argmax_final_kernel<<<1, 256, 0, C().stream>>>(C().blk_val.as<double>(), C().blk_idx.as<long long>(), nb, c.d_best,
+                                                         c.d_bidx);
+          ++C().launches;
+        }
       }
-    }
-    if (a.topk && !screen) {   // the best min(k, seen) of (running set, this chunk)
-      const int tgt = (int)std::min<long long>(a.topk, (long long)tk_r + ch);
-      SelectIn in{tb.run_val[tk_par], tb.run_idx[tk_par], tk_r, tb.scores, m0, ch, 0};
-      int rc = tb.select(in, tgt, tb.run_val[tk_par ^ 1], tb.run_idx[tk_par ^ 1]);
-      if (rc) return rc;
-      tk_par ^= 1;
-      tk_r = tgt;
+      if (a.topk) {
+        rc = tb.absorb(m0, ch);
+        if (rc) return rc;
+      }
     }
     if (a.grad) {
-      AcqGradParams gp2{ap, C().dmu.as<double>(), C().dvar.as<double>(), pmg_dev, grad_dev};
+      AcqGradParams gp2{ap, C().dmu.as<double>(), C().dvar.as<double>(), io.pmg, io.grad};
       acq_grad_kernel<<<(ch + 127) / 128, 128, 0, C().stream>>>(gp2);
       ++C().launches;
     }
-    if (host) {
-      CUDA_TRY(cudaEventRecord(ev_free[slot], C().stream));   // the kernels above were the last readers of the input slot
-      free_rec[slot] = true;
-      if (out_total) {
-        CUDA_TRY(cudaMemcpyAsync(stg.pin_out[slot], dev_out[slot], out_total, cudaMemcpyDeviceToHost, C().stream));
-        CUDA_TRY(cudaEventRecord(ev_out[slot], C().stream));
-      }
-      // while this chunk runs: stage the next chunk's inputs, then hand the previous chunk's outputs to the caller
-      if (m0 + CH < a.M) {
-        int rc = stage_in(m0 + CH, (int)std::min<long long>(CH, a.M - m0 - CH), slot ^ 1);
-        if (rc) return rc;
-      }
-      if (prev_m0 >= 0) {
-        int rc = drain_out(prev_m0, prev_ch, slot ^ 1);
-        if (rc) return rc;
-      }
-      prev_m0 = m0;
-      prev_ch = ch;
+    if (!a.dev) {
+      rc = stg.end_chunk(m0, ch, slot);
+      if (rc) return rc;
     }
   }
   CUDA_TRY(cudaGetLastError());
-  if (screen) {
-    // the pool (survivors in ascending order) through the ordinary path; its first-maximal winner maps back to the
-    // call's index
-    long long npool = 0;
-    CUDA_TRY(cudaMemcpyAsync(&npool, sc.base + (cidx & 1), 8, cudaMemcpyDeviceToHost, C().stream));
-    CUDA_TRY(cudaStreamSynchronize(C().stream));
-    if (host) CUDA_TRY(cudaStreamSynchronize(cp));
-    C().scr_stats[0] = 1;
-    C().scr_stats[1] = a.M;
-    C().scr_stats[2] = npool;
-    if (npool < 1) return fail(BOSS_ERR_STATE, "score: argmax screening kept no candidate");   // the seed's winner always survives
-    if (npool < a.topk) return fail(BOSS_ERR_STATE, "score: top-k screening kept fewer than k candidates");   // the seed's k best survive
-    ScoreArgs s = a;
-    s.Xs = sc.pool_x;
-    s.M = npool;
-    s.prior_mean = sc.pool_pm;
-    s.cons_mask = sc.pool_cm;
-    s.gen = nullptr;
-    s.dev = true;
-    s.internal = true;
-    double bv = 0.0;
-    int64_t bi = -1;
-    s.best_val = &bv;
-    s.best_idx = &bi;
-    s.topk_map = sc.pool_idx;   // top-k: the pool's k best come back with their indices in this call
-    int rc = score_core(s);
-    if (rc) return rc;
-    a.any_fail = s.any_fail;
-    if (a.topk) return 0;
-    long long idx = -1;
-    if (bi >= 0) {
-      CUDA_TRY(cudaMemcpyAsync(&idx, sc.pool_idx + bi, 8, cudaMemcpyDeviceToHost, C().stream));
-      CUDA_TRY(cudaStreamSynchronize(C().stream));
-    }
-    if (a.best_val) *a.best_val = bv;
-    if (a.best_idx) *a.best_idx = idx;
-    return 0;
-  }
+  if (scr.on()) return scr.finish(c, cidx, stg);
+  if (a.internal && !a.want_argmax && !a.topk && !C().timing) return 0;   // a round of the multi-start driver: it synchronises itself
+  // one wait for everything: the (value, index, failure flag) triple -- top-k: the flag behind the k pairs -- is fetched
+  // behind the last chunk's outputs, and the last chunk is handed to the caller after the stream has drained
+  double res[3] = {0.0, 0.0, 0.0};
   if (a.topk) {
-    // the running set, sorted in one CTA, to the caller: k pairs, no M-sized output and no host sort
-    if (tk_r != a.topk) return fail(BOSS_ERR_STATE, "score: top-k set incomplete");
-    int P = 2;
-    while (P < tk_r) P <<= 1;
-    topk_sort_kernel<<<1, 1024, (size_t)P * 12, C().stream>>>(tb.run_val[tk_par], tb.run_idx[tk_par], tk_r, P, a.topk_map,
-                                                             tb.out_val, tb.out_idx);
-    ++C().launches;
-    int af = 0;
-    CUDA_TRY(cudaMemcpyAsync(a.top_val, tb.out_val, (size_t)tk_r * 8, cudaMemcpyDeviceToHost, C().stream));
-    CUDA_TRY(cudaMemcpyAsync(a.top_idx, tb.out_idx, (size_t)tk_r * 8, cudaMemcpyDeviceToHost, C().stream));
-    CUDA_TRY(cudaMemcpyAsync(&af, d_anyfail, 4, cudaMemcpyDeviceToHost, C().stream));
-    CUDA_TRY(cudaStreamSynchronize(C().stream));
-    if (host) CUDA_TRY(cudaStreamSynchronize(cp));
-    timing_end();
-    a.any_fail = af;
-    return 0;
-  }
-  if (a.internal && !a.want_argmax && !C().timing) {   // a round of the multi-start driver: it synchronises itself
-    a.any_fail = 0;
-    return 0;
-  }
-  // one wait for everything: the (value, index, failure flag) triple is fetched behind the last chunk's outputs, and
-  // the last chunk is handed to the caller after the stream has drained (its event has completed by then)
-  double *hres = reinterpret_cast<double *>(hs.data());   // reuse: 3 doubles
-  CUDA_TRY(cudaMemcpyAsync(hres, d_best, 24, cudaMemcpyDeviceToHost, C().stream));
-  CUDA_TRY(cudaStreamSynchronize(C().stream));
-  if (host) CUDA_TRY(cudaStreamSynchronize(cp));
-  if (host && prev_m0 >= 0) {
-    int rc = drain_out(prev_m0, prev_ch, (cidx - 1) & 1);
+    rc = tb.finish(a.topk_map, a.top_val, a.top_idx);
     if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(&res[2], c.d_anyfail, 4, cudaMemcpyDeviceToHost, C().stream));
+  } else {
+    CUDA_TRY(cudaMemcpyAsync(res, c.d_best, 24, cudaMemcpyDeviceToHost, C().stream));
   }
+  CUDA_TRY(cudaStreamSynchronize(C().stream));
+  rc = stg.drain_last();
+  if (rc) return rc;
   timing_end();
   long long bidx;
-  std::memcpy(&bidx, &hres[1], 8);
+  std::memcpy(&bidx, &res[1], 8);
   int af;
-  std::memcpy(&af, &hres[2], 4);
+  std::memcpy(&af, &res[2], 4);
   a.any_fail = af;
   if (a.want_argmax) {
-    if (a.best_val) *a.best_val = hres[0];
+    if (a.best_val) *a.best_val = res[0];
     if (a.best_idx) *a.best_idx = bidx;
   }
   return 0;
@@ -2054,47 +2120,55 @@ int score_dispatch(ScoreArgs &a) {
 
 }  // namespace
 
-int boss_gp_predict(const boss_gp *gp, const double *Xs, int64_t M, const double *prior_mean_s, double *mu,
-                    double *var, int32_t *status) {
-  if (!gp || (!Xs && M > 0)) return fail(BOSS_ERR_ARG, "boss_gp_predict: bad arguments");
-  const boss_gp *sl[1] = {gp};
+// the fields every scoring entry point sets; the others start out null / false / zero
+static ScoreArgs score_args(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
+                            const double *prior_mean, const double *coefs, const double *best, const double *y_max,
+                            const double *lb, const double *ub, const uint8_t *cons_mask) {
   ScoreArgs a{};
-  a.slices = sl;
-  a.y_dim = 1;
-  a.n_samples = 1;
+  a.slices = slices;
+  a.y_dim = y_dim;
+  a.n_samples = n_samples;
   a.Xs = Xs;
   a.M = M;
-  a.prior_mean = prior_mean_s;
+  a.prior_mean = prior_mean;
+  a.coefs = coefs;
+  a.best = best;
+  a.y_max = y_max;
+  a.lb = lb;
+  a.ub = ub;
+  a.cons_mask = cons_mask;
+  return a;
+}
+
+// the box bounds of the acquisition come as a pair or not at all
+static int check_lb_ub(const char *who, const double *lb, const double *ub) {
+  if ((lb == nullptr) != (ub == nullptr)) return fail(BOSS_ERR_ARG, std::string(who) + ": lb and ub must be given together");
+  return 0;
+}
+
+static int predict_impl(const char *who, const boss_gp *gp, const double *Xs, int64_t M, const double *prior_mean_s,
+                        double *mu, double *var, int32_t *status, bool dev, void *stream) {
+  if (!gp || (!Xs && M > 0)) return fail(BOSS_ERR_ARG, std::string(who) + ": bad arguments");
+  const boss_gp *sl[1] = {gp};
+  ScoreArgs a = score_args(sl, 1, 1, Xs, M, prior_mean_s, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
   a.mu_out = mu;
   a.var_out = var;
   a.status_out = status;
-  a.dev = false;
-  a.want_argmax = false;
+  a.dev = dev;
+  a.caller_stream = stream;
   int rc = score_dispatch(a);
   if (rc) return rc;
   return a.any_fail ? BOSS_NEG_VARIANCE : 0;
 }
 
+int boss_gp_predict(const boss_gp *gp, const double *Xs, int64_t M, const double *prior_mean_s, double *mu,
+                    double *var, int32_t *status) {
+  return predict_impl("boss_gp_predict", gp, Xs, M, prior_mean_s, mu, var, status, false, nullptr);
+}
+
 int boss_gp_predict_dev(const boss_gp *gp, const double *Xs_dev, int64_t M, const double *prior_mean_s_dev,
                         double *mu_dev, double *var_dev, int32_t *status_dev, void *stream) {
-  if (!gp || (!Xs_dev && M > 0)) return fail(BOSS_ERR_ARG, "boss_gp_predict_dev: bad arguments");
-  const boss_gp *sl[1] = {gp};
-  ScoreArgs a{};
-  a.slices = sl;
-  a.y_dim = 1;
-  a.n_samples = 1;
-  a.Xs = Xs_dev;
-  a.M = M;
-  a.prior_mean = prior_mean_s_dev;
-  a.mu_out = mu_dev;
-  a.var_out = var_dev;
-  a.status_out = status_dev;
-  a.dev = true;
-  a.caller_stream = stream;
-  a.want_argmax = false;
-  int rc = score_dispatch(a);
-  if (rc) return rc;
-  return a.any_fail ? BOSS_NEG_VARIANCE : 0;
+  return predict_impl("boss_gp_predict_dev", gp, Xs_dev, M, prior_mean_s_dev, mu_dev, var_dev, status_dev, true, stream);
 }
 
 static int ei_score_impl(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
@@ -2104,20 +2178,9 @@ static int ei_score_impl(const boss_gp *const *slices, int y_dim, int n_samples,
                          const double *prior_mean_grad = nullptr, void *stream = nullptr, const MixParams *mix = nullptr) {
   if (!slices || y_dim < 1 || n_samples < 1 || (!Xs && M > 0) || (!fit_coefs && !mix))
     return fail(BOSS_ERR_ARG, "boss_ei_score: bad arguments");
-  if ((lb == nullptr) != (ub == nullptr)) return fail(BOSS_ERR_ARG, "boss_ei_score: lb and ub must be given together");
-  ScoreArgs a{};
-  a.slices = slices;
-  a.y_dim = y_dim;
-  a.n_samples = n_samples;
-  a.Xs = Xs;
-  a.M = M;
-  a.prior_mean = prior_mean_s;
-  a.coefs = fit_coefs;
-  a.best = best;
-  a.y_max = y_max;
-  a.lb = lb;
-  a.ub = ub;
-  a.cons_mask = cons_mask;
+  int rc = check_lb_ub("boss_ei_score", lb, ub);
+  if (rc) return rc;
+  ScoreArgs a = score_args(slices, y_dim, n_samples, Xs, M, prior_mean_s, fit_coefs, best, y_max, lb, ub, cons_mask);
   a.acq = acq;
   a.grad = grad;
   a.prior_mean_grad = prior_mean_grad;
@@ -2155,23 +2218,11 @@ static int ei_score_topk_impl(const boss_gp *const *slices, int y_dim, int n_sam
   if (!slices || y_dim < 1 || n_samples < 1 || !Xs || M < 1 || !fit_coefs || !top_val || !top_idx)
     return fail(BOSS_ERR_ARG, "boss_ei_score_topk: bad arguments");
   if (k < 1 || k > M || k > TOPK_MAX) return fail(BOSS_ERR_ARG, "boss_ei_score_topk: k must be in 1..min(M, 8192)");
-  if ((lb == nullptr) != (ub == nullptr)) return fail(BOSS_ERR_ARG, "boss_ei_score_topk: lb and ub must be given together");
-  ScoreArgs a{};
-  a.slices = slices;
-  a.y_dim = y_dim;
-  a.n_samples = n_samples;
-  a.Xs = Xs;
-  a.M = M;
-  a.prior_mean = prior_mean_s;
-  a.coefs = fit_coefs;
-  a.best = best;
-  a.y_max = y_max;
-  a.lb = lb;
-  a.ub = ub;
-  a.cons_mask = cons_mask;
+  int rc = check_lb_ub("boss_ei_score_topk", lb, ub);
+  if (rc) return rc;
+  ScoreArgs a = score_args(slices, y_dim, n_samples, Xs, M, prior_mean_s, fit_coefs, best, y_max, lb, ub, cons_mask);
   a.dev = dev;
   a.caller_stream = stream;
-  a.want_argmax = false;
   a.topk = k;
   a.top_val = top_val;
   a.top_idx = top_idx;
@@ -2227,30 +2278,18 @@ static int ei_score_generated(const CandGen &gen, int64_t M, const boss_gp *cons
                               const double *lb, const double *ub, const uint8_t *cons_mask, double *acq, double *best_val,
                               int64_t *best_idx, double *best_x) {
   if (!slices || y_dim < 1 || n_samples < 1 || !fit_coefs || !slices[0]) return fail(BOSS_ERR_ARG, "boss_ei_score_*: bad arguments");
-  if ((lb == nullptr) != (ub == nullptr)) return fail(BOSS_ERR_ARG, "boss_ei_score_*: lb and ub must be given together");
+  int rc = check_lb_ub("boss_ei_score_*", lb, ub);
+  if (rc) return rc;
   if (gen.d != slices[0]->d) return fail(BOSS_ERR_ARG, "boss_ei_score_*: x_dim mismatch");
-  ScoreArgs a{};
-  a.slices = slices;
-  a.y_dim = y_dim;
-  a.n_samples = n_samples;
-  a.Xs = nullptr;
-  a.M = M;
-  a.prior_mean = prior_mean_s;
-  a.coefs = fit_coefs;
-  a.best = best;
-  a.y_max = y_max;
-  a.lb = lb;
-  a.ub = ub;
-  a.cons_mask = cons_mask;
+  ScoreArgs a = score_args(slices, y_dim, n_samples, nullptr, M, prior_mean_s, fit_coefs, best, y_max, lb, ub, cons_mask);
   a.acq = acq;
   int64_t bi = -1;
   double bv = 0.0;
   a.best_val = &bv;
   a.best_idx = &bi;
-  a.dev = false;
   a.want_argmax = true;
   a.gen = &gen;
-  int rc = score_dispatch(a);
+  rc = score_dispatch(a);
   if (rc) return rc;
   if (best_val) *best_val = bv;
   if (best_idx) *best_idx = bi < 0 ? bi : gen.first + bi;                  // global index
@@ -2363,12 +2402,7 @@ static int multistart_single(const boss_gp *const *slices, int y_dim, int n_samp
 
   long long evaluated = 0;
   auto eval = [&](const double *Xp, long long Mp, double *fp, double *gp, bool want_best, double *bv, int64_t *bi) -> int {
-    ScoreArgs a{};
-    a.slices = slices;
-    a.y_dim = y_dim;
-    a.n_samples = n_samples;
-    a.Xs = Xp;
-    a.M = Mp;
+    ScoreArgs a = score_args(slices, y_dim, n_samples, Xp, Mp, nullptr, fit_coefs, best, y_max, lb, ub, nullptr);
     evaluated += Mp;
     if (prior_mean_affine) {
       ms_affine_mean_kernel<<<(unsigned)((Mp + 127) / 128), 128, 0, C().stream>>>(Xp, Mp, d, y_dim, aff, pm, pmg);
@@ -2376,11 +2410,6 @@ static int multistart_single(const boss_gp *const *slices, int y_dim, int n_samp
       a.prior_mean = pm;
       a.prior_mean_grad = gp ? pmg : nullptr;
     }
-    a.coefs = fit_coefs;
-    a.best = best;
-    a.y_max = y_max;
-    a.lb = lb;
-    a.ub = ub;
     a.acq = fp;
     a.grad = gp;
     a.best_val = bv;
@@ -2569,22 +2598,7 @@ int boss_gp_cov(const boss_gp *gp, const double *Xs, int64_t M, const double *pr
   const int want = (2 * 148 + ncb - 1) / ncb;
   const int nks = std::max(1, std::min(h->nblk, want));
   const int nsp = pick_row_splits(ncb, h->nblk);
-  XcovParams xp{};
-  xp.Xs = C().xs_stage.as<double>();
-  xp.M = M;
-  xp.d = d;
-  xp.n = h->n;
-  xp.n_pad = h->n_pad;
-  xp.ktiles = h->ktiles;
-  xp.Xt = h->Xt;
-  xp.invl = h->invl;
-  xp.disc_bits = h->disc;
-  xp.alpha = h->alpha;
-  xp.a2 = h->a2;
-  xp.Ks = C().ks.as<double>();
-  xp.mu_part = C().part_mu.as<double>();
-  xp.ld = Mp;
-  launch_xcov(h->kernel_id, h->dp, xp, dim3(ncb, nks), C().stream);
+  launch_xcov(h->kernel_id, h->dp, xcov_params(h, C().xs_stage.as<double>(), M, 0, 0, d, Mp), dim3(ncb, nks), C().stream);
   reduce_rows_kernel<<<(cnt + 255) / 256, 256, 0, C().stream>>>(C().part_mu.as<double>(), 2 * h->nblk, (size_t)Mp,
                                                              C().muv.as<double>(), cnt);
   ScoreParams sp{};

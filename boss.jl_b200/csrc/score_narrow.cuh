@@ -178,7 +178,7 @@ __global__ void __launch_bounds__(256, 1) score_narrow_kernel(const __grid_const
 // ---------------------------------------------------------------------------------------------
 // Quarter-row-block CTAs: built for TINY batches (a handful of unfinished multi-start runs, the reference's one-x-per-call
 // access pattern) and, as it turned out, the fastest shape up to a few thousand candidates (its many short CTAs balance
-// better than the row-split wide kernels: 10 % faster up to 8192 candidates at n = 2048; the cost model in score_core decides).  With one 32-candidate block the kernels above expose only nblk CTAs and the longest of them walks
+// better than the row-split wide kernels: 10 % faster up to 8192 candidates at n = 2048; the cost model in score_slice decides).  With one 32-candidate block the kernels above expose only nblk CTAs and the longest of them walks
 // all 8 nblk stages of the last row block alone: 218 us at n = 4096 whatever the batch holds.  Here a CTA owns 32 rows
 // (4 row slabs) of one row block x 32 candidates (warp = 1 slab x 2 candidate slabs), 4 nblk CTAs per candidate block,
 // launched longest first; the structurally dead head / tail k-tiles of a quarter are not even loaded.
