@@ -67,6 +67,13 @@ EXPORTS = {
                                          _vp, _vp, _vp]),
     "boss_mcei_score": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _vp,
                                   C.c_int, _vp, _vp, _vp, _vp, _vp, _vp, _dp, _i64p]),
+    "boss_mcei_value_grad": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, C.c_int, C.c_double, _vp, _vp,
+                                       _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "boss_mcei_maximize_multistart": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, C.c_int, C.c_int, _vp, C.c_int,
+                                                C.c_double, _vp, _vp, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp,
+                                                _vp, _vp, _dp, _i64p, C.POINTER(C.c_int)]),
+    "boss_mcei_score_topk": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, C.c_int, C.c_double, _vp, _vp, _vp,
+                                       _vp, C.c_int, _vp, _vp, _vp, _vp, _vp, C.c_int64, _vp, _vp]),
     "boss_gp_loglik_batch": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp, C.c_int, _vp, C.c_int64,
                                        _vp]),
     "boss_gp_loglik_batch_dev": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp, C.c_int, _vp,
@@ -345,6 +352,84 @@ def mcei_score(slices, y_dim, n_samples, Xs, fit_kind, eps, best, y_max, c0=0.0,
                                _ptr(tv), _ptr(ep), K, _ptr(b), _ptr(ym), _ptr(lbv), _ptr(ubv), _ptr(cm), _ptr(acq),
                                C.byref(bv), C.byref(bi)), "boss_mcei_score")
     return acq, bv.value, bi.value
+
+
+def _eps_cols(eps, y_dim):
+    """eps (y_dim, K) -> (K, y_dim) C-contiguous = column-major y_dim x K, and K."""
+    ep = np.ascontiguousarray(np.asarray(eps, dtype=np.float64).reshape(y_dim, -1).T)
+    return ep, ep.shape[0]
+
+
+def mcei_value_grad(slices, y_dim, n_samples, Xs, fit_kind, eps, best, y_max, c0=0.0, c=None, q=None, t=None, lb=None,
+                    ub=None, cons_mask=None, prior_mean_s=None, prior_mean_grad_s=None):
+    """Value and x-gradient of mcei_score's Monte-Carlo EI (include/boss_b200.h, boss_mcei_value_grad).
+    -> acq (M,), grad (d, M).  prior_mean_grad_s: (y_dim, d, M)."""
+    Xc = _cols(Xs)
+    M, d = Xc.shape
+    arr = _slice_array(slices)
+    ep, K = _eps_cols(eps, y_dim)
+    cv, qv, tv = _opt(c), _opt(q), _opt(t)
+    b = None if best is None else np.array([best], dtype=np.float64)
+    ym = None if y_max is None else _f64(y_max, (y_dim,))
+    lbv = None if lb is None else _f64(lb, (d,))
+    ubv = None if ub is None else _f64(ub, (d,))
+    cm = None if cons_mask is None else np.ascontiguousarray(cons_mask, dtype=np.uint8)
+    pm = None if prior_mean_s is None else np.ascontiguousarray(np.asarray(prior_mean_s, dtype=np.float64).T)
+    pmg = None if prior_mean_grad_s is None else np.ascontiguousarray(
+        np.transpose(np.asarray(prior_mean_grad_s, dtype=np.float64), (2, 1, 0)))   # (M, d, y_dim)
+    acq = np.empty(M)
+    grad = np.empty((M, d))
+    _check(lib.boss_mcei_value_grad(arr, y_dim, n_samples, _ptr(Xc), M, _ptr(pm), _ptr(pmg), int(fit_kind), float(c0),
+                                    _ptr(cv), _ptr(qv), _ptr(tv), _ptr(ep), K, _ptr(b), _ptr(ym), _ptr(lbv), _ptr(ubv),
+                                    _ptr(cm), _ptr(acq), _ptr(grad)), "boss_mcei_value_grad")
+    return acq, grad.T
+
+
+def mcei_maximize_multistart(slices, y_dim, n_samples, starts, fit_kind, eps, best, y_max, lb, ub, c0=0.0, c=None,
+                             q=None, t=None, iters=60, history=8, discrete_mask=None, prior_mean_affine=None):
+    """ei_maximize_multistart on mcei_score's Monte-Carlo EI (boss_mcei_maximize_multistart).
+    -> X (d, M), f (M,), best_x (d,), best_val, best_idx, evals."""
+    Xc = _cols(starts)
+    M, d = Xc.shape
+    arr = _slice_array(slices)
+    ep, K = _eps_cols(eps, y_dim)
+    cv, qv, tv = _opt(c), _opt(q), _opt(t)
+    b = None if best is None else np.array([best], dtype=np.float64)
+    ym = _opt(y_max)
+    lbv, ubv = _f64(lb, (d,)), _f64(ub, (d,))
+    dm = _opt(discrete_mask, np.uint8)
+    xo = np.empty((M, d)); fo = np.empty(M); bx = np.empty(d)
+    bv, bi, ev = C.c_double(), C.c_int64(), C.c_int()
+    aff = None if prior_mean_affine is None else _f64(prior_mean_affine, (y_dim, d + 1))
+    _check(lib.boss_mcei_maximize_multistart(arr, y_dim, n_samples, _ptr(Xc), M, int(iters), int(history), _ptr(aff),
+                                             int(fit_kind), float(c0), _ptr(cv), _ptr(qv), _ptr(tv), _ptr(ep), K, _ptr(b),
+                                             _ptr(ym), _ptr(lbv), _ptr(ubv), _ptr(dm), _ptr(xo), _ptr(fo), _ptr(bx),
+                                             C.byref(bv), C.byref(bi), C.byref(ev)), "boss_mcei_maximize_multistart")
+    return xo.T, fo, bx, bv.value, bi.value, ev.value
+
+
+def mcei_score_topk(slices, y_dim, n_samples, Xs, fit_kind, eps, best, y_max, k, c0=0.0, c=None, q=None, t=None, lb=None,
+                    ub=None, cons_mask=None, prior_mean_s=None):
+    """The k best candidates of mcei_score's scores, selected on the device (boss_mcei_score_topk; order as
+    ei_score_topk).  -> top_val (k,), top_idx (k,) int64."""
+    Xc = _cols(Xs)
+    M, d = Xc.shape
+    arr = _slice_array(slices)
+    ep, K = _eps_cols(eps, y_dim)
+    cv, qv, tv_ = _opt(c), _opt(q), _opt(t)
+    b = None if best is None else np.array([best], dtype=np.float64)
+    ym = None if y_max is None else _f64(y_max, (y_dim,))
+    lbv = None if lb is None else _f64(lb, (d,))
+    ubv = None if ub is None else _f64(ub, (d,))
+    cm = None if cons_mask is None else np.ascontiguousarray(cons_mask, dtype=np.uint8)
+    pm = None if prior_mean_s is None else np.ascontiguousarray(np.asarray(prior_mean_s, dtype=np.float64).T)
+    k = int(k)
+    top_v = np.empty(max(k, 0))
+    top_i = np.empty(max(k, 0), dtype=np.int64)
+    _check(lib.boss_mcei_score_topk(arr, y_dim, n_samples, _ptr(Xc), M, _ptr(pm), int(fit_kind), float(c0), _ptr(cv),
+                                    _ptr(qv), _ptr(tv_), _ptr(ep), K, _ptr(b), _ptr(ym), _ptr(lbv), _ptr(ubv), _ptr(cm), k,
+                                    _ptr(top_v), _ptr(top_i)), "boss_mcei_score_topk")
+    return top_v, top_i
 
 
 def _opt(a, dtype=np.float64):

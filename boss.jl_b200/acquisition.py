@@ -103,7 +103,8 @@ class Acquisition:
         multi-start driver can run the whole solve."""
         probe = np.zeros((self.problem.data.x_dim, 1))
         no_mean = all(m.mean_at(i, probe) is None for i, m in enumerate(self.models))
-        return no_mean and self.problem.domain.cons is None and self.cons_safe and not self.nonlin
+        return (no_mean and self.problem.domain.cons is None and self.cons_safe
+                and (not self.nonlin or self.expr is not None))
 
     def _fitness_values(self, pred):
         """fitness.(pred_samples): pred is y_dim x P.  A closure written with numpy broadcasting is applied to the
@@ -196,9 +197,17 @@ class Acquisition:
         return int(bi), float(bv)
 
     def topk(self, X, k):
-        """-> (indices (k,), values (k,)) of the k best columns of X in julia_sortperm_rev order.  LinFitness selects on
-        the device (boss_ei_score_topk); a NonlinFitness scores every column and sorts on the host."""
+        """-> (indices (k,), values (k,)) of the k best columns of X in julia_sortperm_rev order.  LinFitness and
+        ExprFitness select on the device (boss_ei_score_topk, boss_mcei_score_topk); an opaque NonlinFitness scores
+        every column and sorts on the host."""
         X = np.asarray(X, dtype=np.float64)
+        if self.expr is not None:
+            lb, ub, cm = self._guards(X)
+            e = self.expr
+            vals, idx = _lib.mcei_score_topk(self.slices, self.y_dim, len(self.posts), X, e.kind_id, self.eps, self.best,
+                                             self.y_max, k, c0=e.c0, c=e.c, q=e.q, t=e.t, lb=lb, ub=ub, cons_mask=cm,
+                                             prior_mean_s=self._prior_mean(X))
+            return idx, vals
         if self.nonlin:
             acq = self._mc_acq(X)
             top = julia_sortperm_rev(acq)[:k]
@@ -211,6 +220,12 @@ class Acquisition:
     def value_and_grad(self, X):
         """-> acq (M,), grad (d, M).  Prior-mean gradients are not propagated for closure means."""
         X = np.asarray(X, dtype=np.float64)
+        if self.expr is not None:     # expression-set fitness: the chain rule through the Monte-Carlo EI on the device
+            lb, ub, cm = self._guards(X)
+            e = self.expr
+            return _lib.mcei_value_grad(self.slices, self.y_dim, len(self.posts), X, e.kind_id, self.eps, self.best,
+                                        self.y_max, c0=e.c0, c=e.c, q=e.q, t=e.t, lb=lb, ub=ub, cons_mask=cm,
+                                        prior_mean_s=self._prior_mean(X))
         if self.nonlin:
             raise NotImplementedError("NonlinFitness: the Monte-Carlo EI of an arbitrary host closure has no analytic "
                                       "gradient here (the reference pushes ForwardDiff duals through the closure); "

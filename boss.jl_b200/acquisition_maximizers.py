@@ -224,9 +224,17 @@ def maximize_acquisition(am, problem: BossProblem, options: BossOptions = BossOp
             starts = np.asarray(am.multistart, dtype=np.float64)
         if acq.device_resident_ok():
             # no host closures on the path (prior mean, cons): the whole multi-start solve stays on the device
-            _, f, bx, bv, _, _ = _lib.ei_maximize_multistart(acq.slices, acq.y_dim, len(acq.posts), starts, acq.coefs,
-                                                             acq.best, acq.y_max, lb, ub, am.iters, am.history,
-                                                             discrete_mask=dom.discrete if dom.discrete.any() else None)
+            dm = dom.discrete if dom.discrete.any() else None
+            if acq.expr is not None:
+                e = acq.expr
+                _, f, bx, bv, _, _ = _lib.mcei_maximize_multistart(acq.slices, acq.y_dim, len(acq.posts), starts, e.kind_id,
+                                                                   acq.eps, acq.best, acq.y_max, lb, ub, c0=e.c0, c=e.c,
+                                                                   q=e.q, t=e.t, iters=am.iters, history=am.history,
+                                                                   discrete_mask=dm)
+            else:
+                _, f, bx, bv, _, _ = _lib.ei_maximize_multistart(acq.slices, acq.y_dim, len(acq.posts), starts, acq.coefs,
+                                                                 acq.best, acq.y_max, lb, ub, am.iters, am.history,
+                                                                 discrete_mask=dm)
             if np.isneginf(bv):
                 raise RuntimeError("All optimization runs failed!")                  # optim_multistart.jl:34
             return bx, bv

@@ -1400,11 +1400,13 @@ struct ScoreCall {
     d_counter = reinterpret_cast<unsigned int *>(small + nsl + 2 * d + 3);
     if (a.mix) {   // MC-EI: the eps matrix (y_dim x n_eps) goes to the device once per call
       mixp = *a.mix;
-      const size_t eb = (size_t)a.y_dim * mixp.n_eps * 8;
-      CUDA_TRY(C().tt.ensure(eb));
-      CUDA_TRY(cudaMemcpyAsync(C().tt.p, mixp.eps_host, eb, cudaMemcpyHostToDevice, C().stream));
-      CUDA_TRY(cudaStreamSynchronize(C().stream));
-      mixp.eps = C().tt.as<double>();
+      if (!mixp.eps) {   // already on the device: the multi-start driver uploads it once per solve
+        const size_t eb = (size_t)a.y_dim * mixp.n_eps * 8;
+        CUDA_TRY(C().tt.ensure(eb));
+        CUDA_TRY(cudaMemcpyAsync(C().tt.p, mixp.eps_host, eb, cudaMemcpyHostToDevice, C().stream));
+        CUDA_TRY(cudaStreamSynchronize(C().stream));
+        mixp.eps = C().tt.as<double>();
+      }
     }
     return 0;
   }
@@ -1977,7 +1979,10 @@ int score_core(ScoreArgs &a) {
     }
     if (a.grad) {
       AcqGradParams gp2{ap, C().dmu.as<double>(), C().dvar.as<double>(), io.pmg, io.grad};
-      acq_grad_kernel<<<(ch + 127) / 128, 128, 0, C().stream>>>(gp2);
+      if (ap.mix.kind != 0 && ap.has_best)   // Monte-Carlo EI; PoF alone has no Monte-Carlo term
+        acq_grad_kernel<true><<<(ch + 127) / 128, 128, 0, C().stream>>>(gp2);
+      else
+        acq_grad_kernel<false><<<(ch + 127) / 128, 128, 0, C().stream>>>(gp2);
       ++C().launches;
     }
     if (!a.dev) {
@@ -2214,8 +2219,9 @@ int boss_ei_score_dev(const boss_gp *const *slices, int y_dim, int n_samples, co
 static int ei_score_topk_impl(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
                               const double *prior_mean_s, const double *fit_coefs, const double *best,
                               const double *y_max, const double *lb, const double *ub, const uint8_t *cons_mask,
-                              int64_t k, double *top_val, int64_t *top_idx, bool dev, void *stream) {
-  if (!slices || y_dim < 1 || n_samples < 1 || !Xs || M < 1 || !fit_coefs || !top_val || !top_idx)
+                              int64_t k, double *top_val, int64_t *top_idx, bool dev, void *stream,
+                              const MixParams *mix = nullptr) {
+  if (!slices || y_dim < 1 || n_samples < 1 || !Xs || M < 1 || (!fit_coefs && !mix) || !top_val || !top_idx)
     return fail(BOSS_ERR_ARG, "boss_ei_score_topk: bad arguments");
   if (k < 1 || k > M || k > TOPK_MAX) return fail(BOSS_ERR_ARG, "boss_ei_score_topk: k must be in 1..min(M, 8192)");
   int rc = check_lb_ub("boss_ei_score_topk", lb, ub);
@@ -2226,6 +2232,7 @@ static int ei_score_topk_impl(const boss_gp *const *slices, int y_dim, int n_sam
   a.topk = k;
   a.top_val = top_val;
   a.top_idx = top_idx;
+  a.mix = mix;
   return score_dispatch(a);
 }
 
@@ -2249,17 +2256,16 @@ int boss_ei_score_topk_dev(const boss_gp *const *slices, int y_dim, int n_sample
 // replaces expected_improvement(::NonlinFitness, ...) (src/acquisitions/expected_improvement.jl:104-111) inside the
 // same construct_ei cases (:68-90).  eps is y_dim x n_eps (column-major, the reference's sample_eps matrix, :119);
 // with n_samples > 1 posteriors (BI) posterior s gets column s (n_eps must equal n_samples, :87-90).
-int boss_mcei_score(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
-                    const double *prior_mean_s, int fit_kind, double fit_c0, const double *fit_c, const double *fit_q,
-                    const double *fit_t, const double *eps, int n_eps, const double *best, const double *y_max,
-                    const double *lb, const double *ub, const uint8_t *cons_mask, double *acq, double *best_val,
-                    int64_t *best_idx) {
-  if (fit_kind < 1 || fit_kind > 4) return fail(BOSS_ERR_ARG, "boss_mcei_score: fit_kind must be 1 (affine), 2 (quadratic), 3 (max) or 4 (min)");
-  if (!eps || n_eps < 1 || y_dim < 1 || y_dim > MAX_YDIM) return fail(BOSS_ERR_ARG, "boss_mcei_score: bad eps / y_dim");
-  if (n_eps > MIX_MAX_EPS) return fail(BOSS_ERR_ARG, "boss_mcei_score: more than 4096 eps samples");
+// The MixParams of one MC-EI call (the validation every boss_mcei_* entry point shares); eps stays a host pointer
+static int mix_params(const char *who, int y_dim, int n_samples, int fit_kind, double fit_c0, const double *fit_c,
+                      const double *fit_q, const double *fit_t, const double *eps, int n_eps, MixParams &mix) {
+  const std::string w(who);
+  if (fit_kind < 1 || fit_kind > 4) return fail(BOSS_ERR_ARG, w + ": fit_kind must be 1 (affine), 2 (quadratic), 3 (max) or 4 (min)");
+  if (!eps || n_eps < 1 || y_dim < 1 || y_dim > MAX_YDIM) return fail(BOSS_ERR_ARG, w + ": bad eps / y_dim");
+  if (n_eps > MIX_MAX_EPS) return fail(BOSS_ERR_ARG, w + ": more than 4096 eps samples");
   if (n_samples > 1 && n_eps != n_samples)
-    return fail(BOSS_ERR_ARG, "boss_mcei_score: with BI posteriors eps must hold one column per posterior");
-  MixParams mix{};
+    return fail(BOSS_ERR_ARG, w + ": with BI posteriors eps must hold one column per posterior");
+  mix = MixParams{};
   mix.kind = fit_kind;
   mix.n_eps = n_eps;
   mix.c0 = fit_c0;
@@ -2269,8 +2275,44 @@ int boss_mcei_score(const boss_gp *const *slices, int y_dim, int n_samples, cons
     mix.t[i] = fit_t ? fit_t[i] : 0.0;
   }
   mix.eps_host = eps;
+  return 0;
+}
+
+int boss_mcei_score(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
+                    const double *prior_mean_s, int fit_kind, double fit_c0, const double *fit_c, const double *fit_q,
+                    const double *fit_t, const double *eps, int n_eps, const double *best, const double *y_max,
+                    const double *lb, const double *ub, const uint8_t *cons_mask, double *acq, double *best_val,
+                    int64_t *best_idx) {
+  MixParams mix;
+  int rc = mix_params("boss_mcei_score", y_dim, n_samples, fit_kind, fit_c0, fit_c, fit_q, fit_t, eps, n_eps, mix);
+  if (rc) return rc;
   return ei_score_impl(slices, y_dim, n_samples, Xs, M, prior_mean_s, nullptr, best, y_max, lb, ub, cons_mask, acq, nullptr,
                        best_val, best_idx, false, nullptr, nullptr, &mix);
+}
+
+int boss_mcei_value_grad(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
+                         const double *prior_mean_s, const double *prior_mean_grad_s, int fit_kind, double fit_c0,
+                         const double *fit_c, const double *fit_q, const double *fit_t, const double *eps, int n_eps,
+                         const double *best, const double *y_max, const double *lb, const double *ub,
+                         const uint8_t *cons_mask, double *acq, double *grad) {
+  if (!grad) return fail(BOSS_ERR_ARG, "boss_mcei_value_grad: grad is NULL");
+  MixParams mix;
+  int rc = mix_params("boss_mcei_value_grad", y_dim, n_samples, fit_kind, fit_c0, fit_c, fit_q, fit_t, eps, n_eps, mix);
+  if (rc) return rc;
+  return ei_score_impl(slices, y_dim, n_samples, Xs, M, prior_mean_s, nullptr, best, y_max, lb, ub, cons_mask, acq, grad,
+                       nullptr, nullptr, false, prior_mean_grad_s, nullptr, &mix);
+}
+
+int boss_mcei_score_topk(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
+                         const double *prior_mean_s, int fit_kind, double fit_c0, const double *fit_c,
+                         const double *fit_q, const double *fit_t, const double *eps, int n_eps, const double *best,
+                         const double *y_max, const double *lb, const double *ub, const uint8_t *cons_mask, int64_t k,
+                         double *top_val, int64_t *top_idx) {
+  MixParams mix;
+  int rc = mix_params("boss_mcei_score_topk", y_dim, n_samples, fit_kind, fit_c0, fit_c, fit_q, fit_t, eps, n_eps, mix);
+  if (rc) return rc;
+  return ei_score_topk_impl(slices, y_dim, n_samples, Xs, M, prior_mean_s, nullptr, best, y_max, lb, ub, cons_mask, k,
+                            top_val, top_idx, false, nullptr, &mix);
 }
 
 static int ei_score_generated(const CandGen &gen, int64_t M, const boss_gp *const *slices, int y_dim, int n_samples,
@@ -2349,7 +2391,7 @@ static int multistart_single(const boss_gp *const *slices, int y_dim, int n_samp
                              int iters, int history, const double *prior_mean_affine, const double *fit_coefs,
                              const double *best, const double *y_max, const double *lb, const double *ub,
                              const uint8_t *discrete_mask, double *x_out, double *f_out, double *best_x,
-                             double *best_val, int64_t *best_idx, int *evals_out) {
+                             double *best_val, int64_t *best_idx, int *evals_out, const MixParams *mix) {
   const int d = slices[0]->d;
   if (d > MS_MAXD) return fail(BOSS_ERR_ARG, "boss_ei_maximize_multistart: x_dim > 32");
   const int H = std::max(1, std::min(history, MS_MAXH - 1));
@@ -2359,9 +2401,10 @@ static int multistart_single(const boss_gp *const *slices, int y_dim, int n_samp
   // the compact batch of a round holds `fan` trial points per unfinished start: up to MS_FAN_BATCH points once the
   // step-size fan is on (few starts left), never more than M points before that
   const size_t cap = (size_t)std::max<long long>(M, MS_FAN_BATCH), capd = cap * d;
-  // carve one workspace: X g dirn | Sh Yh | f t | [affine mean scratch] | Xc gc fc | counters, per-start ints
+  // carve one workspace: X g dirn | Sh Yh | f t | [affine mean scratch] | Xc gc fc | [MC-EI eps] | counters, per-start ints
   const size_t n_aff = prior_mean_affine ? (size_t)y_dim * (d + 1) + cap * y_dim + capd * y_dim : 0;
-  const size_t n_dbl = 3 * Md + 2 * (size_t)RC * Md + 2 * (size_t)M + n_aff + 2 * capd + cap;
+  const size_t n_eps = mix ? (size_t)y_dim * mix->n_eps : 0;
+  const size_t n_dbl = 3 * Md + 2 * (size_t)RC * Md + 2 * (size_t)M + n_aff + 2 * capd + cap + n_eps;
   CUDA_TRY(C().ms_buf.ensure(n_dbl * 8 + (size_t)M * 24 + cap * 4 + 64));
   double *base = C().ms_buf.as<double>();
   MsState st{};
@@ -2382,7 +2425,15 @@ static int multistart_single(const boss_gp *const *slices, int y_dim, int n_samp
   st.Xc = st.t + M + n_aff;
   st.gc = st.Xc + capd;
   st.fc = st.gc + capd;
-  st.counters = reinterpret_cast<int *>(st.fc + cap);
+  // MC-EI: eps goes to the device once per solve; every round's scoring call then skips its own upload and wait
+  MixParams mixd{};
+  if (mix) {
+    mixd = *mix;
+    mixd.eps = st.fc + cap;
+    mixd.eps_host = nullptr;
+    CUDA_TRY(cudaMemcpyAsync(const_cast<double *>(mixd.eps), mix->eps_host, n_eps * 8, cudaMemcpyHostToDevice, C().stream));
+  }
+  st.counters = reinterpret_cast<int *>(st.fc + cap + n_eps);
   st.hist_len = st.counters + 4;
   st.hist_start = st.hist_len + M;
   st.trials = st.hist_start + M;
@@ -2417,6 +2468,7 @@ static int multistart_single(const boss_gp *const *slices, int y_dim, int n_samp
     a.dev = true;
     a.internal = true;
     a.want_argmax = want_best;
+    a.mix = mix ? &mixd : nullptr;
     return score_core(a);
   };
 
@@ -2489,12 +2541,14 @@ static int multistart_single(const boss_gp *const *slices, int y_dim, int n_samp
   return 0;
 }
 
-int boss_ei_maximize_multistart(const boss_gp *const *slices, int y_dim, int n_samples, const double *starts, int64_t M,
-                                int iters, int history, const double *prior_mean_affine, const double *fit_coefs,
-                                const double *best, const double *y_max, const double *lb, const double *ub,
-                                const uint8_t *discrete_mask, double *x_out, double *f_out, double *best_x,
-                                double *best_val, int64_t *best_idx, int *evals_out) {
-  if (!slices || !slices[0] || y_dim < 1 || n_samples < 1 || !starts || M < 1 || !fit_coefs || !lb || !ub)
+// one device, or contiguous ranges of starts dealt to the devices; mix == null: LinFitness (fit_coefs)
+static int maximize_multistart_impl(const boss_gp *const *slices, int y_dim, int n_samples, const double *starts,
+                                    int64_t M, int iters, int history, const double *prior_mean_affine,
+                                    const double *fit_coefs, const double *best, const double *y_max, const double *lb,
+                                    const double *ub, const uint8_t *discrete_mask, double *x_out, double *f_out,
+                                    double *best_x, double *best_val, int64_t *best_idx, int *evals_out,
+                                    const MixParams *mix) {
+  if (!slices || !slices[0] || y_dim < 1 || n_samples < 1 || !starts || M < 1 || (!fit_coefs && !mix) || !lb || !ub)
     return fail(BOSS_ERR_ARG, "boss_ei_maximize_multistart: bad arguments (the box lb/ub is required)");
   const int nsl = y_dim * n_samples;
   for (int q = 0; q < nsl; ++q)
@@ -2513,7 +2567,7 @@ int boss_ei_maximize_multistart(const boss_gp *const *slices, int y_dim, int n_s
     if (!cx) return fail(BOSS_ERR_STATE, "boss_ei_maximize_multistart: no usable device context for the handle");
     Enter en(cx);
     return multistart_single(slices, y_dim, n_samples, starts, M, iters, history, prior_mean_affine, fit_coefs, best, y_max,
-                             lb, ub, discrete_mask, x_out, f_out, best_x, best_val, best_idx, evals_out);
+                             lb, ub, discrete_mask, x_out, f_out, best_x, best_val, best_idx, evals_out, mix);
   }
   // multi-device: the starts are independent local solves (optimize_multistart, src/utils/optim_multistart.jl:10-90):
   // contiguous ranges of starts per device, the winners compared on the host in Julia's argmax order
@@ -2528,7 +2582,7 @@ int boss_ei_maximize_multistart(const boss_gp *const *slices, int y_dim, int n_s
     return multistart_single(slices, y_dim, n_samples, starts + (size_t)first[k] * d, cnt[k], iters, history,
                              prior_mean_affine, fit_coefs, best, y_max, lb, ub, discrete_mask,
                              x_out ? x_out + (size_t)first[k] * d : nullptr, f_out ? f_out + first[k] : nullptr,
-                             bx.data() + (size_t)k * d, &bv[k], &bi[k], &ev[k]);
+                             bx.data() + (size_t)k * d, &bv[k], &bi[k], &ev[k], mix);
   });
   if (rc) return rc;
   double v = -std::numeric_limits<double>::infinity();
@@ -2552,6 +2606,31 @@ int boss_ei_maximize_multistart(const boss_gp *const *slices, int y_dim, int n_s
     for (int k = 0; k < nd; ++k) *evals_out = std::max(*evals_out, ev[k]);
   }
   return 0;
+}
+
+int boss_ei_maximize_multistart(const boss_gp *const *slices, int y_dim, int n_samples, const double *starts, int64_t M,
+                                int iters, int history, const double *prior_mean_affine, const double *fit_coefs,
+                                const double *best, const double *y_max, const double *lb, const double *ub,
+                                const uint8_t *discrete_mask, double *x_out, double *f_out, double *best_x,
+                                double *best_val, int64_t *best_idx, int *evals_out) {
+  if (!fit_coefs) return fail(BOSS_ERR_ARG, "boss_ei_maximize_multistart: bad arguments (the box lb/ub is required)");
+  return maximize_multistart_impl(slices, y_dim, n_samples, starts, M, iters, history, prior_mean_affine, fit_coefs, best,
+                                  y_max, lb, ub, discrete_mask, x_out, f_out, best_x, best_val, best_idx, evals_out,
+                                  nullptr);
+}
+
+int boss_mcei_maximize_multistart(const boss_gp *const *slices, int y_dim, int n_samples, const double *starts,
+                                  int64_t M, int iters, int history, const double *prior_mean_affine, int fit_kind,
+                                  double fit_c0, const double *fit_c, const double *fit_q, const double *fit_t,
+                                  const double *eps, int n_eps, const double *best, const double *y_max,
+                                  const double *lb, const double *ub, const uint8_t *discrete_mask, double *x_out,
+                                  double *f_out, double *best_x, double *best_val, int64_t *best_idx, int *evals_out) {
+  MixParams mix;
+  int rc = mix_params("boss_mcei_maximize_multistart", y_dim, n_samples, fit_kind, fit_c0, fit_c, fit_q, fit_t, eps, n_eps,
+                      mix);
+  if (rc) return rc;
+  return maximize_multistart_impl(slices, y_dim, n_samples, starts, M, iters, history, prior_mean_affine, nullptr, best,
+                                  y_max, lb, ub, discrete_mask, x_out, f_out, best_x, best_val, best_idx, evals_out, &mix);
 }
 
 int boss_ei_value_grad(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,

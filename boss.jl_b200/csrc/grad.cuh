@@ -8,7 +8,7 @@
 //
 // Pipeline per chunk and slice: xcov -> score_trmm (also stores V^T) -> wtv_kernel (U^T = (W^T V)^T, the
 // second triangular product, same DMMA mainloop) -> grad_kernel (kernel derivatives, FP64 pipe) ->
-// acq_grad_kernel (chain rule through EI x PoF).
+// acq_grad_kernel (chain rule through EI x PoF, or through the Monte-Carlo EI of a MixParams expression).
 #pragma once
 #include "score.cuh"
 
@@ -78,6 +78,34 @@ __global__ void __launch_bounds__(256) grad_reduce_kernel(GradReduceParams p) {
   p.dvar[(size_t)j * p.chunk_ld + c] = disc ? 0.0 : -2.0 * av * il;
 }
 
+// MC-EI adjoint weights (DESIGN.md 2.11): for one eps column e with improvement > 0 at y = mu + sd .* e,
+//   A_i += g_i(y),  B_i += g_i(y) e_i,   g_i = df/dy_i of the branch mix_fitness took:
+//   affine c_i;  quadratic c_i + 2 q_i (y_i - t_i);  max / min c_i* for the first extreme output i*, 0 for the others
+__device__ __forceinline__ void mix_adjoint(const MixParams &mx, const double *y, const double *e, int y_dim, double *A,
+                                            double *B) {
+  if (mx.kind == 1 || mx.kind == 2) {
+    for (int i = 0; i < y_dim; ++i) {
+      const double g = mx.kind == 1 ? mx.c[i] : fma(2.0 * mx.q[i], y[i] - mx.t[i], mx.c[i]);
+      A[i] += g;
+      B[i] = fma(g, e[i], B[i]);
+    }
+    return;
+  }
+  int is = -1;   // the selection of mix_fitness: the first output whose term is extreme (NaN terms never reach here)
+  double ext = 0.0;
+  for (int i = 0; i < y_dim; ++i) {
+    if (mx.c[i] == 0.0) continue;
+    const double v = fma(mx.c[i], y[i], mx.t[i]);
+    if (is < 0 || (mx.kind == 3 ? v > ext : v < ext)) {
+      ext = v;
+      is = i;
+    }
+  }
+  if (is < 0) return;   // no output enters f: a constant
+  A[is] += mx.c[is];
+  B[is] = fma(mx.c[is], e[is], B[is]);
+}
+
 // Chain rule through EI x PoF.  dmu / dvar: [(sample*y_dim + slice)][d][chunk_ld].
 struct AcqGradParams {
   AcqParams a;
@@ -86,6 +114,13 @@ struct AcqGradParams {
   double *grad;                   // d x M, indexed by (m - out_off)
 };
 
+// MC = false: the closed-form EI of a LinFitness.  MC = true: the Monte-Carlo EI of a MixParams expression (launched
+// only with `best` set; PoF alone has no Monte-Carlo term and takes MC = false).  Per posterior s with eps columns K_s:
+//   d EI_s = sum_i A_i d mu_i + B_i d sd_i ,  d sd_i = d var_i / (2 sd_i)  (0 when sd_i == 0 or the variance was clipped)
+// with A, B of mix_adjoint averaged over K_s: K_s * y_dim work per posterior, then d * y_dim per candidate.
+// Conventions at the measure-zero kinks: the derivative of the branch the value took (imp == 0 contributes 0, a max /
+// min tie goes to the first output); a NaN improvement makes the gradient NaN.
+template <bool MC>
 __global__ void __launch_bounds__(128) acq_grad_kernel(AcqGradParams q) {
   const AcqParams &p = q.a;
   const int c = blockIdx.x * 128 + threadIdx.x;
@@ -98,6 +133,7 @@ __global__ void __launch_bounds__(128) acq_grad_kernel(AcqGradParams q) {
   for (int s = 0; s < p.n_samples; ++s) {
     // pass 1: scalars
     double cdf_i[MAX_YDIM], wmu_i[MAX_YDIM], wvar_i[MAX_YDIM];
+    double mu_i[MAX_YDIM], sd_i[MAX_YDIM];   // MC only
     bool live_i[MAX_YDIM];
     double mu_f = 0.0, s2 = 0.0, pof = 1.0;
     for (int i = 0; i < p.y_dim; ++i) {
@@ -108,8 +144,13 @@ __global__ void __launch_bounds__(128) acq_grad_kernel(AcqGradParams q) {
       const bool unclipped = var >= 0.0;
       if (!clip_var(var)) failed = true;
       live_i[i] = unclipped;   // the clipped branch of _clip_var returns a constant zero -> zero derivative
-      mu_f = fma(p.coefs[i], mu, mu_f);
-      s2 = fma(p.coefs[i] * p.coefs[i], var, s2);
+      if constexpr (MC) {
+        mu_i[i] = mu;
+        sd_i[i] = sqrt(var);
+      } else {
+        mu_f = fma(p.coefs[i], mu, mu_f);
+        s2 = fma(p.coefs[i] * p.coefs[i], var, s2);
+      }
       cdf_i[i] = 1.0;
       wmu_i[i] = wvar_i[i] = 0.0;
       if (p.has_ymax && !(p.y_max[i] == INFINITY)) {
@@ -126,7 +167,31 @@ __global__ void __launch_bounds__(128) acq_grad_kernel(AcqGradParams q) {
       }
     }
     double ei = 0.0, cphi = 0.0, cpdf_over_2sf = 0.0;   // d ei = cphi * d mu_f + cpdf_over_2sf * d s2
-    if (p.has_best) {
+    double wa[MAX_YDIM], wb[MAX_YDIM];                   // MC: d ei = sum_i wa_i d mu_i + wb_i d var_i
+    if constexpr (MC) {
+      // the value's loop of acq_candidate (same columns, same order), plus the adjoint weights
+      const int k0 = p.n_samples > 1 ? s : 0, k1 = p.n_samples > 1 ? s + 1 : p.mix.n_eps;
+      for (int i = 0; i < p.y_dim; ++i) wa[i] = wb[i] = 0.0;
+      double tot = 0.0;
+      for (int k = k0; k < k1; ++k) {
+        double ys[MAX_YDIM];
+        const double *ek = p.mix.eps + (size_t)k * p.y_dim;
+        for (int i = 0; i < p.y_dim; ++i) ys[i] = mu_i[i] + sd_i[i] * ek[i];
+        const double imp = mix_fitness(p.mix, ys, p.y_dim) - p.best;
+        tot += (imp != imp) ? imp : (imp > 0.0 ? imp : 0.0);
+        if (imp > 0.0) {
+          mix_adjoint(p.mix, ys, ek, p.y_dim, wa, wb);
+        } else if (imp != imp) {
+          for (int i = 0; i < p.y_dim; ++i) wa[i] = wb[i] = NAN;
+        }
+      }
+      const double nk = (double)(k1 - k0);
+      ei = tot / nk;
+      for (int i = 0; i < p.y_dim; ++i) {
+        wa[i] /= nk;
+        wb[i] = sd_i[i] > 0.0 ? wb[i] / nk / (2.0 * sd_i[i]) : 0.0;   // a NaN improvement already made wa NaN
+      }
+    } else if (p.has_best) {
       const double sf = sqrt(s2), diff = mu_f - p.best;
       if (diff == 0.0 && sf == 0.0) {
         ei = 0.0;
@@ -144,14 +209,19 @@ __global__ void __launch_bounds__(128) acq_grad_kernel(AcqGradParams q) {
     }
     // pass 2: per input dimension
     for (int j = 0; j < d; ++j) {
-      double dmu_f = 0.0, ds2 = 0.0, dpof = 0.0;
+      double dmu_f = 0.0, ds2 = 0.0, dpof = 0.0, dei_mc = 0.0;
       for (int i = 0; i < p.y_dim; ++i) {
         const size_t row = ((size_t)(s * p.y_dim + i) * d + j) * p.chunk_ld + c;
         double dm = q.dmu[row];
         if (q.prior_mean_grad) dm += q.prior_mean_grad[((size_t)(m - p.in_off) * d + j) * p.y_dim + i];
         const double dv = live_i[i] ? q.dvar[row] : 0.0;
-        dmu_f = fma(p.coefs[i], dm, dmu_f);
-        ds2 = fma(p.coefs[i] * p.coefs[i], dv, ds2);
+        if constexpr (MC) {
+          dei_mc = fma(wa[i], dm, dei_mc);
+          dei_mc = fma(wb[i], dv, dei_mc);
+        } else {
+          dmu_f = fma(p.coefs[i], dm, dmu_f);
+          ds2 = fma(p.coefs[i] * p.coefs[i], dv, ds2);
+        }
         if (p.has_ymax && !(p.y_max[i] == INFINITY)) {
           double others = 1.0;
           for (int b = 0; b < p.y_dim; ++b)
@@ -159,7 +229,7 @@ __global__ void __launch_bounds__(128) acq_grad_kernel(AcqGradParams q) {
           dpof = fma(wmu_i[i] * dm + wvar_i[i] * dv, others, dpof);
         }
       }
-      const double dei = cphi * dmu_f + cpdf_over_2sf * ds2;
+      const double dei = MC ? dei_mc : cphi * dmu_f + cpdf_over_2sf * ds2;
       double g;
       if (p.has_best)
         g = p.has_ymax ? dei * pof + ei * dpof : dei;

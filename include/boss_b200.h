@@ -160,7 +160,7 @@ int boss_ei_score_dev(const boss_gp *const *slices, int y_dim, int n_samples, co
  *            best_val / best_idx too: top_val[0], top_idx[0] equal boss_ei_score's pair bit for bit.
  *   indices  0-based, into Xs; with boss_init_multi the result is bit-identical to the single-device call.
  * With `best` set and at least 64 Ki candidates the call scores exactly only candidates whose EI upper bound can still
- * reach the k best (DESIGN.md 2.10); the result is the same either way.  MC-EI (boss_mcei_score) has no top-k. */
+ * reach the k best (DESIGN.md 2.10); the result is the same either way. */
 int boss_ei_score_topk(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
                        const double *prior_mean_s, const double *fit_coefs, const double *best, const double *y_max,
                        const double *lb, const double *ub, const uint8_t *cons_mask, int64_t k, double *top_val,
@@ -206,6 +206,40 @@ int boss_mcei_score(const boss_gp *const *slices, int y_dim, int n_samples, cons
                     const double *fit_t, const double *eps, int n_eps, const double *best, const double *y_max,
                     const double *lb, const double *ub, const uint8_t *cons_mask, double *acq, double *best_val,
                     int64_t *best_idx);
+
+/* The same Monte-Carlo EI for OptimizationAM and SampleOptAM (the reference pushes ForwardDiff.Dual numbers through
+ * expected_improvement(::NonlinFitness, ...)).  fit_kind, fit_c0, fit_c, fit_q, fit_t, eps and n_eps as in
+ * boss_mcei_score, with the same limits and error texts; every other argument as in the LinFitness twin.
+ *   boss_mcei_value_grad           as boss_ei_value_grad: acq equals boss_mcei_score's acq bit for bit
+ *   boss_mcei_maximize_multistart  as boss_ei_maximize_multistart; eps is uploaded once per solve and device
+ *   boss_mcei_score_topk           as boss_ei_score_topk (same order and k range); never screened
+ * The x-gradient (DESIGN.md 2.11): for posterior s with eps columns K_s, y_k = mu + sd .* eps_k, imp_k = f(y_k) - best,
+ *   d EI_s / dx_j = sum_i A_i d mu_i/dx_j + B_i d sd_i/dx_j ,
+ *   A_i = 1/|K_s| sum_{k: imp_k > 0} g_i(y_k) ,  B_i = 1/|K_s| sum_{k: imp_k > 0} g_i(y_k) eps_ik ,  g_i = df/dy_i:
+ *   affine c_i;  quadratic c_i + 2 q_i (y_i - t_i);  max / min c_i* for the output i* the value took, 0 for the others.
+ *   d sd_i = d var_i / (2 sd_i) when sd_i > 0 and the variance was not clipped, else 0.  PoF enters by the product rule,
+ *   the result is averaged over s, and the guards of boss_ei_value_grad apply.  With best == NULL (PoF only) the
+ *   gradient equals boss_ei_value_grad's bit for bit.
+ * Conventions at the measure-zero kinks: the derivative of the branch the value took -- imp_k == 0 contributes 0
+ * (the value takes imp > 0 ? imp : 0), a max / min tie goes to the first output.  A candidate whose value is NaN gets a
+ * NaN gradient.  Whether ForwardDiff returns the same numbers at these points has not been checked.
+ * Cost: |K_s| y_dim per candidate and posterior for A and B, then d y_dim for the gradient. */
+int boss_mcei_value_grad(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
+                         const double *prior_mean_s, const double *prior_mean_grad_s, int fit_kind, double fit_c0,
+                         const double *fit_c, const double *fit_q, const double *fit_t, const double *eps, int n_eps,
+                         const double *best, const double *y_max, const double *lb, const double *ub,
+                         const uint8_t *cons_mask, double *acq, double *grad);
+int boss_mcei_maximize_multistart(const boss_gp *const *slices, int y_dim, int n_samples, const double *starts,
+                                  int64_t M, int iters, int history, const double *prior_mean_affine, int fit_kind,
+                                  double fit_c0, const double *fit_c, const double *fit_q, const double *fit_t,
+                                  const double *eps, int n_eps, const double *best, const double *y_max,
+                                  const double *lb, const double *ub, const uint8_t *discrete_mask, double *x_out,
+                                  double *f_out, double *best_x, double *best_val, int64_t *best_idx, int *evals_out);
+int boss_mcei_score_topk(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
+                         const double *prior_mean_s, int fit_kind, double fit_c0, const double *fit_c,
+                         const double *fit_q, const double *fit_t, const double *eps, int n_eps, const double *best,
+                         const double *y_max, const double *lb, const double *ub, const uint8_t *cons_mask, int64_t k,
+                         double *top_val, int64_t *top_idx);
 
 /* Value + analytic x-gradient of the same acquisition for a batch of points: what OptimizationAM's
  * multi-start solver needs per iteration over all starts (src/acquisition_maximizers/optimization.jl:89-118;

@@ -21,12 +21,14 @@
 #   construct_acquisition(::ExpectedImprovement) (expected_improvement.jl:49-90)-> boss_ei_score / boss_mcei_score
 #   maximize_acquisition(::GridAM)        (acquisition_maximizers/grid.jl:45-65)        -> boss_ei_score
 #   maximize_acquisition(::SamplingAM)    (sampling.jl:20-57)                           -> boss_ei_score
-#   maximize_acquisition(::OptimizationAM)(optimization.jl:55-118)                      -> boss_ei_maximize_multistart
-#   maximize_acquisition(::SampleOptAM)   (sample_opt.jl:41-52)                         -> both of the above
+#   maximize_acquisition(::OptimizationAM)(optimization.jl:55-118)                      -> boss_ei_maximize_multistart /
+#                                                                                          boss_mcei_maximize_multistart
+#   maximize_acquisition(::SampleOptAM)   (sample_opt.jl:41-52)                         -> boss_[mc]ei_score_topk + the above
 #   maximize_acquisition(::SequentialBatchAM) (batch.jl:26-38)                          -> boss_gp_append
 #   estimate_parameters(::SamplingMAP)    (model_fitters/sampling.jl:17-78)             -> boss_gp_loglik_batch
 #   data_loglike + ForwardDiff gradient   (model_fitters/optimization.jl:41,153)        -> boss_gp_loglik_grad_batch
-#   acq(x::Vector{<:ForwardDiff.Dual})    (acquisition_maximizers/optimization.jl:36)   -> boss_ei_value_grad
+#   acq(x::Vector{<:ForwardDiff.Dual})    (acquisition_maximizers/optimization.jl:36)   -> boss_ei_value_grad /
+#                                                                                          boss_mcei_value_grad
 module BossB200
 
 using BOSS
@@ -255,35 +257,41 @@ function score(acq::B200Acquisition, X::AbstractMatrix{<:Real}; want_acq::Bool=t
     return out, bv[], Int(bi[]) + 1
 end
 "The k best columns of X: (values, 1-based indices) in descending isless order (NaN first), ties to the lower index --
-`sortperm(vals; rev=true)[1:k]`.  LinFitness selects on the device (boss_ei_score_topk); MC-EI sorts on the host."
+`sortperm(vals; rev=true)[1:k]`, selected on the device (boss_ei_score_topk for LinFitness, boss_mcei_score_topk for
+a B200ExprFitness)."
 function score_topk(acq::B200Acquisition, X::AbstractMatrix{<:Real}, k::Integer)
     Xs = Matrix{Float64}(X)
     M = size(Xs, 2)
     1 <= k <= M || throw(BoundsError(1:M, k))                     # as order[1:multistart] in sample_opt.jl
     f = acq.fitness
-    if !(f isa LinFitness)
-        vals = score(acq, Xs)[1]
-        order = sortperm(vals; rev=true)[1:k]
-        return vals[order], order
-    end
     pm = prior_means(acq, Xs); cm = cons_mask(acq, Xs)
     best = isnothing(acq.best) ? nothing : [acq.best]
-    coefs = Vector{Float64}(f.coefs)
     tv = Vector{Float64}(undef, k); ti = Vector{Int64}(undef, k)
-    GC.@preserve Xs pm cm best coefs check(ccall((:boss_ei_score_topk, LIB), Cint,
-        (Ptr{Ptr{Cvoid}}, Cint, Cint, Ptr{Cdouble}, Int64, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble},
-         Ptr{Cdouble}, Ptr{Cdouble}, Ptr{UInt8}, Int64, Ptr{Cdouble}, Ptr{Int64}),
-        acq.handles, acq.ydim, length(acq.posts), Xs, M, cptr(pm), coefs, cptr(best), cptr(acq.y_max), cptr(acq.lb),
-        cptr(acq.ub), cptr(cm), k, tv, ti))
+    if f isa LinFitness
+        coefs = Vector{Float64}(f.coefs)
+        GC.@preserve Xs pm cm best coefs check(ccall((:boss_ei_score_topk, LIB), Cint,
+            (Ptr{Ptr{Cvoid}}, Cint, Cint, Ptr{Cdouble}, Int64, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble},
+             Ptr{Cdouble}, Ptr{Cdouble}, Ptr{UInt8}, Int64, Ptr{Cdouble}, Ptr{Int64}),
+            acq.handles, acq.ydim, length(acq.posts), Xs, M, cptr(pm), coefs, cptr(best), cptr(acq.y_max), cptr(acq.lb),
+            cptr(acq.ub), cptr(cm), k, tv, ti))
+    else
+        GC.@preserve Xs pm cm best f check(ccall((:boss_mcei_score_topk, LIB), Cint,
+            (Ptr{Ptr{Cvoid}}, Cint, Cint, Ptr{Cdouble}, Int64, Ptr{Cdouble}, Cint, Cdouble, Ptr{Cdouble}, Ptr{Cdouble},
+             Ptr{Cdouble}, Ptr{Cdouble}, Cint, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{UInt8}, Int64,
+             Ptr{Cdouble}, Ptr{Int64}),
+            acq.handles, acq.ydim, length(acq.posts), Xs, M, cptr(pm), f.kind, f.c0, f.c, f.q, f.t, acq.eps,
+            size(acq.eps, 2), cptr(best), cptr(acq.y_max), cptr(acq.lb), cptr(acq.ub), cptr(cm), k, tv, ti))
+    end
     return tv, ti .+ 1
 end
 (acq::B200Acquisition)(X::AbstractMatrix{<:Real}) = score(acq, X)[1]
 (acq::B200Acquisition)(x::AbstractVector{<:Real}) = score(acq, hcat(x))[1][1]
 
-"Value and x-gradient of the acquisition for every column of X (LinFitness; prior-mean closures enter through their
-ForwardDiff Jacobian evaluated on the host)."
+"Value and x-gradient of the acquisition for every column of X (LinFitness: boss_ei_value_grad; B200ExprFitness: the
+chain rule through the Monte-Carlo EI, boss_mcei_value_grad; prior-mean closures enter through their ForwardDiff
+Jacobian evaluated on the host)."
 function value_grad(acq::B200Acquisition, X::AbstractMatrix{<:Real})
-    acq.fitness isa LinFitness || error("BossB200: the x-gradient exists for LinFitness only")
+    f = acq.fitness
     Xs = Matrix{Float64}(X)
     d, M = size(Xs)
     pm = prior_means(acq, Xs); cm = cons_mask(acq, Xs)
@@ -295,13 +303,22 @@ function value_grad(acq::B200Acquisition, X::AbstractMatrix{<:Real})
         end
     end
     vals = Vector{Float64}(undef, M); grad = Matrix{Float64}(undef, d, M)
-    coefs = Vector{Float64}(acq.fitness.coefs)
     best = isnothing(acq.best) ? nothing : [acq.best]
-    GC.@preserve Xs pm pmg cm coefs best check(ccall((:boss_ei_value_grad, LIB), Cint,
-        (Ptr{Ptr{Cvoid}}, Cint, Cint, Ptr{Cdouble}, Int64, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble},
-         Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{UInt8}, Ptr{Cdouble}, Ptr{Cdouble}),
-        acq.handles, acq.ydim, length(acq.posts), Xs, M, cptr(pm), cptr(pmg), coefs, cptr(best), cptr(acq.y_max),
-        cptr(acq.lb), cptr(acq.ub), cptr(cm), vals, grad))
+    if f isa LinFitness
+        coefs = Vector{Float64}(f.coefs)
+        GC.@preserve Xs pm pmg cm coefs best check(ccall((:boss_ei_value_grad, LIB), Cint,
+            (Ptr{Ptr{Cvoid}}, Cint, Cint, Ptr{Cdouble}, Int64, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble},
+             Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{UInt8}, Ptr{Cdouble}, Ptr{Cdouble}),
+            acq.handles, acq.ydim, length(acq.posts), Xs, M, cptr(pm), cptr(pmg), coefs, cptr(best), cptr(acq.y_max),
+            cptr(acq.lb), cptr(acq.ub), cptr(cm), vals, grad))
+    else
+        GC.@preserve Xs pm pmg cm best f check(ccall((:boss_mcei_value_grad, LIB), Cint,
+            (Ptr{Ptr{Cvoid}}, Cint, Cint, Ptr{Cdouble}, Int64, Ptr{Cdouble}, Ptr{Cdouble}, Cint, Cdouble, Ptr{Cdouble},
+             Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Cint, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble},
+             Ptr{UInt8}, Ptr{Cdouble}, Ptr{Cdouble}),
+            acq.handles, acq.ydim, length(acq.posts), Xs, M, cptr(pm), cptr(pmg), f.kind, f.c0, f.c, f.q, f.t, acq.eps,
+            size(acq.eps, 2), cptr(best), cptr(acq.y_max), cptr(acq.lb), cptr(acq.ub), cptr(cm), vals, grad))
+    end
     return vals, grad
 end
 # AutoForwardDiff (the default of OptimizationAM, acquisition_maximizers/optimization.jl:36) calls acq with Dual numbers
@@ -348,8 +365,9 @@ end
 # nothing on the path is a host closure; otherwise the wrapped solver runs with the batched / Dual-aware closure
 function maximize_b200(am::OptimizationAM, problem, options, acq; starts=BOSS.get_starts(am.multistart, problem.domain))
     dom = problem.domain
-    closure_free = isnothing(dom.cons) && all(s -> !(s.mean isa Function), acq.posts[1].slices) && acq.fitness isa LinFitness &&
-                   !isnothing(acq.lb)
+    f = acq.fitness
+    closure_free = isnothing(dom.cons) && all(s -> !(s.mean isa Function), acq.posts[1].slices) &&
+                   (f isa LinFitness || f isa B200ExprFitness) && !isnothing(acq.lb)
     if !closure_free
         cons_func = isnothing(dom.cons) ? nothing : (res, x, p) -> (res .= dom.cons(x))
         return BOSS.optimize(am, acq, cons_func, dom.bounds[1], dom.bounds[2], dom.discrete, BOSS.cons_dim(dom), starts, options)
@@ -363,15 +381,24 @@ function maximize_b200(am::OptimizationAM, problem, options, acq; starts=BOSS.ge
             s.mean isa Real && (aff[1, i] = s.mean)
         end
     end
-    coefs = Vector{Float64}(acq.fitness.coefs)
     best = isnothing(acq.best) ? nothing : [acq.best]
     mask = Vector{UInt8}(dom.discrete)
     bx = Vector{Float64}(undef, d); bv = Ref{Cdouble}(0.0); bi = Ref{Int64}(-1); ev = Ref{Cint}(0)
-    GC.@preserve S aff coefs best mask check(ccall((:boss_ei_maximize_multistart, LIB), Cint,
-        (Ptr{Ptr{Cvoid}}, Cint, Cint, Ptr{Cdouble}, Int64, Cint, Cint, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble},
-         Ptr{Cdouble}, Ptr{Cdouble}, Ptr{UInt8}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ref{Cdouble}, Ref{Int64}, Ref{Cint}),
-        acq.handles, acq.ydim, length(acq.posts), S, M, 60, 8, cptr(aff), coefs, cptr(best), cptr(acq.y_max), acq.lb, acq.ub,
-        mask, C_NULL, C_NULL, bx, bv, bi, ev))
+    if f isa LinFitness
+        coefs = Vector{Float64}(f.coefs)
+        GC.@preserve S aff coefs best mask check(ccall((:boss_ei_maximize_multistart, LIB), Cint,
+            (Ptr{Ptr{Cvoid}}, Cint, Cint, Ptr{Cdouble}, Int64, Cint, Cint, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble},
+             Ptr{Cdouble}, Ptr{Cdouble}, Ptr{UInt8}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ref{Cdouble}, Ref{Int64}, Ref{Cint}),
+            acq.handles, acq.ydim, length(acq.posts), S, M, 60, 8, cptr(aff), coefs, cptr(best), cptr(acq.y_max), acq.lb,
+            acq.ub, mask, C_NULL, C_NULL, bx, bv, bi, ev))
+    else                                                  # B200ExprFitness: the Monte-Carlo EI with this acquisition's eps
+        GC.@preserve S aff f best mask check(ccall((:boss_mcei_maximize_multistart, LIB), Cint,
+            (Ptr{Ptr{Cvoid}}, Cint, Cint, Ptr{Cdouble}, Int64, Cint, Cint, Ptr{Cdouble}, Cint, Cdouble, Ptr{Cdouble},
+             Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Cint, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble},
+             Ptr{UInt8}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ref{Cdouble}, Ref{Int64}, Ref{Cint}),
+            acq.handles, acq.ydim, length(acq.posts), S, M, 60, 8, cptr(aff), f.kind, f.c0, f.c, f.q, f.t, acq.eps,
+            size(acq.eps, 2), cptr(best), cptr(acq.y_max), acq.lb, acq.ub, mask, C_NULL, C_NULL, bx, bv, bi, ev))
+    end
     bv[] == -Inf && error("All optimization runs failed!")        # optim_multistart.jl:34
     return bx, bv[]
 end

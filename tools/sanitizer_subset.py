@@ -6,7 +6,7 @@
 
 Families: build_k, potrf_tile (+ fused diagonal step), chol_trsm, chol_update, chol_panel, chol_update_rl, trtri_*_rl,
 trtri_fused, kinv_wtw, loglik_grad_tile, loglik_small (warp path), matvec, xcov, score_trmm (plain and row-split),
-wtv, grad, acq (+ MC-EI), argmax, cov (gemm_nt + cov_finish), candidate generators, append (+ capacity growth),
+wtv, grad (+ MC-EI gradient), acq (+ MC-EI), argmax, top-k, cov (gemm_nt + cov_finish), candidate generators, append (+ capacity growth),
 multi-start driver.  Results are checked against the oracle so that a run that "passes" the sanitizer by computing
 nothing is caught.  Prints one JSON line.
 """
@@ -74,6 +74,25 @@ def main():
     r_mc = O.mc_ei_acquisition([posts], Xs[:, :256], f, eps, best, y_max)
     assert np.max(np.abs(a_mc - r_mc)) <= 1e-9 * np.max(np.abs(r_mc))
     done.append("mcei")
+    # --- MC-EI value + gradient, its multi-start driver and top-k (acq_grad_kernel<true>) ---
+    from tests import mcei_grad_oracle as MO
+    mc_kw = dict(c=coefs, q=np.array([0.0, -0.3]), t=np.zeros(2))
+    best_mc = float(np.median([f(Y[:, j]) for j in range(n)]))      # most candidates improve on it: a non-trivial gradient
+    a_mg, g_mg = _lib.mcei_value_grad(gps, 2, 1, Xs[:, :200], 2, eps, best_mc, y_max, **mc_kw)
+    a_mr, g_mr = MO.mc_ei_value_grad([posts], Xs[:, :200], 2, 0.0, coefs, mc_kw["q"], mc_kw["t"], eps, best_mc, y_max)
+    g_scale = np.max(np.abs(g_mr), axis=1, keepdims=True)
+    assert np.all(g_scale > 0)
+    assert np.max(np.abs(a_mg - a_mr)) <= 1e-9 * np.max(np.abs(a_mr))
+    assert np.max(np.abs(g_mg - g_mr) / g_scale) <= 1e-7
+    ms_starts = rng.random((d, 64))
+    _, fo_mc, _, _, _, _ = _lib.mcei_maximize_multistart(gps, 2, 1, ms_starts, 2, eps, best_mc, y_max, lb, ub, iters=4,
+                                                         **mc_kw)
+    f0_mc, _, _ = _lib.mcei_score(gps, 2, 1, ms_starts, 2, eps, best_mc, y_max, lb=lb, ub=ub, **mc_kw)
+    assert np.all(fo_mc >= f0_mc - 1e-15) and np.max(fo_mc) > 0
+    a_tk, _, _ = _lib.mcei_score(gps, 2, 1, Xs[:, :256], 2, eps, best_mc, y_max, **mc_kw)
+    tv_mc, ti_mc = _lib.mcei_score_topk(gps, 2, 1, Xs[:, :256], 2, eps, best_mc, y_max, 10, **mc_kw)
+    assert np.array_equal(ti_mc, np.argsort(-a_tk, kind="stable")[:10]) and np.array_equal(tv_mc, a_tk[ti_mc])
+    done.append("mcei_grad+multistart+topk")
     # --- full covariance ---
     mu_c, cov, _ = _lib.gp_cov(gps[0], Xs[:, :40])
     cref, _ = O.posterior_cov(posts[0], Xs[:, :40])
