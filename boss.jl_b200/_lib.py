@@ -92,6 +92,9 @@ EXPORTS = {
     "boss_dbg_check_redzones": (C.c_int64, [_i64p]),
     "boss_dbg_redzone_selftest": (C.c_int64, []),
     "boss_dbg_screen_stats": (C.c_int, [_i64p]),
+    "boss_dbg_screen_ambiguous": (C.c_int, [_i64p]),
+    "boss_dbg_screen_mean": (C.c_int, [_vp, _vp, C.c_int64, _vp, _vp, _vp]),
+    "boss_dbg_kappa_f32": (C.c_int, [C.c_int, _vp, C.c_int, _vp]),
 }
 for _name, (_res, _args) in EXPORTS.items():
     _f = getattr(lib, _name)          # AttributeError here = header and library disagree
@@ -674,3 +677,29 @@ def dbg_screen_stats():
     out = (C.c_int64 * 3)()
     _check(lib.boss_dbg_screen_stats(out), "boss_dbg_screen_stats")
     return int(out[0]), int(out[1]), int(out[2])
+
+
+def dbg_screen_ambiguous():
+    """The FP32 mean tier of the last screened call: (candidates in the ambiguous band, pool as the chunks left it --
+    definite keeps plus ambiguous candidates -- before the FP64 refinement and the re-seed)."""
+    out = (C.c_int64 * 2)()
+    _check(lib.boss_dbg_screen_ambiguous(out), "boss_dbg_screen_ambiguous")
+    return int(out[0]), int(out[1])
+
+
+def dbg_screen_mean(gp: GP, Xs):
+    """(mu~, E, mu64) of the candidates Xs (d x M) under gp: the FP32 tier's mean and error bound, and the FP64 mean
+    (K*^T alpha, no prior mean)."""
+    Xc = _cols(Xs)
+    M = Xc.shape[0]
+    mu32, E, mu64 = np.empty(M), np.empty(M), np.empty(M)
+    _check(lib.boss_dbg_screen_mean(gp.handle, _ptr(Xc), M, _ptr(mu32), _ptr(E), _ptr(mu64)), "boss_dbg_screen_mean")
+    return mu32, E, mu64
+
+
+def dbg_kappa_f32(kid, r):
+    """The FP32 tier's kappa at d2 = float32(r^2) (kid 0 SE, 1 Matern32, 2 Matern52)."""
+    r = _f64(r)
+    out = np.empty_like(r)
+    _check(lib.boss_dbg_kappa_f32(int(kid), _ptr(r), r.size, _ptr(out)), "boss_dbg_kappa_f32")
+    return out

@@ -136,8 +136,10 @@ struct Ctx {
   DevBuf blk_val, blk_idx, small, chol_L, chol_Winv, chol_misc, tt, vt, ut, dmu, dvar;
   DevBuf part_mu, part_ss, part_gm, part_gv, cov_p, cov_stage, chol_W, chol_WT, ll_vec, ll_part, ms_buf;   // split-invariant partial sums (score.cuh / grad.cuh)
   DevBuf scr_misc, scr_pool;         // argmax screening: bounds, counts, seed batch / survivor pool (Screen)
+  DevBuf scr_pool2;                  // argmax screening: the pool re-compacted after refinement and re-seed
   DevBuf topk;                       // top-k calls: running set, chunk scores, selection state, sorted result
   int64_t scr_stats[3] = {0, 0, 0};  // last scoring call: screened (1) or fell back (2), candidates bounded, pool size
+  int64_t scr_amb[2] = {0, 0};       // last screened call: ambiguous candidates of the FP32 tier, pool before refinement and re-seed
   // event pool for per-kernel-class timing
   cudaEvent_t ev_a[EV_POOL], ev_b[EV_POOL];
   int ev_class[EV_POOL];
@@ -1717,21 +1719,33 @@ long long screen_min_m() {
 struct Screen {
   enum State { OFF, SCREENING, FELL_BACK } state = OFF;   // scr_stats[0]: 1 once a screened call finished, 2 fell back
   double thr = -INFINITY;   // survivors: bound >= thr or NaN
-  // device buffers: the bounds of one chunk, per-256 survivor counts, the pool size (two slots), the seed selection
-  // (two ping-pong rounds), the seed batch and the survivor pool
-  double *bound = nullptr, *seed_x = nullptr, *seed_pm = nullptr, *pool_x = nullptr, *pool_pm = nullptr;
-  int *cnt = nullptr, *ti[2] = {};
+  double T = 0.0;           // the seed batch's best (argmax) or k-th best (top-k) score
+  // FP32 mean tier from the second chunk on (BOSS_SCREEN_F64=1: the FP64 tier throughout); the threshold re-seeded
+  // from the whole pool before it is scored (BOSS_SCREEN_NO_RESEED=1: not)
+  bool f32 = false, reseed = false;
+  long long n0 = 0, n_amb = 0;   // pool rows of the first chunk; ambiguous candidates of the call
+  // device buffers: the bounds of one chunk (hi in the FP32 tier) and lo, per-256 survivor counts, the pool sizes (two
+  // slots for the chunks, two for the re-compaction), the seed selection (two ping-pong rounds), the seed batch, the
+  // refinement batch, the survivor pool with each row's bound and verdict, and the re-compacted pool
+  double *bound = nullptr, *lo = nullptr, *seed_x = nullptr, *seed_pm = nullptr, *pool_x = nullptr, *pool_pm = nullptr;
+  double *pool_bound = nullptr, *ref_x = nullptr, *ref_pm = nullptr, *consts = nullptr;
+  int *cnt = nullptr, *ti[2] = {}, *ref_row = nullptr, *ref_cnt = nullptr;
   unsigned long long *tk[2] = {};
   long long *base = nullptr, *pool_idx = nullptr;
-  unsigned char *seed_cm = nullptr, *pool_cm = nullptr;
+  unsigned char *seed_cm = nullptr, *pool_cm = nullptr, *pool_ver = nullptr;
+  std::vector<float *> xt32, al32;   // per slice: FP32 copies of the scaled training inputs (negated) and of alpha
 
   bool on() const { return state == SCREENING; }
 
+  // bytes of one pool row: candidate, index, bound, verdict, prior means, constraint-mask entry
+  static size_t pool_row(const ScoreArgs &a, int d) {
+    return (size_t)d * 8 + 8 + 8 + 1 + (a.prior_mean ? (size_t)a.y_dim * 8 : 0) + (a.cons_mask ? 1 : 0);
+  }
+
   // ch0: the first chunk, which the seed batch is drawn from
   static bool eligible(const ScoreArgs &a, int ch0, int d) {
-    const size_t pool_row = (size_t)d * 8 + (a.prior_mean ? (size_t)a.y_dim * 8 : 0) + 8 + (a.cons_mask ? 1 : 0);
     return (a.want_argmax || a.topk) && a.best && !a.internal && !a.acq && !a.grad && !a.mu_out && !a.var_out &&
-           !a.status_out && !a.mix && a.M >= screen_min_m() && (size_t)a.M * pool_row <= SCREEN_POOL_BYTES &&
+           !a.status_out && !a.mix && a.M >= screen_min_m() && (size_t)a.M * pool_row(a, d) <= SCREEN_POOL_BYTES &&
            a.topk <= ch0 && getenv("BOSS_NO_SCREEN") == nullptr;
   }
 
@@ -1740,14 +1754,25 @@ struct Screen {
     const long long M = a.M;
     const int CH = c.CH, d = c.d, y_dim = a.y_dim, ns_max = a.topk ? topk_seed_n(a.topk, ch0) : SEED_N;
     const bool pm = a.prior_mean != nullptr, cm = a.cons_mask != nullptr;
+    f32 = getenv("BOSS_SCREEN_F64") == nullptr;
+    reseed = getenv("BOSS_SCREEN_NO_RESEED") == nullptr;
     size_t tot = 0;
     const size_t ntk = (size_t)(CH + TOPK_IN - 1) / TOPK_IN * SEED_N;
-    const size_t o_bound = take(tot, (size_t)CH * 8), o_cnt = take(tot, (size_t)(CH + 255) / 256 * 4), o_base = take(tot, 16);
+    const size_t o_bound = take(tot, (size_t)CH * 8), o_lo = take(tot, (size_t)CH * 8);
+    const size_t o_cnt = take(tot, (size_t)(CH + 255) / 256 * 4), o_base = take(tot, 32);
     const size_t o_tk0 = take(tot, ntk * 8), o_tk1 = take(tot, ntk * 8), o_ti0 = take(tot, ntk * 4), o_ti1 = take(tot, ntk * 4);
     const size_t o_sx = take(tot, (size_t)ns_max * d * 8), o_spm = take(tot, (size_t)ns_max * y_dim * 8), o_scm = take(tot, ns_max);
+    const size_t o_rx = take(tot, (size_t)CH * d * 8), o_rpm = take(tot, pm ? (size_t)CH * y_dim * 8 : 0);
+    const size_t o_rrow = take(tot, (size_t)CH * 4), o_rcnt = take(tot, 8), o_consts = take(tot, (size_t)c.nsl * 16);
+    std::vector<size_t> o_xt(c.nsl), o_al(c.nsl);
+    for (int q = 0; q < c.nsl; ++q) {
+      o_xt[q] = take(tot, f32 ? (size_t)c.sl[q]->n_pad * c.sl[q]->dp * 4 : 0);
+      o_al[q] = take(tot, f32 ? (size_t)c.sl[q]->n_pad * 4 : 0);
+    }
     CUDA_TRY(C().scr_misc.ensure(tot));
     unsigned char *b = C().scr_misc.as<unsigned char>();
     bound = reinterpret_cast<double *>(b + o_bound);
+    lo = reinterpret_cast<double *>(b + o_lo);
     cnt = reinterpret_cast<int *>(b + o_cnt);
     base = reinterpret_cast<long long *>(b + o_base);
     tk[0] = reinterpret_cast<unsigned long long *>(b + o_tk0);
@@ -1757,16 +1782,33 @@ struct Screen {
     seed_x = reinterpret_cast<double *>(b + o_sx);
     seed_pm = reinterpret_cast<double *>(b + o_spm);
     seed_cm = b + o_scm;
+    ref_x = reinterpret_cast<double *>(b + o_rx);
+    ref_pm = pm ? reinterpret_cast<double *>(b + o_rpm) : nullptr;
+    ref_row = reinterpret_cast<int *>(b + o_rrow);
+    ref_cnt = reinterpret_cast<int *>(b + o_rcnt);
+    consts = reinterpret_cast<double *>(b + o_consts);
+    xt32.assign(c.nsl, nullptr);
+    al32.assign(c.nsl, nullptr);
+    for (int q = 0; q < c.nsl && f32; ++q) {   // per call, so that an appended point or a refit is never missed
+      const boss_gp *h = c.sl[q];
+      xt32[q] = reinterpret_cast<float *>(b + o_xt[q]);
+      al32[q] = reinterpret_cast<float *>(b + o_al[q]);
+      screen_consts_kernel<<<1, 1024, 0, C().stream>>>(h->Xt, h->alpha, h->n_pad, h->dp, xt32[q], al32[q], consts + 2 * q);
+      ++C().launches;
+    }
     tot = 0;
     const size_t o_px = take(tot, (size_t)M * d * 8), o_pidx = take(tot, (size_t)M * 8);
+    const size_t o_pb = take(tot, (size_t)M * 8), o_pv = take(tot, (size_t)M);
     const size_t o_ppm = pm ? take(tot, (size_t)M * y_dim * 8) : 0, o_pcm = cm ? take(tot, (size_t)M) : 0;
     CUDA_TRY(C().scr_pool.ensure(tot));
     b = C().scr_pool.as<unsigned char>();
     pool_x = reinterpret_cast<double *>(b + o_px);
     pool_idx = reinterpret_cast<long long *>(b + o_pidx);
+    pool_bound = reinterpret_cast<double *>(b + o_pb);
+    pool_ver = b + o_pv;
     pool_pm = pm ? reinterpret_cast<double *>(b + o_ppm) : nullptr;
     pool_cm = cm ? b + o_pcm : nullptr;
-    CUDA_TRY(cudaMemsetAsync(base, 0, 16, C().stream));
+    CUDA_TRY(cudaMemsetAsync(base, 0, 32, C().stream));
     state = SCREENING;
     return 0;
   }
@@ -1774,18 +1816,25 @@ struct Screen {
   // One chunk: the means of every slice (xcov without K*^T), the bounds, the survivors appended to the pool.  The first
   // chunk also sets the threshold from the seed batch and ends screening (the chunk is then scored on the full path
   // from the same staged inputs) when the bound does not separate: T not positive, or more than a quarter of the chunk
-  // surviving.
+  // surviving.  The first chunk takes the FP64 means, so the seed batch, T and that decision are those of the FP64
+  // tier; later chunks of the FP32 tier bound EI from mu~ +- E' and leave the ambiguous ones to Screen::finish.
   int chunk(const ScoreCall &c, const AcqParams &ap, const ChunkIO &io, int cidx, TopkBufs &tb) {
     const ScoreArgs &a = c.a;
     const long long m0 = ap.m0;
     const int ch = ap.chunk, ncb = (ch + 127) / 128, nb = (ch + 255) / 256;
+    const bool t32 = f32 && cidx > 0;
     for (int q = 0; q < c.nsl; ++q) {
       const boss_gp *h = c.sl[q];
       const int nks = std::max(1, std::min(h->nblk, (16 * 148 + ncb - 1) / ncb));
+      const XcovParams xp = xcov_params(h, io.xs, a.M, m0, io.off, c.d, c.CH);
       {
         Timed t(1);
-        launch_xcov_mean(h->kernel_id, h->dp, xcov_params(h, io.xs, a.M, m0, io.off, c.d, c.CH), dim3(ncb, nks),
-                         C().stream);
+        if (t32)
+          launch_xcov_mean_f32(h->kernel_id, h->dp, XcovF32Params{xp, xt32[q], al32[q], consts + 2 * q,
+                                                                  C().sumsq.as<double>() + (size_t)q * c.CH},
+                               dim3(ncb, nks), C().stream);
+        else
+          launch_xcov_mean(h->kernel_id, h->dp, xp, dim3(ncb, nks), C().stream);
       }
       reduce_rows_kernel<<<(ncb * 128 + 255) / 256, 256, 0, C().stream>>>(C().part_mu.as<double>(), 2 * h->nblk, (size_t)c.CH,
                                                                         C().muv.as<double>() + (size_t)q * c.CH, ncb * 128);
@@ -1799,6 +1848,15 @@ struct Screen {
     bp.out_off = m0;
     bp.blk_val = nullptr;
     bp.blk_idx = nullptr;
+    if (t32) {   // muv <- mu~ + E', sumsq <- mu~ - E'; bound = EI at the first (hi), lo = EI at the second
+      BandParams bd{C().muv.as<double>(), C().sumsq.as<double>(), c.nsl, a.y_dim, c.CH, ch, {}};
+      for (int i = 0; i < a.y_dim; ++i) bd.coefs[i] = ap.coefs[i];
+      screen_band_kernel<<<nb, 256, 0, C().stream>>>(bd);
+      acq_kernel<<<nb, 256, 0, C().stream>>>(bp);
+      bp.mu = C().sumsq.as<double>();
+      bp.acq = lo;
+      C().launches += 2;
+    }
     acq_kernel<<<nb, 256, 0, C().stream>>>(bp);
     C().launches += 2 * c.nsl + 1;
     const size_t c0 = (size_t)(m0 - ap.in_off);   // the chunk's first candidate in the input arrays
@@ -1809,9 +1867,11 @@ struct Screen {
       int rc = seed(c, ch, xs_c, pm_c, cm_c, tb);
       if (rc || !on()) return rc;
     }
-    screen_count_kernel<<<nb, 256, 0, C().stream>>>(bound, ch, thr, cnt);
-    CompactParams cpar{bound, ch, thr, cnt, m0, xs_c, pm_c, cm_c, c.d, a.y_dim, base, cidx & 1,
-                       pool_x, pool_pm, pool_cm, pool_idx};
+    // FP32 tier: hi < thr (1 - 2^-32) drops, lo >= thr (1 + 2^-32) keeps, anything else (NaN too) is ambiguous
+    const double thr_drop = t32 ? thr * (1.0 - 0x1p-32) : thr;
+    screen_count_kernel<<<nb, 256, 0, C().stream>>>(bound, nullptr, ch, thr_drop, cnt);
+    CompactParams cpar{bound, nullptr, ch, thr_drop, t32 ? lo : nullptr, thr * (1.0 + 0x1p-32), cnt, m0, xs_c, pm_c, cm_c,
+                       c.d, a.y_dim, base, cidx & 1, pool_x, pool_pm, pool_cm, pool_idx, nullptr, pool_bound, pool_ver};
     screen_compact_kernel<<<nb, 256, 0, C().stream>>>(cpar);
     C().launches += 2;
     if (cidx == 0) {
@@ -1819,13 +1879,15 @@ struct Screen {
       CUDA_TRY(cudaMemcpyAsync(&surv, base + 1, 8, cudaMemcpyDeviceToHost, C().stream));
       CUDA_TRY(cudaStreamSynchronize(C().stream));
       C().scr_stats[2] = surv;
+      n0 = surv;
       if (4 * surv > ch) fall_back();
     }
     return 0;
   }
 
-  // After the last chunk: the pool (survivors in ascending order) through the ordinary path; its first-maximal winner
-  // (or its k best) map back to the call's indices.
+  // After the last chunk: the ambiguous rows refined in FP64, the threshold re-seeded from the pool's highest bounds,
+  // the pool re-compacted; then the pool (survivors in ascending order) through the ordinary path, its first-maximal
+  // winner (or its k best) mapped back to the call's indices.
   int finish(const ScoreCall &c, int nchunks, HostStaging &stg) {
     ScoreArgs &a = c.a;
     long long npool = 0;
@@ -1835,17 +1897,43 @@ struct Screen {
     if (rc) return rc;
     C().scr_stats[0] = 1;
     C().scr_stats[1] = a.M;
-    C().scr_stats[2] = npool;
-    if (npool < 1) return fail(BOSS_ERR_STATE, "score: argmax screening kept no candidate");   // the seed's winner always survives
-    if (npool < a.topk) return fail(BOSS_ERR_STATE, "score: top-k screening kept fewer than k candidates");   // the seed's k best survive
+    n_amb = 0;
+    for (long long r0 = n0; f32 && r0 < npool; r0 += c.CH) {
+      rc = refine(c, r0, (int)std::min<long long>(c.CH, npool - r0));
+      if (rc) return rc;
+    }
+    const double *px = pool_x, *ppm = pool_pm;
+    const unsigned char *pcm = pool_cm;
+    const long long *pidx = pool_idx;
+    long long nfin = npool;
+    double thr2 = thr;
+    const int ns_max = a.topk ? topk_seed_n(a.topk, (int)std::min<long long>(c.CH, a.M)) : SEED_N;
+    if (reseed && npool > ns_max) {
+      rc = reseed_thr(c, (int)std::min<long long>(npool, c.CH), thr2);
+      if (rc) return rc;
+    }
+    if (n_amb > 0 || thr2 > thr) {   // keep rows with verdict 1 and bound >= thr2 (or NaN), in order
+      rc = recompact(c, npool, thr2, nfin);
+      if (rc) return rc;
+      unsigned char *b = C().scr_pool2.as<unsigned char>();
+      px = reinterpret_cast<double *>(b);
+      pidx = reinterpret_cast<long long *>(b + p2_off[0]);
+      ppm = pool_pm ? reinterpret_cast<double *>(b + p2_off[1]) : nullptr;
+      pcm = pool_cm ? b + p2_off[2] : nullptr;
+    }
+    C().scr_stats[2] = nfin;
+    C().scr_amb[0] = n_amb;
+    C().scr_amb[1] = npool;
+    if (nfin < 1) return fail(BOSS_ERR_STATE, "score: argmax screening kept no candidate");   // the seed's winner always survives
+    if (nfin < a.topk) return fail(BOSS_ERR_STATE, "score: top-k screening kept fewer than k candidates");   // the seed's k best survive
     SubsetResult r;
-    rc = score_subset(c, pool_x, pool_pm, pool_cm, npool, a.top_val, a.top_idx, pool_idx, false, r);
+    rc = score_subset(c, px, ppm, pcm, nfin, a.top_val, a.top_idx, pidx, false, r);
     if (rc) return rc;
     a.any_fail = r.any_fail;
     if (a.topk) return 0;
     long long idx = -1;
     if (r.best_idx >= 0) {
-      CUDA_TRY(cudaMemcpyAsync(&idx, pool_idx + r.best_idx, 8, cudaMemcpyDeviceToHost, C().stream));
+      CUDA_TRY(cudaMemcpyAsync(&idx, pidx + r.best_idx, 8, cudaMemcpyDeviceToHost, C().stream));
       CUDA_TRY(cudaStreamSynchronize(C().stream));
     }
     if (a.best_val) *a.best_val = r.best_val;
@@ -1854,6 +1942,8 @@ struct Screen {
   }
 
  private:
+  size_t p2_off[3] = {0, 0, 0};   // re-compacted pool: offsets of the indices, prior means, mask entries
+
   void fall_back() {
     C().scr_stats[0] = 2;
     state = FELL_BACK;
@@ -1862,45 +1952,143 @@ struct Screen {
   // The seed batch of the first chunk: the exact scores of its highest bounds.  Their best (argmax) or k-th best
   // (top-k) score T is a lower bound of the call's best or k-th best score; bounds below T (1 - 2^-30) cannot reach it.
   int seed(const ScoreCall &c, int ch, const double *xs_c, const double *pm_c, const unsigned char *cm_c, TopkBufs &tb) {
+    double Ts;
+    int rc = score_seed(c, ch, bound, xs_c, pm_c, cm_c, tb, Ts);
+    if (rc) return rc;
+    C().scr_stats[1] = ch;
+    if (!(Ts >= SCREEN_MIN_T)) {
+      fall_back();
+      return 0;
+    }
+    T = Ts;
+    thr = T * (1.0 - 0x1p-30);
+    return 0;
+  }
+
+  // the exact scores of the highest of the n bounds b (candidate i at xs + i d, pm + i y_dim, cm + i): their best
+  // (argmax) or k-th best (top-k) score
+  int score_seed(const ScoreCall &c, int n, const double *b, const double *xs, const double *pm, const unsigned char *cm,
+                 TopkBufs &tb, double &Ts) {
     const ScoreArgs &a = c.a;
     int ns;
     if (a.topk) {   // the S_k highest bounds (NaN bounds last), selected into the top-k buffers
-      ns = topk_seed_n(a.topk, ch);
-      SelectIn in{nullptr, nullptr, 0, bound, 0, ch, 1};
+      ns = topk_seed_n(a.topk, n);
+      SelectIn in{nullptr, nullptr, 0, b, 0, n, 1};
       int rc = tb.select(in, ns, tb.run_val[0], tb.run_idx[0]);
       if (rc) return rc;
-      seed_gather_kernel<<<(ns + 255) / 256, 256, 0, C().stream>>>(tb.run_idx[0], ns, xs_c, pm_c, cm_c, c.d, a.y_dim,
+      seed_gather_kernel<<<(ns + 255) / 256, 256, 0, C().stream>>>(tb.run_idx[0], ns, xs, pm, cm, c.d, a.y_dim,
                                                                     seed_x, seed_pm, seed_cm);
     } else {        // the SEED_N highest bounds: bitonic rounds over TOPK_IN-element blocks
-      int n = ch, par = 0;
+      int m = n, par = 0;
       const unsigned long long *kin = nullptr;
       const int *iin = nullptr;
       do {
-        const int nbk = (n + TOPK_IN - 1) / TOPK_IN;
-        seed_topk_kernel<<<nbk, 1024, 0, C().stream>>>(kin ? nullptr : bound, kin, iin, n, tk[par], ti[par]);
+        const int nbk = (m + TOPK_IN - 1) / TOPK_IN;
+        seed_topk_kernel<<<nbk, 1024, 0, C().stream>>>(kin ? nullptr : b, kin, iin, m, tk[par], ti[par]);
         ++C().launches;
         kin = tk[par];
         iin = ti[par];
         par ^= 1;
-        n = nbk * SEED_N;
-      } while (n > SEED_N);
-      ns = std::min(SEED_N, ch);
-      seed_gather_kernel<<<1, SEED_N, 0, C().stream>>>(iin, ns, xs_c, pm_c, cm_c, c.d, a.y_dim, seed_x, seed_pm, seed_cm);
+        m = nbk * SEED_N;
+      } while (m > SEED_N);
+      ns = std::min(SEED_N, n);
+      seed_gather_kernel<<<1, SEED_N, 0, C().stream>>>(iin, ns, xs, pm, cm, c.d, a.y_dim, seed_x, seed_pm, seed_cm);
     }
     ++C().launches;
     std::vector<double> sv((size_t)a.topk);
     std::vector<int64_t> si((size_t)a.topk);
     SubsetResult r;
-    int rc = score_subset(c, seed_x, pm_c ? seed_pm : nullptr, cm_c ? seed_cm : nullptr, ns, sv.data(), si.data(),
-                          nullptr, true, r);
+    int rc = score_subset(c, seed_x, pm ? seed_pm : nullptr, cm ? seed_cm : nullptr, ns, sv.data(), si.data(), nullptr,
+                          true, r);
     if (rc) return rc;
-    C().scr_stats[1] = ch;
-    const double T = a.topk ? sv[(size_t)a.topk - 1] : r.best_val;
-    if (!(T >= SCREEN_MIN_T)) {
-      fall_back();
-      return 0;
+    Ts = a.topk ? sv[(size_t)a.topk - 1] : r.best_val;
+    return 0;
+  }
+
+  // Pool rows [r0, r0 + n) (n <= CH): the ambiguous ones gathered, their FP64 means and bounds (xcov_kernel<.., false>,
+  // reduce_rows and the bound of the FP64 tier, so bit for bit the bound that tier computes), today's rule as verdict.
+  int refine(const ScoreCall &c, long long r0, int n) {
+    const ScoreArgs &a = c.a;
+    CUDA_TRY(cudaMemsetAsync(ref_cnt, 0, 4, C().stream));
+    screen_amb_gather_kernel<<<(n + 255) / 256, 256, 0, C().stream>>>(
+        pool_ver + r0, n, pool_x + (size_t)r0 * c.d, pool_pm ? pool_pm + (size_t)r0 * a.y_dim : nullptr, c.d, a.y_dim,
+        (int)r0, ref_x, ref_pm, ref_row, ref_cnt);
+    int namb = 0;
+    CUDA_TRY(cudaMemcpyAsync(&namb, ref_cnt, 4, cudaMemcpyDeviceToHost, C().stream));
+    CUDA_TRY(cudaStreamSynchronize(C().stream));
+    C().launches += 1;
+    n_amb += namb;
+    if (namb == 0) return 0;
+    const int ncb = (namb + 127) / 128, nb = (namb + 255) / 256;
+    for (int q = 0; q < c.nsl; ++q) {
+      const boss_gp *h = c.sl[q];
+      const int nks = std::max(1, std::min(h->nblk, (16 * 148 + ncb - 1) / ncb));
+      launch_xcov_mean(h->kernel_id, h->dp, xcov_params(h, ref_x, namb, 0, 0, c.d, c.CH), dim3(ncb, nks), C().stream);
+      reduce_rows_kernel<<<(ncb * 128 + 255) / 256, 256, 0, C().stream>>>(C().part_mu.as<double>(), 2 * h->nblk, (size_t)c.CH,
+                                                                        C().muv.as<double>() + (size_t)q * c.CH, ncb * 128);
     }
-    thr = T * (1.0 - 0x1p-30);
+    ChunkIO io;
+    io.xs = ref_x;
+    io.pm = ref_pm;
+    AcqParams bp = c.acq_params(0, namb, io);
+    bp.M = namb;
+    bp.sumsq = nullptr;
+    bp.has_ymax = 0;
+    bp.lb = bp.ub = nullptr;
+    bp.cons_mask = nullptr;
+    bp.acq = bound;
+    bp.out_off = 0;
+    bp.blk_val = nullptr;
+    bp.blk_idx = nullptr;
+    acq_kernel<<<nb, 256, 0, C().stream>>>(bp);
+    screen_amb_scatter_kernel<<<nb, 256, 0, C().stream>>>(bound, ref_row, namb, thr, pool_bound, pool_ver);
+    C().launches += 2 * c.nsl + 2;
+    return 0;
+  }
+
+  // Re-seed (DESIGN.md 2.9): the exact scores of the highest bounds among the first n pool rows still kept.  Any set of
+  // real candidates gives a valid threshold; the pool's highest bounds give one close to the call's best score.
+  int reseed_thr(const ScoreCall &c, int n, double &thr2) {
+    screen_sel_bound_kernel<<<(n + 255) / 256, 256, 0, C().stream>>>(pool_bound, pool_ver, n, bound);
+    ++C().launches;
+    TopkBufs tb;
+    if (c.a.topk) {
+      int rc = tb.setup(c.a.topk, c.CH, (int)std::min<long long>(c.CH, c.a.M));
+      if (rc) return rc;
+    }
+    double Ts;
+    int rc = score_seed(c, n, bound, pool_x, pool_pm, pool_cm, tb, Ts);
+    if (rc) return rc;
+    if (Ts > T) thr2 = Ts * (1.0 - 0x1p-30);
+    return 0;
+  }
+
+  // pool rows with verdict 1 and bound >= thr2 (or NaN), in order, into the second pool buffer; their count -> nfin
+  int recompact(const ScoreCall &c, long long npool, double thr2, long long &nfin) {
+    const ScoreArgs &a = c.a;
+    size_t tot = 0;
+    const size_t o_x = take(tot, (size_t)npool * c.d * 8);
+    p2_off[0] = take(tot, (size_t)npool * 8);
+    p2_off[1] = take(tot, pool_pm ? (size_t)npool * a.y_dim * 8 : 0);
+    p2_off[2] = take(tot, pool_cm ? (size_t)npool : 0);
+    (void)o_x;
+    CUDA_TRY(C().scr_pool2.ensure(tot));
+    unsigned char *b = C().scr_pool2.as<unsigned char>();
+    int par = 0;
+    for (long long r0 = 0; r0 < npool; r0 += c.CH, par ^= 1) {
+      const int n = (int)std::min<long long>(c.CH, npool - r0), nb = (n + 255) / 256;
+      screen_count_kernel<<<nb, 256, 0, C().stream>>>(pool_bound + r0, pool_ver + r0, n, thr2, cnt);
+      CompactParams cp{pool_bound + r0, pool_ver + r0, n, thr2, nullptr, 0.0, cnt, 0,
+                       pool_x + (size_t)r0 * c.d, pool_pm ? pool_pm + (size_t)r0 * a.y_dim : nullptr,
+                       pool_cm ? pool_cm + r0 : nullptr, c.d, a.y_dim, base + 2, par,
+                       reinterpret_cast<double *>(b), pool_pm ? reinterpret_cast<double *>(b + p2_off[1]) : nullptr,
+                       pool_cm ? b + p2_off[2] : nullptr, reinterpret_cast<long long *>(b + p2_off[0]), pool_idx + r0,
+                       nullptr, nullptr};
+      screen_compact_kernel<<<nb, 256, 0, C().stream>>>(cp);
+      C().launches += 2;
+    }
+    CUDA_TRY(cudaMemcpyAsync(&nfin, base + 2 + par, 8, cudaMemcpyDeviceToHost, C().stream));
+    CUDA_TRY(cudaStreamSynchronize(C().stream));
     return 0;
   }
 };
@@ -1920,7 +2108,7 @@ int score_core(ScoreArgs &a) {
   }
   rc = c.setup();
   if (rc) return rc;
-  if (!a.internal) C().scr_stats[0] = C().scr_stats[1] = C().scr_stats[2] = 0;
+  if (!a.internal) C().scr_stats[0] = C().scr_stats[1] = C().scr_stats[2] = C().scr_amb[0] = C().scr_amb[1] = 0;
   const int ch0 = (int)std::min<long long>(c.CH, a.M);   // the first chunk
   Screen scr;
   if (Screen::eligible(a, ch0, c.d)) {
@@ -3309,6 +3497,73 @@ int boss_dbg_factors(const boss_gp *gp, double *L, double *W, double *alpha) {
 int boss_dbg_screen_stats(int64_t *out) {
   REQUIRE_INIT();
   for (int i = 0; i < 3; ++i) out[i] = C().scr_stats[i];
+  return 0;
+}
+
+// The FP32 mean tier of the last screened call (DESIGN.md 2.9): out[0] = candidates in the ambiguous band (refined in
+// FP64), out[1] = the pool as the chunks left it (definite keeps and ambiguous candidates), before refinement and re-seed.
+int boss_dbg_screen_ambiguous(int64_t *out) {
+  REQUIRE_INIT();
+  out[0] = C().scr_amb[0];
+  out[1] = C().scr_amb[1];
+  return 0;
+}
+
+// For M candidates (column-major d x M host array): the FP32 tier's mean mu~ and bound E, and the FP64 tier's mean
+// (K*^T alpha, without a prior mean), computed by the kernels the screen runs.
+int boss_dbg_screen_mean(const boss_gp *gp, const double *Xs, int64_t M, double *mu32, double *E, double *mu64) {
+  if (!gp || M < 1 || M > (1 << 22) || !Xs) return fail(BOSS_ERR_ARG, "boss_dbg_screen_mean: bad argument");
+  REQUIRE_HANDLE_CTX(gp);
+  const int d = gp->d, ld = (int)((M + 127) / 128 * 128), ncb = ld / 128;
+  const int nks = std::max(1, std::min(gp->nblk, (16 * 148 + ncb - 1) / ncb));
+  double *dx = nullptr, *dpart = nullptr, *dout = nullptr, *dA = nullptr;
+  float *dxt = nullptr, *dal = nullptr;
+  CUDA_TRY(cudaMalloc(&dx, (size_t)M * d * 8));
+  CUDA_TRY(cudaMalloc(&dpart, (size_t)2 * gp->nblk * ld * 8));
+  CUDA_TRY(cudaMalloc(&dout, (size_t)3 * ld * 8));
+  CUDA_TRY(cudaMalloc(&dA, 16));
+  CUDA_TRY(cudaMalloc(&dxt, (size_t)gp->n_pad * gp->dp * 4));
+  CUDA_TRY(cudaMalloc(&dal, (size_t)gp->n_pad * 4));
+  CUDA_TRY(cudaMemcpyAsync(dx, Xs, (size_t)M * d * 8, cudaMemcpyHostToDevice, C().stream));
+  screen_consts_kernel<<<1, 1024, 0, C().stream>>>(gp->Xt, gp->alpha, gp->n_pad, gp->dp, dxt, dal, dA);
+  XcovParams xp = xcov_params(gp, dx, M, 0, 0, d, ld);
+  xp.mu_part = dpart;
+  launch_xcov_mean_f32(gp->kernel_id, gp->dp, XcovF32Params{xp, dxt, dal, dA, dout + ld}, dim3(ncb, nks), C().stream);
+  reduce_rows_kernel<<<(ld + 255) / 256, 256, 0, C().stream>>>(dpart, 2 * gp->nblk, (size_t)ld, dout, ld);
+  launch_xcov_mean(gp->kernel_id, gp->dp, xp, dim3(ncb, nks), C().stream);
+  reduce_rows_kernel<<<(ld + 255) / 256, 256, 0, C().stream>>>(dpart, 2 * gp->nblk, (size_t)ld, dout + 2 * ld, ld);
+  CUDA_TRY(cudaGetLastError());
+  std::vector<double> h((size_t)3 * ld);
+  CUDA_TRY(cudaMemcpyAsync(h.data(), dout, h.size() * 8, cudaMemcpyDeviceToHost, C().stream));
+  CUDA_TRY(cudaStreamSynchronize(C().stream));
+  for (int64_t i = 0; i < M; ++i) {
+    if (mu32) mu32[i] = h[i];
+    if (E) E[i] = h[ld + i];
+    if (mu64) mu64[i] = h[2 * (size_t)ld + i];
+  }
+  cudaFree(dx);
+  cudaFree(dpart);
+  cudaFree(dout);
+  cudaFree(dA);
+  cudaFree(dxt);
+  cudaFree(dal);
+  return 0;
+}
+
+// kappa_f32<kid>((float)(r^2)) of the FP32 mean tier for n distances r (kid 0 SE, 1 Matern32, 2 Matern52)
+int boss_dbg_kappa_f32(int kid, const double *r, int n, double *out) {
+  REQUIRE_INIT();
+  if (kid < 0 || kid > 2 || n < 0) return fail(BOSS_ERR_ARG, "boss_dbg_kappa_f32: bad argument");
+  double *dr, *dout;
+  CUDA_TRY(cudaMalloc(&dr, (size_t)n * 8 + 8));
+  CUDA_TRY(cudaMalloc(&dout, (size_t)n * 8 + 8));
+  // on the library stream: a pageable cudaMemcpy may return before its DMA lands, and that stream does not wait for it
+  CUDA_TRY(cudaMemcpyAsync(dr, r, (size_t)n * 8, cudaMemcpyHostToDevice, C().stream));
+  launch_kappa_f32_sweep(kid, dr, n, dout, C().stream);
+  CUDA_TRY(cudaMemcpyAsync(out, dout, (size_t)n * 8, cudaMemcpyDeviceToHost, C().stream));
+  CUDA_TRY(cudaStreamSynchronize(C().stream));
+  cudaFree(dr);
+  cudaFree(dout);
   return 0;
 }
 

@@ -105,6 +105,30 @@ __device__ __forceinline__ double kappa(double d2) {
   }
 }
 
+// FP32 kappa for the FP32 mean tier of argmax screening (DESIGN.md 2.9): one MUFU.RSQ (Matern only) and one MUFU.EX2.
+// r = d2 rsqrt(max(d2, 1e-30)) is 0 at d2 = 0 (|r~ - r| <= 1e-15 below the floor); t >= ~87 flushes exp to 0.
+// Absolute error against kappa at the same d2, measured over r in [0, 40]: tests/test_gpu_screen_f32.py.
+template <int KID>
+__device__ __forceinline__ float kappa_f32(float d2) {
+  float e;
+  if (KID == 0) {
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(d2 * -0.72134752044448170f /* -log2(e)/2 */));
+    return e;
+  }
+  float y;
+  asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(fmaxf(d2, 1e-30f)));
+  const float r = d2 * y;
+  if (KID == 1) {
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(r * -2.4988211106473432f /* -sqrt3 log2(e) */));
+    const float t = 1.7320508075688772f * r;
+    return fmaf(t, e, e);
+  } else {
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(r * -3.2259641822295610f /* -sqrt5 log2(e) */));
+    const float t = 2.2360679774997896f * r;
+    return fmaf(fmaf(1.6666666666666667f, d2, t), e, e);
+  }
+}
+
 // (d kappa / d r) / r as a function of d2 = r^2 : finite at r = 0 for all three kernels.
 template <int KID>
 __device__ __forceinline__ double kappa_dr_over_r(double d2) {

@@ -349,20 +349,110 @@ __global__ void seed_gather_kernel(const I *sel, int ns, const double *xs, const
   if (cm) scm[s] = cm[c];
 }
 
-// a candidate stays unless its bound is below thr = T (1 - 2^-30); a NaN bound stays
-__device__ __forceinline__ bool screen_keep(const double *bound, int c, int ch, double thr) {
-  return c < ch && !(bound[c] < thr);
+// a candidate stays unless its bound is below thr = T (1 - 2^-30); a NaN bound stays.  With a verdict array (the
+// re-compaction of the pool), rows whose verdict is not 1 (dropped by the FP64 refinement) go too.
+__device__ __forceinline__ bool screen_keep(const double *bound, const unsigned char *ver, int c, int ch, double thr) {
+  return c < ch && !(bound[c] < thr) && (!ver || ver[c] == 1);
 }
 
-__global__ void __launch_bounds__(256) screen_count_kernel(const double *bound, int ch, double thr, int *cnt) {
-  const int k = __syncthreads_count(screen_keep(bound, blockIdx.x * 256 + threadIdx.x, ch, thr));
+__global__ void __launch_bounds__(256) screen_count_kernel(const double *bound, const unsigned char *ver, int ch, double thr,
+                                                           int *cnt) {
+  const int k = __syncthreads_count(screen_keep(bound, ver, blockIdx.x * 256 + threadIdx.x, ch, thr));
   if (threadIdx.x == 0) cnt[blockIdx.x] = k;
+}
+
+// ---- the FP32 mean tier (DESIGN.md 2.9) ----
+
+// Per call and slice: the FP32 copies of the scaled training inputs (negated) and of alpha, and the constants of the
+// error bound, A1 = sum_j |alpha_j| and A2 = sum_j |alpha_j| |ut_j|, summed in a fixed order (one CTA of 1024 threads).
+__global__ void __launch_bounds__(1024) screen_consts_kernel(const double *Xt, const double *alpha, int n_pad, int DP,
+                                                             float *xt_neg, float *al, double *A) {
+  __shared__ double s1[1024], s2[1024];
+  const int tid = threadIdx.x;
+  for (int e = tid; e < n_pad * DP; e += 1024) xt_neg[e] = -(float)Xt[e];
+  double a1 = 0.0, a2 = 0.0;
+  for (int j = tid; j < n_pad; j += 1024) {
+    const double aj = fabs(alpha[j]);
+    double n2 = 0.0;
+    for (int i = 0; i < DP; ++i) n2 = fma(Xt[(size_t)j * DP + i], Xt[(size_t)j * DP + i], n2);
+    al[j] = (float)alpha[j];
+    a1 += aj;
+    a2 = fma(aj, sqrt(n2), a2);
+  }
+  s1[tid] = a1;
+  s2[tid] = a2;
+  __syncthreads();
+  for (int o = 512; o > 0; o >>= 1) {
+    if (tid < o) {
+      s1[tid] += s1[tid + o];
+      s2[tid] += s2[tid + o];
+    }
+    __syncthreads();
+  }
+  if (tid == 0) {
+    A[0] = s1[0];
+    A[1] = s2[0];
+  }
+}
+
+// mu (mu~ of each slice) and e (its bound E) become mu~ + E' and mu~ - E', E' = E with the sign of the slice's output
+// coefficient, so that EI is at least as large at the first as at the FP64 mean and no larger at the second.  A
+// non-finite mu~ or E gives NaN for both (the candidate is then ambiguous).
+struct BandParams {
+  double *mu, *e;
+  int nsl, y_dim, ld, n;
+  double coefs[MAX_YDIM];
+};
+__global__ void __launch_bounds__(256) screen_band_kernel(BandParams p) {
+  const int c = blockIdx.x * 256 + threadIdx.x;
+  if (c >= p.n) return;
+  for (int q = 0; q < p.nsl; ++q) {
+    const size_t o = (size_t)q * p.ld + c;
+    const double m = p.mu[o], E = p.coefs[q % p.y_dim] < 0.0 ? -p.e[o] : p.e[o];
+    const bool ok = isfinite(m) && isfinite(E);
+    p.mu[o] = ok ? m + E : NAN;
+    p.e[o] = ok ? m - E : NAN;
+  }
+}
+
+// The ambiguous rows (verdict 2) among pool rows [0, n) of a piece: their candidates, prior means and rows, in any order
+// (each gets its own verdict back); the count goes to cnt[0].
+__global__ void __launch_bounds__(256) screen_amb_gather_kernel(const unsigned char *ver, int n, const double *px,
+                                                                const double *ppm, int d, int y_dim, int r0, double *rx,
+                                                                double *rpm, int *rrow, int *cnt) {
+  const int i = blockIdx.x * 256 + threadIdx.x;
+  if (i >= n || ver[i] != 2) return;
+  const int s = atomicAdd(cnt, 1);
+  for (int j = 0; j < d; ++j) rx[(size_t)s * d + j] = px[(size_t)i * d + j];
+  if (ppm)
+    for (int k = 0; k < y_dim; ++k) rpm[(size_t)s * y_dim + k] = ppm[(size_t)i * y_dim + k];
+  rrow[s] = r0 + i;
+}
+
+// today's rule on the FP64 bounds of the gathered rows: verdict 1 (keep) unless bound < thr; the bound goes with it
+__global__ void __launch_bounds__(256) screen_amb_scatter_kernel(const double *b, const int *rrow, int n, double thr,
+                                                                 double *pbound, unsigned char *pver) {
+  const int s = blockIdx.x * 256 + threadIdx.x;
+  if (s >= n) return;
+  const int row = rrow[s];
+  pbound[row] = b[s];
+  pver[row] = !(b[s] < thr) ? 1 : 0;
+}
+
+// the bounds the re-seed selects from: dropped rows count as NaN (lowest)
+__global__ void __launch_bounds__(256) screen_sel_bound_kernel(const double *pbound, const unsigned char *pver, int n,
+                                                               double *out) {
+  const int i = blockIdx.x * 256 + threadIdx.x;
+  if (i < n) out[i] = pver[i] == 1 ? pbound[i] : NAN;
 }
 
 struct CompactParams {
   const double *bound;
+  const unsigned char *ver;      // re-compaction: the rows' verdicts (keep only 1), else null
   int ch;
   double thr;
+  const double *lo;              // FP32 tier: EI at mu~ - E' (survivors with lo >= thr_keep are definite keeps), else null
+  double thr_keep;
   const int *cnt;                // survivors per 256 candidates (screen_count_kernel)
   long long m0;                  // index (within the call) of the chunk's first candidate
   const double *xs, *pm;         // the chunk's first candidate (pm may be null)
@@ -372,7 +462,10 @@ struct CompactParams {
   int par;
   double *px, *ppm;              // pool: candidates, prior means,
   unsigned char *pcm;            //       constraint-mask entries,
-  long long *pidx;               //       index within the call
+  long long *pidx;               //       index within the call (m0 + position, or sidx[position] if sidx is set)
+  const long long *sidx;
+  double *pbound;                //       bounds (or null): hi in the FP32 tier, the FP64 bound otherwise
+  unsigned char *pver;           //       verdicts (or null): 1 keep, 2 ambiguous (refined in Screen::finish)
 };
 
 // ordered compaction: survivors keep their relative order, so the pool's first-maximal argmax is the call's
@@ -390,7 +483,7 @@ __global__ void __launch_bounds__(256) screen_compact_kernel(CompactParams p) {
     }
   }
   const int c = b * 256 + tid;
-  const bool keep = screen_keep(p.bound, c, p.ch, p.thr);
+  const bool keep = screen_keep(p.bound, p.ver, c, p.ch, p.thr);
   const unsigned bal = __ballot_sync(0xffffffffu, keep);
   if (lane == 0) s_warp[w] = __popc(bal);
   __syncthreads();
@@ -401,7 +494,9 @@ __global__ void __launch_bounds__(256) screen_compact_kernel(CompactParams p) {
   if (p.pm)
     for (int i = 0; i < p.y_dim; ++i) p.ppm[o * p.y_dim + i] = p.pm[(size_t)c * p.y_dim + i];
   if (p.cm) p.pcm[o] = p.cm[c];
-  p.pidx[o] = p.m0 + c;
+  p.pidx[o] = p.sidx ? p.sidx[c] : p.m0 + c;
+  if (p.pbound) p.pbound[o] = p.bound[c];
+  if (p.pver) p.pver[o] = (!p.lo || p.lo[c] >= p.thr_keep) ? 1 : 2;
 }
 
 // ---------------------------------------------------------------------------------------------

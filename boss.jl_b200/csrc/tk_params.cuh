@@ -47,6 +47,19 @@ struct XcovParams {
 
 constexpr int XCOV_KC = 128;  // training points staged per shared-memory pass
 
+// The FP32 mean tier of argmax screening (DESIGN.md 2.9): mu~ with a proven bound E on |mu~ - mu|, from an FP32 copy
+// of the training inputs and weights.  x.Xt / x.alpha are unused; x.mu_part receives the partials (FP64, same layout).
+struct XcovF32Params {
+  XcovParams x;
+  const float *Xt_neg;   // [n_pad][DP] -(scaled training inputs), rounded to FP32
+  const float *alpha;    // [n_pad] alpha rounded to FP32
+  const double *A;       // [2] A1 = sum |alpha_j|, A2 = sum |alpha_j| |ut_j|  (screen_consts_kernel)
+  double *E;             // [ld] the error bound of each candidate's mean
+};
+// E = a^2 2^-24 (SCREEN_C_EVAL A1 + SCREEN_L_KAPPA (|u| A1 + A2))   (DESIGN.md 2.9)
+constexpr double SCREEN_C_EVAL = 64.0;
+constexpr double SCREEN_L_KAPPA = 0.65;
+
 struct CovFinishParams {
   const double *Xs;     // d x M raw candidates
   int M, d, ktilesC;    // ktilesC = M_pad / 16
@@ -92,6 +105,8 @@ bool launch_build_k(int kid, int dp, const BuildKParams &p, dim3 grid, cudaStrea
 bool launch_loglik_grad_tile(int kid, int dp, const LlGradParams &p, dim3 grid, cudaStream_t st);
 bool launch_xcov(int kid, int dp, const XcovParams &p, dim3 grid, cudaStream_t st);
 bool launch_xcov_mean(int kid, int dp, const XcovParams &p, dim3 grid, cudaStream_t st);   // mu partials only (p.Ks unused)
+bool launch_xcov_mean_f32(int kid, int dp, const XcovF32Params &p, dim3 grid, cudaStream_t st);
+bool launch_kappa_f32_sweep(int kid, const double *r, int n, double *out, cudaStream_t st);
 bool launch_cov_finish(int kid, int dp, const CovFinishParams &p, dim3 grid, cudaStream_t st);
 bool launch_grad(int kid, int dp, const GradParams &p, dim3 grid, cudaStream_t st);
 bool launch_loglik_small(int kid, int dp, const SmallLoglikParams &p, int nblocks, cudaStream_t st);

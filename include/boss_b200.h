@@ -334,8 +334,18 @@ int boss_dbg_factors(const boss_gp *gp, double *L, double *W, double *alpha);   
 int64_t boss_dbg_check_redzones(int64_t *n_allocs);
 int64_t boss_dbg_redzone_selftest(void);   /* negative control: writes 2 guard bytes on purpose, returns how many the scan found */
 /* argmax / top-k screening of the last scoring call on the current device: out[0] = 0 not screened, 1 screened, 2 fell back
- * to the full path after the first chunk; out[1] = candidates bounded; out[2] = candidates that survived the bound */
+ * to the full path after the first chunk; out[1] = candidates bounded; out[2] = candidates that survived the bound and
+ * the re-seeded threshold (the pool scored exactly) */
 int boss_dbg_screen_stats(int64_t *out);
+/* the FP32 mean tier of the last screened call: out[0] = candidates in the ambiguous band (their means were recomputed in
+ * FP64), out[1] = the pool as the chunks left it (definite keeps plus ambiguous candidates), before the FP64 refinement
+ * and the re-seeded threshold */
+int boss_dbg_screen_ambiguous(int64_t *out);
+/* the FP32 tier's mean mu~ and error bound E, and the FP64 mean, of M candidates (d x M column-major) under gp
+ * (K*^T alpha, no prior mean) */
+int boss_dbg_screen_mean(const boss_gp *gp, const double *Xs, int64_t M, double *mu32, double *E, double *mu64);
+/* the FP32 tier's kappa at d2 = (float)(r^2), kid 0 SE, 1 Matern32, 2 Matern52 */
+int boss_dbg_kappa_f32(int kid, const double *r, int n, double *out);
 
 #ifdef __cplusplus
 }
