@@ -46,6 +46,7 @@ EXPORTS = {
     "boss_gp_d": (C.c_int, [_vp]),
     "boss_gp_predict": (C.c_int, [_vp, _vp, C.c_int64, _vp, _vp, _vp, _vp]),
     "boss_gp_predict_dev": (C.c_int, [_vp, _vp, C.c_int64, _vp, _vp, _vp, _vp, _vp]),
+    "boss_gp_predict_grad": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "boss_gp_cov": (C.c_int, [_vp, _vp, C.c_int64, _vp, _vp, _vp]),
     "boss_ei_score": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                 _dp, _i64p]),
@@ -246,6 +247,28 @@ def gp_predict(gp: GP, Xs, prior_mean_s=None):
     st = np.empty(M, dtype=np.int32)
     _check(lib.boss_gp_predict(gp.handle, _ptr(Xc), M, _ptr(pm), _ptr(mu), _ptr(var), _ptr(st)), "boss_gp_predict")
     return mu, var, st
+
+
+def gp_predict_grad(slices, y_dim, n_samples, Xs, prior_mean_s=None, prior_mean_grad_s=None):
+    """Posterior means, variances and their x-gradients of all P = n_samples * y_dim posteriors in one call
+    (include/boss_b200.h, boss_gp_predict_grad).  slices: flat list, sample-major (slices[s*y_dim+i]);
+    prior_mean_s (y_dim, M) and prior_mean_grad_s (y_dim, d, M) are shared by the samples.
+    -> mu (P, M), var (P, M), dmu (P, d, M), dvar (P, d, M), status (P, M) int32; mu, var and status equal
+    gp_predict's per slice bit for bit."""
+    Xc = _cols(Xs)
+    M, d = Xc.shape
+    assert len(slices) == y_dim * n_samples
+    P = y_dim * n_samples
+    arr = _slice_array(slices)
+    pm = None if prior_mean_s is None else np.ascontiguousarray(np.asarray(prior_mean_s, dtype=np.float64).T)
+    pmg = None if prior_mean_grad_s is None else np.ascontiguousarray(
+        np.transpose(np.asarray(prior_mean_grad_s, dtype=np.float64), (2, 1, 0)))   # (M, d, y_dim)
+    mu = np.empty((M, P)); var = np.empty((M, P))
+    dmu = np.empty((M, d, P)); dvar = np.empty((M, d, P))
+    st = np.empty((M, P), dtype=np.int32)
+    _check(lib.boss_gp_predict_grad(arr, y_dim, n_samples, _ptr(Xc), M, _ptr(pm), _ptr(pmg), _ptr(mu), _ptr(var),
+                                    _ptr(dmu), _ptr(dvar), _ptr(st)), "boss_gp_predict_grad")
+    return mu.T, var.T, np.transpose(dmu, (2, 1, 0)), np.transpose(dvar, (2, 1, 0)), st.T
 
 
 def gp_cov(gp: GP, Xs, prior_mean_s=None):

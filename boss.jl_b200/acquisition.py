@@ -48,6 +48,73 @@ def julia_sortperm_rev(v):
     return np.argsort(~key, kind="stable")
 
 
+def _pof_grad(mu, var, sd, dmu, dvar, y_max):
+    """d PoF / dx for one posterior: PoF = prod_i cdf(Normal(mu_i, sd_i), y_max_i), by the product rule over the outputs;
+    d cdf_i = pdf(z_i) (-d mu_i / sd_i - (y_max_i - mu_i) d var_i / (2 sd_i var_i)), 0 where sd_i == 0 or y_max_i = +Inf.
+    mu, var, sd (y_dim, M); dmu, dvar (y_dim, d, M) -> (d, M)."""
+    ym = np.asarray(y_max, dtype=np.float64)[:, None]
+    cdf = _normal_cdf(mu, sd, ym)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        z = (ym - mu) / sd
+        pdf = np.exp(-0.5 * z * z) * 0.3989422804014327
+        dc = pdf[:, None, :] * (-dmu / sd[:, None, :] - (ym - mu)[:, None, :] * dvar / (2.0 * sd * var)[:, None, :])
+    dc = np.where(((sd > 0.0) & ~np.isposinf(ym))[:, None, :], dc, 0.0)
+    dpof = np.zeros(dmu.shape[1:])
+    for i in range(mu.shape[0]):
+        others = np.prod(np.delete(cdf, i, axis=0), axis=0)
+        dpof += dc[i] * others
+    return dpof
+
+
+def mc_ei_value_grad(mu, var, dmu, dvar, eps, f, g, best, y_max, status=None):
+    """Value and x-gradient of the Monte-Carlo EI (x PoF) of a NonlinFitness closure (expected_improvement.jl:104-111)
+    from the posteriors and their x-gradients, by the chain rule of DESIGN.md 2.11 with g = df/dy taken from the caller:
+      y_k = mu + sd .* eps_k,  imp_k = f(y_k) - best,  EI_s = 1/K sum_k max(0, imp_k)
+      d EI_s = sum_i A_i d mu_i + B_i d sd_i,  A_i = 1/K sum_{imp_k > 0} g_i(y_k),  B_i = 1/K sum_{imp_k > 0} g_i(y_k) eps_ik
+    d sd_i = d var_i / (2 sd_i) where sd_i > 0 (dvar is already 0 where the variance was clipped); a NaN improvement gives
+    a NaN gradient; PoF enters by the product rule; the BI samples are averaged.
+      mu, var (S, y_dim, M); dmu, dvar (S, y_dim, d, M); eps (y_dim, K) (S > 1: posterior s takes column s);
+      f(Y) -> (P,), g(Y) -> (y_dim, P) for Y (y_dim, P); best / y_max None or as Acquisition; status (S, y_dim, M) or None.
+    -> val (M,) (-inf where a status is non-zero; bit for bit Acquisition's value path), grad (d, M) (0 there).
+    No domain guards."""
+    S, y_dim, M = mu.shape
+    d = dmu.shape[2]
+    acc = np.zeros(M)
+    gacc = np.zeros((d, M))
+    failed = np.zeros(M, dtype=bool) if status is None else np.any(np.asarray(status) != 0, axis=(0, 1))
+    for s in range(S):
+        m, v, dm, dv = mu[s], var[s], dmu[s], dvar[s]
+        if best is None and y_max is None:
+            continue
+        with np.errstate(invalid="ignore"):
+            sd = np.sqrt(v)
+        # the value: the expressions of Acquisition._mc_acq, so the bits agree
+        pof = 1.0 if y_max is None else np.prod(_normal_cdf(m, sd, y_max[:, None]), axis=0)
+        dpof = 0.0 if y_max is None else _pof_grad(m, v, sd, dm, dv, y_max)
+        if best is None:
+            acc += pof
+            gacc += dpof
+            continue
+        e = eps if S == 1 else eps[:, s:s + 1]
+        K = e.shape[1]
+        pred = (m[:, :, None] + sd[:, :, None] * e[:, None, :]).reshape(y_dim, M * K)      # y_dim x M x K
+        imp = f(pred).reshape(M, K) - best
+        ei = np.maximum(0.0, imp).sum(axis=1) / K
+        acc += ei * pof
+        pos = (imp > 0.0)[None]
+        G = np.where(pos, np.asarray(g(pred), dtype=np.float64).reshape(y_dim, M, K), 0.0)
+        A = G.sum(axis=2) / K
+        B = (G * e[:, None, :]).sum(axis=2) / K
+        A = np.where(np.isnan(imp).any(axis=1)[None], np.nan, A)
+        with np.errstate(divide="ignore", invalid="ignore"):
+            dsd = np.where(sd[:, None, :] > 0, dv / (2.0 * sd[:, None, :]), 0.0)
+        dei = np.einsum("im,idm->dm", A, dm) + np.einsum("im,idm->dm", B, dsd)
+        gacc += dei if y_max is None else dei * pof + ei * dpof
+    val = np.where(failed, -np.inf, acc / S)
+    grad = np.where(failed[None], 0.0, gacc / S)
+    return val, grad
+
+
 def sample_eps(y_dim: int, count: int, rng=None):
     """sample_ϵs (expected_improvement.jl:118): y_dim x count standard normal draws."""
     rng = np.random.default_rng() if rng is None else rng
@@ -118,6 +185,42 @@ class Acquisition:
             pass
         return np.array([float(self.fitness(pred[:, k])) for k in range(P)])
 
+    def _fitness_grads(self, pred):
+        """fitness.grad at the columns of pred (y_dim x P) -> y_dim x P; column by column for a closure that does not
+        broadcast, like _fitness_values."""
+        P = pred.shape[1]
+        g = self.fitness.grad
+        try:
+            v = np.asarray(g(pred), dtype=np.float64)
+            if v.shape == (self.y_dim, P):
+                return v
+        except Exception:
+            pass
+        return np.stack([np.asarray(g(pred[:, k]), dtype=np.float64).reshape(self.y_dim) for k in range(P)], axis=1)
+
+    def _apply_guards(self, X, acq, grad=None):
+        """make_safe (expected_improvement.jl:58-65): 0 outside the bounds or `cons` (the gradient too)."""
+        lb, ub, cm = self._guards(X)
+        keep = np.ones(X.shape[1], dtype=bool)
+        if lb is not None:
+            keep &= np.all((X >= np.asarray(lb)[:, None]) & (X <= np.asarray(ub)[:, None]), axis=0)
+        if cm is not None:
+            keep &= np.asarray(cm, dtype=bool)
+        acq = np.where(keep, acq, 0.0)
+        return acq if grad is None else (acq, np.where(keep[None], grad, 0.0))
+
+    def _mc_value_grad(self, X):
+        """Value and x-gradient of the Monte-Carlo EI of a NonlinFitness closure with `grad`: the posteriors and their
+        x-gradients of all S*y_dim slices in one boss_gp_predict_grad call, the chain rule on the host
+        (mc_ei_value_grad).  The value equals acq(X) bit for bit."""
+        S, M, d = len(self.posts), X.shape[1], X.shape[0]
+        mu, var, dmu, dvar, st = _lib.gp_predict_grad(self.slices, self.y_dim, S, X, self._prior_mean(X))
+        acq, grad = mc_ei_value_grad(mu.reshape(S, self.y_dim, M), var.reshape(S, self.y_dim, M),
+                                     dmu.reshape(S, self.y_dim, d, M), dvar.reshape(S, self.y_dim, d, M), self.eps,
+                                     self._fitness_values, self._fitness_grads, self.best, self.y_max,
+                                     status=st.reshape(S, self.y_dim, M))
+        return self._apply_guards(X, acq, grad)
+
     def _mc_acq(self, X, want_argmax=False):
         """construct_ei for a NonlinFitness (expected_improvement.jl:68-90, :104-111)."""
         M = X.shape[1]
@@ -151,12 +254,7 @@ class Acquisition:
             f = self._fitness_values(pred.reshape(self.y_dim, M * K)).reshape(M, K)
             acc += np.maximum(0.0, f - self.best).sum(axis=1) / K * pof
         acq = np.where(failed, -np.inf, acc / len(self.posts))
-        lb, ub, cm = self._guards(X)
-        if lb is not None:
-            acq = np.where(np.all((X >= np.asarray(lb)[:, None]) & (X <= np.asarray(ub)[:, None]), axis=0), acq, 0.0)
-        if cm is not None:
-            acq = np.where(np.asarray(cm, dtype=bool), acq, 0.0)
-        return acq
+        return self._apply_guards(X, acq)
 
     def _prior_mean(self, X):
         ms = [m.mean_at(i, X) for i, m in enumerate(self.models)]
@@ -218,7 +316,8 @@ class Acquisition:
         return idx, vals
 
     def value_and_grad(self, X):
-        """-> acq (M,), grad (d, M).  Prior-mean gradients are not propagated for closure means."""
+        """-> acq (M,), grad (d, M).  Prior-mean gradients are not propagated for closure means.  A NonlinFitness needs
+        `grad` (df/dy) unless it is an ExprFitness."""
         X = np.asarray(X, dtype=np.float64)
         if self.expr is not None:     # expression-set fitness: the chain rule through the Monte-Carlo EI on the device
             lb, ub, cm = self._guards(X)
@@ -226,6 +325,8 @@ class Acquisition:
             return _lib.mcei_value_grad(self.slices, self.y_dim, len(self.posts), X, e.kind_id, self.eps, self.best,
                                         self.y_max, c0=e.c0, c=e.c, q=e.q, t=e.t, lb=lb, ub=ub, cons_mask=cm,
                                         prior_mean_s=self._prior_mean(X))
+        if self.nonlin and getattr(self.fitness, "grad", None) is not None:
+            return self._mc_value_grad(X)       # a closure with df/dy: the chain rule on the host
         if self.nonlin:
             raise NotImplementedError("NonlinFitness: the Monte-Carlo EI of an arbitrary host closure has no analytic "
                                       "gradient here (the reference pushes ForwardDiff duals through the closure); "

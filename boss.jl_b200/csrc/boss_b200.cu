@@ -1068,8 +1068,9 @@ struct ScoreArgs {
   const uint8_t *cons_mask;                      // host or device
   double *acq, *grad;                            // host or device
   const double *prior_mean_grad;                 // y_dim x d x M (host or device) or null
-  double *mu_out, *var_out;                      // predict mode (single slice), host or device
+  double *mu_out, *var_out;                      // predict mode, host or device: P x M (P = n_samples*y_dim)
   int32_t *status_out;
+  double *dmu_out = nullptr, *dvar_out = nullptr; // predict mode with x-gradients (boss_gp_predict_grad): P x d x M
   double *best_val;  // host
   int64_t *best_idx; // host
   bool dev;          // arrays are device pointers
@@ -1083,6 +1084,11 @@ struct ScoreArgs {
   double *top_val = nullptr;
   int64_t *top_idx = nullptr;
   const long long *topk_map = nullptr;   // device, or null: returned indices are topk_map[i] (the screened pool's origins)
+
+  // boss_gp_predict_grad: the posterior gradients themselves are the output (predict_grad_kernel)
+  bool pgrad() const { return dmu_out || dvar_out; }
+  // the x-gradient pipeline runs (V^T store, wtv, grad, grad_reduce): for the acquisition or for the posteriors
+  bool xgrad() const { return grad || pgrad(); }
 };
 
 // Julia's isless order on (value, index): NaN maximal, -0.0 < +0.0, ties -> lowest index (host twin of acq_better)
@@ -1156,6 +1162,7 @@ struct ChunkIO {
   double *acq = nullptr, *mu = nullptr, *var = nullptr, *grad = nullptr;
   int *st = nullptr;
   long long off = 0;
+  double *dmu = nullptr, *dvar = nullptr;
 };
 
 // Host <-> device staging of a chunked call with HOST arrays.  The caller's arrays are ordinary pageable memory in
@@ -1170,7 +1177,8 @@ struct HostStaging {
   bool xs_direct = false;   // the caller's candidate matrix is pinned already: DMA straight from it
   // byte offsets of every array inside a slot
   size_t in_xs = 0, in_pm = 0, in_cm = 0, in_pmg = 0, in_total = 0;
-  size_t out_acq = 0, out_mu = 0, out_var = 0, out_st = 0, out_gr = 0, out_total = 0;
+  size_t out_acq = 0, out_mu = 0, out_var = 0, out_st = 0, out_gr = 0, out_dmu = 0, out_dvar = 0, out_total = 0;
+  int P = 1;   // posteriors per candidate in the predict outputs (1 for boss_gp_predict)
   unsigned char *pin_in[2] = {}, *pin_out[2] = {}, *dev_in[2] = {}, *dev_out[2] = {};
   cudaStream_t cp = C().ll_stream[LL_GROUPS - 1];   // copy stream (the last log-likelihood group stream is idle here)
   cudaEvent_t ev_in[2] = {C().ll_join[LL_GROUPS - 1], C().ll_join[LL_GROUPS - 2]};     // H2D of the slot done
@@ -1184,17 +1192,20 @@ struct HostStaging {
     a = &args;
     CH = ch_cap;
     d = dim;
-    has_pmg = a->grad && a->prior_mean_grad;
+    P = a->y_dim * a->n_samples;
+    has_pmg = a->xgrad() && a->prior_mean_grad;
     xs_direct = !a->gen && is_pinned_host(a->Xs);
     in_xs = take(in_total, (size_t)CH * d * 8);   // device slot always holds the candidates
     if (a->prior_mean) in_pm = take(in_total, (size_t)CH * a->y_dim * 8);
     if (a->cons_mask) in_cm = take(in_total, (size_t)CH);
     if (has_pmg) in_pmg = take(in_total, (size_t)CH * d * a->y_dim * 8);
     if (a->acq) out_acq = take(out_total, (size_t)CH * 8);
-    if (a->mu_out) out_mu = take(out_total, (size_t)CH * 8);
-    if (a->var_out) out_var = take(out_total, (size_t)CH * 8);
-    if (a->status_out) out_st = take(out_total, (size_t)CH * 4);
+    if (a->mu_out) out_mu = take(out_total, (size_t)P * CH * 8);
+    if (a->var_out) out_var = take(out_total, (size_t)P * CH * 8);
+    if (a->status_out) out_st = take(out_total, (size_t)P * CH * 4);
     if (a->grad) out_gr = take(out_total, (size_t)CH * d * 8);
+    if (a->dmu_out) out_dmu = take(out_total, (size_t)P * d * CH * 8);
+    if (a->dvar_out) out_dvar = take(out_total, (size_t)P * d * CH * 8);
     const size_t out_slot = std::max<size_t>(out_total, 256);
     CUDA_TRY(C().xs_stage.ensure(2 * in_total));    // both device input slots
     CUDA_TRY(C().acq_stage.ensure(2 * out_slot));   // both device output slots
@@ -1241,6 +1252,8 @@ struct HostStaging {
     if (a->var_out) io.var = reinterpret_cast<double *>(dev_out[slot] + out_var);
     if (a->status_out) io.st = reinterpret_cast<int *>(dev_out[slot] + out_st);
     if (a->grad) io.grad = reinterpret_cast<double *>(dev_out[slot] + out_gr);
+    if (a->dmu_out) io.dmu = reinterpret_cast<double *>(dev_out[slot] + out_dmu);
+    if (a->dvar_out) io.dvar = reinterpret_cast<double *>(dev_out[slot] + out_dvar);
     return 0;
   }
 
@@ -1305,13 +1318,19 @@ struct HostStaging {
     CUDA_TRY(cudaEventSynchronize(ev_out[slot]));
     const unsigned char *pin = pin_out[slot];
     if (a->acq) std::memcpy(a->acq + m0, pin + out_acq, (size_t)ch * 8);
-    if (a->mu_out) std::memcpy(a->mu_out + m0, pin + out_mu, (size_t)ch * 8);
-    if (a->var_out) std::memcpy(a->var_out + m0, pin + out_var, (size_t)ch * 8);
-    if (a->status_out) std::memcpy(a->status_out + m0, pin + out_st, (size_t)ch * 4);
+    if (a->mu_out) std::memcpy(a->mu_out + (size_t)m0 * P, pin + out_mu, (size_t)ch * P * 8);
+    if (a->var_out) std::memcpy(a->var_out + (size_t)m0 * P, pin + out_var, (size_t)ch * P * 8);
+    if (a->status_out) std::memcpy(a->status_out + (size_t)m0 * P, pin + out_st, (size_t)ch * P * 4);
     if (a->grad) std::memcpy(a->grad + (size_t)m0 * d, pin + out_gr, (size_t)ch * d * 8);
+    if (a->dmu_out) std::memcpy(a->dmu_out + (size_t)m0 * d * P, pin + out_dmu, (size_t)ch * d * P * 8);
+    if (a->dvar_out) std::memcpy(a->dvar_out + (size_t)m0 * d * P, pin + out_dvar, (size_t)ch * d * P * 8);
     return 0;
   }
 };
+
+// boss_gp_predict_grad: the chunk is capped so that one output slot (P x M values, P x d x M gradients, pinned and on
+// the device, two of each) stays within this budget; at P = 16, d = 32 that is 246 candidate blocks instead of 296
+constexpr size_t PGRAD_SLOT_BYTES = (size_t)256 << 20;
 
 // What every stage of one scoring call reads: its arguments, the slices' replicas on this device, the chunk capacity
 // and the small block of per-call device scalars.
@@ -1354,7 +1373,11 @@ struct ScoreCall {
     ncb_max = std::min<long long>(ncb_max, 592);
     if (ncb_max >= 148) ncb_max = ncb_max / 148 * 148;
     if (ncb_max < 1) return fail(BOSS_ERR_ARG, "score: n too large for the scratch budget");
-    if (a.grad) ncb_max = std::max<long long>(1, std::min<long long>(ncb_max, ncb_max >= 296 ? 296 : ncb_max));
+    if (a.xgrad()) ncb_max = std::max<long long>(1, std::min<long long>(ncb_max, ncb_max >= 296 ? 296 : ncb_max));
+    if (a.pgrad()) {   // one output slot (pinned and device) within PGRAD_SLOT_BYTES (DESIGN.md 2.12)
+      const long long per_block = 128ll * nsl * (20 + 16ll * d);   // mu, var, status, dmu, dvar of 128 candidates
+      ncb_max = std::max<long long>(1, std::min<long long>(ncb_max, (long long)(PGRAD_SLOT_BYTES / per_block)));
+    }
     const long long need_cb = (a.M + 127) / 128;
     const int ncb_cap = (int)std::min<long long>(ncb_max, need_cb);
     CH = ncb_cap * 128;
@@ -1367,9 +1390,9 @@ struct ScoreCall {
     CUDA_TRY(C().part_ss.ensure((size_t)2 * max_nblk * CH * 8));
     // batches up to 8192 candidates keep V^T even without gradients: the quarter-row kernels (10 % faster than the
     // row-split wide kernels up to there) reduce the variance from the stored tile
-    have_vt = a.grad || CH <= 8192;
-    if (have_vt && !a.grad) CUDA_TRY(C().vt.ensure((size_t)CH * max_npad * 8));
-    if (a.grad) {
+    have_vt = a.xgrad() || CH <= 8192;
+    if (have_vt && !a.xgrad()) CUDA_TRY(C().vt.ensure((size_t)CH * max_npad * 8));
+    if (a.xgrad()) {
       if (d > 32) return fail(BOSS_ERR_ARG, "score: gradients need x_dim <= 32");
       CUDA_TRY(C().vt.ensure((size_t)CH * max_npad * 8));
       CUDA_TRY(C().ut.ensure((size_t)CH * max_npad * 8));
@@ -1448,9 +1471,11 @@ struct ScoreCall {
     ap.ub = (a.lb && a.ub) ? small + nsl + d : nullptr;
     ap.cons_mask = io.cm;
     ap.acq = io.acq;
-    ap.mu_out = io.mu;
-    ap.var_out = io.var;
-    ap.status_out = io.st;
+    if (!a.pgrad()) {   // predict_grad_kernel writes boss_gp_predict_grad's P x M layout
+      ap.mu_out = io.mu;
+      ap.var_out = io.var;
+      ap.status_out = io.st;
+    }
     ap.any_fail = d_anyfail;
     ap.blk_val = a.want_argmax ? C().blk_val.as<double>() : nullptr;
     ap.blk_idx = a.want_argmax ? C().blk_idx.as<long long>() : nullptr;
@@ -1506,7 +1531,7 @@ bool score_slice(const ScoreCall &c, int q, const AcqParams &ap, const ChunkIO &
   sp.ktiles = h->ktiles;
   sp.ss_part = C().part_ss.as<double>();
   sp.ld = CH;
-  sp.VT = a.grad ? C().vt.as<double>() : nullptr;
+  sp.VT = a.xgrad() ? C().vt.as<double>() : nullptr;
   if (fuse) {
     sp.fused = 1;
     sp.ap = ap;
@@ -1526,7 +1551,7 @@ bool score_slice(const ScoreCall &c, int q, const AcqParams &ap, const ChunkIO &
                                                                      C().part_ss.as<double>(), CH);
   } else if (narrow) {
     NarrowParams np{h->W, C().ks.as<double>(), h->nblk, h->ktiles, C().part_ss.as<double>(), CH,
-                    a.grad ? C().vt.as<double>() : nullptr};
+                    a.xgrad() ? C().vt.as<double>() : nullptr};
     Timed t(0);
     score_narrow_kernel<0><<<dim3(ncb32, nsp32), 256, NW_SMEM_BYTES, C().stream>>>(np);
   } else {
@@ -1541,7 +1566,7 @@ bool score_slice(const ScoreCall &c, int q, const AcqParams &ap, const ChunkIO &
     reduce_rows2_kernel<<<(cnt + 255) / 256, 256, 0, C().stream>>>(C().part_ss.as<double>(), 2 * h->nblk, (size_t)CH,
                                                                 C().sumsq.as<double>() + (size_t)q * CH, cnt);
   C().launches += fuse ? 2 : 4;
-  if (a.grad) {
+  if (a.xgrad()) {
     WtvParams wp{h->WT, C().vt.as<double>(), C().ut.as<double>(), h->nblk, h->ktiles};
     NarrowParams np{h->WT, C().vt.as<double>(), h->nblk, h->ktiles, nullptr, CH, C().ut.as<double>()};
     if (quarter) {
@@ -1744,7 +1769,7 @@ struct Screen {
 
   // ch0: the first chunk, which the seed batch is drawn from
   static bool eligible(const ScoreArgs &a, int ch0, int d) {
-    return (a.want_argmax || a.topk) && a.best && !a.internal && !a.acq && !a.grad && !a.mu_out && !a.var_out &&
+    return (a.want_argmax || a.topk) && a.best && !a.internal && !a.acq && !a.xgrad() && !a.mu_out && !a.var_out &&
            !a.status_out && !a.mix && a.M >= screen_min_m() && (size_t)a.M * pool_row(a, d) <= SCREEN_POOL_BYTES &&
            a.topk <= ch0 && getenv("BOSS_NO_SCREEN") == nullptr;
   }
@@ -2133,7 +2158,8 @@ int score_core(ScoreArgs &a) {
     const int slot = cidx & 1;
     ChunkIO io;
     if (a.dev) {
-      io = {a.Xs, a.prior_mean, a.prior_mean_grad, a.cons_mask, a.acq, a.mu_out, a.var_out, a.grad, a.status_out, 0};
+      io = {a.Xs, a.prior_mean, a.prior_mean_grad, a.cons_mask, a.acq, a.mu_out, a.var_out, a.grad, a.status_out, 0,
+            a.dmu_out, a.dvar_out};
     } else {
       rc = stg.chunk_inputs(m0, ch, slot, io);
       if (rc) return rc;
@@ -2150,7 +2176,12 @@ int score_core(ScoreArgs &a) {
     if (!scr.on()) {   // the full path (screening did not take the chunk)
       bool fused = false;
       for (int q = 0; q < c.nsl; ++q) fused = score_slice(c, q, ap, io);
-      if (!fused) {
+      if (a.pgrad()) {   // the posteriors and their gradients are the output: no acquisition
+        PredictGradParams pg{ap, C().dmu.as<double>(), C().dvar.as<double>(), io.pmg, io.mu, io.var, io.dmu, io.dvar, io.st};
+        const long long ne = (long long)ch * c.d * c.nsl;
+        predict_grad_kernel<<<(unsigned)((ne + 255) / 256), 256, 0, C().stream>>>(pg);
+        ++C().launches;
+      } else if (!fused) {
         const int nb = (ch + 255) / 256;
         acq_kernel<<<nb, 256, 0, C().stream>>>(ap);
         ++C().launches;
@@ -2263,9 +2294,11 @@ int score_dispatch(ScoreArgs &a) {
     if (a.cons_mask) s.cons_mask = a.cons_mask + off;
     if (a.acq) s.acq = a.acq + off;
     if (a.grad) s.grad = a.grad + (size_t)off * d;
-    if (a.mu_out) s.mu_out = a.mu_out + off;
-    if (a.var_out) s.var_out = a.var_out + off;
-    if (a.status_out) s.status_out = a.status_out + off;
+    if (a.mu_out) s.mu_out = a.mu_out + (size_t)off * nsl;   // predict outputs: nsl per candidate (1 for boss_gp_predict)
+    if (a.var_out) s.var_out = a.var_out + (size_t)off * nsl;
+    if (a.status_out) s.status_out = a.status_out + (size_t)off * nsl;
+    if (a.dmu_out) s.dmu_out = a.dmu_out + (size_t)off * d * nsl;
+    if (a.dvar_out) s.dvar_out = a.dvar_out + (size_t)off * d * nsl;
     s.best_val = &bv[k];
     s.best_idx = &bi[k];
     if (a.topk) {
@@ -2838,6 +2871,26 @@ int boss_ei_value_grad_dev(const boss_gp *const *slices, int y_dim, int n_sample
   if (!grad_dev) return fail(BOSS_ERR_ARG, "boss_ei_value_grad_dev: grad is NULL");
   return ei_score_impl(slices, y_dim, n_samples, Xs_dev, M, prior_mean_s_dev, fit_coefs, best, y_max, lb, ub,
                        cons_mask_dev, acq_dev, grad_dev, nullptr, nullptr, true, prior_mean_grad_s_dev, stream);
+}
+
+int boss_gp_predict_grad(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
+                         const double *prior_mean_s, const double *prior_mean_grad_s, double *mu, double *var,
+                         double *dmu, double *dvar, int32_t *status) {
+  if (!slices || y_dim < 1 || n_samples < 1 || (!Xs && M > 0))
+    return fail(BOSS_ERR_ARG, "boss_gp_predict_grad: bad arguments");
+  if (!dmu && !dvar)
+    return fail(BOSS_ERR_ARG, "boss_gp_predict_grad: dmu and dvar are both NULL (boss_gp_predict gives mu and var alone)");
+  ScoreArgs a = score_args(slices, y_dim, n_samples, Xs, M, prior_mean_s, nullptr, nullptr, nullptr, nullptr, nullptr,
+                           nullptr);
+  a.prior_mean_grad = prior_mean_grad_s;
+  a.mu_out = mu;
+  a.var_out = var;
+  a.status_out = status;
+  a.dmu_out = dmu;
+  a.dvar_out = dvar;
+  int rc = score_dispatch(a);
+  if (rc) return rc;
+  return a.any_fail ? BOSS_NEG_VARIANCE : 0;
 }
 
 int boss_gp_cov(const boss_gp *gp, const double *Xs, int64_t M, const double *prior_mean_s, double *mu, double *cov) {

@@ -8,7 +8,8 @@
 //
 // Pipeline per chunk and slice: xcov -> score_trmm (also stores V^T) -> wtv_kernel (U^T = (W^T V)^T, the
 // second triangular product, same DMMA mainloop) -> grad_kernel (kernel derivatives, FP64 pipe) ->
-// acq_grad_kernel (chain rule through EI x PoF, or through the Monte-Carlo EI of a MixParams expression).
+// acq_grad_kernel (chain rule through EI x PoF, or through the Monte-Carlo EI of a MixParams expression), or
+// predict_grad_kernel (boss_gp_predict_grad: mu, var and their gradients themselves, in the caller's layout).
 #pragma once
 #include "score.cuh"
 
@@ -247,6 +248,52 @@ __global__ void __launch_bounds__(128) acq_grad_kernel(AcqGradParams q) {
   }
   if (p.cons_mask && p.cons_mask[m - p.in_off] == 0) zero = true;
   for (int j = 0; j < d; ++j) q.grad[(size_t)(m - p.out_off) * d + j] = zero ? 0.0 : gacc[j] / (double)p.n_samples;
+}
+
+// boss_gp_predict_grad's output stage (in place of acq_kernel + acq_grad_kernel): the P = n_samples * y_dim posteriors
+// of the chunk, from [q][chunk_ld] rows and [q][j][chunk_ld] sections to the caller's candidate-major layout
+//   mu / var / status  at (m - out_off) * P + q ,   dmu / dvar  at ((m - out_off) * d + j) * P + q .
+// One thread per output element in output order, so every store is coalesced; the strided loads hit the chunk's
+// sections, which the reductions just wrote.  mu and var use acq_candidate's expressions (same bits as boss_gp_predict).
+struct PredictGradParams {
+  AcqParams a;                     // mu / sumsq rows, a2, prior_mean, any_fail, chunk geometry
+  const double *dmu, *dvar;        // [q][d][chunk_ld]
+  const double *prior_mean_grad;   // y_dim x d x M (index ((m - in_off) * d + j) * y_dim + i) or null
+  double *mu_out, *var_out, *dmu_out, *dvar_out;   // each may be null
+  int *status_out;
+};
+__global__ void __launch_bounds__(256) predict_grad_kernel(PredictGradParams q) {
+  const AcqParams &p = q.a;
+  const int P = p.n_samples * p.y_dim, d = p.d;
+  const int e = blockIdx.x * 256 + threadIdx.x;   // element of the chunk's dmu / dvar output (chunk * d * P < 2^31)
+  if (e >= p.chunk * d * P) return;
+  const int qi = e % P, j = e / P % d, c = e / (P * d);
+  const int i = qi % p.y_dim;
+  const size_t row = (size_t)qi * p.chunk_ld + c;
+  const long long m = p.m0 + c;
+  const double var_raw = p.a2[qi] - p.sumsq[row] + VAR_JITTER;
+  const size_t sec = ((size_t)qi * d + j) * p.chunk_ld + c;
+  const size_t o = (size_t)(m - p.out_off) * d * P + ((size_t)j * P + qi);   // == ((m - out_off) * d + j) * P + q
+  if (q.dmu_out) {
+    double dm = q.dmu[sec];
+    if (q.prior_mean_grad) dm += q.prior_mean_grad[((size_t)(m - p.in_off) * d + j) * p.y_dim + i];
+    q.dmu_out[o] = dm;
+  }
+  if (q.dvar_out) q.dvar_out[o] = var_raw >= 0.0 ? q.dvar[sec] : 0.0;   // the clipped branch of _clip_var is a constant
+  // the first chunk * P threads also write the value outputs, element e of those (candidate-major as well)
+  if (e >= p.chunk * P) return;
+  const int q2 = e % P, c2 = e / P;
+  const size_t row2 = (size_t)q2 * p.chunk_ld + c2;
+  const long long m2 = p.m0 + c2;
+  double mu = p.mu[row2];
+  if (p.prior_mean) mu = p.prior_mean[(size_t)(m2 - p.in_off) * p.y_dim + q2 % p.y_dim] + mu;
+  double var = p.a2[q2] - p.sumsq[row2] + VAR_JITTER;
+  const bool ok = clip_var(var);
+  if (!ok) *p.any_fail = 1;
+  const size_t o2 = (size_t)(m2 - p.out_off) * P + q2;
+  if (q.mu_out) q.mu_out[o2] = mu;
+  if (q.var_out) q.var_out[o2] = var;
+  if (q.status_out) q.status_out[o2] = ok ? 0 : 2;
 }
 
 }  // namespace boss

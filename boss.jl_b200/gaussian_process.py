@@ -99,6 +99,13 @@ class GaussianProcess:
         return ll
 
 
+def _raise_domain_error(var, status):
+    """The DomainError of _clip_var (gaussian_process.jl:186-194) for the first failed variance, as a ValueError."""
+    if np.any(status != 0):
+        bad = var[np.nonzero(status)][0]
+        raise ValueError(f"DomainError: The posterior GP predicted variance {bad} but only values above -1e-8 are tolerated.")
+
+
 class GaussianProcessPosterior:
     """One output slice: handle to the device-resident factor cache (replaces the AbstractGPs.PosteriorGP wrapper,
     gaussian_process.jl:127-131)."""
@@ -116,10 +123,23 @@ class GaussianProcessPosterior:
         X = x[:, None] if vec else x
         pm = self.model.mean_at(self.slice_idx, X)
         mu, var, st = _lib.gp_predict(self.gp, X, pm)
-        if np.any(st != 0):
-            bad = var[np.flatnonzero(st)[0]]
-            raise ValueError(f"DomainError: The posterior GP predicted variance {bad} but only values above -1e-8 are tolerated.")
+        _raise_domain_error(var, st)
         return (float(mu[0]), float(var[0])) if vec else (mu, var)
+
+    def mean_and_var_grad(self, x):
+        """mean_and_var with the x-gradients (the mirror's stand-in for ForwardDiff through mean_and_var; one
+        boss_gp_predict_grad call): vector x -> (mu, var, dmu (d,), dvar (d,)); matrix X (d x M) -> (mu (M,), var (M,),
+        dmu (d, M), dvar (d, M)).  mu and var equal mean_and_var's bit for bit.  The gradient of a prior-mean closure is
+        not included (the constant and zero means have none).  Raises ValueError where mean_and_var does."""
+        x = np.asarray(x, dtype=np.float64)
+        vec = x.ndim == 1
+        X = x[:, None] if vec else x
+        pm = self.model.mean_at(self.slice_idx, X)
+        mu, var, dmu, dvar, st = _lib.gp_predict_grad([self.gp], 1, 1, X, None if pm is None else pm[None])
+        _raise_domain_error(var, st)
+        if vec:
+            return float(mu[0, 0]), float(var[0, 0]), dmu[0, :, 0].copy(), dvar[0, :, 0].copy()
+        return mu[0], var[0], dmu[0], dvar[0]
 
     def mean(self, x):
         return self.mean_and_var(x)[0]

@@ -4,7 +4,7 @@ from __future__ import annotations
 import numpy as np
 
 from . import _lib
-from .gaussian_process import GaussianProcessPosterior, _as_gp, _kernel_parts, model_posterior_slice
+from .gaussian_process import GaussianProcessPosterior, _as_gp, _kernel_parts, _raise_domain_error, model_posterior_slice
 from .types import BossProblem, get_params
 
 
@@ -20,6 +20,22 @@ class DefaultModelPosterior:
         if x.ndim == 1:
             return np.array([r[0] for r in res]), np.array([r[1] for r in res])
         return np.stack([r[0] for r in res]), np.stack([r[1] for r in res])      # y_dim x M
+
+    def mean_and_var_grad(self, x):
+        """mean_and_var with the x-gradients of every output slice in one boss_gp_predict_grad call (the mirror's
+        stand-in for ForwardDiff through mean_and_var): vector x -> (mu (y_dim,), var (y_dim,), dmu (y_dim, d),
+        dvar (y_dim, d)); matrix X (d x M) -> (mu (y_dim, M), var (y_dim, M), dmu (y_dim, d, M), dvar (y_dim, d, M)).
+        Prior-mean closures are not differentiated.  Raises ValueError where mean_and_var does."""
+        x = np.asarray(x, dtype=np.float64)
+        vec = x.ndim == 1
+        X = x[:, None] if vec else x
+        ms = [s.model.mean_at(s.slice_idx, X) for s in self.slices]
+        pm = None if all(m is None for m in ms) else np.stack([np.zeros(X.shape[1]) if m is None else m for m in ms])
+        mu, var, dmu, dvar, st = _lib.gp_predict_grad([s.gp for s in self.slices], len(self.slices), 1, X, pm)
+        _raise_domain_error(var, st)
+        if vec:
+            return mu[:, 0].copy(), var[:, 0].copy(), dmu[:, :, 0].copy(), dvar[:, :, 0].copy()
+        return mu, var, dmu, dvar
 
     def mean(self, x):
         return self.mean_and_var(x)[0]

@@ -79,7 +79,11 @@ class LinFitness:
 
 @dataclass
 class NonlinFitness:
+    """fitness(y) -> Real.  `grad` (optional): grad(Y) -> df/dy (y_dim x P) at the columns of a y_dim x P matrix Y --
+    what ForwardDiff does to the closure in the reference.  With it, Acquisition.value_and_grad (and so OptimizationAM
+    and SampleOptAM) can differentiate the Monte-Carlo EI of the closure; the closure itself stays on the host."""
     fitness: Callable
+    grad: Optional[Callable] = None
 
     def __call__(self, y):
         return self.fitness(y)

@@ -119,6 +119,22 @@ int boss_gp_predict(const boss_gp *gp, const double *Xs, int64_t M, const double
 int boss_gp_predict_dev(const boss_gp *gp, const double *Xs_dev, int64_t M, const double *prior_mean_s_dev,
                         double *mu_dev, double *var_dev, int32_t *status_dev, void *stream);
 
+/* Posterior mean and variance with their x-gradients, for every posterior of a BI model in one call: what BOSS.jl
+ * obtains by pushing ForwardDiff.Dual numbers through mean_and_var (gaussian_process.jl:169-178), e.g. to
+ * differentiate an arbitrary NonlinFitness closure on the host (DESIGN.md 2.12).
+ *   slices, y_dim, n_samples, Xs, prior_mean_s, prior_mean_grad_s  as boss_ei_value_grad (the prior mean and its
+ *       gradient, y_dim x M and y_dim x d x M, are shared by the BI samples)
+ *   P = n_samples * y_dim posteriors, q = s*y_dim + i;  outputs candidate-major, any of them may be NULL:
+ *   mu, var, status  P x M at index m*P + q: bit for bit what boss_gp_predict gives for slices[q] (_clip_var included)
+ *   dmu, dvar        P x d x M at index (m*d + j)*P + q;  at least one of the two must be given (else BOSS_ERR_ARG:
+ *       boss_gp_predict gives mu and var alone)
+ * Gradient conventions: dvar is 0 where the raw variance was < 0 (the clipped branch is a constant), discrete
+ * (rounded) dims have zero derivative, dmu includes prior_mean_grad_s when given.  Limits as the gradient path:
+ * x_dim <= 32, y_dim <= 16.  Returns 0, or BOSS_NEG_VARIANCE if any status is non-zero; M = 0 returns 0. */
+int boss_gp_predict_grad(const boss_gp *const *slices, int y_dim, int n_samples, const double *Xs, int64_t M,
+                         const double *prior_mean_s, const double *prior_mean_grad_s, double *mu, double *var,
+                         double *dmu, double *dvar, int32_t *status);
+
 /* Replaces cov / mean_and_cov(::GaussianProcessPosterior, X) (gaussian_process.jl:163-167,180-184):
  * full M x M posterior covariance (column-major), diagonal clipped.  Intended for small M. */
 int boss_gp_cov(const boss_gp *gp, const double *Xs, int64_t M, const double *prior_mean_s,

@@ -18,6 +18,7 @@
 #   reference function                                                          -> library entry point
 #   model_posterior_slice (src/models/gaussian_process.jl:133-141)              -> boss_gp_fit / boss_gp_fit_batch
 #   mean / var / mean_and_var / cov / mean_and_cov (:143-184)                   -> boss_gp_predict / boss_gp_cov
+#   mean_and_var(post, X::Matrix{<:ForwardDiff.Dual})                           -> boss_gp_predict_grad
 #   construct_acquisition(::ExpectedImprovement) (expected_improvement.jl:49-90)-> boss_ei_score / boss_mcei_score
 #   maximize_acquisition(::GridAM)        (acquisition_maximizers/grid.jl:45-65)        -> boss_ei_score
 #   maximize_acquisition(::SamplingAM)    (sampling.jl:20-57)                           -> boss_ei_score
@@ -154,6 +155,36 @@ function mean_and_var(post::B200Posterior, X::AbstractMatrix{<:Real})
         throw(DomainError(σ2[i], "The posterior GP predicted variance $(σ2[i]) but only values above -1e-8 are tolerated."))
     end
     return μ, σ2
+end
+
+# ForwardDiff through the posterior (a Dual sweep through mean / var, a custom acquisition built on b200_posterior):
+# one boss_gp_predict_grad call on the values gives mu, var and their x-Jacobians (the prior mean left out); the
+# partials of every column follow by the chain rule, and the slice mean is added by evaluating it on the Duals, which
+# also differentiates a mean closure.  The values equal the Real method's (prior + mu in the same order).  The vector
+# method below reaches this one through hcat for Dual vectors too.
+dual_mean(::Nothing, X::AbstractMatrix) = nothing
+dual_mean(m::Real, X::AbstractMatrix) = fill(Float64(m), size(X, 2))
+dual_mean(m::Function, X::AbstractMatrix) = [m(x) for x in eachcol(X)]
+function mean_and_var(post::B200Posterior, X::AbstractMatrix{D}) where {T, V, N, D<:ForwardDiff.Dual{T, V, N}}
+    Xs = Matrix{Float64}(ForwardDiff.value.(X))
+    d, M = size(Xs)
+    μ = Vector{Float64}(undef, M); σ2 = Vector{Float64}(undef, M); st = Vector{Int32}(undef, M)
+    dμ = Matrix{Float64}(undef, d, M); dσ2 = Matrix{Float64}(undef, d, M)   # one posterior: index (m*d + j)
+    h = Ptr{Cvoid}[post.handle]
+    rc = GC.@preserve Xs h check(ccall((:boss_gp_predict_grad, LIB), Cint,
+        (Ptr{Ptr{Cvoid}}, Cint, Cint, Ptr{Cdouble}, Int64, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble},
+         Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int32}),
+        h, 1, 1, Xs, M, C_NULL, C_NULL, μ, σ2, dμ, dσ2, st))
+    if rc == 2   # the Real method's DomainError
+        i = findfirst(!=(0), st)
+        throw(DomainError(σ2[i], "The posterior GP predicted variance $(σ2[i]) but only values above -1e-8 are tolerated."))
+    end
+    dual(v, J, m) = ForwardDiff.Dual{T}(v, ForwardDiff.Partials(ntuple(k -> sum(J[j, m] * ForwardDiff.partials(X[j, m], k)
+                                                                                  for j in 1:d), N)))
+    μd = [dual(μ[m], dμ, m) for m in 1:M]
+    σ2d = [dual(σ2[m], dσ2, m) for m in 1:M]
+    pm = dual_mean(post.mean, X)
+    return (isnothing(pm) ? μd : pm .+ μd), σ2d
 end
 mean_and_var(post::B200Posterior, x::AbstractVector{<:Real}) = first.(mean_and_var(post, hcat(x)))
 mean(post::B200Posterior, x) = mean_and_var(post, x)[1]

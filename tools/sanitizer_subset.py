@@ -6,7 +6,7 @@
 
 Families: build_k, potrf_tile (+ fused diagonal step), chol_trsm, chol_update, chol_panel, chol_update_rl, trtri_*_rl,
 trtri_fused, kinv_wtw, loglik_grad_tile, loglik_small (warp path), matvec, xcov, score_trmm (plain and row-split),
-wtv, grad (+ MC-EI gradient), acq (+ MC-EI), argmax, top-k, cov (gemm_nt + cov_finish), candidate generators, append (+ capacity growth),
+wtv, grad (+ MC-EI gradient, + posterior gradients), acq (+ MC-EI), argmax, top-k, cov (gemm_nt + cov_finish), candidate generators, append (+ capacity growth),
 multi-start driver.  Results are checked against the oracle so that a run that "passes" the sanitizer by computing
 nothing is caught.  Prints one JSON line.
 """
@@ -58,6 +58,14 @@ def main():
     assert relerr(a_g[mm], a_r[mm]) <= 1e-9
     assert np.max(np.abs(g_g[:, mm] - g_r[:, mm]) / np.max(np.abs(g_r[:, mm]), axis=0)) <= 1e-7
     done.append("value_grad")
+    # --- posterior x-gradients (predict_grad_kernel) for both slices in one call ---
+    pmu, pvar, pdm, pdv, pst = _lib.gp_predict_grad(gps, 2, 1, Xs[:, :200])
+    for i in range(2):
+        mo, vo, dmo, dvo, _ = O.mean_var_grad(posts[i], Xs[:, :200])
+        assert relerr(pvar[i], vo) <= 1e-9 and np.max(np.abs(pmu[i] - mo)) <= 1e-9 * np.max(np.abs(mo))
+        assert np.max(np.abs(pdm[i] - dmo)) <= 1e-8 * np.max(np.abs(dmo))
+        assert np.max(np.abs(pdv[i] - dvo)) <= 1e-8 * np.max(np.abs(dvo))
+    done.append("predict_grad")
     # --- device candidate generators ---
     _, gv, gi, gx = _lib.ei_score_uniform(gps, 2, 1, 5, M, lb, ub, coefs, best, y_max)
     pts = _lib.uniform_candidates(5, 0, M, lb, ub)
