@@ -83,6 +83,10 @@ EXPORTS = {
                                             _vp, _vp]),
     "boss_gp_loglik_grad_batch_dev": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp, C.c_int, _vp,
                                                 C.c_int64, _vp, _vp, _vp]),
+    "boss_gp_loglik_grad_batch_mean": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, C.c_int, C.c_int64, _vp, _vp,
+                                                 _vp, C.c_int, _vp, C.c_int64, _vp, _vp, _vp]),
+    "boss_gp_loglik_grad_batch_mean_dev": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, C.c_int, C.c_int64, _vp,
+                                                     _vp, _vp, C.c_int, _vp, C.c_int64, _vp, _vp, _vp, _vp]),
     "boss_set_timing": (None, [C.c_int]),
     "boss_last_kernel_ms": (C.c_double, [C.c_int]),
     "boss_last_kernel_count": (C.c_int, [C.c_int]),
@@ -639,6 +643,44 @@ def loglik_grad_batch_dev(X_ptr, d, n, Y_ptr, ldy, ls_ptr, amp_ptr, noise_ptr, k
                                              int(kernel_id), None, int(S), _vp(out_ptr), _vp(grad_ptr),
                                              _vp(stream) if stream else None),
            "boss_gp_loglik_grad_batch_dev")
+
+
+def loglik_grad_batch_mean(X, Y_minus_mean, J, lengthscales, amplitude, noise_std, kernel_id=KERNEL_MATERN52,
+                           discrete_mask=None):
+    """loglik_grad_batch plus the gradient w.r.t. the parameters theta of the prior mean, alpha^T J per sample.
+    J = dm(X; theta)/dtheta at the training inputs: (k, n) shared by all samples or (S, k, n) per sample (row c of a
+    sample is column c of ForwardDiff.jacobian's n x k matrix).  -> loglik (S,), grad (S, d + 2), grad_mean (S, k)."""
+    Xc = _cols(X)
+    n, d = Xc.shape
+    ls = _f64(lengthscales)
+    S = ls.shape[0]
+    assert ls.shape == (S, d)
+    amp = _f64(amplitude, (S,))
+    ns = _f64(noise_std, (S,))
+    Y = _f64(Y_minus_mean)
+    ldy = 0 if Y.ndim == 1 else n
+    Jc = _f64(J)
+    assert Jc.ndim in (2, 3) and Jc.shape[-1] == n and (Jc.ndim == 2 or Jc.shape[0] == S)
+    k = Jc.shape[-2]
+    ldj = 0 if Jc.ndim == 2 else k * n
+    dm = None if discrete_mask is None else np.ascontiguousarray(discrete_mask, dtype=np.uint8)
+    out = np.empty(S)
+    grad = np.empty((S, d + 2))
+    gm = np.empty((S, k))
+    _check(lib.boss_gp_loglik_grad_batch_mean(_ptr(Xc), d, n, _ptr(Y), ldy, _ptr(Jc), k, ldj, _ptr(ls), _ptr(amp), _ptr(ns),
+                                              int(kernel_id), _ptr(dm), S, _ptr(out), _ptr(grad), _ptr(gm)),
+           "boss_gp_loglik_grad_batch_mean")
+    return out, grad, gm
+
+
+def loglik_grad_batch_mean_dev(X_ptr, d, n, Y_ptr, ldy, J_ptr, k, ldj, ls_ptr, amp_ptr, noise_ptr, kernel_id, S, out_ptr,
+                               grad_ptr, grad_mean_ptr, discrete_mask=None, stream=None):
+    dm = None if discrete_mask is None else np.ascontiguousarray(discrete_mask, dtype=np.uint8)
+    _check(lib.boss_gp_loglik_grad_batch_mean_dev(_vp(X_ptr), d, n, _vp(Y_ptr), ldy, _vp(J_ptr), int(k), int(ldj),
+                                                  _vp(ls_ptr), _vp(amp_ptr), _vp(noise_ptr), int(kernel_id), _ptr(dm),
+                                                  int(S), _vp(out_ptr), _vp(grad_ptr), _vp(grad_mean_ptr),
+                                                  _vp(stream) if stream else None),
+           "boss_gp_loglik_grad_batch_mean_dev")
 
 
 def loglik_batch_dev(X_ptr, d, n, Y_ptr, ldy, ls_ptr, amp_ptr, noise_ptr, kernel_id, S, out_ptr, discrete_mask=None,

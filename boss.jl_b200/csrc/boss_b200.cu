@@ -2967,10 +2967,20 @@ struct StreamGuard {
   ~StreamGuard() { C().stream = keep; }
 };
 
+// Prior-mean Jacobian of boss_gp_loglik_grad_batch_mean: J (sample s at J + s*ldj, ldj == 0 shared, n x k column-major
+// inside a sample) in, alpha^T J (S x k) out.  Only the gradient mode takes one.
+struct MeanJac {
+  const double *J;
+  int k;
+  int64_t ldj;
+  double *grad_mean;
+};
+
 // one batch inside the current context
 static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t ldy, const double *ls,
                        const double *amp, const double *noise, int kernel_id, const uint8_t *discrete_mask, int64_t S,
-                       double *loglik, bool dev, double *grad, boss_gp **fit_out, void *caller_stream) {
+                       double *loglik, bool dev, double *grad, boss_gp **fit_out, void *caller_stream,
+                       const MeanJac *mj = nullptr) {
   const int dp = pick_dp(d);
   if (S == 0) return 0;
   if (dev) {
@@ -3003,22 +3013,29 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
   }
 
   // device copies of the inputs when called with host pointers
-  const double *dX = X, *dY = Ymm, *dls = ls, *damp = amp, *dnoise = noise;
+  const double *dX = X, *dY = Ymm, *dls = ls, *damp = amp, *dnoise = noise, *dJ = mj ? mj->J : nullptr;
   double *dll = loglik;
   const size_t ycount = ldy ? (size_t)S * ldy : (size_t)n;
-  // misc: [X | Y | ls | amp | noise | ll] (host variant) then logdet_blk[Sb*nblk] | ssq_blk[Sb*nblk] | r, w [Sb*n_pad] | status[Sb]
-  size_t off = 0, oX = 0, oY = 0, ols = 0, oamp = 0, onoise = 0, oll = 0;
+  // the last sample's Jacobian ends at k*n: a caller stride ldj > k*n need not be padded after it
+  const size_t jcount = !mj ? 0 : (size_t)mj->k * n + (mj->ldj ? (size_t)(S - 1) * mj->ldj : 0);
+  // misc: [X | Y | J | ls | amp | noise | ll] (host variant) then grad | grad_mean (host variant, gradient mode) then
+  // logdet_blk[Sb*nblk] | ssq_blk[Sb*nblk] | r, w [Sb*n_pad] | status[Sb]
+  size_t off = 0, oX = 0, oY = 0, oJ = 0, ols = 0, oamp = 0, onoise = 0, oll = 0;
   if (!dev) {
     oX = off; off += (size_t)n * d;
     oY = off; off += ycount;
+    oJ = off; off += jcount;
     ols = off; off += (size_t)S * d;
     oamp = off; off += S;
     onoise = off; off += S;
     oll = off; off += S;
   }
-  size_t ogr = 0;
+  size_t ogr = 0, ogm = 0;
   if (!dev && grad) {
     ogr = off; off += (size_t)S * (d + 2);
+  }
+  if (!dev && mj) {
+    ogm = off; off += (size_t)S * mj->k;
   }
   const size_t old_ = off;
   off += (size_t)Sb * nblk;
@@ -3035,12 +3052,17 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
   if (!dev) {
     CUDA_TRY(cudaMemcpyAsync(misc + oX, X, (size_t)n * d * 8, cudaMemcpyHostToDevice, C().stream));
     CUDA_TRY(cudaMemcpyAsync(misc + oY, Ymm, ycount * 8, cudaMemcpyHostToDevice, C().stream));
+    if (mj) {
+      CUDA_TRY(cudaMemcpyAsync(misc + oJ, mj->J, jcount * 8, cudaMemcpyHostToDevice, C().stream));
+      dJ = misc + oJ;
+    }
     CUDA_TRY(cudaMemcpyAsync(misc + ols, ls, (size_t)S * d * 8, cudaMemcpyHostToDevice, C().stream));
     CUDA_TRY(cudaMemcpyAsync(misc + oamp, amp, (size_t)S * 8, cudaMemcpyHostToDevice, C().stream));
     CUDA_TRY(cudaMemcpyAsync(misc + onoise, noise, (size_t)S * 8, cudaMemcpyHostToDevice, C().stream));
     dX = misc + oX; dY = misc + oY; dls = misc + ols; damp = misc + oamp; dnoise = misc + onoise; dll = misc + oll;
   }
   double *dgrad = (grad && !dev) ? misc + ogr : grad;
+  double *dgm = !mj ? nullptr : dev ? mj->grad_mean : misc + ogm;
   double *logdet_blk = misc + old_;
   int *status = reinterpret_cast<int *>(misc + ost);
 
@@ -3182,6 +3204,11 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
         matvec_p_kernel<<<dim3(n_pad / 64, gs), 256, 0, C().stream>>>(WTg, wv, al, ktiles, mat, n_pad, n_pad);
         C().launches += 3;
       }
+      if (mj) {   // prior-mean gradient alpha^T J: reads alpha only, so the hyper-parameter gradient below is unchanged
+        loglik_mean_grad_kernel<<<dim3(mj->k, gs), 128, 0, C().stream>>>(al, n_pad, dJ + (size_t)so * mj->ldj, mj->ldj, n,
+                                                                        mj->k, stg, dgm + (size_t)so * mj->k);
+        ++C().launches;
+      }
       if (grad) {
         // K^-1 = W^T W over the factor's storage;  tile partial sums;  final scaling
         double *partg = C().ll_part.as<double>() + (size_t)wo * ntiles * (dp + 2);
@@ -3274,6 +3301,8 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
   CUDA_TRY(cudaGetLastError());
   if (!dev) CUDA_TRY(cudaMemcpyAsync(loglik, dll, (size_t)S * 8, cudaMemcpyDeviceToHost, C().stream));
   if (!dev && grad) CUDA_TRY(cudaMemcpyAsync(grad, dgrad, (size_t)S * (d + 2) * 8, cudaMemcpyDeviceToHost, C().stream));
+  if (!dev && mj)
+    CUDA_TRY(cudaMemcpyAsync(mj->grad_mean, dgm, (size_t)S * mj->k * 8, cudaMemcpyDeviceToHost, C().stream));
   CUDA_TRY(cudaStreamSynchronize(C().stream));
   timing_end();
   if (!dev) {
@@ -3292,7 +3321,7 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
 static int loglik_impl(const double *X, int d, int n, const double *Ymm, int64_t ldy, const double *ls,
                        const double *amp, const double *noise, int kernel_id, const uint8_t *discrete_mask, int64_t S,
                        double *loglik, bool dev, double *grad = nullptr, boss_gp **fit_out = nullptr,
-                       void *caller_stream = nullptr) {
+                       void *caller_stream = nullptr, const MeanJac *mj = nullptr) {
   if (!X || !Ymm || !ls || !amp || !noise || !loglik || d < 1 || n < 1 || S < 0)
     return fail(BOSS_ERR_ARG, "boss_gp_loglik_batch: bad arguments");
   if (kernel_id < 0 || kernel_id > 2) return fail(BOSS_ERR_ARG, "boss_gp_loglik_batch: unknown kernel_id");
@@ -3308,15 +3337,18 @@ static int loglik_impl(const double *X, int d, int n, const double *Ymm, int64_t
   const int nd = (g_ndev > 1 && tl_dev < 0 && !dev && !fit_out && S >= 2LL * g_ndev) ? g_ndev : 1;
   if (nd <= 1) {
     REQUIRE_INIT();
-    return loglik_core(X, d, n, Ymm, ldy, ls, amp, noise, kernel_id, discrete_mask, S, loglik, dev, grad, fit_out, caller_stream);
+    return loglik_core(X, d, n, Ymm, ldy, ls, amp, noise, kernel_id, discrete_mask, S, loglik, dev, grad, fit_out, caller_stream,
+                       mj);
   }
   const int64_t per = (S + nd - 1) / nd;
   int rc = for_each_device(nd, [&](int k, Ctx *) {
     const int64_t s0 = std::min<int64_t>(S, (int64_t)k * per), cnt = std::min<int64_t>(per, S - s0);
     if (cnt <= 0) return 0;
+    MeanJac mjk{};
+    if (mj) mjk = MeanJac{mj->J + (size_t)s0 * mj->ldj, mj->k, mj->ldj, mj->grad_mean + (size_t)s0 * mj->k};
     return loglik_core(X, d, n, ldy ? Ymm + (size_t)s0 * ldy : Ymm, ldy, ls + (size_t)s0 * d, amp + s0, noise + s0, kernel_id,
                        discrete_mask, cnt, loglik + s0, false, grad ? grad + (size_t)s0 * (d + 2) : nullptr,
-                       fit_out ? fit_out + s0 : nullptr, nullptr);
+                       fit_out ? fit_out + s0 : nullptr, nullptr, mj ? &mjk : nullptr);
   });
   return rc;
 }
@@ -3401,6 +3433,37 @@ int boss_gp_loglik_grad_batch_dev(const double *X_dev, int d, int n, const doubl
   if (!grad_dev) return fail(BOSS_ERR_ARG, "boss_gp_loglik_grad_batch_dev: grad is NULL");
   return loglik_impl(X_dev, d, n, Y_minus_mean_dev, ldy, lengthscales_dev, amplitude_dev, noise_std_dev, kernel_id,
                      discrete_mask, S, loglik_dev, true, grad_dev, nullptr, stream);
+}
+
+static int check_mean_jac(const char *who, int n, const double *grad, const double *mean_jac, int k, int64_t ldj,
+                          const double *grad_mean) {
+  if (!grad) return fail(BOSS_ERR_ARG, std::string(who) + ": grad is NULL");
+  if (!mean_jac || !grad_mean) return fail(BOSS_ERR_ARG, std::string(who) + ": mean_jac or grad_mean is NULL");
+  if (k < 1) return fail(BOSS_ERR_ARG, std::string(who) + ": k < 1");
+  if (ldj != 0 && ldj < (int64_t)k * n) return fail(BOSS_ERR_ARG, std::string(who) + ": ldj is neither 0 nor >= k*n");
+  return 0;
+}
+
+int boss_gp_loglik_grad_batch_mean(const double *X, int d, int n, const double *Y_minus_mean, int64_t ldy,
+                                   const double *mean_jac, int k, int64_t ldj, const double *lengthscales,
+                                   const double *amplitude, const double *noise_std, int kernel_id,
+                                   const uint8_t *discrete_mask, int64_t S, double *loglik, double *grad,
+                                   double *grad_mean) {
+  if (int rc = check_mean_jac("boss_gp_loglik_grad_batch_mean", n, grad, mean_jac, k, ldj, grad_mean)) return rc;
+  const MeanJac mj{mean_jac, k, ldj, grad_mean};
+  return loglik_impl(X, d, n, Y_minus_mean, ldy, lengthscales, amplitude, noise_std, kernel_id, discrete_mask, S, loglik,
+                     false, grad, nullptr, nullptr, &mj);
+}
+int boss_gp_loglik_grad_batch_mean_dev(const double *X_dev, int d, int n, const double *Y_minus_mean_dev, int64_t ldy,
+                                       const double *mean_jac_dev, int k, int64_t ldj, const double *lengthscales_dev,
+                                       const double *amplitude_dev, const double *noise_std_dev, int kernel_id,
+                                       const uint8_t *discrete_mask, int64_t S, double *loglik_dev, double *grad_dev,
+                                       double *grad_mean_dev, void *stream) {
+  if (int rc = check_mean_jac("boss_gp_loglik_grad_batch_mean_dev", n, grad_dev, mean_jac_dev, k, ldj, grad_mean_dev))
+    return rc;
+  const MeanJac mj{mean_jac_dev, k, ldj, grad_mean_dev};
+  return loglik_impl(X_dev, d, n, Y_minus_mean_dev, ldy, lengthscales_dev, amplitude_dev, noise_std_dev, kernel_id,
+                     discrete_mask, S, loglik_dev, true, grad_dev, nullptr, stream, &mj);
 }
 
 // ---------------------------------------------------------------------------------------------

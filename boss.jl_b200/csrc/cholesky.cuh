@@ -548,4 +548,27 @@ __global__ void loglik_grad_final_kernel(const double *part, int ntiles, int DP,
   grad[(size_t)s * (d + 2) + d + 1] = ok ? sn * a2 : 0.0;
 }
 
+// Gradient w.r.t. the parameters of the prior mean (DESIGN.md 2.13):  d LML / d theta_c = alpha^T J[:, c],  J = dm/dtheta
+// at the training inputs, n x k column-major per sample (sample s at J + s*ldj; ldj == 0: shared).  Grid (k, S).  Thread t
+// sums alpha_i J_ic over i = t, t + 128, ... < n in ascending i, then a fixed-order tree finishes: the result depends on
+// the sample's alpha and J alone, never on the batch, window, stream group or device it was evaluated in.
+__global__ void __launch_bounds__(128) loglik_mean_grad_kernel(const double *__restrict__ alpha, int n_pad,
+                                                               const double *__restrict__ J, long long ldj, int n, int k,
+                                                               const int *__restrict__ status, double *__restrict__ grad_mean) {
+  __shared__ double red[128];
+  const int c = blockIdx.x, s = blockIdx.y, t = threadIdx.x;
+  const double *a = alpha + (size_t)s * n_pad;
+  const double *Jc = J + (size_t)s * ldj + (size_t)c * n;
+  double acc = 0.0;
+  for (int i = t; i < n; i += 128) acc = fma(a[i], Jc[i], acc);
+  red[t] = acc;
+  __syncthreads();
+#pragma unroll
+  for (int w = 64; w > 0; w >>= 1) {
+    if (t < w) red[t] += red[t + w];
+    __syncthreads();
+  }
+  if (t == 0) grad_mean[(size_t)s * k + c] = status[s] == 0 ? red[0] : 0.0;   // not PD: alpha is garbage, the gradient 0
+}
+
 }  // namespace boss

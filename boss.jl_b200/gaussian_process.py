@@ -213,29 +213,46 @@ def data_loglike(model, data: ExperimentData):
 
 
 def data_loglike_and_grad(model, data: ExperimentData):
-    """(params | list of params) -> (loglik, grad): the data log-likelihood and its gradient w.r.t. the GP
-    hyper-parameters as GaussianProcessParams-shaped arrays (d lengthscales x y_dim, amplitudes, noise_std).
-    What `AutoForwardDiff` gives OptimizationMAP / NUTS in the reference (src/model_fitters/optimization.jl:41,153),
-    evaluated as one batched device call per output slice.  GaussianProcess models only (a Semiparametric
-    model's theta-gradient would need the user's predict closure differentiated on the host)."""
-    if isinstance(model, Semiparametric):
-        raise NotImplementedError("data_loglike_and_grad: GaussianProcess models only")
+    """(params | list of params) -> (loglik, grad): the data log-likelihood and its gradient w.r.t. the model
+    parameters, shaped like the parameters: GaussianProcessParams (d lengthscales x y_dim, amplitudes, noise_std), or
+    SemiparametricParams with d/dtheta in front.  What `AutoForwardDiff` gives OptimizationMAP / NUTS in the reference
+    (src/model_fitters/optimization.jl:41,153), evaluated as one batched device call per output slice.
+    A Semiparametric model needs Parametric(jacobian=...): its theta-gradient is alpha^T J summed over the output slices,
+    J the Jacobian of the parametric mean at the training inputs (boss_gp_loglik_grad_batch_mean)."""
+    semi = isinstance(model, Semiparametric)
+    if semi and model.parametric.jacobian is None:
+        raise NotImplementedError("data_loglike_and_grad: a Semiparametric model needs Parametric(jacobian=...)")
+    gp_model = model.nonparametric if semi else model
 
     def llg(params):
         single = not isinstance(params, (list, tuple))
         plist = [params] if single else list(params)
-        S, d = len(plist), data.x_dim
+        S, d, n = len(plist), data.x_dim, data.X.shape[1]
         total = np.zeros(S)
         grads = [GaussianProcessParams(np.zeros((d, data.y_dim)), np.zeros(data.y_dim), np.zeros(data.y_dim))
                  for _ in range(S)]
-        kid, mask = _kernel_parts(model.kernel)
+        kid, mask = _kernel_parts(gp_model.kernel)
+        if semi:
+            k = len(plist[0].theta)
+            jac = model.parametric.jacobian
+            # S x n x y_dim x k: d predict / d theta of every sample at every training input
+            Jall = np.array([[np.asarray(jac(data.X[:, j], p.theta), dtype=np.float64).reshape(data.y_dim, k)
+                              for j in range(n)] for p in plist])
+            grads = [SemiparametricParams(np.zeros(k), g.lengthscales, g.amplitudes, g.noise_std) for g in grads]
         for i in range(data.y_dim):
-            m = model.mean_at(i, data.X)
-            Ymm = data.Y[i] if m is None else data.Y[i] - m
             L = np.stack([p.lengthscales[:, i] for p in plist])
             A = np.array([p.amplitudes[i] for p in plist])
             N = np.array([p.noise_std[i] for p in plist])
-            ll, g = _lib.loglik_grad_batch(data.X, Ymm, L, A, N, kid, mask)
+            if semi:
+                Ymm = np.stack([data.Y[i] - _as_gp(model, p)[0].mean_at(i, data.X) for p in plist])   # as data_loglike
+                J = Jall[:, :, i, :].transpose(0, 2, 1)                                               # S x k x n
+                ll, g, gm = _lib.loglik_grad_batch_mean(data.X, Ymm, J, L, A, N, kid, mask)
+                for s in range(S):
+                    grads[s].theta += gm[s]
+            else:
+                m = model.mean_at(i, data.X)
+                Ymm = data.Y[i] if m is None else data.Y[i] - m
+                ll, g = _lib.loglik_grad_batch(data.X, Ymm, L, A, N, kid, mask)
             total += ll
             for s in range(S):
                 grads[s].lengthscales[:, i] = g[s, :d]
@@ -255,11 +272,15 @@ class SemiparametricParams:
 
 
 class Parametric:
-    """Minimal parametric model: predict(x, theta) -> y (src/models/parametric.jl); evaluated on the host."""
+    """Minimal parametric model: predict(x, theta) -> y (src/models/parametric.jl); evaluated on the host.
+    jacobian(x, theta), optional: the (y_dim, k) array d predict / d theta at one point -- the mirror's stand-in for the
+    ForwardDiff sweep through `predict`.  With it, a Semiparametric model has data_loglike_and_grad and gradient
+    OptimizationMAP."""
 
-    def __init__(self, predict: Callable, theta_priors: Optional[List[Prior]] = None):
+    def __init__(self, predict: Callable, theta_priors: Optional[List[Prior]] = None, jacobian: Optional[Callable] = None):
         self.predict = predict
         self.theta_priors = theta_priors
+        self.jacobian = jacobian
 
 
 class Semiparametric:

@@ -25,7 +25,9 @@ class OptimizationMAP:
       "lbfgs"    gradient-based (the reference's default autodiff = AutoForwardDiff(), optimization.jl:41,153): batched
                  L-BFGS in log-parameter space on boss_gp_loglik_grad_batch (value + analytic gradient of the data
                  log-likelihood for all starts at once; the prior term's gradient is a host-side central difference).
-                 GaussianProcess models; a Semiparametric model falls back to "compass".
+                 GaussianProcess models, and Semiparametric models whose Parametric has a `jacobian` (theta enters raw,
+                 its gradient from boss_gp_loglik_grad_batch_mean); a Semiparametric model without one falls back to
+                 "compass".
       "compass"  derivative-free compass search in log space (what NEWUOA / BOBYQA are used for in the examples)."""
 
     def __init__(self, multistart=20, iters: int = 40, step0: float = 0.5, seed: Optional[int] = None,
@@ -161,8 +163,9 @@ def estimate_parameters(fitter, problem: BossProblem, options: BossOptions = Bos
             b = int(np.argmax(f0))
             return MAPParams(starts[b], float(f0[b]))
         _devectorize_rows = lambda rows, owners: [_devec_free(o, v) for v, o in zip(rows, owners)]
-        if fitter.algorithm == "lbfgs" and not isinstance(model, Semiparametric):
-            return _lbfgs_map(fitter, model, data, V, free, tmpl, _devec_free, return_all)
+        if fitter.algorithm == "lbfgs" and (not isinstance(model, Semiparametric) or model.parametric.jacobian is not None):
+            lo, hi = _search_box(model, V0)
+            return _lbfgs_map(fitter, model, data, V, free, tmpl, _devec_free, return_all, lo[free], hi[free])
         f = ll(_devectorize_rows(V, range(S)))
         step = np.full(S, fitter.step0)
         for _ in range(fitter.iters):
@@ -191,10 +194,32 @@ def estimate_parameters(fitter, problem: BossProblem, options: BossOptions = Bos
     raise TypeError(f"unsupported model fitter {type(fitter).__name__}")
 
 
-def _lbfgs_map(fitter, model, data, V, free, tmpl, devec_free, return_all):
-    """Gradient OptimizationMAP: maximise data_loglike + params_loglike over the free log-parameters of all starts with
-    the batched L-BFGS of acquisition_maximizers.batched_lbfgs_maximize.  One value + gradient evaluation of all
-    unfinished starts = one boss_gp_loglik_grad_batch call per output slice."""
+def _search_box(model, V0):
+    """Box of the gradient search over the whole vectorised parameters (_vectorize order), from the starts V0 (S x P_all).
+    batched_lbfgs_maximize needs a finite box, and its first trial step is a tenth of the widest side.  The log-parameters
+    get [-30, 30] (e^30: effectively unbounded).  theta enters raw, on a scale only the starts reveal: it gets
+    [min over starts - 30, max over starts + 30], cut to the support of a Uniform prior (outside it the prior term is
+    -inf).  Its sides are 60 + the spread of the starts in that entry, so starts spread wider than a few units (a wide
+    Normal prior) enlarge the first trial step of every entry, log-parameters included; the Armijo backtracking then
+    halves the step until it is accepted, at the cost of extra evaluations in the first rounds."""
+    from .types import Uniform
+    lo = np.full(V0.shape[1], -30.0)
+    hi = np.full(V0.shape[1], 30.0)
+    if isinstance(model, Semiparametric):
+        k = len(model.parametric.theta_priors)
+        lo[:k] = V0[:, :k].min(axis=0) - 30.0
+        hi[:k] = V0[:, :k].max(axis=0) + 30.0
+        for c, pr in enumerate(model.parametric.theta_priors):
+            if isinstance(pr, Uniform):
+                lo[c], hi[c] = max(lo[c], pr.lo), min(hi[c], pr.hi)
+    return lo, hi
+
+
+def _lbfgs_map(fitter, model, data, V, free, tmpl, devec_free, return_all, lo, hi):
+    """Gradient OptimizationMAP: maximise data_loglike + params_loglike over the free parameters of all starts (log
+    scale for lambda, alpha, sigma; raw theta) inside the box [lo, hi] with the batched L-BFGS of
+    acquisition_maximizers.batched_lbfgs_maximize.  One value + gradient evaluation of all unfinished starts = one
+    boss_gp_loglik_grad_batch (Semiparametric: boss_gp_loglik_grad_batch_mean) call per output slice."""
     from .acquisition_maximizers import batched_lbfgs_maximize
     llg = data_loglike_and_grad(model, data)
     pll = model.params_loglike()
@@ -221,8 +246,11 @@ def _lbfgs_map(fitter, model, data, V, free, tmpl, devec_free, return_all):
         ll_d, grads = llg(plist)
         f = np.empty(len(cols)); G = np.zeros((P, len(cols)))
         for c, (s, p) in enumerate(zip(cols, plist)):
-            full = np.concatenate([grads[c].lengthscales.ravel(order="F") * p.lengthscales.ravel(order="F"),
-                                   grads[c].amplitudes * p.amplitudes, grads[c].noise_std * p.noise_std])   # d/d log(theta)
+            parts = [grads[c].lengthscales.ravel(order="F") * p.lengthscales.ravel(order="F"),
+                     grads[c].amplitudes * p.amplitudes, grads[c].noise_std * p.noise_std]          # d/d log(lambda, alpha, sigma)
+            if isinstance(p, SemiparametricParams):
+                parts.insert(0, grads[c].theta)                                                     # theta is not log-scaled
+            full = np.concatenate(parts)
             pr, gpr = prior_and_grad(p, Z[:, c], s)
             f[c] = ll_d[c] + pr if np.isfinite(pr) else -np.inf
             G[:, c] = full[free] + gpr
@@ -230,7 +258,6 @@ def _lbfgs_map(fitter, model, data, V, free, tmpl, devec_free, return_all):
 
     # batched_lbfgs_maximize calls value_and_grad on the columns of the unfinished starts; it needs to know which
     # starts those are (Dirac-pinned entries are rebuilt per start), so the driver publishes the active set
-    lo = np.full(P, -30.0); hi = np.full(P, 30.0)          # log-parameters: an effectively unbounded box
     X, f = batched_lbfgs_maximize(value_and_grad, V.T.copy(), lo, hi, iters=fitter.iters, publish_active=value_and_grad)
     if np.all(np.isneginf(f)):
         raise RuntimeError("All optimization runs failed!")

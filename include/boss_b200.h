@@ -328,6 +328,28 @@ int boss_gp_loglik_grad_batch_dev(const double *X_dev, int d, int n, const doubl
                                   const double *noise_std_dev, int kernel_id, const uint8_t *discrete_mask,
                                   int64_t S, double *loglik_dev, double *grad_dev, void *stream);
 
+/* Same batch and outputs, plus the gradient w.r.t. the parameters theta of a parametric prior mean m(x; theta) -- the
+ * Semiparametric model's part of what ForwardDiff differentiates in OptimizationMAP / NUTS:
+ *   d LML / d theta_c = alpha^T J[:, c],   alpha = K^-1 (y - m(X; theta)),   J = dm(X; theta)/dtheta   (DESIGN.md 2.13)
+ * The caller differentiates m on the host (ForwardDiff.jacobian's n x k layout) and passes Y_minus_mean per sample.
+ *   mean_jac   n x k column-major per sample (element (i, c) at i + c*n), sample s at mean_jac + s*ldj;
+ *              ldj == 0: one Jacobian shared by all samples (a mean linear in theta)
+ *   grad_mean  S x k, sample s at grad_mean + s*k: sum over the n rows of alpha_i J_ic; zeros where the sample is not
+ *              positive definite
+ * loglik and grad equal boss_gp_loglik_grad_batch's bit for bit, and a sample's grad_mean does not depend on the batch it
+ * is evaluated in.  BOSS_ERR_ARG also for k < 1, a NULL grad / mean_jac / grad_mean, and 0 < ldj < k*n. */
+int boss_gp_loglik_grad_batch_mean(const double *X, int d, int n, const double *Y_minus_mean, int64_t ldy,
+                                   const double *mean_jac, int k, int64_t ldj,
+                                   const double *lengthscales, const double *amplitude, const double *noise_std,
+                                   int kernel_id, const uint8_t *discrete_mask, int64_t S,
+                                   double *loglik, double *grad, double *grad_mean);
+int boss_gp_loglik_grad_batch_mean_dev(const double *X_dev, int d, int n, const double *Y_minus_mean_dev, int64_t ldy,
+                                       const double *mean_jac_dev, int k, int64_t ldj,
+                                       const double *lengthscales_dev, const double *amplitude_dev,
+                                       const double *noise_std_dev, int kernel_id, const uint8_t *discrete_mask,
+                                       int64_t S, double *loglik_dev, double *grad_dev, double *grad_mean_dev,
+                                       void *stream);
+
 /* ---- instrumentation ---------------------------------------------------------------------
  * CUDA-event time (ms) of the dominant kernel class inside the last scoring / loglik call, and the
  * number of kernel launches the library has issued since boss_init (bench.py's gpu_launches). */

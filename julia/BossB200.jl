@@ -28,6 +28,7 @@
 #   maximize_acquisition(::SequentialBatchAM) (batch.jl:26-38)                          -> boss_gp_append
 #   estimate_parameters(::SamplingMAP)    (model_fitters/sampling.jl:17-78)             -> boss_gp_loglik_batch
 #   data_loglike + ForwardDiff gradient   (model_fitters/optimization.jl:41,153)        -> boss_gp_loglik_grad_batch
+#     (Semiparametric: θ through ForwardDiff.jacobian of the parametric mean)             -> boss_gp_loglik_grad_batch_mean
 #   acq(x::Vector{<:ForwardDiff.Dual})    (acquisition_maximizers/optimization.jl:36)   -> boss_ei_value_grad /
 #                                                                                          boss_mcei_value_grad
 module BossB200
@@ -512,6 +513,42 @@ function data_loglike_grad_batch(model::GaussianProcess, data::ExperimentData, p
         total .+= ll
         for s in 1:S
             grads[s][1][:, i] .= G[1:d, s]; grads[s][2][i] = G[d + 1, s]; grads[s][3][i] = G[d + 2, s]
+        end
+    end
+    return total, grads
+end
+
+"The same for a Semiparametric model, plus the gradient w.r.t. the parametric mean's θ (DESIGN.md 2.13): per output
+slice, δ = y - m(X; θ) and the n × k Jacobian J = ∂m(X; θ)/∂θ of every sample (ForwardDiff.jacobian, the layout the C
+ABI takes) go to one boss_gp_loglik_grad_batch_mean call, which returns αᵀJ beside the (λ, α, σ) gradient; dθ is summed
+over the slices.  Returns (loglik::Vector, grads::Vector of (dθ, dλ d×y_dim, dα, dσ)).
+No Julia installation was available when this method was written: it has been reviewed, not run."
+function data_loglike_grad_batch(model::Semiparametric, data::ExperimentData, ps::AbstractVector{<:SemiparametricParams})
+    supported(model) || throw(ArgumentError("data_loglike_grad_batch: the nonparametric part must be a GaussianProcess " *
+                                            "with an SE / Matern32 / Matern52 kernel (possibly discrete)"))
+    g = gp_part(model)
+    X = Matrix{Float64}(data.X)
+    d, n = size(X)
+    S = length(ps); yd = y_dim(data); k = length(ps[1].θ)
+    total = zeros(S)
+    grads = [(zeros(k), zeros(d, yd), zeros(yd), zeros(yd)) for _ in 1:S]
+    mask = discrete_mask(g.kernel)
+    for i in 1:yd
+        L = Matrix{Float64}(reduce(hcat, [p.λ[:, i] for p in ps])); A = Float64[p.α[i] for p in ps]; N = Float64[p.σ[i] for p in ps]
+        Ys = reduce(hcat, [Vector{Float64}(data.Y[i, :]) .- eval_mean(slice_mean(model, p, i), X) for p in ps])   # n x S
+        Js = Array{Float64}(undef, n, k, S)
+        for (s, p) in enumerate(ps)
+            Js[:, :, s] .= ForwardDiff.jacobian(θ -> [model.parametric(x, θ)[i] for x in eachcol(X)], p.θ)
+        end
+        ll = Vector{Float64}(undef, S); G = Matrix{Float64}(undef, d + 2, S); Gm = Matrix{Float64}(undef, k, S)
+        GC.@preserve X Ys Js L A N mask check(ccall((:boss_gp_loglik_grad_batch_mean, LIB), Cint,
+            (Ptr{Cdouble}, Cint, Cint, Ptr{Cdouble}, Int64, Ptr{Cdouble}, Cint, Int64, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble},
+             Cint, Ptr{UInt8}, Int64, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}),
+            X, d, n, Ys, n, Js, k, k * n, L, A, N, kernel_id(g.kernel), cptr(mask), S, ll, G, Gm))
+        total .+= ll
+        for s in 1:S
+            grads[s][1] .+= Gm[:, s]
+            grads[s][2][:, i] .= G[1:d, s]; grads[s][3][i] = G[d + 1, s]; grads[s][4][i] = G[d + 2, s]
         end
     end
     return total, grads

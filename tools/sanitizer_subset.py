@@ -5,7 +5,7 @@
     compute-sanitizer --tool racecheck --error-exitcode 1 python tools/sanitizer_subset.py --tiny
 
 Families: build_k, potrf_tile (+ fused diagonal step), chol_trsm, chol_update, chol_panel, chol_update_rl, trtri_*_rl,
-trtri_fused, kinv_wtw, loglik_grad_tile, loglik_small (warp path), matvec, xcov, score_trmm (plain and row-split),
+trtri_fused, kinv_wtw, loglik_grad_tile, loglik_mean_grad, loglik_small (warp path), matvec, xcov, score_trmm (plain and row-split),
 wtv, grad (+ MC-EI gradient, + posterior gradients), acq (+ MC-EI), argmax, top-k, cov (gemm_nt + cov_finish), candidate generators, append (+ capacity growth),
 multi-start driver.  Results are checked against the oracle so that a run that "passes" the sanitizer by computing
 nothing is caught.  Prints one JSON line.
@@ -116,9 +116,16 @@ def main():
     llr, grr = O.gp_loglik_grad_batch(X, Y[0], L, A, N, 0)
     assert relerr(llg, llr) <= 1e-8
     assert np.max(np.abs(gr - grr) / np.linalg.norm(grr, axis=1, keepdims=True)) <= 1e-8
+    # prior-mean gradient (loglik_mean_grad_kernel), per-sample Jacobians: loglik and grad unchanged, alpha^T J
+    from tests import loglik_mean_grad_oracle as MG
+    Jm = np.random.default_rng(8).standard_normal((S, 3, n))
+    llm, grm, gmm = _lib.loglik_grad_batch_mean(X, Y[0], Jm, L, A, N, 0)
+    assert np.array_equal(llm, llg) and np.array_equal(grm, gr)
+    _, gmr = MG.gp_loglik_mean_grad_batch(X, Y[0], Jm, L, A, N, 0)
+    assert np.max(np.abs(gmm - gmr) / np.linalg.norm(gmr, axis=1, keepdims=True)) <= 1e-9
     fb = _lib.gp_fit_batch(X, Y[0], L[:3], A[:3], N[:3], 2)
     assert all(g is not None for g in fb)
-    done.append("loglik+grad+fit_batch")
+    done.append("loglik+grad+mean_grad+fit_batch")
     # --- warp-register small-n path ---
     Xsm, Ysm, _, _, _ = make_problem(24, 2, seed=4)
     Ls, As, Ns = make_hyper_samples(40, 2, seed=5)
