@@ -100,6 +100,7 @@ EXPORTS = {
     "boss_dbg_screen_ambiguous": (C.c_int, [_i64p]),
     "boss_dbg_screen_mean": (C.c_int, [_vp, _vp, C.c_int64, _vp, _vp, _vp]),
     "boss_dbg_kappa_f32": (C.c_int, [C.c_int, _vp, C.c_int, _vp]),
+    "boss_dbg_mma_d2": (C.c_int, [C.c_int, _vp, _vp, _vp, _vp, C.c_int, C.c_int, _vp]),
 }
 for _name, (_res, _args) in EXPORTS.items():
     _f = getattr(lib, _name)          # AttributeError here = header and library disagree
@@ -767,4 +768,16 @@ def dbg_kappa_f32(kid, r):
     r = _f64(r)
     out = np.empty_like(r)
     _check(lib.boss_dbg_kappa_f32(int(kid), _ptr(r), r.size, _ptr(out)), "boss_dbg_kappa_f32")
+    return out
+
+
+def dbg_mma_d2(dp, u, t, nu, nt):
+    """The FP32 tier's tensor-core d2 = nu + nt - 2 u.t (before the clamp at 0) for FP32 points u (m x kp, m a
+    multiple of 16) and t (n x kp, n a multiple of 8), kp = dp rounded up to the kernels' 8, 16 or 32."""
+    u, t = np.ascontiguousarray(u, np.float32), np.ascontiguousarray(t, np.float32)
+    nu, nt = np.ascontiguousarray(nu, np.float32), np.ascontiguousarray(nt, np.float32)
+    m, n = u.shape[0], t.shape[0]
+    out = np.empty((m, n), np.float32)
+    _check(lib.boss_dbg_mma_d2(int(dp), u.ctypes.data, t.ctypes.data, nu.ctypes.data, nt.ctypes.data, m // 16, n // 8,
+                               out.ctypes.data), "boss_dbg_mma_d2")
     return out

@@ -1758,7 +1758,7 @@ struct Screen {
   unsigned long long *tk[2] = {};
   long long *base = nullptr, *pool_idx = nullptr;
   unsigned char *seed_cm = nullptr, *pool_cm = nullptr, *pool_ver = nullptr;
-  std::vector<float *> xt32, al32;   // per slice: FP32 copies of the scaled training inputs (negated) and of alpha
+  std::vector<float *> xt32, al32;   // per slice: the MMA tier's B fragments of the centred training inputs, |t~|^2 and alpha
 
   bool on() const { return state == SCREENING; }
 
@@ -1788,11 +1788,12 @@ struct Screen {
     const size_t o_tk0 = take(tot, ntk * 8), o_tk1 = take(tot, ntk * 8), o_ti0 = take(tot, ntk * 4), o_ti1 = take(tot, ntk * 4);
     const size_t o_sx = take(tot, (size_t)ns_max * d * 8), o_spm = take(tot, (size_t)ns_max * y_dim * 8), o_scm = take(tot, ns_max);
     const size_t o_rx = take(tot, (size_t)CH * d * 8), o_rpm = take(tot, pm ? (size_t)CH * y_dim * 8 : 0);
-    const size_t o_rrow = take(tot, (size_t)CH * 4), o_rcnt = take(tot, 8), o_consts = take(tot, (size_t)c.nsl * 16);
+    const size_t o_rrow = take(tot, (size_t)CH * 4), o_rcnt = take(tot, 8);
+    const size_t o_consts = take(tot, (size_t)c.nsl * SCREEN_NCONST * 8);
     std::vector<size_t> o_xt(c.nsl), o_al(c.nsl);
     for (int q = 0; q < c.nsl; ++q) {
-      o_xt[q] = take(tot, f32 ? (size_t)c.sl[q]->n_pad * c.sl[q]->dp * 4 : 0);
-      o_al[q] = take(tot, f32 ? (size_t)c.sl[q]->n_pad * 4 : 0);
+      o_xt[q] = take(tot, f32 ? (size_t)c.sl[q]->n_pad * ((c.sl[q]->dp + 7) / 8 * 8) * 8 : 0);
+      o_al[q] = take(tot, f32 ? (size_t)c.sl[q]->n_pad * 8 : 0);
     }
     CUDA_TRY(C().scr_misc.ensure(tot));
     unsigned char *b = C().scr_misc.as<unsigned char>();
@@ -1818,7 +1819,8 @@ struct Screen {
       const boss_gp *h = c.sl[q];
       xt32[q] = reinterpret_cast<float *>(b + o_xt[q]);
       al32[q] = reinterpret_cast<float *>(b + o_al[q]);
-      screen_consts_kernel<<<1, 1024, 0, C().stream>>>(h->Xt, h->alpha, h->n_pad, h->dp, xt32[q], al32[q], consts + 2 * q);
+      screen_consts_kernel<<<1, 1024, 0, C().stream>>>(h->Xt, h->alpha, h->n, h->n_pad, h->dp, xt32[q], al32[q],
+                                                       consts + (size_t)SCREEN_NCONST * q);
       ++C().launches;
     }
     tot = 0;
@@ -1855,12 +1857,15 @@ struct Screen {
       {
         Timed t(1);
         if (t32)
-          launch_xcov_mean_f32(h->kernel_id, h->dp, XcovF32Params{xp, xt32[q], al32[q], consts + 2 * q,
-                                                                  C().sumsq.as<double>() + (size_t)q * c.CH},
+          launch_xcov_mean_f32(h->kernel_id, h->dp,
+                               XcovF32Params{xp, reinterpret_cast<const float4 *>(xt32[q]),
+                                             reinterpret_cast<const float4 *>(al32[q]), consts + (size_t)SCREEN_NCONST * q,
+                                             C().sumsq.as<double>() + (size_t)q * c.CH},
                                dim3(ncb, nks), C().stream);
         else
           launch_xcov_mean(h->kernel_id, h->dp, xp, dim3(ncb, nks), C().stream);
       }
+      if (t32 && q == c.nsl - 1) break;   // the tail kernel sums the last slice's partials
       reduce_rows_kernel<<<(ncb * 128 + 255) / 256, 256, 0, C().stream>>>(C().part_mu.as<double>(), 2 * h->nblk, (size_t)c.CH,
                                                                         C().muv.as<double>() + (size_t)q * c.CH, ncb * 128);
     }
@@ -1873,17 +1878,18 @@ struct Screen {
     bp.out_off = m0;
     bp.blk_val = nullptr;
     bp.blk_idx = nullptr;
-    if (t32) {   // muv <- mu~ + E', sumsq <- mu~ - E'; bound = EI at the first (hi), lo = EI at the second
-      BandParams bd{C().muv.as<double>(), C().sumsq.as<double>(), c.nsl, a.y_dim, c.CH, ch, {}};
-      for (int i = 0; i < a.y_dim; ++i) bd.coefs[i] = ap.coefs[i];
-      screen_band_kernel<<<nb, 256, 0, C().stream>>>(bd);
+    // FP32 tier: hi < thr (1 - 2^-32) drops, lo >= thr (1 + 2^-32) keeps, anything else (NaN too) is ambiguous.  The
+    // first chunk (FP64 tier) sets thr in seed().
+    if (t32) {   // muv <- mu~ + E', sumsq <- mu~ - E'; bound = EI at the first (hi), lo = EI at the second; the counts
+      TailParams tp{bp, bp, C().part_mu.as<double>(), 2 * c.sl[c.nsl - 1]->nblk, c.nsl, thr * (1.0 - 0x1p-32), cnt};
+      tp.lo.mu = C().sumsq.as<double>();
+      tp.lo.acq = lo;
+      screen_tail_kernel<<<nb, 256, 0, C().stream>>>(tp);
+      C().launches += 2 * c.nsl;
+    } else {
       acq_kernel<<<nb, 256, 0, C().stream>>>(bp);
-      bp.mu = C().sumsq.as<double>();
-      bp.acq = lo;
-      C().launches += 2;
+      C().launches += 2 * c.nsl + 1;
     }
-    acq_kernel<<<nb, 256, 0, C().stream>>>(bp);
-    C().launches += 2 * c.nsl + 1;
     const size_t c0 = (size_t)(m0 - ap.in_off);   // the chunk's first candidate in the input arrays
     const double *xs_c = ap.Xs + c0 * c.d;
     const double *pm_c = ap.prior_mean ? ap.prior_mean + c0 * a.y_dim : nullptr;
@@ -1892,13 +1898,15 @@ struct Screen {
       int rc = seed(c, ch, xs_c, pm_c, cm_c, tb);
       if (rc || !on()) return rc;
     }
-    // FP32 tier: hi < thr (1 - 2^-32) drops, lo >= thr (1 + 2^-32) keeps, anything else (NaN too) is ambiguous
     const double thr_drop = t32 ? thr * (1.0 - 0x1p-32) : thr;
-    screen_count_kernel<<<nb, 256, 0, C().stream>>>(bound, nullptr, ch, thr_drop, cnt);
+    if (!t32) {
+      screen_count_kernel<<<nb, 256, 0, C().stream>>>(bound, nullptr, ch, thr_drop, cnt);
+      ++C().launches;
+    }
     CompactParams cpar{bound, nullptr, ch, thr_drop, t32 ? lo : nullptr, thr * (1.0 + 0x1p-32), cnt, m0, xs_c, pm_c, cm_c,
                        c.d, a.y_dim, base, cidx & 1, pool_x, pool_pm, pool_cm, pool_idx, nullptr, pool_bound, pool_ver};
     screen_compact_kernel<<<nb, 256, 0, C().stream>>>(cpar);
-    C().launches += 2;
+    ++C().launches;
     if (cidx == 0) {
       long long surv = 0;
       CUDA_TRY(cudaMemcpyAsync(&surv, base + 1, 8, cudaMemcpyDeviceToHost, C().stream));
@@ -3637,14 +3645,17 @@ int boss_dbg_screen_mean(const boss_gp *gp, const double *Xs, int64_t M, double 
   CUDA_TRY(cudaMalloc(&dx, (size_t)M * d * 8));
   CUDA_TRY(cudaMalloc(&dpart, (size_t)2 * gp->nblk * ld * 8));
   CUDA_TRY(cudaMalloc(&dout, (size_t)3 * ld * 8));
-  CUDA_TRY(cudaMalloc(&dA, 16));
-  CUDA_TRY(cudaMalloc(&dxt, (size_t)gp->n_pad * gp->dp * 4));
-  CUDA_TRY(cudaMalloc(&dal, (size_t)gp->n_pad * 4));
+  CUDA_TRY(cudaMalloc(&dA, SCREEN_NCONST * 8));
+  CUDA_TRY(cudaMalloc(&dxt, (size_t)gp->n_pad * ((gp->dp + 7) / 8 * 8) * 8));
+  CUDA_TRY(cudaMalloc(&dal, (size_t)gp->n_pad * 8));
   CUDA_TRY(cudaMemcpyAsync(dx, Xs, (size_t)M * d * 8, cudaMemcpyHostToDevice, C().stream));
-  screen_consts_kernel<<<1, 1024, 0, C().stream>>>(gp->Xt, gp->alpha, gp->n_pad, gp->dp, dxt, dal, dA);
+  screen_consts_kernel<<<1, 1024, 0, C().stream>>>(gp->Xt, gp->alpha, gp->n, gp->n_pad, gp->dp, dxt, dal, dA);
   XcovParams xp = xcov_params(gp, dx, M, 0, 0, d, ld);
   xp.mu_part = dpart;
-  launch_xcov_mean_f32(gp->kernel_id, gp->dp, XcovF32Params{xp, dxt, dal, dA, dout + ld}, dim3(ncb, nks), C().stream);
+  launch_xcov_mean_f32(gp->kernel_id, gp->dp,
+                       XcovF32Params{xp, reinterpret_cast<const float4 *>(dxt), reinterpret_cast<const float4 *>(dal), dA,
+                                     dout + ld},
+                       dim3(ncb, nks), C().stream);
   reduce_rows_kernel<<<(ld + 255) / 256, 256, 0, C().stream>>>(dpart, 2 * gp->nblk, (size_t)ld, dout, ld);
   launch_xcov_mean(gp->kernel_id, gp->dp, xp, dim3(ncb, nks), C().stream);
   reduce_rows_kernel<<<(ld + 255) / 256, 256, 0, C().stream>>>(dpart, 2 * gp->nblk, (size_t)ld, dout + 2 * ld, ld);
@@ -3680,6 +3691,35 @@ int boss_dbg_kappa_f32(int kid, const double *r, int n, double *out) {
   CUDA_TRY(cudaStreamSynchronize(C().stream));
   cudaFree(dr);
   cudaFree(dout);
+  return 0;
+}
+
+int boss_dbg_mma_d2(int dp, const float *u, const float *t, const float *nu, const float *nt, int mt, int nt_tiles,
+                    float *d2) {
+  REQUIRE_INIT();
+  if (dp < 1 || dp > 32 || mt < 1 || nt_tiles < 1 || mt > 4096 || nt_tiles > 4096 || !u || !t || !nu || !nt || !d2)
+    return fail(BOSS_ERR_ARG, "boss_dbg_mma_d2: bad argument");
+  const int dpp = dp <= 8 ? 8 : dp <= 16 ? 16 : 32;   // the kernels' k-steps: padded dimensions 2-8, 12-16, 32
+  const size_t m = (size_t)16 * mt, n = (size_t)8 * nt_tiles;
+  float *du, *dt, *dnu, *dnt, *dd;
+  CUDA_TRY(cudaMalloc(&du, m * dpp * 4));
+  CUDA_TRY(cudaMalloc(&dt, n * dpp * 4));
+  CUDA_TRY(cudaMalloc(&dnu, m * 4));
+  CUDA_TRY(cudaMalloc(&dnt, n * 4));
+  CUDA_TRY(cudaMalloc(&dd, m * n * 4));
+  CUDA_TRY(cudaMemcpyAsync(du, u, m * dpp * 4, cudaMemcpyHostToDevice, C().stream));
+  CUDA_TRY(cudaMemcpyAsync(dt, t, n * dpp * 4, cudaMemcpyHostToDevice, C().stream));
+  CUDA_TRY(cudaMemcpyAsync(dnu, nu, m * 4, cudaMemcpyHostToDevice, C().stream));
+  CUDA_TRY(cudaMemcpyAsync(dnt, nt, n * 4, cudaMemcpyHostToDevice, C().stream));
+  launch_mma_d2(dpp, du, dt, dnu, dnt, mt, nt_tiles, dd, C().stream);
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaMemcpyAsync(d2, dd, m * n * 4, cudaMemcpyDeviceToHost, C().stream));
+  CUDA_TRY(cudaStreamSynchronize(C().stream));
+  cudaFree(du);
+  cudaFree(dt);
+  cudaFree(dnu);
+  cudaFree(dnt);
+  cudaFree(dd);
   return 0;
 }
 

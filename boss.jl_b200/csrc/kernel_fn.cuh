@@ -129,6 +129,16 @@ __device__ __forceinline__ float kappa_f32(float d2) {
   }
 }
 
+// x = hi + lo + r with hi, lo TF32 (round to nearest, ties away): |x - hi| <= 2^-11 |x|, |r| <= 2^-22 |x|.  x - hi is
+// exact in FP32.  Non-finite x gives lo = NaN.
+__device__ __forceinline__ void tf32_split(float x, float &hi, float &lo) {
+  unsigned h, l;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(h) : "f"(x));
+  hi = __uint_as_float(h);
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(l) : "f"(x - hi));
+  lo = __uint_as_float(l);
+}
+
 // (d kappa / d r) / r as a function of d2 = r^2 : finite at r = 0 for all three kernels.
 template <int KID>
 __device__ __forceinline__ double kappa_dr_over_r(double d2) {

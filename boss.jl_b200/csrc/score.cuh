@@ -363,21 +363,47 @@ __global__ void __launch_bounds__(256) screen_count_kernel(const double *bound, 
 
 // ---- the FP32 mean tier (DESIGN.md 2.9) ----
 
-// Per call and slice: the FP32 copies of the scaled training inputs (negated) and of alpha, and the constants of the
-// error bound, A1 = sum_j |alpha_j| and A2 = sum_j |alpha_j| |ut_j|, summed in a fixed order (one CTA of 1024 threads).
-__global__ void __launch_bounds__(1024) screen_consts_kernel(const double *Xt, const double *alpha, int n_pad, int DP,
-                                                             float *xt_neg, float *al, double *A) {
+// Per call and slice (one CTA of 1024 threads, every sum in a fixed order): the centre c = the mean of the n scaled
+// training inputs; the FP32 copies the MMA tier reads (XcovF32Params: the TF32-split B fragments of t~ = fp32(ut - c),
+// |t~|^2 and alpha); and the constants of the error bound, A1 = sum_j |alpha_j| and A3 = sum_j |alpha_j| |ut_j - c|^2.
+// A = [A1, A3, c_0 .. c_{DP-1}].
+__global__ void __launch_bounds__(1024) screen_consts_kernel(const double *Xt, const double *alpha, int n, int n_pad,
+                                                             int DP, float *tfrag, float *tn_al, double *A) {
   __shared__ double s1[1024], s2[1024];
-  const int tid = threadIdx.x;
-  for (int e = tid; e < n_pad * DP; e += 1024) xt_neg[e] = -(float)Xt[e];
+  __shared__ double wsum[32][32], cen[32];
+  const int tid = threadIdx.x, KS = (DP + 7) / 8;
+  for (int i = 0; i < DP; ++i) {   // per dimension: strided per-thread sums, a warp butterfly, the 32 warps in order
+    double s = 0.0;
+    for (int j = tid; j < n; j += 1024) s += Xt[(size_t)j * DP + i];
+    for (int o = 1; o < 32; o <<= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if ((tid & 31) == 0) wsum[tid >> 5][i] = s;
+  }
+  __syncthreads();
+  if (tid < DP) {
+    double s = 0.0;
+    for (int k = 0; k < 32; ++k) s += wsum[k][tid];
+    cen[tid] = s / n;
+    A[2 + tid] = cen[tid];
+  }
+  __syncthreads();
   double a1 = 0.0, a2 = 0.0;
   for (int j = tid; j < n_pad; j += 1024) {
     const double aj = fabs(alpha[j]);
     double n2 = 0.0;
-    for (int i = 0; i < DP; ++i) n2 = fma(Xt[(size_t)j * DP + i], Xt[(size_t)j * DP + i], n2);
-    al[j] = (float)alpha[j];
+    for (int i = 0; i < 8 * KS; ++i) {
+      const double v = i < DP ? Xt[(size_t)j * DP + i] - cen[i] : 0.0;
+      n2 = fma(v, v, n2);
+      float hi, lo;
+      tf32_split((float)v, hi, lo);
+      // tile j / 8, k-step i / 8, lane 4 (j % 8) + i % 4; b0 holds dimension i % 8 < 4, b1 the others
+      const size_t f = (((size_t)(j >> 3) * KS + (i >> 3)) * 32 + 4 * (j & 7) + (i & 3)) * 4 + ((i >> 2) & 1);
+      tfrag[f] = hi;
+      tfrag[f + 2] = lo;
+    }
+    tn_al[2 * j] = (float)n2;
+    tn_al[2 * j + 1] = (float)alpha[j];
     a1 += aj;
-    a2 = fma(aj, sqrt(n2), a2);
+    a2 = fma(aj, n2, a2);
   }
   s1[tid] = a1;
   s2[tid] = a2;
@@ -395,24 +421,41 @@ __global__ void __launch_bounds__(1024) screen_consts_kernel(const double *Xt, c
   }
 }
 
-// mu (mu~ of each slice) and e (its bound E) become mu~ + E' and mu~ - E', E' = E with the sign of the slice's output
-// coefficient, so that EI is at least as large at the first as at the FP64 mean and no larger at the second.  A
-// non-finite mu~ or E gives NaN for both (the candidate is then ambiguous).
-struct BandParams {
-  double *mu, *e;
-  int nsl, y_dim, ld, n;
-  double coefs[MAX_YDIM];
+// The tail of an FP32-tier chunk, one thread per candidate c:
+//  - the last slice's mean partials summed into hi.mu in reduce_rows_kernel's order (the earlier slices' are there);
+//  - per slice, mu~ (in hi.mu) and its bound E (in lo.mu) become mu~ + E' and mu~ - E', E' = E with the sign of the
+//    slice's output coefficient, so that EI is at least as large at the first as at the FP64 mean and no larger at the
+//    second; a non-finite mu~ or E gives NaN for both (the candidate is then ambiguous);
+//  - the EI bound at each (acq_candidate, into hi.acq and lo.acq);
+//  - the survivors per 256 candidates, screen_count_kernel's rule with hi.acq as the bound.
+struct TailParams {
+  AcqParams hi, lo;     // the bound pass at mu~ + E' and at mu~ - E' (same rows, chunk_ld and coefficients)
+  const double *part;   // the last slice's partials, [P][hi.chunk_ld]
+  int P, nsl;
+  double thr;           // drop threshold of the count
+  int *cnt;
 };
-__global__ void __launch_bounds__(256) screen_band_kernel(BandParams p) {
+__global__ void __launch_bounds__(256) screen_tail_kernel(TailParams p) {
   const int c = blockIdx.x * 256 + threadIdx.x;
-  if (c >= p.n) return;
-  for (int q = 0; q < p.nsl; ++q) {
-    const size_t o = (size_t)q * p.ld + c;
-    const double m = p.mu[o], E = p.coefs[q % p.y_dim] < 0.0 ? -p.e[o] : p.e[o];
-    const bool ok = isfinite(m) && isfinite(E);
-    p.mu[o] = ok ? m + E : NAN;
-    p.e[o] = ok ? m - E : NAN;
+  const long long m = p.hi.m0 + c;
+  const bool active = c < p.hi.chunk && m < p.hi.M;
+  bool keep = false;
+  if (active) {
+    double *mu = const_cast<double *>(p.hi.mu), *e = const_cast<double *>(p.lo.mu);
+    const size_t ld = (size_t)p.hi.chunk_ld;
+    mu[(size_t)(p.nsl - 1) * ld + c] = ordered_sum(p.part + c, ld, p.P);
+    for (int q = 0; q < p.nsl; ++q) {
+      const size_t o = (size_t)q * ld + c;
+      const double mq = mu[o], E = p.hi.coefs[q % p.hi.y_dim] < 0.0 ? -e[o] : e[o];
+      const bool ok = isfinite(mq) && isfinite(E);
+      mu[o] = ok ? mq + E : NAN;
+      e[o] = ok ? mq - E : NAN;
+    }
+    keep = !(acq_candidate(p.hi, c, m) < p.thr);
+    acq_candidate(p.lo, c, m);
   }
+  const int k = __syncthreads_count(keep);
+  if (threadIdx.x == 0) p.cnt[blockIdx.x] = k;
 }
 
 // The ambiguous rows (verdict 2) among pool rows [0, n) of a piece: their candidates, prior means and rows, in any order

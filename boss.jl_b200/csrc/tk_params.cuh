@@ -47,18 +47,23 @@ struct XcovParams {
 
 constexpr int XCOV_KC = 128;  // training points staged per shared-memory pass
 
-// The FP32 mean tier of argmax screening (DESIGN.md 2.9): mu~ with a proven bound E on |mu~ - mu|, from an FP32 copy
-// of the training inputs and weights.  x.Xt / x.alpha are unused; x.mu_part receives the partials (FP64, same layout).
+// The FP32 mean tier of argmax screening (DESIGN.md 2.9): mu~ with a proven bound E on |mu~ - mu|, from per-call FP32
+// copies of the centred training inputs and of alpha (screen_consts_kernel).  x.Xt / x.alpha are unused; x.mu_part
+// receives the partials (FP64, same layout).
 struct XcovF32Params {
   XcovParams x;
-  const float *Xt_neg;   // [n_pad][DP] -(scaled training inputs), rounded to FP32
-  const float *alpha;    // [n_pad] alpha rounded to FP32
-  const double *A;       // [2] A1 = sum |alpha_j|, A2 = sum |alpha_j| |ut_j|  (screen_consts_kernel)
+  const float4 *tfrag;   // [n_pad / 8][KP / 8][32] per eight-point tile, k-step and lane: the MMA's B fragments of the
+                         // centred training inputs t~ = fp32(ut - c), TF32-split: (b0 hi, b1 hi, b0 lo, b1 lo)
+  const float4 *tn_al;   // [n_pad / 2] (|t~_j|^2, alpha_j, |t~_j+1|^2, alpha_j+1) rounded to FP32
+  const double *A;       // [SCREEN_NCONST] A1 = sum |alpha_j|, A3 = sum |alpha_j| |ut_j - c|^2, the centre c (DP)
   double *E;             // [ld] the error bound of each candidate's mean
 };
-// E = a^2 2^-24 (SCREEN_C_EVAL A1 + SCREEN_L_KAPPA (|u| A1 + A2))   (DESIGN.md 2.9)
+constexpr int SCREEN_NCONST = 2 + 32;
+// E = a^2 2^-24 (SCREEN_C_EVAL A1 + L2 k (|u - c|^2 A1 + A3))   (DESIGN.md 2.9), L2 = sup |d kappa / d(d2)|, and
+// k 2^-24 (|u - c|^2 + |ut_j - c|^2) bounds the error of the tensor-core d2 with KP = DP rounded up to 8
 constexpr double SCREEN_C_EVAL = 64.0;
-constexpr double SCREEN_L_KAPPA = 0.65;
+__host__ __device__ constexpr double screen_l2(int kid) { return kid == 0 ? 0.5 : kid == 1 ? 1.5 : 5.0 / 6.0; }
+__host__ __device__ constexpr double screen_k_dot(int dp) { return 24.0 + 7.5 * (8 * ((dp + 7) / 8)); }
 
 struct CovFinishParams {
   const double *Xs;     // d x M raw candidates
@@ -107,6 +112,8 @@ bool launch_xcov(int kid, int dp, const XcovParams &p, dim3 grid, cudaStream_t s
 bool launch_xcov_mean(int kid, int dp, const XcovParams &p, dim3 grid, cudaStream_t st);   // mu partials only (p.Ks unused)
 bool launch_xcov_mean_f32(int kid, int dp, const XcovF32Params &p, dim3 grid, cudaStream_t st);
 bool launch_kappa_f32_sweep(int kid, const double *r, int n, double *out, cudaStream_t st);
+bool launch_mma_d2(int dp, const float *u, const float *t, const float *nu, const float *nt, int mt, int nt_, float *d2,
+                   cudaStream_t st);
 bool launch_cov_finish(int kid, int dp, const CovFinishParams &p, dim3 grid, cudaStream_t st);
 bool launch_grad(int kid, int dp, const GradParams &p, dim3 grid, cudaStream_t st);
 bool launch_loglik_small(int kid, int dp, const SmallLoglikParams &p, int nblocks, cudaStream_t st);

@@ -59,55 +59,156 @@ __global__ void __launch_bounds__(256) xcov_kernel(XcovParams p) {
   }
 }
 
-// The FP32 mean tier of argmax screening (DESIGN.md 2.9): xcov_kernel<KID, DP, false>'s grid, partial layout and
-// reduction order, with the distances and kappa in FP32 (packed f32x2 differences, MUFU rsqrt / ex2).  Each run of 8
-// training points is summed in FP32 and added to an FP64 accumulator (one conversion per 8 pairs).  Blocks of split 0
-// also write each candidate's error bound E (tk_params.cuh), from |u| in FP64 and the per-call constants A1, A2.
+// D += A B for one m16n8k8 tile: A (16 x 8, row-major) and B (8 x 8, column-major) in TF32, D in FP32
+__device__ __forceinline__ void mma_tf32(float (&d)[4], const unsigned (&a)[4], unsigned b0, unsigned b1) {
+  asm("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, "
+      "{%0, %1, %2, %3};"
+      : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
+
+// The FP32 mean tier of argmax screening (DESIGN.md 2.9): xcov_kernel<KID, DP, false>'s grid and partial layout, with
+// d2 = |u~|^2 + |t~_j|^2 - 2 u~.t~_j from centred FP32 points.  The cross term runs on the tensor cores (mma.sync TF32,
+// 3-term hi / lo split, accumulated in FP32); the norms are added and kappa_f32 evaluated on the accumulator fragments.
+// Warp w takes candidates 16w..16w+15 of the block against the 16 eight-point tiles of a 128-point training chunk,
+// tiles 0-7 into partial 2 (k0 / 128) and tiles 8-15 into partial 2 (k0 / 128) + 1.  A thread holds candidates g and
+// g + 8 (g = lane / 4) against training points 2t, 2t + 1 of each tile (t = lane % 4); each run of 4 tiles (8 points
+// per candidate) is summed in FP32 and added to an FP64 accumulator, and the four lanes of a candidate are combined
+// by a fixed butterfly, so the partials do not depend on scheduling.  Blocks of split 0 also write each candidate's
+// error bound E (tk_params.cuh).
 template <int KID, int DP>
-__global__ void __launch_bounds__(256) xcov_mean_f32_kernel(XcovF32Params q) {
-  static_assert(DP % 2 == 0, "padded dimensions are even");
+__global__ void __launch_bounds__(256) xcov_mean_mma_kernel(XcovF32Params q) {
+  constexpr int KS = (DP + 7) / 8, KP = 8 * KS;   // k-steps of the MMA, the padded dimension
   const XcovParams &p = q.x;
-  __shared__ float2 xt[XCOV_KC * DP / 2];
-  __shared__ float al[XCOV_KC];
-  const int tid = threadIdx.x, r = tid & 127, kh = tid >> 7;
+  // the candidates' -2 u~ (hi, lo; [128][KP] each) before the loop, the chunk's B fragments in it
+  __shared__ float4 sbuf[XCOV_KC / 8 * KS * 32];
+  __shared__ float4 snt[XCOV_KC / 2];   // (|t~|^2, alpha) of training points 2i, 2i + 1
+  __shared__ float snu[128];
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5, g = lane >> 2, t = lane & 3;
   const int cb = blockIdx.x;
-  const long long m = p.m0 + (long long)cb * 128 + r;
-  float2 xc[DP / 2];
-  {
+  if (tid < 128) {
+    const long long m = p.m0 + (long long)cb * 128 + tid;
     double x64[DP];
     load_scaled_point<DP>(x64, p.Xs + (size_t)(m - p.in_off) * p.d, p.d, p.invl, p.disc_bits, m < p.M);
     double n2 = 0.0;
 #pragma unroll
-    for (int i = 0; i < DP; ++i) n2 = fma(x64[i], x64[i], n2);
-#pragma unroll
-    for (int i = 0; i < DP / 2; ++i) xc[i] = make_float2((float)x64[2 * i], (float)x64[2 * i + 1]);
-    if (blockIdx.y == 0 && kh == 0)
-      q.E[(size_t)cb * 128 + r] =
-          p.a2 * 0x1p-24 * (SCREEN_C_EVAL * q.A[0] + SCREEN_L_KAPPA * fma(sqrt(n2), q.A[0], q.A[1]));
-  }
-  const float2 *xg = reinterpret_cast<const float2 *>(q.Xt_neg);
-  for (int k0 = blockIdx.y * XCOV_KC; k0 < p.n_pad; k0 += gridDim.y * XCOV_KC) {
-    double mu_acc = 0.0;
-    __syncthreads();
-    for (int e = tid; e < XCOV_KC * DP / 2; e += 256) xt[e] = xg[(size_t)k0 * (DP / 2) + e];
-    if (tid < XCOV_KC) al[tid] = q.alpha[k0 + tid];
-    __syncthreads();
-    for (int mcol = kh; mcol < XCOV_KC / 8; mcol += 2) {
-      float s8 = 0.0f;
-#pragma unroll
-      for (int kk = 0; kk < 8; ++kk) {   // eight independent chains; padded columns have alpha = 0 and Xt = 0
-        const int kl = mcol * 8 + kk;
-        float2 acc = make_float2(0.0f, 0.0f);
-#pragma unroll
-        for (int i = 0; i < DP / 2; ++i) {
-          const float2 df = __fadd2_rn(xc[i], xt[kl * (DP / 2) + i]);
-          acc = __ffma2_rn(df, df, acc);
-        }
-        s8 = fmaf(al[kl], kappa_f32<KID>(acc.x + acc.y), s8);
-      }
-      mu_acc += (double)s8;
+    for (int i = 0; i < DP; ++i) {
+      x64[i] -= q.A[2 + i];
+      n2 = fma(x64[i], x64[i], n2);
     }
-    p.mu_part[(size_t)(2 * (k0 / XCOV_KC) + kh) * p.ld + (size_t)cb * 128 + r] = p.a2 * mu_acc;
+    float *ua = reinterpret_cast<float *>(sbuf);
+#pragma unroll
+    for (int i = 0; i < KP; ++i) {
+      float hi, lo;
+      tf32_split(i < DP ? (float)x64[i] : 0.0f, hi, lo);
+      ua[tid * KP + i] = -2.0f * hi;
+      ua[128 * KP + tid * KP + i] = -2.0f * lo;
+    }
+    snu[tid] = (float)n2;
+    if (blockIdx.y == 0)
+      q.E[(size_t)cb * 128 + tid] =
+          p.a2 * 0x1p-24 * (SCREEN_C_EVAL * q.A[0] + screen_l2(KID) * screen_k_dot(DP) * fma(n2, q.A[0], q.A[1]));
+  }
+  __syncthreads();
+  unsigned ahi[KS][4], alo[KS][4];
+  {
+    const float *ua = reinterpret_cast<const float *>(sbuf);
+    const int r0 = 16 * w + g;
+#pragma unroll
+    for (int ks = 0; ks < KS; ++ks)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {   // a0: (g, t), a1: (g + 8, t), a2: (g, t + 4), a3: (g + 8, t + 4)
+        const int o = (r0 + 8 * (e & 1)) * KP + ks * 8 + t + 4 * (e >> 1);
+        ahi[ks][e] = __float_as_uint(ua[o]);
+        alo[ks][e] = __float_as_uint(ua[128 * KP + o]);
+      }
+  }
+  const float nu0 = snu[16 * w + g], nu1 = snu[16 * w + g + 8];
+  for (int k0 = blockIdx.y * XCOV_KC; k0 < p.n_pad; k0 += gridDim.y * XCOV_KC) {
+    __syncthreads();
+    for (int e = tid; e < XCOV_KC / 8 * KS * 32; e += 256) sbuf[e] = q.tfrag[(size_t)(k0 / 8) * KS * 32 + e];
+    if (tid < XCOV_KC / 2) snt[tid] = q.tn_al[k0 / 2 + tid];
+    __syncthreads();
+#pragma unroll
+    for (int kh = 0; kh < 2; ++kh) {
+      double acc0 = 0.0, acc1 = 0.0;   // candidates g and g + 8
+#pragma unroll
+      for (int run = 0; run < 2; ++run) {
+        float s0 = 0.0f, s1 = 0.0f;
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          const int nt = kh * 8 + run * 4 + u;
+          float c[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+#pragma unroll
+          for (int ks = 0; ks < KS; ++ks) {   // b = (b0 hi, b1 hi, b0 lo, b1 lo): B(t, g), B(t + 4, g)
+            const float4 b = sbuf[(nt * KS + ks) * 32 + lane];
+            mma_tf32(c, alo[ks], __float_as_uint(b.x), __float_as_uint(b.y));
+            mma_tf32(c, ahi[ks], __float_as_uint(b.z), __float_as_uint(b.w));
+            mma_tf32(c, ahi[ks], __float_as_uint(b.x), __float_as_uint(b.y));
+          }
+          const float4 na = snt[nt * 4 + t];   // points 2t, 2t + 1 of the tile
+          s0 = fmaf(na.y, kappa_f32<KID>(fmaxf(c[0] + nu0 + na.x, 0.0f)), s0);
+          s0 = fmaf(na.w, kappa_f32<KID>(fmaxf(c[1] + nu0 + na.z, 0.0f)), s0);
+          s1 = fmaf(na.y, kappa_f32<KID>(fmaxf(c[2] + nu1 + na.x, 0.0f)), s1);
+          s1 = fmaf(na.w, kappa_f32<KID>(fmaxf(c[3] + nu1 + na.z, 0.0f)), s1);
+        }
+        acc0 += (double)s0;
+        acc1 += (double)s1;
+      }
+      acc0 += __shfl_xor_sync(0xffffffffu, acc0, 1);
+      acc1 += __shfl_xor_sync(0xffffffffu, acc1, 1);
+      acc0 += __shfl_xor_sync(0xffffffffu, acc0, 2);
+      acc1 += __shfl_xor_sync(0xffffffffu, acc1, 2);
+      if (t == 0) {
+        double *dst = p.mu_part + (size_t)(2 * (k0 / XCOV_KC) + kh) * p.ld + (size_t)cb * 128 + 16 * w + g;
+        dst[0] = p.a2 * acc0;
+        dst[8] = p.a2 * acc1;
+      }
+    }
+  }
+}
+
+// The tensor-core d2 of xcov_mean_mma_kernel for given FP32 points, for the tests of its error model: u [16 gridDim.x]
+// [8 KS] and t [8 gridDim.y][8 KS] row-major, nu / nt their norms; one warp per 16 x 8 tile, the same split, MMA chain
+// and assembly (without the clamp at 0), d2 [16 gridDim.x][8 gridDim.y] row-major.
+template <int KS>
+__global__ void mma_d2_kernel(const float *u, const float *t, const float *nu, const float *nt, float *d2) {
+  const int lane = threadIdx.x, g = lane >> 2, tq = lane & 3, KP = 8 * KS;
+  const int r0 = blockIdx.x * 16 + g, j = blockIdx.y * 8 + g, N = gridDim.y * 8;
+  float c[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+  for (int ks = 0; ks < KS; ++ks) {
+    unsigned ahi[4], alo[4], bhi[2], blo[2];
+    for (int e = 0; e < 4; ++e) {
+      float hi, lo;
+      tf32_split(u[(size_t)(r0 + 8 * (e & 1)) * KP + ks * 8 + tq + 4 * (e >> 1)], hi, lo);
+      ahi[e] = __float_as_uint(-2.0f * hi);
+      alo[e] = __float_as_uint(-2.0f * lo);
+    }
+    for (int e = 0; e < 2; ++e) {
+      float hi, lo;
+      tf32_split(t[(size_t)j * KP + ks * 8 + tq + 4 * e], hi, lo);
+      bhi[e] = __float_as_uint(hi);
+      blo[e] = __float_as_uint(lo);
+    }
+    mma_tf32(c, alo, bhi[0], bhi[1]);
+    mma_tf32(c, ahi, blo[0], blo[1]);
+    mma_tf32(c, ahi, bhi[0], bhi[1]);
+  }
+  const int row = blockIdx.x * 16 + g, col = blockIdx.y * 8 + 2 * tq;
+  for (int e = 0; e < 4; ++e) {
+    const int rr = row + 8 * (e >> 1), cc = col + (e & 1);
+    d2[(size_t)rr * N + cc] = c[e] + nu[rr] + nt[cc];
+  }
+}
+
+bool launch_mma_d2(int dp, const float *u, const float *t, const float *nu, const float *nt, int mt, int nt_, float *d2,
+                   cudaStream_t st) {
+  const dim3 grid(mt, nt_);
+  switch ((dp + 7) / 8) {
+    case 1: mma_d2_kernel<1><<<grid, 32, 0, st>>>(u, t, nu, nt, d2); return true;
+    case 2: mma_d2_kernel<2><<<grid, 32, 0, st>>>(u, t, nu, nt, d2); return true;
+    case 4: mma_d2_kernel<4><<<grid, 32, 0, st>>>(u, t, nu, nt, d2); return true;
+    default: return false;
   }
 }
 
@@ -227,7 +328,7 @@ bool launch_xcov_mean(int kid, int dp, const XcovParams &p, dim3 grid, cudaStrea
 #undef CALL
 }
 bool launch_xcov_mean_f32(int kid, int dp, const XcovF32Params &p, dim3 grid, cudaStream_t st) {
-#define CALL(K, D) xcov_mean_f32_kernel<K, D><<<grid, 256, 0, st>>>(p)
+#define CALL(K, D) xcov_mean_mma_kernel<K, D><<<grid, 256, 0, st>>>(p)
   BOSS_DISPATCH_KID_DP(CALL, kid, dp)
 #undef CALL
 }

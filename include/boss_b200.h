@@ -384,6 +384,11 @@ int boss_dbg_screen_ambiguous(int64_t *out);
 int boss_dbg_screen_mean(const boss_gp *gp, const double *Xs, int64_t M, double *mu32, double *E, double *mu64);
 /* the FP32 tier's kappa at d2 = (float)(r^2), kid 0 SE, 1 Matern32, 2 Matern52 */
 int boss_dbg_kappa_f32(int kid, const double *r, int n, double *out);
+/* the FP32 tier's tensor-core d2 = |u|^2 + |t|^2 - 2 u.t (before the clamp at 0) of m = 16 mt FP32 points u (m x kp
+ * row-major, kp = dp rounded up to 8) against n = 8 nt points t (n x kp), with their norms nu (m) and nt (n) as given:
+ * d2 is m x n row-major */
+int boss_dbg_mma_d2(int dp, const float *u, const float *t, const float *nu, const float *nt, int mt, int nt_tiles,
+                    float *d2);
 
 #ifdef __cplusplus
 }

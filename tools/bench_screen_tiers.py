@@ -8,10 +8,12 @@ BOSS_SCREEN_NO_RESEED=1) and "f32_reseed" (the default).  Cases: bench.py's prob
 candidates) with the candidates resident on the device, in pinned and in pageable host memory; C5's shape (n = 1024,
 d = 10, 4 outputs, EI x PoF, 512 Ki candidates, argmax only); and the bench problem refitted with noise 1e-4, where
 the larger sum |alpha| widens E and more candidates need the FP64 refinement.  Each round times `steps` calls of every
-tier in turn; printed per case and tier: ms per call, pool size, ambiguous candidates, and whether the (value, index)
-pairs are bit-identical to the f64 tier's.  One JSON line, with the card name and power limit it was measured at.
+tier in turn; printed per case and tier: ms per call, kernel launches per call, pool size, ambiguous candidates, and
+whether the (value, index) pairs are bit-identical to the f64 tier's.  One JSON line, with the card name and power limit
+it was measured at.
 --profile FILE: afterwards, one resident bench call per tier under torch.profiler (a run of its own, after the timed
-rounds); the CUDA time per kernel name and tier goes to FILE as JSON."""
+rounds); the CUDA time per kernel name and tier goes to FILE as JSON, with the FP32 tier's mean kernel per chunk and
+its (candidate, training point) pairs per second beside two bounds whose rates are assumptions, not measurements."""
 import argparse
 import json
 import os
@@ -22,6 +24,8 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+CH0 = 75_776                 # the first chunk of the bench problem (FP64 tier), candidates
+SASS_INSTR_PER_PAIR = 14.0   # xcov_mean_mma_kernel<2, 8>: about 900 instructions per 64 pairs a thread (cuobjdump -sass)
 sys.path.insert(0, ROOT)
 sys.dont_write_bytecode = True
 
@@ -103,7 +107,10 @@ def main():
                 ms_t, r = timed(fn, args.steps)
                 ms[t].append(ms_t)
                 st, amb = _lib.dbg_screen_stats(), _lib.dbg_screen_ambiguous()
-                info[t] = {"screen_state": st[0], "bounded": st[1], "pool": st[2], "ambiguous": amb[0]}
+                l0 = _lib.launch_count()
+                fn()
+                info[t] = {"screen_state": st[0], "bounded": st[1], "pool": st[2], "ambiguous": amb[0],
+                           "launches_per_call": _lib.launch_count() - l0}
                 key = (np.float64(r[0]).view(np.int64), r[1])
                 ref = key if ref is None else ref
                 same = same and key == ref
@@ -136,6 +143,18 @@ def main():
                     if us > 0:
                         ker[e.key] = {"us": us, "count": e.count}
             prof_out["tiers"][t] = dict(sorted(ker.items(), key=lambda kv: -kv[1]["us"])[:25])
+            mean_k = [(k, v) for k, v in ker.items() if "xcov_mean_mma_kernel" in k]
+            if mean_k:
+                k, v = mean_k[0]
+                per_chunk = v["us"] / v["count"]
+                pairs = (M - CH0) * 2048                 # every candidate after the first chunk, n = 2048
+                clk = 1.965e9                            # the card's maximum SM clock (sm_max_clock)
+                prof_out["tiers"][t]["mean_tier"] = {
+                    "kernel": k, "us_per_chunk": per_chunk, "chunks": v["count"],
+                    "pairs_per_s": pairs / (v["us"] * 1e-6),
+                    "bound_issue_pairs_per_s (assumed: 1 warp instruction / clock / SM sub-partition, "
+                    "SASS_INSTR_PER_PAIR from cuobjdump)": 4 * 148 * clk * 32 / SASS_INSTR_PER_PAIR,
+                    "bound_mufu_pairs_per_s (assumed: 16 MUFU results / clock / SM, 2 per pair)": 16 * 148 * clk / 2}
         for k in ("BOSS_SCREEN_F64", "BOSS_SCREEN_NO_RESEED"):
             os.environ.pop(k, None)
         with open(args.profile, "w") as f:
