@@ -10,9 +10,10 @@ from . import _lib  # noqa: F401  (raises loudly when the CUDA library has not b
 from .types import (BIParams, BossOptions, BossProblem, Dirac, Domain, ExperimentData, ExprFitness, FixedParams, LinFitness,  # noqa: F401
                     LogNormal, MAPParams, NonlinFitness, Normal, Product, Uniform, generate_LHC, in_bounds, in_domain,
                     mvlognormal)
-from .gaussian_process import (DiscreteKernel, GaussianProcess, GaussianProcessParams, GaussianProcessPosterior,  # noqa: F401
-                               Matern32Kernel, Matern52Kernel, Parametric, Semiparametric, SemiparametricParams,
-                               SqExponentialKernel, data_loglike, data_loglike_and_grad, model_posterior_slice)
+from .gaussian_process import (DiscreteKernel, ExponentialKernel, GaussianProcess, GaussianProcessParams,  # noqa: F401
+                               GaussianProcessPosterior, Matern12Kernel, Matern32Kernel, Matern52Kernel, Parametric,
+                               RationalQuadraticKernel, Semiparametric, SemiparametricParams, SqExponentialKernel,
+                               data_loglike, data_loglike_and_grad, model_posterior_slice)
 from .posterior import DefaultModelPosterior, average_mean, model_posterior  # noqa: F401
 from .acquisition import (Acquisition, ExpectedImprovement, best_so_far, construct_acquisition,  # noqa: F401
                           construct_safe_acquisition)

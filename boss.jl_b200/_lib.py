@@ -18,7 +18,8 @@ if not os.path.exists(LIB_PATH):
 lib = C.CDLL(LIB_PATH)
 
 BOSS_OK, BOSS_NOT_POSDEF, BOSS_NEG_VARIANCE = 0, 1, 2
-KERNEL_SE, KERNEL_MATERN32, KERNEL_MATERN52 = 0, 1, 2
+KERNEL_SE, KERNEL_MATERN32, KERNEL_MATERN52, KERNEL_MATERN12 = 0, 1, 2, 3
+RQ_SLOTS = 512   # BOSS_RQ_SLOTS: distinct RationalQuadratic shape parameters a process can register
 
 _dp = C.POINTER(C.c_double)
 _u8p = C.POINTER(C.c_uint8)
@@ -94,6 +95,8 @@ EXPORTS = {
     "boss_dbg_gemm_nt": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_int, _vp]),
     "boss_dbg_factors": (C.c_int, [_vp, _vp, _vp, _vp]),
     "boss_dbg_kernel_fn": (C.c_int, [C.c_int, _vp, C.c_int, _vp]),
+    "boss_kernel_rational_quadratic": (C.c_int, [C.c_double, C.POINTER(C.c_int)]),
+    "boss_dbg_kernel_fn_id": (C.c_int, [C.c_int, C.c_int, _vp, C.c_int, _vp]),
     "boss_dbg_check_redzones": (C.c_int64, [_i64p]),
     "boss_dbg_redzone_selftest": (C.c_int64, []),
     "boss_dbg_screen_stats": (C.c_int, [_i64p]),
@@ -120,6 +123,21 @@ def _check(rc: int, what: str) -> int:
     if rc < 0:
         raise BossError(f"{what} failed ({rc}): {last_error()}")
     return rc
+
+
+_rq_ids: dict[float, int] = {}
+
+
+def kernel_rational_quadratic(rq_a: float) -> int:
+    """The kernel_id of RationalQuadraticKernel(alpha = rq_a): (1 + r^2 / (2 rq_a))^-rq_a.  Ids come from a
+    process-lifetime table in the library (no device needed) and are cached here per value."""
+    a = float(rq_a)
+    kid = _rq_ids.get(a)
+    if kid is None:
+        out = C.c_int(-1)
+        _check(lib.boss_kernel_rational_quadratic(a, C.byref(out)), "boss_kernel_rational_quadratic")
+        kid = _rq_ids[a] = int(out.value)
+    return kid
 
 
 def init(device: int = 0) -> None:
@@ -718,6 +736,15 @@ def dbg_kernel_fn(which, t):
     t = _f64(t)
     out = np.empty_like(t)
     _check(lib.boss_dbg_kernel_fn(int(which), _ptr(t), t.size, _ptr(out)), "boss_dbg_kernel_fn")
+    return out
+
+
+def dbg_kernel_fn_id(kernel_id, which, d2):
+    """The covariance function of kernel_id at squared distances d2: which = 0 kappa_fast, 1 kappa'(r)/r fast,
+    2 kappa (libm), 3 kappa'(r)/r (libm)."""
+    d2 = _f64(d2)
+    out = np.empty_like(d2)
+    _check(lib.boss_dbg_kernel_fn_id(int(kernel_id), int(which), _ptr(d2), d2.size, _ptr(out)), "boss_dbg_kernel_fn_id")
     return out
 
 

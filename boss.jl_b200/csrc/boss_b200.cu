@@ -366,6 +366,8 @@ int set_kernel_attrs() {
   CUDA_TRY(cudaFuncSetAttribute(chol_matrix_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, CM_SMEM_BYTES));
   CUDA_TRY(cudaFuncSetAttribute(chol_matrix_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, CM_SMEM_BYTES));
   CUDA_TRY(cudaFuncSetAttribute(chol_matrix_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, CM_SMEM_BYTES));
+  CUDA_TRY(cudaFuncSetAttribute(chol_matrix_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, CM_SMEM_BYTES));
+  CUDA_TRY(cudaFuncSetAttribute(chol_matrix_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, CM_SMEM_BYTES));
   C().attrs_done = true;
   return 0;
 }
@@ -442,6 +444,7 @@ int run_cholesky(double *L, size_t L_stride, double *Winv, size_t Winv_stride, i
     pp.gen_dp = gen_dp;
     pp.gen_n = gen->n;
     pp.gen_kid = gen_kid;
+    pp.gen_rq_a = gen->rq_a;
     pp.gen_ls = gen->ls;
     pp.gen_amp = gen->amp;
     pp.gen_noise = gen->noise;
@@ -507,7 +510,8 @@ int run_cholesky(double *L, size_t L_stride, double *Winv, size_t Winv_stride, i
 // handle
 // ---------------------------------------------------------------------------------------------
 struct boss_gp {
-  int n = 0, d = 0, n_pad = 0, nblk = 0, ktiles = 0, kernel_id = 0, dp = 0;
+  int n = 0, d = 0, n_pad = 0, nblk = 0, ktiles = 0, kernel_id = 0, dp = 0;   // kernel_id: the decoded KID (0-4)
+  double rq_a = 0.0;                                                         // RationalQuadratic shape (KID 4)
   unsigned long long disc = 0;
   double amp = 0, noise = 0, a2 = 0;
   double loglik = 0;
@@ -637,9 +641,73 @@ int for_each_device(int ndev, const std::function<int(int, Ctx *)> &fn) {
   return 0;
 }
 
+// Kernel ids: 0-3 name a covariance function directly; 256 + slot names RationalQuadratic with the rq_a registered in
+// that slot (boss_kernel_rational_quadratic).  The table lives for the process and holds no device state; a slot is
+// written once, under the mutex, before its id is handed out.
+constexpr int RQ_ID0 = 256;
+std::mutex g_rq_mu;
+uint64_t g_rq_bits[BOSS_RQ_SLOTS];
+int g_rq_n = 0;
+
+struct KernelSpec {
+  int kid = 0;        // template KID of the device kernels (tk_params.cuh)
+  double rq_a = 0.0;  // RationalQuadratic shape parameter (kid 4)
+};
+
+// kernel_id -> (KID, rq_a); false for an unknown id
+bool decode_kernel(int kernel_id, KernelSpec *ks) {
+  if (kernel_id >= 0 && kernel_id <= BOSS_KERNEL_MATERN12) {
+    *ks = KernelSpec{kernel_id, 0.0};
+    return true;
+  }
+  if (kernel_id < RQ_ID0 || kernel_id >= RQ_ID0 + BOSS_RQ_SLOTS) return false;
+  std::lock_guard<std::mutex> lk(g_rq_mu);
+  const int slot = kernel_id - RQ_ID0;
+  if (slot >= g_rq_n) return false;
+  double a;
+  std::memcpy(&a, &g_rq_bits[slot], 8);
+  *ks = KernelSpec{4, a};
+  return true;
+}
+
+// boss_dbg_kernel_fn_id: the four covariance-function variants of one KID at n squared distances
+template <int KID>
+__global__ void dbg_kernel_fn_id_kernel(int which, double rq_a, const double *d2, double *out, int n) {
+  __shared__ double tab[EXPTAB_N];
+  exptab_init(tab);
+  __syncthreads();
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const double x = d2[i];
+    out[i] = which == 0 ? kappa_fast<KID>(x, tab, rq_a)
+             : which == 1 ? kappa_dr_over_r_fast<KID>(x, tab, rq_a)
+             : which == 2 ? kappa<KID>(x, rq_a)
+                          : kappa_dr_over_r<KID>(x, rq_a);
+  }
+}
+
 }  // namespace
 
 extern "C" {
+
+int boss_kernel_rational_quadratic(double rq_a, int *kernel_id) {
+  if (!kernel_id) return fail(BOSS_ERR_ARG, "boss_kernel_rational_quadratic: kernel_id is NULL");
+  if (!std::isfinite(rq_a) || !(rq_a > 0.0))
+    return fail(BOSS_ERR_ARG, "boss_kernel_rational_quadratic: rq_a must be finite and > 0");
+  uint64_t bits;
+  std::memcpy(&bits, &rq_a, 8);
+  std::lock_guard<std::mutex> lk(g_rq_mu);
+  for (int i = 0; i < g_rq_n; ++i)
+    if (g_rq_bits[i] == bits) {
+      *kernel_id = RQ_ID0 + i;
+      return 0;
+    }
+  if (g_rq_n >= BOSS_RQ_SLOTS)
+    return fail(BOSS_ERR_ARG, "boss_kernel_rational_quadratic: all " + std::to_string(BOSS_RQ_SLOTS) +
+                                  " rational-quadratic slots are in use");
+  g_rq_bits[g_rq_n] = bits;
+  *kernel_id = RQ_ID0 + g_rq_n++;
+  return 0;
+}
 
 int boss_version(void) { return 200; }
 int boss_device(void) {
@@ -735,12 +803,12 @@ void boss_shutdown(void) {
 // ---------------------------------------------------------------------------------------------
 // one posterior fit inside the current context
 static int fit_single(const double *X, int d, int n, const double *y_minus_mean, const double *lengthscales,
-                      double amplitude, double noise_std, int kernel_id, const uint8_t *discrete_mask, boss_gp **out,
+                      double amplitude, double noise_std, KernelSpec ks, const uint8_t *discrete_mask, boss_gp **out,
                       double *loglik_out) {
   if (!out) return fail(BOSS_ERR_ARG, "boss_gp_fit: out is NULL");
   *out = nullptr;
   if (!X || !y_minus_mean || !lengthscales || d < 1 || n < 1) return fail(BOSS_ERR_ARG, "boss_gp_fit: bad arguments");
-  if (kernel_id < 0 || kernel_id > 2) return fail(BOSS_ERR_ARG, "boss_gp_fit: unknown kernel_id");
+  const int kernel_id = ks.kid;
   const int dp = pick_dp(d);
   if (dp < 0) return fail(BOSS_ERR_ARG, "boss_gp_fit: x_dim > 32 is not supported");
   // reference asserts (src/models/gaussian_process.jl:227-229)
@@ -755,6 +823,7 @@ static int fit_single(const double *X, int d, int n, const double *y_minus_mean,
   h->nblk = h->n_pad / TM;
   h->ktiles = h->n_pad / TK;
   h->kernel_id = kernel_id;
+  h->rq_a = ks.rq_a;
   h->dp = dp;
   h->disc = mask_bits(discrete_mask, d);
   h->amp = amplitude + MIN_PARAM_VALUE;
@@ -821,6 +890,7 @@ static int fit_single(const double *X, int d, int n, const double *y_minus_mean,
   bk.K = h->L;
   bk.K_stride = mat;
   bk.status = status;
+  bk.rq_a = ks.rq_a;
   {
     Timed t(1);
     launch_build_k(kernel_id, dp, bk, dim3(nblk * (nblk + 1) / 2, 1), C().stream);
@@ -890,6 +960,8 @@ int boss_gp_fit(const double *X, int d, int n, const double *y_minus_mean, const
                 double *loglik_out) {
   if (!out) return fail(BOSS_ERR_ARG, "boss_gp_fit: out is NULL");
   *out = nullptr;
+  KernelSpec ks;
+  if (!decode_kernel(kernel_id, &ks)) return fail(BOSS_ERR_ARG, "boss_gp_fit: unknown kernel_id");
   if (g_ndev > 1 && tl_dev < 0) {
     // multi-device mode: the same deterministic fit on every device (2.9 GF at n = 2048 - cheaper than shipping
     // 3 x 32 MB of factors over NVLink, and it needs no peer access)
@@ -897,7 +969,7 @@ int boss_gp_fit(const double *X, int d, int n, const double *y_minus_mean, const
     std::vector<boss_gp *> reps(nd, nullptr);
     std::vector<double> ll(nd, 0.0);
     int rc = for_each_device(nd, [&](int k, Ctx *) {
-      return fit_single(X, d, n, y_minus_mean, lengthscales, amplitude, noise_std, kernel_id, discrete_mask, &reps[k], &ll[k]);
+      return fit_single(X, d, n, y_minus_mean, lengthscales, amplitude, noise_std, ks, discrete_mask, &reps[k], &ll[k]);
     });
     if (loglik_out) *loglik_out = ll[0];
     if (rc) {
@@ -910,7 +982,7 @@ int boss_gp_fit(const double *X, int d, int n, const double *y_minus_mean, const
     return 0;
   }
   REQUIRE_INIT();
-  return fit_single(X, d, n, y_minus_mean, lengthscales, amplitude, noise_std, kernel_id, discrete_mask, out, loglik_out);
+  return fit_single(X, d, n, y_minus_mean, lengthscales, amplitude, noise_std, ks, discrete_mask, out, loglik_out);
 }
 
 void boss_gp_free(boss_gp *gp) {
@@ -984,7 +1056,7 @@ static int append_single(boss_gp *h, const double *x_new, double y_minus_mean_ne
   int *status = reinterpret_cast<int *>(ws + o_st);
   CUDA_TRY(cudaMemsetAsync(status, 0, 8, C().stream));
   CUDA_TRY(cudaMemcpyAsync(ws, x_new, (size_t)d * 8, cudaMemcpyHostToDevice, C().stream));
-  launch_append_kvec(h->kernel_id, h->dp, ws, d, n, npad, h->invl, h->disc, h->a2, h->Xt, ws + o_k, C().stream);
+  launch_append_kvec(h->kernel_id, h->dp, ws, d, n, npad, h->invl, h->disc, h->a2, h->rq_a, h->Xt, ws + o_k, C().stream);
   matvec_p_kernel<<<npad / 64, 256, 0, C().stream>>>(h->W, ws + o_k, ws + o_l, h->ktiles);
   append_scalars_kernel<<<1, 256, 0, C().stream>>>(ws + o_l, h->wvec, n, h->a2 + h->noise * h->noise, y_minus_mean_new,
                                                  ws + o_sc, status);
@@ -1152,6 +1224,7 @@ XcovParams xcov_params(const boss_gp *h, const double *xs, long long M, long lon
   xp.Ks = C().ks.as<double>();
   xp.mu_part = C().part_mu.as<double>();
   xp.ld = ld;
+  xp.rq_a = h->rq_a;
   return xp;
 }
 
@@ -1597,6 +1670,7 @@ bool score_slice(const ScoreCall &c, int q, const AcqParams &ap, const ChunkIO &
     gq.UT = C().ut.as<double>();
     gq.gm_part = C().part_gm.as<double>();
     gq.gv_part = C().part_gv.as<double>();
+    gq.rq_a = h->rq_a;
     {
       Timed t(1);
       launch_grad(h->kernel_id, h->dp, gq, dim3(ncb, nks), C().stream);
@@ -1779,7 +1853,9 @@ struct Screen {
     const long long M = a.M;
     const int CH = c.CH, d = c.d, y_dim = a.y_dim, ns_max = a.topk ? topk_seed_n(a.topk, ch0) : SEED_N;
     const bool pm = a.prior_mean != nullptr, cm = a.cons_mask != nullptr;
-    f32 = getenv("BOSS_SCREEN_F64") == nullptr;
+    // the FP32 tier's error bound is proven for KIDs 0-2 only; a call with any other slice keeps FP64 means throughout
+    f32 = getenv("BOSS_SCREEN_F64") == nullptr &&
+          std::all_of(c.sl.begin(), c.sl.begin() + c.nsl, [](const boss_gp *h) { return kid_has_f32_tier(h->kernel_id); });
     reseed = getenv("BOSS_SCREEN_NO_RESEED") == nullptr;
     size_t tot = 0;
     const size_t ntk = (size_t)(CH + TOPK_IN - 1) / TOPK_IN * SEED_N;
@@ -2954,6 +3030,7 @@ int boss_gp_cov(const boss_gp *gp, const double *Xs, int64_t M, const double *pr
   cf.mu_out = mu ? C().mu_stage.as<double>() : nullptr;
   cf.cov = C().cov_stage.as<double>();
   cf.any_fail = d_fail;
+  cf.rq_a = h->rq_a;
   launch_cov_finish(h->kernel_id, h->dp, cf, dim3((unsigned)((M + 15) / 16), (unsigned)((M + 15) / 16)), C().stream);
   C().launches += 5;
   CUDA_TRY(cudaGetLastError());
@@ -2986,10 +3063,10 @@ struct MeanJac {
 
 // one batch inside the current context
 static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t ldy, const double *ls,
-                       const double *amp, const double *noise, int kernel_id, const uint8_t *discrete_mask, int64_t S,
+                       const double *amp, const double *noise, KernelSpec ks, const uint8_t *discrete_mask, int64_t S,
                        double *loglik, bool dev, double *grad, boss_gp **fit_out, void *caller_stream,
                        const MeanJac *mj = nullptr) {
-  const int dp = pick_dp(d);
+  const int dp = pick_dp(d), kernel_id = ks.kid;
   if (S == 0) return 0;
   if (dev) {
     int rc = wait_for_caller(caller_stream);
@@ -3088,6 +3165,7 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
     sp.disc_bits = disc;
     sp.S = S;
     sp.loglik = dll;
+    sp.rq_a = ks.rq_a;
     Timed t(2);
     launch_loglik_small(kernel_id, dp, sp, (int)((S + SMALL_WARPS - 1) / SMALL_WARPS), C().stream);
     ++C().launches;
@@ -3124,6 +3202,7 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
     pp.gen_dp = dp;
     pp.gen_n = n;
     pp.gen_kid = kernel_id;
+    pp.gen_rq_a = ks.rq_a;
     pp.gen_ls = dls + (size_t)s0 * d;
     pp.gen_amp = damp + s0;
     pp.gen_noise = dnoise + s0;
@@ -3132,12 +3211,14 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
     {
       Timed t(2);
       const unsigned grid = (unsigned)std::min<long long>(sb, 2 * 148);
-      if (kernel_id == 0)
-        chol_matrix_kernel<0><<<grid, 256, CM_SMEM_BYTES, C().stream>>>(cp);
-      else if (kernel_id == 1)
-        chol_matrix_kernel<1><<<grid, 256, CM_SMEM_BYTES, C().stream>>>(cp);
-      else
-        chol_matrix_kernel<2><<<grid, 256, CM_SMEM_BYTES, C().stream>>>(cp);
+      switch (kernel_id) {   // every KID explicitly (ids were decoded by loglik_impl)
+        case 0: chol_matrix_kernel<0><<<grid, 256, CM_SMEM_BYTES, C().stream>>>(cp); break;
+        case 1: chol_matrix_kernel<1><<<grid, 256, CM_SMEM_BYTES, C().stream>>>(cp); break;
+        case 2: chol_matrix_kernel<2><<<grid, 256, CM_SMEM_BYTES, C().stream>>>(cp); break;
+        case 3: chol_matrix_kernel<3><<<grid, 256, CM_SMEM_BYTES, C().stream>>>(cp); break;
+        case 4: chol_matrix_kernel<4><<<grid, 256, CM_SMEM_BYTES, C().stream>>>(cp); break;
+        default: return fail(BOSS_ERR_ARG, "boss_gp_loglik_batch: unknown kernel");
+      }
     }
     loglik_finish_kernel<<<(sb + 127) / 128, 128, 0, C().stream>>>(logdet_blk, pp.fwd_ssq, status, nblk, n, sb, dll + s0);
     C().launches += 2;
@@ -3182,6 +3263,7 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
       bk.K = Lg;
       bk.K_stride = mat;
       bk.status = stg;
+      bk.rq_a = ks.rq_a;
       // Fused diagonal step (K_jj generated on chip + SYRK + potrf in one 2-CTA/SM kernel) for small matrices, where the
       // three short launches and the tile's HBM trip dominate (C3, n = 512: 1.61 -> 1.55 ms); for long k-ranges the
       // dedicated SYRK kernel (5-stage ring, 218 registers) runs its DMMAs at 75 % of the SM's rate against 51 % for the
@@ -3239,6 +3321,7 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
         lg.K_stride = mat;
         lg.alpha = al;
         lg.part = partg;
+        lg.rq_a = ks.rq_a;
         {
           Timed t(1);
           launch_loglik_grad_tile(kernel_id, dp, lg, dim3(ntiles, gs), C().stream);
@@ -3269,6 +3352,7 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
         if (hst[q] != 0) continue;
         boss_gp *h = new boss_gp();
         h->n = n; h->d = d; h->n_pad = n_pad; h->nblk = nblk; h->ktiles = ktiles; h->kernel_id = kernel_id; h->dp = dp;
+        h->rq_a = ks.rq_a;
         h->disc = disc;
         h->amp = amp[sidx] + MIN_PARAM_VALUE;
         h->noise = noise[sidx] + MIN_PARAM_VALUE;
@@ -3332,7 +3416,8 @@ static int loglik_impl(const double *X, int d, int n, const double *Ymm, int64_t
                        void *caller_stream = nullptr, const MeanJac *mj = nullptr) {
   if (!X || !Ymm || !ls || !amp || !noise || !loglik || d < 1 || n < 1 || S < 0)
     return fail(BOSS_ERR_ARG, "boss_gp_loglik_batch: bad arguments");
-  if (kernel_id < 0 || kernel_id > 2) return fail(BOSS_ERR_ARG, "boss_gp_loglik_batch: unknown kernel_id");
+  KernelSpec ks;
+  if (!decode_kernel(kernel_id, &ks)) return fail(BOSS_ERR_ARG, "boss_gp_loglik_batch: unknown kernel_id");
   if (pick_dp(d) < 0) return fail(BOSS_ERR_ARG, "boss_gp_loglik_batch: x_dim > 32 is not supported");
   if (!dev) {
     for (int64_t s = 0; s < S; ++s) {
@@ -3345,7 +3430,7 @@ static int loglik_impl(const double *X, int d, int n, const double *Ymm, int64_t
   const int nd = (g_ndev > 1 && tl_dev < 0 && !dev && !fit_out && S >= 2LL * g_ndev) ? g_ndev : 1;
   if (nd <= 1) {
     REQUIRE_INIT();
-    return loglik_core(X, d, n, Ymm, ldy, ls, amp, noise, kernel_id, discrete_mask, S, loglik, dev, grad, fit_out, caller_stream,
+    return loglik_core(X, d, n, Ymm, ldy, ls, amp, noise, ks, discrete_mask, S, loglik, dev, grad, fit_out, caller_stream,
                        mj);
   }
   const int64_t per = (S + nd - 1) / nd;
@@ -3354,7 +3439,7 @@ static int loglik_impl(const double *X, int d, int n, const double *Ymm, int64_t
     if (cnt <= 0) return 0;
     MeanJac mjk{};
     if (mj) mjk = MeanJac{mj->J + (size_t)s0 * mj->ldj, mj->k, mj->ldj, mj->grad_mean + (size_t)s0 * mj->k};
-    return loglik_core(X, d, n, ldy ? Ymm + (size_t)s0 * ldy : Ymm, ldy, ls + (size_t)s0 * d, amp + s0, noise + s0, kernel_id,
+    return loglik_core(X, d, n, ldy ? Ymm + (size_t)s0 * ldy : Ymm, ldy, ls + (size_t)s0 * d, amp + s0, noise + s0, ks,
                        discrete_mask, cnt, loglik + s0, false, grad ? grad + (size_t)s0 * (d + 2) : nullptr,
                        fit_out ? fit_out + s0 : nullptr, nullptr, mj ? &mjk : nullptr);
   });
@@ -3386,11 +3471,12 @@ int boss_gp_fit_batch(const double *X, int d, int n, const double *Y_minus_mean,
     const int nd = g_ndev;
     std::vector<std::vector<boss_gp *>> reps(nd, std::vector<boss_gp *>((size_t)S, nullptr));
     std::vector<std::vector<double>> lls(nd, std::vector<double>((size_t)S, 0.0));
-    if (!X || !Y_minus_mean || !lengthscales || !amplitude || !noise_std || d < 1 || n < 1 || kernel_id < 0 ||
-        kernel_id > 2 || pick_dp(d) < 0)
+    KernelSpec ks;
+    if (!X || !Y_minus_mean || !lengthscales || !amplitude || !noise_std || d < 1 || n < 1 ||
+        !decode_kernel(kernel_id, &ks) || pick_dp(d) < 0)
       return fail(BOSS_ERR_ARG, "boss_gp_fit_batch: bad arguments");
     rc = for_each_device(nd, [&](int k, Ctx *) {
-      return loglik_core(X, d, n, Y_minus_mean, ldy, lengthscales, amplitude, noise_std, kernel_id, discrete_mask, S,
+      return loglik_core(X, d, n, Y_minus_mean, ldy, lengthscales, amplitude, noise_std, ks, discrete_mask, S,
                          lls[k].data(), false, nullptr, reps[k].data(), nullptr);
     });
     ll = lls[0];
@@ -3521,12 +3607,12 @@ __global__ void dbg_kernel_fn_kernel(int which, const double *t, double *out, in
     switch (which) {
       case 0: v = fast_exp_neg(x, tab); break;
       case 1: v = fast_sqrt(x); break;
-      case 2: v = kappa_fast<0>(x, tab); break;
-      case 3: v = kappa_fast<1>(x, tab); break;
-      case 4: v = kappa_fast<2>(x, tab); break;
-      case 5: v = kappa_dr_over_r_fast<0>(x, tab); break;
-      case 6: v = kappa_dr_over_r_fast<1>(x, tab); break;
-      default: v = kappa_dr_over_r_fast<2>(x, tab); break;
+      case 2: v = kappa_fast<0>(x, tab, 0.0); break;
+      case 3: v = kappa_fast<1>(x, tab, 0.0); break;
+      case 4: v = kappa_fast<2>(x, tab, 0.0); break;
+      case 5: v = kappa_dr_over_r_fast<0>(x, tab, 0.0); break;
+      case 6: v = kappa_dr_over_r_fast<1>(x, tab, 0.0); break;
+      default: v = kappa_dr_over_r_fast<2>(x, tab, 0.0); break;
     }
     out[i] = v;
   }
@@ -3541,6 +3627,32 @@ int boss_dbg_kernel_fn(int which, const double *t, int n, double *out) {
   dbg_kernel_fn_kernel<<<148, 256, 0, C().stream>>>(which, dt, dout, n);
   CUDA_TRY(cudaStreamSynchronize(C().stream));
   CUDA_TRY(cudaMemcpy(out, dout, (size_t)n * 8, cudaMemcpyDeviceToHost));
+  cudaFree(dt);
+  cudaFree(dout);
+  return 0;
+}
+
+int boss_dbg_kernel_fn_id(int kernel_id, int which, const double *d2, int n, double *out) {
+  REQUIRE_INIT();
+  KernelSpec ks;
+  if (!decode_kernel(kernel_id, &ks)) return fail(BOSS_ERR_ARG, "boss_dbg_kernel_fn_id: unknown kernel_id");
+  if (which < 0 || which > 3 || n < 0 || (n > 0 && (!d2 || !out)))
+    return fail(BOSS_ERR_ARG, "boss_dbg_kernel_fn_id: bad argument");
+  if (n == 0) return 0;
+  double *dt, *dout;
+  CUDA_TRY(cudaMalloc(&dt, (size_t)n * 8));
+  CUDA_TRY(cudaMalloc(&dout, (size_t)n * 8));
+  CUDA_TRY(cudaMemcpyAsync(dt, d2, (size_t)n * 8, cudaMemcpyHostToDevice, C().stream));
+  switch (ks.kid) {
+    case 0: dbg_kernel_fn_id_kernel<0><<<148, 256, 0, C().stream>>>(which, ks.rq_a, dt, dout, n); break;
+    case 1: dbg_kernel_fn_id_kernel<1><<<148, 256, 0, C().stream>>>(which, ks.rq_a, dt, dout, n); break;
+    case 2: dbg_kernel_fn_id_kernel<2><<<148, 256, 0, C().stream>>>(which, ks.rq_a, dt, dout, n); break;
+    case 3: dbg_kernel_fn_id_kernel<3><<<148, 256, 0, C().stream>>>(which, ks.rq_a, dt, dout, n); break;
+    default: dbg_kernel_fn_id_kernel<4><<<148, 256, 0, C().stream>>>(which, ks.rq_a, dt, dout, n); break;
+  }
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaMemcpyAsync(out, dout, (size_t)n * 8, cudaMemcpyDeviceToHost, C().stream));
+  CUDA_TRY(cudaStreamSynchronize(C().stream));
   cudaFree(dt);
   cudaFree(dout);
   return 0;
@@ -3637,6 +3749,8 @@ int boss_dbg_screen_ambiguous(int64_t *out) {
 // (K*^T alpha, without a prior mean), computed by the kernels the screen runs.
 int boss_dbg_screen_mean(const boss_gp *gp, const double *Xs, int64_t M, double *mu32, double *E, double *mu64) {
   if (!gp || M < 1 || M > (1 << 22) || !Xs) return fail(BOSS_ERR_ARG, "boss_dbg_screen_mean: bad argument");
+  if (!kid_has_f32_tier(gp->kernel_id))
+    return fail(BOSS_ERR_ARG, "boss_dbg_screen_mean: the FP32 mean tier does not exist for this kernel");
   REQUIRE_HANDLE_CTX(gp);
   const int d = gp->d, ld = (int)((M + 127) / 128 * 128), ncb = ld / 128;
   const int nks = std::max(1, std::min(gp->nblk, (16 * 148 + ncb - 1) / ncb));

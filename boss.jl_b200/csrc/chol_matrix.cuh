@@ -178,7 +178,7 @@ __device__ __forceinline__ void cm_update_job(const PotrfParams &p, const int s_
       d20 = fma(df0, df0, d20);
       d21 = fma(df1, df1, d21);
     }
-    double v0 = a2 * kappa_fast<KID>(d20, etab), v1 = a2 * kappa_fast<KID>(d21, etab);
+    double v0 = a2 * kappa_fast<KID>(d20, etab, p.gen_rq_a), v1 = a2 * kappa_fast<KID>(d21, etab, p.gen_rq_a);
     const bool row_live = i * 128 + r < p.gen_n;
     const int gj = j * 128 + 64 * h + c;
     if (!(row_live && gj < p.gen_n)) v0 = 0.0;            // padding rows / columns of an off-diagonal block are zero

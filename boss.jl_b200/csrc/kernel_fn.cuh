@@ -1,6 +1,6 @@
 // kernel_fn.cuh -- covariance function evaluation shared by the kernel-matrix builder (a1) and the
 // cross-covariance generator (a3).  Mirrors KernelFunctions' kappa for SqExponential / Matern32 /
-// Matern52 composed with ARDTransform(1/l) and ScaledKernel(a^2)  (reference call site:
+// Matern52 / Exponential (Matern12) / RationalQuadratic composed with ARDTransform(1/l) and ScaledKernel(a^2)  (reference call site:
 // src/models/gaussian_process.jl:243), optional DiscreteKernel rounding (src/models/utils/kernels.jl:56-64).
 #pragma once
 #include "common.cuh"
@@ -66,42 +66,126 @@ __device__ __forceinline__ double fast_sqrt(double x) {
   return fma(fma(-g, g, x), h, g);
 }
 
+// 1/sqrt(x) for x >= 0: MUFU.RSQ64H seed (~2^-22) and two Newton steps, a few ulp for every normal x.  The seed flushes
+// subnormals, so x is raised to the smallest normal double first: x = 0 returns 6.7e153 (the one caller selects 0 there).
+__device__ __forceinline__ double fast_rsqrt(double x) {
+  x = fmax(x, 2.2250738585072014e-308);
+  double y;
+  asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(x));
+  const double h = 0.5 * x;
+  y = y * fma(-h * y, y, 1.5);
+  return y * fma(-h * y, y, 1.5);
+}
+
+// log1p(u) for u >= 0 without branches (libm's log1p inlines a slow path that, eight chains wide, costs the tile kernels
+// their registers): w = 1 + u = 2^k m with m in [sqrt(1/2), sqrt(2)), log m = 2 atanh(s), s = (m - 1) / (m + 1), |s| <=
+// 0.172, by an odd series through s^21; the reciprocals are MUFU.RCP64H seeds refined by Newton steps, and the
+// rounding of 1 + u is put back as -((w - 1) - u) / w.  A few ulp (measured against mpmath,
+// tests/test_gpu_kernels_more.py::test_kernel_functions).  Finite u only.
+__device__ __forceinline__ double rcp_newton(double x, int steps) {
+  double y;
+  asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(x));
+  for (int i = 0; i < steps; ++i) y = fma(y, fma(-x, y, 1.0), y);
+  return y;
+}
+__device__ __forceinline__ double fast_log1p(double u) {
+  const double w = 1.0 + u, c = (w - 1.0) - u;
+  const int hi = __double2hiint(w);
+  const int k = ((hi + (0x3FF00000 - 0x3FE6A09E)) >> 20) - 1023;
+  const double m = __hiloint2double(hi - (k << 20), __double2loint(w));
+  const double f = m - 1.0, q = 2.0 + f;
+  const double rq = rcp_newton(q, 2);
+  double sv = f * rq;
+  sv = fma(fma(-sv, q, f), rq, sv);
+  const double z = sv * sv;
+  double p = fma(z, 1.0 / 21.0, 1.0 / 19.0);
+  p = fma(p, z, 1.0 / 17.0);
+  p = fma(p, z, 1.0 / 15.0);
+  p = fma(p, z, 1.0 / 13.0);
+  p = fma(p, z, 1.0 / 11.0);
+  p = fma(p, z, 1.0 / 9.0);
+  p = fma(p, z, 1.0 / 7.0);
+  p = fma(p, z, 1.0 / 5.0);
+  p = fma(p, z, 1.0 / 3.0);
+  const double s2 = 2.0 * sv, lm = fma(s2 * z, p, s2);
+  const double kd = (double)k;
+  const double corr = fma(kd, 1.9082149292705877e-10 /* ln2 - ln2_hi */, lm) - c * rcp_newton(w, 1);
+  return fma(kd, 6.93147180369123816490e-01 /* ln2_hi: 32 bits, kd * ln2_hi is exact */, corr);
+}
+
+// The covariance functions kappa(d2) of the ARD-scaled squared distance d2 = r^2 (DESIGN.md 2.14 for KIDs 3 and 4):
+//   KID 0 SqExponential  exp(-r^2 / 2)          KID 3 Matern12 / Exponential  exp(-r)
+//   KID 1 Matern32       (1 + sqrt3 r) exp(-sqrt3 r)   KID 4 RationalQuadratic  (1 + r^2 / (2 a))^-a,  a = rq_a > 0
+//   KID 2 Matern52       (1 + sqrt5 r + 5 r^2 / 3) exp(-sqrt5 r)
+// rq_a is the RQ shape parameter (KernelFunctions' alpha, not BOSS's amplitude); KIDs 0-3 ignore it.  kappa(0) = 1 for
+// every KID.  RQ's 0.5 / rq_a is loop-invariant in every caller and hoisted out of the training-point loops.
 template <int KID>
-__device__ __forceinline__ double kappa_fast(double d2, const double *tab) {
+__device__ __forceinline__ double kappa_fast(double d2, const double *tab, double rq_a) {
   if (KID == 0) {
     return fast_exp_neg(0.5 * d2, tab);
   } else if (KID == 1) {
     const double t = 1.7320508075688772 * fast_sqrt(d2);
     return (1.0 + t) * fast_exp_neg(t, tab);
-  } else {
+  } else if (KID == 2) {
     const double t = 2.23606797749979 * fast_sqrt(d2);
     return (1.0 + t + (5.0 / 3.0) * d2) * fast_exp_neg(t, tab);
+  } else if (KID == 3) {
+    return fast_exp_neg(fast_sqrt(d2), tab);
+  } else {
+    static_assert(KID >= 0 && KID <= 4, "kernel id");
+    return fast_exp_neg(rq_a * fast_log1p(d2 * (0.5 / rq_a)), tab);
   }
 }
 
 // (d kappa / d r) / r, fast variant (see kappa_dr_over_r below)
 template <int KID>
-__device__ __forceinline__ double kappa_dr_over_r_fast(double d2, const double *tab) {
+__device__ __forceinline__ double kappa_dr_over_r_fast(double d2, const double *tab, double rq_a) {
   if (KID == 0) {
     return -fast_exp_neg(0.5 * d2, tab);
   } else if (KID == 1) {
     return -3.0 * fast_exp_neg(1.7320508075688772 * fast_sqrt(d2), tab);
-  } else {
+  } else if (KID == 2) {
     const double t = 2.23606797749979 * fast_sqrt(d2);
     return -(5.0 / 3.0) * (1.0 + t) * fast_exp_neg(t, tab);
+  } else if (KID == 3) {
+    const double ri = fast_rsqrt(d2);
+    const double v = -fast_exp_neg(d2 * ri, tab) * ri;
+    return d2 == 0.0 ? 0.0 : v;   // the r = 0 convention (DESIGN.md 2.14): a select, not a branch
+  } else {
+    static_assert(KID >= 0 && KID <= 4, "kernel id");
+    return -fast_exp_neg((rq_a + 1.0) * fast_log1p(d2 * (0.5 / rq_a)), tab);
+  }
+}
+
+// kappa_fast and kappa_dr_over_r_fast at the same d2 (the log-likelihood gradient's tile pass needs both): RQ shares
+// its log1p between the two, every other KID evaluates the two functions above unchanged.
+template <int KID>
+__device__ __forceinline__ void kappa_and_dr_fast(double d2, const double *tab, double rq_a, double &k, double &g) {
+  if (KID == 4) {
+    const double l = fast_log1p(d2 * (0.5 / rq_a));
+    k = fast_exp_neg(rq_a * l, tab);
+    g = -fast_exp_neg((rq_a + 1.0) * l, tab);
+  } else {
+    k = kappa_fast<KID>(d2, tab, rq_a);
+    g = kappa_dr_over_r_fast<KID>(d2, tab, rq_a);
   }
 }
 
 template <int KID>
-__device__ __forceinline__ double kappa(double d2) {
+__device__ __forceinline__ double kappa(double d2, double rq_a) {
   if (KID == 0) {
     return exp(-0.5 * d2);
   } else if (KID == 1) {
     const double t = 1.7320508075688772 * sqrt(d2);
     return (1.0 + t) * exp(-t);
-  } else {
+  } else if (KID == 2) {
     const double t = 2.23606797749979 * sqrt(d2);
     return (1.0 + t + (5.0 / 3.0) * d2) * exp(-t);
+  } else if (KID == 3) {
+    return exp(-sqrt(d2));
+  } else {
+    static_assert(KID >= 0 && KID <= 4, "kernel id");
+    return exp(-rq_a * log1p(d2 * (0.5 / rq_a)));
   }
 }
 
@@ -139,16 +223,25 @@ __device__ __forceinline__ void tf32_split(float x, float &hi, float &lo) {
   lo = __uint_as_float(l);
 }
 
-// (d kappa / d r) / r as a function of d2 = r^2 : finite at r = 0 for all three kernels.
+// (d kappa / d r) / r as a function of d2 = r^2: finite at r = 0 for KIDs 0-2 and 4.  Matern12's -exp(-r) / r is
+// unbounded there; it is defined as 0 at d2 == 0 (DESIGN.md 2.14), as a select, so no -Inf * 0 = NaN can reach a sum.
+// RQ: -kappa / (1 + r^2 / (2a)) = -(1 + r^2 / (2a))^-(a+1).
 template <int KID>
-__device__ __forceinline__ double kappa_dr_over_r(double d2) {
+__device__ __forceinline__ double kappa_dr_over_r(double d2, double rq_a) {
   if (KID == 0) {
     return -exp(-0.5 * d2);
   } else if (KID == 1) {
     return -3.0 * exp(-1.7320508075688772 * sqrt(d2));
-  } else {
+  } else if (KID == 2) {
     const double t = 2.23606797749979 * sqrt(d2);
     return -(5.0 / 3.0) * (1.0 + t) * exp(-t);
+  } else if (KID == 3) {
+    const double r = sqrt(d2);
+    const double v = -exp(-r) / r;
+    return d2 == 0.0 ? 0.0 : v;
+  } else {
+    static_assert(KID >= 0 && KID <= 4, "kernel id");
+    return -exp(-(rq_a + 1.0) * log1p(d2 * (0.5 / rq_a)));
   }
 }
 

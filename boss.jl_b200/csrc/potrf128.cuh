@@ -50,6 +50,7 @@ struct PotrfParams {
   int gen_d, gen_dp, gen_n, gen_kid;
   const double *gen_ls, *gen_amp, *gen_noise;   // per-matrix raw hyper-parameters
   unsigned long long gen_disc;
+  double gen_rq_a;         // RationalQuadratic shape parameter (gen_kid 4)
   int store_L;             // also write L_jj back to global (batched posterior fit: L is part of the handle)
 };
 
@@ -105,7 +106,7 @@ __device__ __forceinline__ int pt_cpos(int lane, int e) {
 // and a dynamically indexed accumulator array would be demoted to local memory for the whole kernel).
 template <int KID>
 __device__ __forceinline__ void pf_generate_tile(double *T, const double *xs, int dp, int warp, int lane, int row0, int n,
-                                                 double a2, double s2, const double *etab) {
+                                                 double a2, double s2, const double *etab, double rq_a) {
 #pragma unroll 1
   for (int t = 0; t < 17; ++t) {
     const int R = t < 16 - warp ? warp + t : t - 1, Cs = t < 16 - warp ? warp : 15 - warp;
@@ -117,7 +118,7 @@ __device__ __forceinline__ void pf_generate_tile(double *T, const double *xs, in
       d20 = fma(df0, df0, d20);
       d21 = fma(df1, df1, d21);
     }
-    double v0 = a2 * kappa_fast<KID>(d20, etab), v1 = a2 * kappa_fast<KID>(d21, etab);
+    double v0 = a2 * kappa_fast<KID>(d20, etab, rq_a), v1 = a2 * kappa_fast<KID>(d21, etab, rq_a);
     const int gi = row0 + r, gj = row0 + c0;
     if (gi < n && gj < n) {
       if (gi == gj) v0 += s2;
@@ -310,12 +311,14 @@ __device__ __forceinline__ void potrf_tile_body(const PotrfParams &p, const int 
       dst[pt_cpos(lane, 1)] = acc[t][1];
     }
     const double a2 = amp * amp, s2 = sn * sn;
-    if (p.gen_kid == 0)
-      pf_generate_tile<0>(T, tmp, dp, warp, lane, row0, p.gen_n, a2, s2, etab);
-    else if (p.gen_kid == 1)
-      pf_generate_tile<1>(T, tmp, dp, warp, lane, row0, p.gen_n, a2, s2, etab);
-    else
-      pf_generate_tile<2>(T, tmp, dp, warp, lane, row0, p.gen_n, a2, s2, etab);
+    switch (p.gen_kid) {   // every KID explicitly: an unknown id generates nothing (the host decodes ids first)
+      case 0: pf_generate_tile<0>(T, tmp, dp, warp, lane, row0, p.gen_n, a2, s2, etab, p.gen_rq_a); break;
+      case 1: pf_generate_tile<1>(T, tmp, dp, warp, lane, row0, p.gen_n, a2, s2, etab, p.gen_rq_a); break;
+      case 2: pf_generate_tile<2>(T, tmp, dp, warp, lane, row0, p.gen_n, a2, s2, etab, p.gen_rq_a); break;
+      case 3: pf_generate_tile<3>(T, tmp, dp, warp, lane, row0, p.gen_n, a2, s2, etab, p.gen_rq_a); break;
+      case 4: pf_generate_tile<4>(T, tmp, dp, warp, lane, row0, p.gen_n, a2, s2, etab, p.gen_rq_a); break;
+      default: break;
+    }
   }
   __syncthreads();
 

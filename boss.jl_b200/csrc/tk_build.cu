@@ -69,7 +69,7 @@ __global__ void __launch_bounds__(256) build_k_kernel(BuildKParams p) {
         const double df = xr[i] - xcol[jj * DP + i];
         d2 = fma(df, df, d2);
       }
-      v[kk] = a2 * kappa_fast<KID>(d2, etab);
+      v[kk] = a2 * kappa_fast<KID>(d2, etab, p.rq_a);
     }
     if (rb == cb || rb == p.nblk - 1) {   // diagonal tile (noise) or last row block (padding): per-element fix-up
 #pragma unroll
@@ -149,8 +149,7 @@ __global__ void __launch_bounds__(256) loglik_grad_tile_kernel(LlGradParams p) {
         const double df = xr[q] - xcol[jj * DP + q];
         d2 = fma(df, df, d2);
       }
-      kap[kk] = kappa_fast<KID>(d2, etab);
-      wgt[kk] = kappa_dr_over_r_fast<KID>(d2, etab);
+      kappa_and_dr_fast<KID>(d2, etab, p.rq_a, kap[kk], wgt[kk]);
     }
 #pragma unroll
     for (int kk = 0; kk < 8; ++kk) {

@@ -1,5 +1,5 @@
 // tk_params.cuh -- parameter blocks and host launchers of the kernels that are templated on
-// (covariance function KID, padded input dimension DP).  Those 7 kernel families x 21 instantiations are most of the
+// (covariance function KID, padded input dimension DP).  Those 7 kernel families x 35 instantiations are most of the
 // library's compile time, so they live in their own translation units (tk_build.cu, tk_score.cu, tk_small.cu) and are
 // reached through the plain launch_* functions declared at the end of this file.
 #pragma once
@@ -18,6 +18,7 @@ struct BuildKParams {
   size_t K_stride;
   int *status;              // S; set to -1 on negative hyper-parameters (reference asserts)
   int skip_diag;            // diagonal tiles are produced elsewhere (potrf_fused_kernel generates K_jj on chip)
+  double rq_a;              // RationalQuadratic shape parameter (KID 4; ignored by the other kernels)
 };
 
 struct LlGradParams {
@@ -29,6 +30,7 @@ struct LlGradParams {
   size_t K_stride;
   const double *alpha;   // [S][n_pad]
   double *part;          // [S][ntiles][DP + 2]
+  double rq_a;
 };
 
 struct XcovParams {
@@ -43,6 +45,7 @@ struct XcovParams {
   double *Ks;              // chunk scratch, P-layout: rows = candidates of the chunk, cols = training index
   double *mu_part;         // [2*nblk][ld] per-(128-chunk of training points, k-half) partials of K*^T alpha
   int ld;                  // leading dimension of mu_part (= chunk capacity)
+  double rq_a;
 };
 
 constexpr int XCOV_KC = 128;  // training points staged per shared-memory pass
@@ -77,6 +80,7 @@ struct CovFinishParams {
   double *mu_out;       // [M] or null
   double *cov;          // M x M column-major
   int *any_fail;
+  double rq_a;
 };
 
 struct GradParams {
@@ -88,6 +92,7 @@ struct GradParams {
   double a2;
   const double *UT;    // chunk scratch (P-layout), u = K^-1 k*
   double *gm_part, *gv_part;  // [2*nblk][d][chunk_ld] per-(training chunk, k-half) partial sums (unscaled)
+  double rq_a;
 };
 
 constexpr int SMALL_N = 32;
@@ -103,9 +108,15 @@ struct SmallLoglikParams {
   unsigned long long disc_bits;
   long long S;
   double *loglik;       // S: value, -Inf (not positive definite) or NaN (negative hyper-parameter)
+  double rq_a;
 };
 
-// ---- host launchers: dispatch on (kernel_id 0..2, dp in {2,4,6,8,12,16,32}); false = unsupported combination ----
+// ---- host launchers: dispatch on (KID 0..4, dp in {2,4,6,8,12,16,32}); false = unsupported combination ----
+// KIDs: 0 SqExponential, 1 Matern32, 2 Matern52, 3 Matern12, 4 RationalQuadratic (kernel_fn.cuh).  The FP32 mean tier
+// (launch_xcov_mean_f32) exists for KIDs 0-2 only: its error bound needs sup |d kappa / d(d2)|, which is infinite for
+// Matern12 and not derived for RQ's FP32 evaluation, so those kernels screen with FP64 means (DESIGN.md 2.14).
+constexpr int NUM_KID = 5;
+__host__ __device__ constexpr bool kid_has_f32_tier(int kid) { return kid >= 0 && kid <= 2; }
 bool launch_build_k(int kid, int dp, const BuildKParams &p, dim3 grid, cudaStream_t st);
 bool launch_loglik_grad_tile(int kid, int dp, const LlGradParams &p, dim3 grid, cudaStream_t st);
 bool launch_xcov(int kid, int dp, const XcovParams &p, dim3 grid, cudaStream_t st);
@@ -118,32 +129,34 @@ bool launch_cov_finish(int kid, int dp, const CovFinishParams &p, dim3 grid, cud
 bool launch_grad(int kid, int dp, const GradParams &p, dim3 grid, cudaStream_t st);
 bool launch_loglik_small(int kid, int dp, const SmallLoglikParams &p, int nblocks, cudaStream_t st);
 bool launch_append_kvec(int kid, int dp, const double *xnew, int d, int n, int n_pad, const double *invl,
-                        unsigned long long disc_bits, double a2, double *Xt, double *kvec, cudaStream_t st);
+                        unsigned long long disc_bits, double a2, double rq_a, double *Xt, double *kvec, cudaStream_t st);
 
-#define BOSS_DISPATCH_KID_DP(CALL, kid, dp)       \
-  switch ((kid) * 100 + (dp)) {                   \
-    case 2: CALL(0, 2); return true;              \
-    case 4: CALL(0, 4); return true;              \
-    case 6: CALL(0, 6); return true;              \
-    case 8: CALL(0, 8); return true;              \
-    case 12: CALL(0, 12); return true;            \
-    case 16: CALL(0, 16); return true;            \
-    case 32: CALL(0, 32); return true;            \
-    case 102: CALL(1, 2); return true;            \
-    case 104: CALL(1, 4); return true;            \
-    case 106: CALL(1, 6); return true;            \
-    case 108: CALL(1, 8); return true;            \
-    case 112: CALL(1, 12); return true;           \
-    case 116: CALL(1, 16); return true;           \
-    case 132: CALL(1, 32); return true;           \
-    case 202: CALL(2, 2); return true;            \
-    case 204: CALL(2, 4); return true;            \
-    case 206: CALL(2, 6); return true;            \
-    case 208: CALL(2, 8); return true;            \
-    case 212: CALL(2, 12); return true;           \
-    case 216: CALL(2, 16); return true;           \
-    case 232: CALL(2, 32); return true;           \
-    default: return false;                        \
+#define BOSS_DISPATCH_DP_CASES(CALL, K)  \
+  case (K) * 100 + 2: CALL(K, 2); return true;     \
+  case (K) * 100 + 4: CALL(K, 4); return true;     \
+  case (K) * 100 + 6: CALL(K, 6); return true;     \
+  case (K) * 100 + 8: CALL(K, 8); return true;     \
+  case (K) * 100 + 12: CALL(K, 12); return true;   \
+  case (K) * 100 + 16: CALL(K, 16); return true;   \
+  case (K) * 100 + 32: CALL(K, 32); return true;
+
+#define BOSS_DISPATCH_KID_DP(CALL, kid, dp) \
+  switch ((kid) * 100 + (dp)) {             \
+    BOSS_DISPATCH_DP_CASES(CALL, 0)         \
+    BOSS_DISPATCH_DP_CASES(CALL, 1)         \
+    BOSS_DISPATCH_DP_CASES(CALL, 2)         \
+    BOSS_DISPATCH_DP_CASES(CALL, 3)         \
+    BOSS_DISPATCH_DP_CASES(CALL, 4)         \
+    default: return false;                  \
+  }
+
+// the kernels of the FP32 mean tier: KIDs 0-2 only (see kid_has_f32_tier)
+#define BOSS_DISPATCH_KID_DP_F32(CALL, kid, dp) \
+  switch ((kid) * 100 + (dp)) {                 \
+    BOSS_DISPATCH_DP_CASES(CALL, 0)             \
+    BOSS_DISPATCH_DP_CASES(CALL, 1)             \
+    BOSS_DISPATCH_DP_CASES(CALL, 2)             \
+    default: return false;                      \
   }
 
 }  // namespace boss

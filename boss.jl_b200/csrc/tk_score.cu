@@ -1,6 +1,7 @@
 // tk_score.cu -- the FP64-pipe kernels of the scoring path that evaluate the covariance function: cross-covariance
 // K*^T + posterior mean (row a3), the finish of the full posterior covariance, and the kernel derivatives of the
-// x-gradient (row g1); instantiated for every (covariance function, padded input dimension).
+// x-gradient (row g1); instantiated for every (covariance function, padded input dimension), the FP32 mean tier for
+// KIDs 0-2 only.
 #include "common.cuh"
 #include "tk_params.cuh"
 
@@ -41,7 +42,7 @@ __global__ void __launch_bounds__(256) xcov_kernel(XcovParams p) {
           const double df = xc[i] - xt[kl * DP + i];
           d2 = fma(df, df, d2);
         }
-        v[kk] = p.a2 * kappa_fast<KID>(d2, etab);
+        v[kk] = p.a2 * kappa_fast<KID>(d2, etab, p.rq_a);
       }
       if (live < XCOV_KC) {
 #pragma unroll
@@ -238,7 +239,7 @@ __global__ void __launch_bounds__(256) cov_finish_kernel(CovFinishParams p) {
     d2 = fma(df, df, d2);
   }
   const int hi = max(i, j), lo = min(i, j);
-  double v = p.a2 * kappa_fast<KID>(d2, etab) - p.C[p_index(hi, lo, p.ktilesC)];
+  double v = p.a2 * kappa_fast<KID>(d2, etab, p.rq_a) - p.C[p_index(hi, lo, p.ktilesC)];
   if (i == j) {
     v += VAR_JITTER;
     if (!clip_var(v)) *p.any_fail = 1;
@@ -288,7 +289,7 @@ __global__ void __launch_bounds__(256) grad_kernel(GradParams p) {
           const double df = xc[i] - xt[kl * DP + i];
           d2 = fma(df, df, d2);
         }
-        gk[kk] = p.a2 * kappa_dr_over_r_fast<KID>(d2, etab);
+        gk[kk] = p.a2 * kappa_dr_over_r_fast<KID>(d2, etab, p.rq_a);
       }
       if (p.n - k0 < XCOV_KC) {
 #pragma unroll
@@ -329,7 +330,7 @@ bool launch_xcov_mean(int kid, int dp, const XcovParams &p, dim3 grid, cudaStrea
 }
 bool launch_xcov_mean_f32(int kid, int dp, const XcovF32Params &p, dim3 grid, cudaStream_t st) {
 #define CALL(K, D) xcov_mean_mma_kernel<K, D><<<grid, 256, 0, st>>>(p)
-  BOSS_DISPATCH_KID_DP(CALL, kid, dp)
+  BOSS_DISPATCH_KID_DP_F32(CALL, kid, dp)
 #undef CALL
 }
 bool launch_kappa_f32_sweep(int kid, const double *r, int n, double *out, cudaStream_t st) {

@@ -64,7 +64,7 @@ __global__ void __launch_bounds__(SMALL_WARPS * 32) loglik_small_kernel(SmallLog
         const double df = xi[q] - __dmul_rn(xs[j * DP + q], invl[q]);
         d2 = fma(df, df, d2);
       }
-      v = a2 * kappa<KID>(d2);
+      v = a2 * kappa<KID>(d2, p.rq_a);
       if (j == lane) v += s2;
     }
     a[j] = v;
@@ -109,7 +109,8 @@ __global__ void __launch_bounds__(SMALL_WARPS * 32) loglik_small_kernel(SmallLog
 // k[i] = a^2 kappa(|x~_i - x~+|), i < n (zero beyond); also appends the scaled point as row n of Xt.
 template <int KID, int DP>
 __global__ void append_kvec_kernel(const double *xnew, int d, int n, int n_pad, const double *invl,
-                                   unsigned long long disc_bits, double a2, double *Xt, double *kvec) {
+                                   unsigned long long disc_bits, double a2, double rq_a, double *Xt,
+                                   double *kvec) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n_pad) return;
   double xn[DP];
@@ -122,7 +123,7 @@ __global__ void append_kvec_kernel(const double *xnew, int d, int n, int n_pad, 
       const double df = Xt[(size_t)i * DP + q] - xn[q];
       d2 = fma(df, df, d2);
     }
-    val = a2 * kappa<KID>(d2);
+    val = a2 * kappa<KID>(d2, rq_a);
   }
   kvec[i] = val;
   if (i == n) {
@@ -137,8 +138,9 @@ bool launch_loglik_small(int kid, int dp, const SmallLoglikParams &p, int nblock
 #undef CALL
 }
 bool launch_append_kvec(int kid, int dp, const double *xnew, int d, int n, int n_pad, const double *invl,
-                        unsigned long long disc_bits, double a2, double *Xt, double *kvec, cudaStream_t st) {
-#define CALL(K, D) append_kvec_kernel<K, D><<<(n_pad + 255) / 256, 256, 0, st>>>(xnew, d, n, n_pad, invl, disc_bits, a2, Xt, kvec)
+                        unsigned long long disc_bits, double a2, double rq_a, double *Xt, double *kvec, cudaStream_t st) {
+#define CALL(K, D) append_kvec_kernel<K, D><<<(n_pad + 255) / 256, 256, 0, st>>>(xnew, d, n, n_pad, invl, disc_bits, a2, rq_a, Xt, \
+                                                                             kvec)
   BOSS_DISPATCH_KID_DP(CALL, kid, dp)
 #undef CALL
 }

@@ -28,6 +28,26 @@ class Matern52Kernel:
 
 
 @dataclass(frozen=True)
+class ExponentialKernel:
+    """exp(-r): the Matern-1/2 kernel, for rough objectives."""
+    kernel_id: int = _lib.KERNEL_MATERN12
+
+
+Matern12Kernel = ExponentialKernel   # KernelFunctions' alias
+
+
+@dataclass(frozen=True)
+class RationalQuadraticKernel:
+    """(1 + r^2 / (2 alpha))^-alpha, alpha > 0: a scale mixture of squared exponentials (KernelFunctions' default
+    alpha = 2).  alpha is the kernel's fixed shape parameter, not BOSS's amplitude and not a hyper-parameter."""
+    alpha: float = 2.0
+
+    @property
+    def kernel_id(self):
+        return _lib.kernel_rational_quadratic(self.alpha)
+
+
+@dataclass(frozen=True)
 class DiscreteKernel:
     """src/models/utils/kernels.jl:43-69: round the flagged dims before evaluating the kernel."""
     kernel: object

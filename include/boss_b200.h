@@ -57,6 +57,21 @@ extern "C" {
 #define BOSS_KERNEL_SE 0        /* SqExponentialKernel                         */
 #define BOSS_KERNEL_MATERN32 1  /* Matern32Kernel (examples/example.jl:88)     */
 #define BOSS_KERNEL_MATERN52 2  /* Matern52Kernel (default, src/deprecated.jl:34) */
+#define BOSS_KERNEL_MATERN12 3  /* ExponentialKernel = Matern12Kernel: exp(-r)   */
+/* RationalQuadraticKernel(alpha = rq_a): kappa = (1 + r^2 / (2 rq_a))^-rq_a.  rq_a is KernelFunctions' shape parameter
+ * (not BOSS's amplitude) and is part of the kernel, so it has no fixed id: boss_kernel_rational_quadratic registers it
+ * in a process-lifetime host table and writes an id (256 + slot) that boss_gp_fit, boss_gp_fit_batch and the
+ * boss_gp_loglik* entry points accept.  The same bits of rq_a always give the same id.  Thread-safe, callable before
+ * boss_init and after boss_shutdown (no device state).  A non-finite or non-positive rq_a, or a full table
+ * (BOSS_RQ_SLOTS distinct values), is BOSS_ERR_ARG.  A handle keeps the kernel family and rq_a it was fitted with.
+ * Ids 4-255 and unassigned slots are unknown kernel ids.
+ * r = 0 convention of Matern12 (DESIGN.md 2.14): exp(-r) has a cusp there, and kappa'(r)/r = -exp(-r)/r is taken as 0
+ * at r == 0.  A duplicated training point then adds 0 to the log-likelihood gradient (its per-pair term g dq^2 has limit
+ * 0 anyway), and a candidate that coincides with a training point in scaled coordinates gets 0 from that point in
+ * d mu / dx and d var / dx (the symmetric subgradient).  This is believed to match ForwardDiff under the reference's
+ * nansafe_mode = true (sqrt'(0) * 0 -> 0); it has not been checked against Julia. */
+#define BOSS_RQ_SLOTS 512
+int boss_kernel_rational_quadratic(double rq_a, int *kernel_id);
 
 typedef struct boss_gp boss_gp; /* opaque: one fitted GP = one output slice x one hyper-parameter vector */
 
@@ -363,6 +378,9 @@ int boss_dbg_gemm_nt(const double *A, const double *B, int M, int N, int K, doub
 /* device scalar functions of the kernel-matrix stages: which = 0 exp(-t), 1 sqrt(t), 2-4 kappa(d2) SE / Matern32 /
  * Matern52, 5-7 kappa'(r)/r of the same */
 int boss_dbg_kernel_fn(int which, const double *t, int n, double *out);
+/* the covariance function of any accepted kernel_id (registered RQ ids included) at n squared distances d2:
+ * which = 0 kappa_fast, 1 kappa'(r)/r fast, 2 kappa (libm), 3 kappa'(r)/r (libm) */
+int boss_dbg_kernel_fn_id(int kernel_id, int which, const double *d2, int n, double *out);
 int boss_dbg_factors(const boss_gp *gp, double *L, double *W, double *alpha);          /* dense row-major n x n, n   */
 /* BOSS_DEBUG_REDZONE=1 (environment, read at the first allocation): every device allocation is exact-sized and
  * bracketed by 64 KB guard bands of 0xA5.  Returns the number of guard bytes overwritten so far on the calling

@@ -38,7 +38,8 @@ using BOSS: GaussianProcess, GaussianProcessParams, Semiparametric, Semiparametr
             ModelPosteriorSlice, DefaultModelPosterior, BossProblem, BossOptions, AcquisitionMaximizer, ModelFitter,
             GridAM, SamplingAM, OptimizationAM, SampleOptAM, SequentialBatchAM, SamplingMAP, ExpectedImprovement,
             LinFitness, NonlinFitness, MAPParams, BIParams, Infinity, mean_getindex, best_so_far, get_params, y_dim
-using KernelFunctions: SqExponentialKernel, Matern32Kernel, Matern52Kernel
+using KernelFunctions: SqExponentialKernel, Matern32Kernel, Matern52Kernel, ExponentialKernel, RationalQuadraticKernel
+using Distances: Euclidean
 using LinearAlgebra: diag, PosDefException
 using Random: shuffle
 using ForwardDiff
@@ -66,6 +67,23 @@ shutdown() = ccall((:boss_shutdown, LIB), Cvoid, ())
 kernel_id(::SqExponentialKernel) = 0
 kernel_id(::Matern32Kernel) = 1
 kernel_id(::Matern52Kernel) = 2
+# ExponentialKernel (= Matern12Kernel) and RationalQuadraticKernel: the device evaluates them on the Euclidean distance
+# only; any other metric keeps the stock path.  An RQ kernel's shape α is registered once per value with the library
+# (boss_kernel_rational_quadratic, host-only, thread-safe) and the id is cached here.
+kernel_id(k::ExponentialKernel) = k.metric isa Euclidean ? 3 : nothing
+const RQ_IDS = Dict{Float64,Cint}()
+const RQ_LOCK = ReentrantLock()
+function kernel_id(k::RationalQuadraticKernel)
+    k.metric isa Euclidean || return nothing
+    a = Float64(only(k.α))
+    lock(RQ_LOCK) do
+        get!(RQ_IDS, a) do
+            id = Ref{Cint}(-1)
+            check(ccall((:boss_kernel_rational_quadratic, LIB), Cint, (Cdouble, Ref{Cint}), a, id))
+            id[]
+        end
+    end
+end
 kernel_id(k::BOSS.DiscreteKernel) = kernel_id(k.kernel)
 kernel_id(k) = nothing                                  # CustomKernel etc.: not accelerated -> stock BOSS.jl path
 discrete_mask(k::BOSS.DiscreteKernel) = k.dims isa Missing ? nothing : Vector{UInt8}(k.dims)
