@@ -1828,9 +1828,9 @@ struct Screen {
   // refinement batch, the survivor pool with each row's bound and verdict, and the re-compacted pool
   double *bound = nullptr, *lo = nullptr, *seed_x = nullptr, *seed_pm = nullptr, *pool_x = nullptr, *pool_pm = nullptr;
   double *pool_bound = nullptr, *ref_x = nullptr, *ref_pm = nullptr, *consts = nullptr;
-  int *cnt = nullptr, *ti[2] = {}, *ref_row = nullptr, *ref_cnt = nullptr;
+  int *ti[2] = {}, *ref_row = nullptr, *ref_cnt = nullptr;
   unsigned long long *tk[2] = {};
-  long long *base = nullptr, *pool_idx = nullptr;
+  long long *cnt = nullptr, *base = nullptr, *pool_idx = nullptr;   // cnt: survivors per 128 candidates, then offsets
   unsigned char *seed_cm = nullptr, *pool_cm = nullptr, *pool_ver = nullptr;
   std::vector<float *> xt32, al32;   // per slice: the MMA tier's B fragments of the centred training inputs, |t~|^2 and alpha
 
@@ -1853,14 +1853,18 @@ struct Screen {
     const long long M = a.M;
     const int CH = c.CH, d = c.d, y_dim = a.y_dim, ns_max = a.topk ? topk_seed_n(a.topk, ch0) : SEED_N;
     const bool pm = a.prior_mean != nullptr, cm = a.cons_mask != nullptr;
-    // the FP32 tier's error bound is proven for KIDs 0-2 only; a call with any other slice keeps FP64 means throughout
-    f32 = getenv("BOSS_SCREEN_F64") == nullptr &&
-          std::all_of(c.sl.begin(), c.sl.begin() + c.nsl, [](const boss_gp *h) { return kid_has_f32_tier(h->kernel_id); });
+    // the FP32 tier's error bound is proven for KIDs 0-2 only, and its kernel takes up to SCREEN_F32_MAX_SL slices of one
+    // covariance function: any other call keeps FP64 means throughout
+    const int kid0 = c.sl[0]->kernel_id;
+    f32 = getenv("BOSS_SCREEN_F64") == nullptr && kid_has_f32_tier(kid0) && c.nsl <= SCREEN_F32_MAX_SL &&
+          std::all_of(c.sl.begin(), c.sl.begin() + c.nsl, [&](const boss_gp *h) { return h->kernel_id == kid0; });
     reseed = getenv("BOSS_SCREEN_NO_RESEED") == nullptr;
     size_t tot = 0;
     const size_t ntk = (size_t)(CH + TOPK_IN - 1) / TOPK_IN * SEED_N;
-    const size_t o_bound = take(tot, (size_t)CH * 8), o_lo = take(tot, (size_t)CH * 8);
-    const size_t o_cnt = take(tot, (size_t)(CH + 255) / 256 * 4), o_base = take(tot, 32);
+    // bounds and counts for one chunk, or for all candidates after the first when they are on the device (FP32 tier)
+    const size_t span = a.dev && f32 ? std::max<long long>(CH, M) : CH;
+    const size_t o_bound = take(tot, span * 8), o_lo = take(tot, span * 8);
+    const size_t o_cnt = take(tot, (span + 127) / 128 * 8), o_base = take(tot, 32);
     const size_t o_tk0 = take(tot, ntk * 8), o_tk1 = take(tot, ntk * 8), o_ti0 = take(tot, ntk * 4), o_ti1 = take(tot, ntk * 4);
     const size_t o_sx = take(tot, (size_t)ns_max * d * 8), o_spm = take(tot, (size_t)ns_max * y_dim * 8), o_scm = take(tot, ns_max);
     const size_t o_rx = take(tot, (size_t)CH * d * 8), o_rpm = take(tot, pm ? (size_t)CH * y_dim * 8 : 0);
@@ -1875,7 +1879,7 @@ struct Screen {
     unsigned char *b = C().scr_misc.as<unsigned char>();
     bound = reinterpret_cast<double *>(b + o_bound);
     lo = reinterpret_cast<double *>(b + o_lo);
-    cnt = reinterpret_cast<int *>(b + o_cnt);
+    cnt = reinterpret_cast<long long *>(b + o_cnt);
     base = reinterpret_cast<long long *>(b + o_base);
     tk[0] = reinterpret_cast<unsigned long long *>(b + o_tk0);
     tk[1] = reinterpret_cast<unsigned long long *>(b + o_tk1);
@@ -1920,31 +1924,14 @@ struct Screen {
   // chunk also sets the threshold from the seed batch and ends screening (the chunk is then scored on the full path
   // from the same staged inputs) when the bound does not separate: T not positive, or more than a quarter of the chunk
   // surviving.  The first chunk takes the FP64 means, so the seed batch, T and that decision are those of the FP64
-  // tier; later chunks of the FP32 tier bound EI from mu~ +- E' and leave the ambiguous ones to Screen::finish.
+  // tier; later chunks of the FP32 tier bound EI from mu~ +- E' in one launch of screen_mean_bound_kernel and leave the
+  // ambiguous ones to Screen::finish.  With device-resident candidates, the FP32 tier's "chunk" is everything after the
+  // first chunk (see score_core).
   int chunk(const ScoreCall &c, const AcqParams &ap, const ChunkIO &io, int cidx, TopkBufs &tb) {
     const ScoreArgs &a = c.a;
     const long long m0 = ap.m0;
     const int ch = ap.chunk, ncb = (ch + 127) / 128, nb = (ch + 255) / 256;
     const bool t32 = f32 && cidx > 0;
-    for (int q = 0; q < c.nsl; ++q) {
-      const boss_gp *h = c.sl[q];
-      const int nks = std::max(1, std::min(h->nblk, (16 * 148 + ncb - 1) / ncb));
-      const XcovParams xp = xcov_params(h, io.xs, a.M, m0, io.off, c.d, c.CH);
-      {
-        Timed t(1);
-        if (t32)
-          launch_xcov_mean_f32(h->kernel_id, h->dp,
-                               XcovF32Params{xp, reinterpret_cast<const float4 *>(xt32[q]),
-                                             reinterpret_cast<const float4 *>(al32[q]), consts + (size_t)SCREEN_NCONST * q,
-                                             C().sumsq.as<double>() + (size_t)q * c.CH},
-                               dim3(ncb, nks), C().stream);
-        else
-          launch_xcov_mean(h->kernel_id, h->dp, xp, dim3(ncb, nks), C().stream);
-      }
-      if (t32 && q == c.nsl - 1) break;   // the tail kernel sums the last slice's partials
-      reduce_rows_kernel<<<(ncb * 128 + 255) / 256, 256, 0, C().stream>>>(C().part_mu.as<double>(), 2 * h->nblk, (size_t)c.CH,
-                                                                        C().muv.as<double>() + (size_t)q * c.CH, ncb * 128);
-    }
     AcqParams bp = ap;   // EI at the prior variance, PoF = 1, no guards -> bound[c]
     bp.sumsq = nullptr;
     bp.has_ymax = 0;
@@ -1956,13 +1943,41 @@ struct Screen {
     bp.blk_idx = nullptr;
     // FP32 tier: hi < thr (1 - 2^-32) drops, lo >= thr (1 + 2^-32) keeps, anything else (NaN too) is ambiguous.  The
     // first chunk (FP64 tier) sets thr in seed().
-    if (t32) {   // muv <- mu~ + E', sumsq <- mu~ - E'; bound = EI at the first (hi), lo = EI at the second; the counts
-      TailParams tp{bp, bp, C().part_mu.as<double>(), 2 * c.sl[c.nsl - 1]->nblk, c.nsl, thr * (1.0 - 0x1p-32), cnt};
-      tp.lo.mu = C().sumsq.as<double>();
-      tp.lo.acq = lo;
-      screen_tail_kernel<<<nb, 256, 0, C().stream>>>(tp);
-      C().launches += 2 * c.nsl;
+    if (t32) {
+      ScreenF32Params sp{};
+      sp.Xs = io.xs;
+      sp.m0 = m0;
+      sp.M = m0 + ch;
+      sp.in_off = io.off;
+      sp.d = c.d;
+      sp.nsl = c.nsl;
+      for (int q = 0; q < c.nsl; ++q) {
+        const boss_gp *h = c.sl[q];
+        sp.sl[q] = ScreenSlice{reinterpret_cast<const float4 *>(xt32[q]), reinterpret_cast<const float4 *>(al32[q]),
+                               consts + (size_t)SCREEN_NCONST * q, h->invl, h->disc, h->a2, h->n_pad};
+      }
+      sp.hi = bp;
+      sp.lo = bp;
+      sp.lo.acq = lo;
+      sp.thr = thr * (1.0 - 0x1p-32);
+      sp.cnt = cnt;
+      {
+        Timed t(1);
+        launch_screen_mean_bound(c.sl[0]->kernel_id, c.sl[0]->dp, sp, ncb, C().stream);
+      }
+      ++C().launches;
     } else {
+      for (int q = 0; q < c.nsl; ++q) {
+        const boss_gp *h = c.sl[q];
+        const int nks = std::max(1, std::min(h->nblk, (16 * 148 + ncb - 1) / ncb));
+        {
+          Timed t(1);
+          launch_xcov_mean(h->kernel_id, h->dp, xcov_params(h, io.xs, a.M, m0, io.off, c.d, c.CH), dim3(ncb, nks),
+                           C().stream);
+        }
+        reduce_rows_kernel<<<(ncb * 128 + 255) / 256, 256, 0, C().stream>>>(
+            C().part_mu.as<double>(), 2 * h->nblk, (size_t)c.CH, C().muv.as<double>() + (size_t)q * c.CH, ncb * 128);
+      }
       acq_kernel<<<nb, 256, 0, C().stream>>>(bp);
       C().launches += 2 * c.nsl + 1;
     }
@@ -1976,13 +1991,14 @@ struct Screen {
     }
     const double thr_drop = t32 ? thr * (1.0 - 0x1p-32) : thr;
     if (!t32) {
-      screen_count_kernel<<<nb, 256, 0, C().stream>>>(bound, nullptr, ch, thr_drop, cnt);
+      screen_count_kernel<<<ncb, 128, 0, C().stream>>>(bound, nullptr, ch, thr_drop, cnt);
       ++C().launches;
     }
+    screen_scan_kernel<<<1, 1024, 0, C().stream>>>(cnt, ncb, base, cidx & 1);
     CompactParams cpar{bound, nullptr, ch, thr_drop, t32 ? lo : nullptr, thr * (1.0 + 0x1p-32), cnt, m0, xs_c, pm_c, cm_c,
-                       c.d, a.y_dim, base, cidx & 1, pool_x, pool_pm, pool_cm, pool_idx, nullptr, pool_bound, pool_ver};
-    screen_compact_kernel<<<nb, 256, 0, C().stream>>>(cpar);
-    ++C().launches;
+                       c.d, a.y_dim, pool_x, pool_pm, pool_cm, pool_idx, nullptr, pool_bound, pool_ver};
+    screen_compact_kernel<<<ncb, 128, 0, C().stream>>>(cpar);
+    C().launches += 2;
     if (cidx == 0) {
       long long surv = 0;
       CUDA_TRY(cudaMemcpyAsync(&surv, base + 1, 8, cudaMemcpyDeviceToHost, C().stream));
@@ -2185,16 +2201,17 @@ struct Screen {
     unsigned char *b = C().scr_pool2.as<unsigned char>();
     int par = 0;
     for (long long r0 = 0; r0 < npool; r0 += c.CH, par ^= 1) {
-      const int n = (int)std::min<long long>(c.CH, npool - r0), nb = (n + 255) / 256;
-      screen_count_kernel<<<nb, 256, 0, C().stream>>>(pool_bound + r0, pool_ver + r0, n, thr2, cnt);
+      const int n = (int)std::min<long long>(c.CH, npool - r0), ncb = (n + 127) / 128;
+      screen_count_kernel<<<ncb, 128, 0, C().stream>>>(pool_bound + r0, pool_ver + r0, n, thr2, cnt);
+      screen_scan_kernel<<<1, 1024, 0, C().stream>>>(cnt, ncb, base + 2, par);
       CompactParams cp{pool_bound + r0, pool_ver + r0, n, thr2, nullptr, 0.0, cnt, 0,
                        pool_x + (size_t)r0 * c.d, pool_pm ? pool_pm + (size_t)r0 * a.y_dim : nullptr,
-                       pool_cm ? pool_cm + r0 : nullptr, c.d, a.y_dim, base + 2, par,
+                       pool_cm ? pool_cm + r0 : nullptr, c.d, a.y_dim,
                        reinterpret_cast<double *>(b), pool_pm ? reinterpret_cast<double *>(b + p2_off[1]) : nullptr,
                        pool_cm ? b + p2_off[2] : nullptr, reinterpret_cast<long long *>(b + p2_off[0]), pool_idx + r0,
                        nullptr, nullptr};
-      screen_compact_kernel<<<nb, 256, 0, C().stream>>>(cp);
-      C().launches += 2;
+      screen_compact_kernel<<<ncb, 128, 0, C().stream>>>(cp);
+      C().launches += 3;
     }
     CUDA_TRY(cudaMemcpyAsync(&nfin, base + 2 + par, 8, cudaMemcpyDeviceToHost, C().stream));
     CUDA_TRY(cudaStreamSynchronize(C().stream));
@@ -2237,8 +2254,11 @@ int score_core(ScoreArgs &a) {
 
   timing_begin();
   int cidx = 0;
-  for (long long m0 = 0; m0 < a.M; m0 += c.CH, ++cidx) {
-    const int ch = (int)std::min<long long>(c.CH, a.M - m0);
+  for (long long m0 = 0, step = 0; m0 < a.M; m0 += step, ++cidx) {
+    // device-resident candidates on the FP32 screening tier: everything after the first chunk in one piece (the
+    // screened call's M fits the pool, so an int)
+    const int ch = (int)std::min<long long>(scr.on() && scr.f32 && a.dev && cidx > 0 ? a.M : c.CH, a.M - m0);
+    step = ch;
     const int slot = cidx & 1;
     ChunkIO io;
     if (a.dev) {
@@ -3580,15 +3600,17 @@ int boss_dbg_gemm_nt(const double *A, const double *B, int M, int N, int K, doub
   CUDA_TRY(cudaMalloc(&dA, pa.size() * 8));
   CUDA_TRY(cudaMalloc(&dB, pb.size() * 8));
   CUDA_TRY(cudaMalloc(&dC, (size_t)Mp * Np * 8));
-  CUDA_TRY(cudaMemcpy(dA, pa.data(), pa.size() * 8, cudaMemcpyHostToDevice));
-  CUDA_TRY(cudaMemcpy(dB, pb.data(), pb.size() * 8, cudaMemcpyHostToDevice));
+  // copies on the context's stream: it does not synchronise with the legacy default stream, so a plain cudaMemcpy
+  // from pageable memory could still be in flight when the kernel reads its destination
+  CUDA_TRY(cudaMemcpyAsync(dA, pa.data(), pa.size() * 8, cudaMemcpyHostToDevice, C().stream));
+  CUDA_TRY(cudaMemcpyAsync(dB, pb.data(), pb.size() * 8, cudaMemcpyHostToDevice, C().stream));
   GemmNtParams p{dA, dB, dC, Kp / TK, Np / TK, 0};
   gemm_nt_kernel<<<dim3(Np / TM, Mp / TM), GEMM_THREADS, GEMM_SMEM_BYTES, C().stream>>>(p);
   ++C().launches;
   CUDA_TRY(cudaGetLastError());
-  CUDA_TRY(cudaStreamSynchronize(C().stream));
   std::vector<double> pc((size_t)Mp * Np);
-  CUDA_TRY(cudaMemcpy(pc.data(), dC, pc.size() * 8, cudaMemcpyDeviceToHost));
+  CUDA_TRY(cudaMemcpyAsync(pc.data(), dC, pc.size() * 8, cudaMemcpyDeviceToHost, C().stream));
+  CUDA_TRY(cudaStreamSynchronize(C().stream));
   for (int r = 0; r < M; ++r)
     for (int c = 0; c < N; ++c) Cout[(size_t)r * N + c] = pc[p_index(r, c, Np / TK)];
   cudaFree(dA);
@@ -3623,10 +3645,11 @@ int boss_dbg_kernel_fn(int which, const double *t, int n, double *out) {
   double *dt, *dout;
   CUDA_TRY(cudaMalloc(&dt, (size_t)n * 8 + 8));
   CUDA_TRY(cudaMalloc(&dout, (size_t)n * 8 + 8));
-  CUDA_TRY(cudaMemcpy(dt, t, (size_t)n * 8, cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpyAsync(dt, t, (size_t)n * 8, cudaMemcpyHostToDevice, C().stream));   // stream-ordered, as above
   dbg_kernel_fn_kernel<<<148, 256, 0, C().stream>>>(which, dt, dout, n);
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaMemcpyAsync(out, dout, (size_t)n * 8, cudaMemcpyDeviceToHost, C().stream));
   CUDA_TRY(cudaStreamSynchronize(C().stream));
-  CUDA_TRY(cudaMemcpy(out, dout, (size_t)n * 8, cudaMemcpyDeviceToHost));
   cudaFree(dt);
   cudaFree(dout);
   return 0;
@@ -3764,13 +3787,19 @@ int boss_dbg_screen_mean(const boss_gp *gp, const double *Xs, int64_t M, double 
   CUDA_TRY(cudaMalloc(&dal, (size_t)gp->n_pad * 8));
   CUDA_TRY(cudaMemcpyAsync(dx, Xs, (size_t)M * d * 8, cudaMemcpyHostToDevice, C().stream));
   screen_consts_kernel<<<1, 1024, 0, C().stream>>>(gp->Xt, gp->alpha, gp->n, gp->n_pad, gp->dp, dxt, dal, dA);
+  ScreenF32Params sp{};
+  sp.Xs = dx;
+  sp.M = M;
+  sp.d = d;
+  sp.nsl = 1;
+  sp.sl[0] = ScreenSlice{reinterpret_cast<const float4 *>(dxt), reinterpret_cast<const float4 *>(dal), dA, gp->invl,
+                         gp->disc, gp->a2, gp->n_pad};
+  sp.mu_out = dout;
+  sp.e_out = dout + ld;
+  sp.ld = ld;
+  launch_screen_mean_bound(gp->kernel_id, gp->dp, sp, ncb, C().stream);
   XcovParams xp = xcov_params(gp, dx, M, 0, 0, d, ld);
   xp.mu_part = dpart;
-  launch_xcov_mean_f32(gp->kernel_id, gp->dp,
-                       XcovF32Params{xp, reinterpret_cast<const float4 *>(dxt), reinterpret_cast<const float4 *>(dal), dA,
-                                     dout + ld},
-                       dim3(ncb, nks), C().stream);
-  reduce_rows_kernel<<<(ld + 255) / 256, 256, 0, C().stream>>>(dpart, 2 * gp->nblk, (size_t)ld, dout, ld);
   launch_xcov_mean(gp->kernel_id, gp->dp, xp, dim3(ncb, nks), C().stream);
   reduce_rows_kernel<<<(ld + 255) / 256, 256, 0, C().stream>>>(dpart, 2 * gp->nblk, (size_t)ld, dout + 2 * ld, ld);
   CUDA_TRY(cudaGetLastError());

@@ -10,6 +10,7 @@
 // argmax loops grid.jl:52-65, sampling.jl:37-48.  W = L^-1 is formed once per fit, so the per-candidate
 // triangular solve of the reference becomes a triangular matrix product.
 #pragma once
+#include "acq.cuh"
 #include "gemm_core.cuh"
 #include "kernel_fn.cuh"
 #include "tk_params.cuh"
@@ -52,168 +53,6 @@ __global__ void __launch_bounds__(256) reduce_rows_kernel(const double *__restri
 // ---------------------------------------------------------------------------------------------
 // elementwise acquisition stage + block argmax
 // ---------------------------------------------------------------------------------------------
-constexpr int MAX_YDIM = 16;
-
-// Monte-Carlo expected improvement for a NonlinFitness drawn from a small expression set
-// (expected_improvement(::NonlinFitness, ...), src/acquisitions/expected_improvement.jl:104-111):
-//   EI = 1/K sum_k max(0, f(mu + sqrt(var) .* eps_k) - best),   f one of
-//   kind 1  affine     f(y) = c0 + sum_i c_i y_i
-//   kind 2  quadratic  f(y) = c0 + sum_i c_i y_i + sum_i q_i (y_i - t_i)^2
-//   kind 3  max        f(y) = c0 + max_i (c_i y_i + t_i)   over the outputs with c_i != 0
-//   kind 4  min        f(y) = c0 + min_i (c_i y_i + t_i)   over the outputs with c_i != 0
-// kind 0 = off (LinFitness closed form).  An arbitrary Julia closure stays a host job (INTEGRATION.md).
-constexpr int MIX_MAX_EPS = 4096;
-struct MixParams {
-  int kind = 0, n_eps = 0;
-  double c0 = 0.0;
-  double c[MAX_YDIM] = {}, q[MAX_YDIM] = {}, t[MAX_YDIM] = {};
-  const double *eps = nullptr;        // device, y_dim x n_eps column-major
-  const double *eps_host = nullptr;   // host copy handed in by the caller (uploaded by score_core)
-};
-__host__ __device__ __forceinline__ double mix_fitness(const MixParams &mx, const double *y, int y_dim) {
-  double f = mx.c0;
-  if (mx.kind == 1) {
-    for (int i = 0; i < y_dim; ++i) f = fma(mx.c[i], y[i], f);
-  } else if (mx.kind == 2) {
-    for (int i = 0; i < y_dim; ++i) {
-      const double dv = y[i] - mx.t[i];
-      f = fma(mx.c[i], y[i], f);
-      f = fma(mx.q[i] * dv, dv, f);
-    }
-  } else {
-    bool any = false;
-    double ext = 0.0;
-    for (int i = 0; i < y_dim; ++i) {
-      if (mx.c[i] == 0.0) continue;
-      const double v = fma(mx.c[i], y[i], mx.t[i]);
-      if (!any) {
-        ext = v;
-        any = true;
-      } else if (v != v || ext != ext) {
-        ext = NAN;
-      } else {
-        ext = mx.kind == 3 ? (v > ext ? v : ext) : (v < ext ? v : ext);
-      }
-    }
-    f += ext;
-  }
-  return f;
-}
-
-struct AcqParams {
-  int y_dim, n_samples, d;
-  long long M, m0;       // global candidate count / chunk start
-  long long in_off;      // Xs / prior_mean / cons_mask are indexed by (m - in_off)
-  long long out_off;     // acq / mu_out / var_out / status_out are indexed by (m - out_off)
-  int chunk;             // candidates in this chunk
-  int chunk_ld;          // leading dimension of mu / sumsq ([n_samples*y_dim][chunk_ld])
-  const double *mu;      // K*^T alpha per (sample, slice)
-  const double *sumsq;   // |W k*|^2 per (sample, slice)
-  const double *a2;      // [n_samples*y_dim] prior variance a^2 (device)
-  const double *prior_mean;  // y_dim x M or null
-  double coefs[MAX_YDIM];
-  double y_max[MAX_YDIM];
-  int has_best, has_ymax;
-  double best;
-  const double *Xs;      // d x M for the bounds check (null if no bounds)
-  const double *lb, *ub; // device, d each (null if no bounds)
-  const unsigned char *cons_mask;  // or null
-  double *acq;           // or null
-  double *mu_out, *var_out;  // predict mode (single slice) or null
-  int *status_out;       // predict mode or null
-  int *any_fail;         // device flag
-  double *blk_val;       // per-block winners
-  long long *blk_idx;
-  MixParams mix;         // kind != 0: Monte-Carlo EI of a NonlinFitness expression instead of the closed form
-};
-
-__device__ __forceinline__ double norm_cdf(double z) { return 0.5 * erfc(-z * 0.7071067811865476); }
-__device__ __forceinline__ double norm_pdf(double z) { return exp(-0.5 * z * z) * 0.3989422804014327; }
-
-
-// The acquisition value of candidate c of the chunk (global index m): slices x BI samples -> EI x PoF, guards.
-// Writes the optional per-candidate outputs.  Shared by acq_kernel and the fused epilogue of score_trmm_kernel.
-__device__ __forceinline__ double acq_candidate(const AcqParams &p, const int c, const long long m) {
-  double result;
-  {
-    double accum = 0.0;
-    bool failed = false;
-    for (int s = 0; s < p.n_samples; ++s) {
-      double mu_f = 0.0, s2 = 0.0, pof = 1.0;
-      double mu_i[MAX_YDIM], sd_i[MAX_YDIM];
-      for (int i = 0; i < p.y_dim; ++i) {
-        const size_t row = (size_t)(s * p.y_dim + i) * p.chunk_ld + c;
-        double mu = p.mu[row];
-        if (p.prior_mean) mu = p.prior_mean[(size_t)(m - p.in_off) * p.y_dim + i] + mu;
-        // sumsq == null: the prior variance a^2 + 1e-18, an upper bound of the posterior one (argmax screening)
-        double var = p.a2[s * p.y_dim + i] - (p.sumsq ? p.sumsq[row] : 0.0) + VAR_JITTER;
-        const bool ok = clip_var(var);
-        if (!ok) failed = true;
-        if (p.mu_out) p.mu_out[m - p.out_off] = mu;
-        if (p.var_out) p.var_out[m - p.out_off] = var;
-        if (p.status_out) p.status_out[m - p.out_off] = ok ? 0 : 2;
-        mu_f = fma(p.coefs[i], mu, mu_f);
-        s2 = fma(p.coefs[i] * p.coefs[i], var, s2);
-        mu_i[i] = mu;
-        sd_i[i] = sqrt(var);
-        if (p.has_ymax) {
-          const double ym = p.y_max[i];
-          if (!(ym == INFINITY)) {                 // cdf(., Infinity()) == 1 exactly (src/utils/inf.jl:13-15)
-            const double sd = sqrt(var);
-            double z = (ym - mu) / sd;
-            if (sd == 0.0 && ym == mu) z = INFINITY;   // StatsFuns: x == mu, sigma == 0 -> cdf 1
-            pof *= norm_cdf(z);
-          }
-        }
-      }
-      double a;
-      if (p.has_best && p.mix.kind != 0) {
-        // one posterior: all eps columns; BI posteriors: posterior s takes column s (expected_improvement.jl:87-90,108-111)
-        const int k0 = p.n_samples > 1 ? s : 0, k1 = p.n_samples > 1 ? s + 1 : p.mix.n_eps;
-        double tot = 0.0;
-        for (int k = k0; k < k1; ++k) {
-          double ys[MAX_YDIM];
-          for (int i = 0; i < p.y_dim; ++i) ys[i] = mu_i[i] + sd_i[i] * p.mix.eps[(size_t)k * p.y_dim + i];
-          const double imp = mix_fitness(p.mix, ys, p.y_dim) - p.best;
-          tot += (imp != imp) ? imp : (imp > 0.0 ? imp : 0.0);   // max(0, NaN) = NaN in Julia
-        }
-        const double ei = tot / (double)(k1 - k0);
-        a = p.has_ymax ? ei * pof : ei;
-      } else if (p.has_best) {
-        const double sf = sqrt(s2);
-        const double diff = mu_f - p.best;
-        double ei;
-        if (diff == 0.0 && sf == 0.0) {
-          ei = 0.0;
-        } else {
-          const double z = diff / sf;
-          ei = diff * norm_cdf(z) + sf * norm_pdf(z);
-        }
-        a = p.has_ymax ? ei * pof : ei;
-      } else {
-        a = p.has_ymax ? pof : 0.0;
-      }
-      accum += a;
-    }
-    result = accum / (double)p.n_samples;
-    if (failed) {
-      result = -INFINITY;
-      *p.any_fail = 1;
-    }
-    if (p.lb) {
-      bool inb = true;
-      for (int i = 0; i < p.d; ++i) {
-        const double x = p.Xs[(size_t)(m - p.in_off) * p.d + i];
-        if (x < p.lb[i] || x > p.ub[i]) inb = false;
-      }
-      if (!inb) result = 0.0;
-    }
-    if (p.cons_mask && p.cons_mask[m - p.in_off] == 0) result = 0.0;
-    if (p.acq) p.acq[m - p.out_off] = result;
-  }
-  return result;
-}
-
 __global__ void __launch_bounds__(256) acq_kernel(AcqParams p) {
   __shared__ double sv[256];
   __shared__ long long si[256];
@@ -355,16 +194,50 @@ __device__ __forceinline__ bool screen_keep(const double *bound, const unsigned 
   return c < ch && !(bound[c] < thr) && (!ver || ver[c] == 1);
 }
 
-__global__ void __launch_bounds__(256) screen_count_kernel(const double *bound, const unsigned char *ver, int ch, double thr,
-                                                           int *cnt) {
-  const int k = __syncthreads_count(screen_keep(bound, ver, blockIdx.x * 256 + threadIdx.x, ch, thr));
+// survivors per 128 candidates (launched with 128 threads)
+__global__ void __launch_bounds__(128) screen_count_kernel(const double *bound, const unsigned char *ver, int ch, double thr,
+                                                           long long *cnt) {
+  const int k = __syncthreads_count(screen_keep(bound, ver, blockIdx.x * 128 + threadIdx.x, ch, thr));
   if (threadIdx.x == 0) cnt[blockIdx.x] = k;
+}
+
+// The n per-128 survivor counts become, in place, the pool offsets of their candidate blocks: base[par] plus the
+// exclusive prefix sum.  base[par ^ 1] gets the pool size after them.  One CTA; each thread takes a contiguous run.
+__global__ void __launch_bounds__(1024) screen_scan_kernel(long long *cnt, int n, long long *base, int par) {
+  __shared__ long long ws[32];
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5, per = (n + 1023) / 1024;
+  const int j0 = min(n, tid * per), j1 = min(n, j0 + per);
+  long long s = 0;
+  for (int j = j0; j < j1; ++j) s += cnt[j];
+  long long v = s;   // inclusive scan: within the warp, then over the warps
+  for (int o = 1; o < 32; o <<= 1) {
+    const long long u = __shfl_up_sync(0xffffffffu, v, o);
+    if (lane >= o) v += u;
+  }
+  if (lane == 31) ws[w] = v;
+  __syncthreads();
+  if (w == 0) {
+    long long x = ws[lane];
+    for (int o = 1; o < 32; o <<= 1) {
+      const long long u = __shfl_up_sync(0xffffffffu, x, o);
+      if (lane >= o) x += u;
+    }
+    ws[lane] = x;
+  }
+  __syncthreads();
+  long long off = base[par] + (w ? ws[w - 1] : 0) + v - s;
+  for (int j = j0; j < j1; ++j) {
+    const long long k = cnt[j];
+    cnt[j] = off;
+    off += k;
+  }
+  if (tid == 1023) base[par ^ 1] = off;
 }
 
 // ---- the FP32 mean tier (DESIGN.md 2.9) ----
 
 // Per call and slice (one CTA of 1024 threads, every sum in a fixed order): the centre c = the mean of the n scaled
-// training inputs; the FP32 copies the MMA tier reads (XcovF32Params: the TF32-split B fragments of t~ = fp32(ut - c),
+// training inputs; the FP32 copies the MMA tier reads (ScreenSlice: the TF32-split B fragments of t~ = fp32(ut - c),
 // |t~|^2 and alpha); and the constants of the error bound, A1 = sum_j |alpha_j| and A3 = sum_j |alpha_j| |ut_j - c|^2.
 // A = [A1, A3, c_0 .. c_{DP-1}].
 __global__ void __launch_bounds__(1024) screen_consts_kernel(const double *Xt, const double *alpha, int n, int n_pad,
@@ -421,43 +294,6 @@ __global__ void __launch_bounds__(1024) screen_consts_kernel(const double *Xt, c
   }
 }
 
-// The tail of an FP32-tier chunk, one thread per candidate c:
-//  - the last slice's mean partials summed into hi.mu in reduce_rows_kernel's order (the earlier slices' are there);
-//  - per slice, mu~ (in hi.mu) and its bound E (in lo.mu) become mu~ + E' and mu~ - E', E' = E with the sign of the
-//    slice's output coefficient, so that EI is at least as large at the first as at the FP64 mean and no larger at the
-//    second; a non-finite mu~ or E gives NaN for both (the candidate is then ambiguous);
-//  - the EI bound at each (acq_candidate, into hi.acq and lo.acq);
-//  - the survivors per 256 candidates, screen_count_kernel's rule with hi.acq as the bound.
-struct TailParams {
-  AcqParams hi, lo;     // the bound pass at mu~ + E' and at mu~ - E' (same rows, chunk_ld and coefficients)
-  const double *part;   // the last slice's partials, [P][hi.chunk_ld]
-  int P, nsl;
-  double thr;           // drop threshold of the count
-  int *cnt;
-};
-__global__ void __launch_bounds__(256) screen_tail_kernel(TailParams p) {
-  const int c = blockIdx.x * 256 + threadIdx.x;
-  const long long m = p.hi.m0 + c;
-  const bool active = c < p.hi.chunk && m < p.hi.M;
-  bool keep = false;
-  if (active) {
-    double *mu = const_cast<double *>(p.hi.mu), *e = const_cast<double *>(p.lo.mu);
-    const size_t ld = (size_t)p.hi.chunk_ld;
-    mu[(size_t)(p.nsl - 1) * ld + c] = ordered_sum(p.part + c, ld, p.P);
-    for (int q = 0; q < p.nsl; ++q) {
-      const size_t o = (size_t)q * ld + c;
-      const double mq = mu[o], E = p.hi.coefs[q % p.hi.y_dim] < 0.0 ? -e[o] : e[o];
-      const bool ok = isfinite(mq) && isfinite(E);
-      mu[o] = ok ? mq + E : NAN;
-      e[o] = ok ? mq - E : NAN;
-    }
-    keep = !(acq_candidate(p.hi, c, m) < p.thr);
-    acq_candidate(p.lo, c, m);
-  }
-  const int k = __syncthreads_count(keep);
-  if (threadIdx.x == 0) p.cnt[blockIdx.x] = k;
-}
-
 // The ambiguous rows (verdict 2) among pool rows [0, n) of a piece: their candidates, prior means and rows, in any order
 // (each gets its own verdict back); the count goes to cnt[0].
 __global__ void __launch_bounds__(256) screen_amb_gather_kernel(const unsigned char *ver, int n, const double *px,
@@ -496,13 +332,11 @@ struct CompactParams {
   double thr;
   const double *lo;              // FP32 tier: EI at mu~ - E' (survivors with lo >= thr_keep are definite keeps), else null
   double thr_keep;
-  const int *cnt;                // survivors per 256 candidates (screen_count_kernel)
+  const long long *off;          // pool offset of each 128 candidates (screen_scan_kernel)
   long long m0;                  // index (within the call) of the chunk's first candidate
   const double *xs, *pm;         // the chunk's first candidate (pm may be null)
   const unsigned char *cm;       // or null
   int d, y_dim;
-  long long *base;               // pool size before this chunk in base[par]; the last CTA writes the size after it to base[par ^ 1]
-  int par;
   double *px, *ppm;              // pool: candidates, prior means,
   unsigned char *pcm;            //       constraint-mask entries,
   long long *pidx;               //       index within the call (m0 + position, or sidx[position] if sidx is set)
@@ -511,27 +345,17 @@ struct CompactParams {
   unsigned char *pver;           //       verdicts (or null): 1 keep, 2 ambiguous (refined in Screen::finish)
 };
 
-// ordered compaction: survivors keep their relative order, so the pool's first-maximal argmax is the call's
-__global__ void __launch_bounds__(256) screen_compact_kernel(CompactParams p) {
-  __shared__ long long s_off;
-  __shared__ int s_warp[8];
-  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5, b = blockIdx.x;
-  if (w == 0) {
-    long long s = 0;
-    for (int j = lane; j < b; j += 32) s += p.cnt[j];
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    if (lane == 0) {
-      s_off = p.base[p.par] + s;
-      if (b == (int)gridDim.x - 1) p.base[p.par ^ 1] = s_off + p.cnt[b];
-    }
-  }
-  const int c = b * 256 + tid;
+// ordered compaction, 128 candidates per CTA: survivors keep their relative order, so the pool's first-maximal argmax
+// is the call's
+__global__ void __launch_bounds__(128) screen_compact_kernel(CompactParams p) {
+  __shared__ int s_warp[4];
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5, c = blockIdx.x * 128 + tid;
   const bool keep = screen_keep(p.bound, p.ver, c, p.ch, p.thr);
   const unsigned bal = __ballot_sync(0xffffffffu, keep);
   if (lane == 0) s_warp[w] = __popc(bal);
   __syncthreads();
   if (!keep) return;
-  long long o = s_off + __popc(bal & ((1u << lane) - 1u));
+  long long o = p.off[blockIdx.x] + __popc(bal & ((1u << lane) - 1u));
   for (int q = 0; q < w; ++q) o += s_warp[q];
   for (int j = 0; j < p.d; ++j) p.px[o * p.d + j] = p.xs[(size_t)c * p.d + j];
   if (p.pm)

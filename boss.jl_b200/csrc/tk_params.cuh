@@ -3,7 +3,7 @@
 // library's compile time, so they live in their own translation units (tk_build.cu, tk_score.cu, tk_small.cu) and are
 // reached through the plain launch_* functions declared at the end of this file.
 #pragma once
-#include "kernel_fn.cuh"
+#include "acq.cuh"
 
 namespace boss {
 
@@ -51,15 +51,30 @@ struct XcovParams {
 constexpr int XCOV_KC = 128;  // training points staged per shared-memory pass
 
 // The FP32 mean tier of argmax screening (DESIGN.md 2.9): mu~ with a proven bound E on |mu~ - mu|, from per-call FP32
-// copies of the centred training inputs and of alpha (screen_consts_kernel).  x.Xt / x.alpha are unused; x.mu_part
-// receives the partials (FP64, same layout).
-struct XcovF32Params {
-  XcovParams x;
+// copies of the centred training inputs and of alpha (screen_consts_kernel), and the bound verdicts of the candidates
+// (screen_mean_bound_kernel in tk_score.cu).  One launch covers every slice of a call, up to SCREEN_F32_MAX_SL of them,
+// all of one covariance function.
+struct ScreenSlice {
   const float4 *tfrag;   // [n_pad / 8][KP / 8][32] per eight-point tile, k-step and lane: the MMA's B fragments of the
                          // centred training inputs t~ = fp32(ut - c), TF32-split: (b0 hi, b1 hi, b0 lo, b1 lo)
   const float4 *tn_al;   // [n_pad / 2] (|t~_j|^2, alpha_j, |t~_j+1|^2, alpha_j+1) rounded to FP32
   const double *A;       // [SCREEN_NCONST] A1 = sum |alpha_j|, A3 = sum |alpha_j| |ut_j - c|^2, the centre c (DP)
-  double *E;             // [ld] the error bound of each candidate's mean
+  const double *invl;    // [DP]
+  unsigned long long disc_bits;
+  double a2;
+  int n_pad;
+};
+constexpr int SCREEN_F32_MAX_SL = 16;
+struct ScreenF32Params {
+  const double *Xs;       // d x . raw candidates (device), candidate m at column (m - in_off)
+  long long m0, M, in_off;   // candidates [m0, M)
+  int d, nsl;
+  ScreenSlice sl[SCREEN_F32_MAX_SL];
+  AcqParams hi, lo;       // the bound pass at mu~ + E' and at mu~ - E' (mu / sumsq unused; hi.acq, lo.acq get the bounds)
+  double thr;             // a candidate survives unless its hi bound is below thr
+  long long *cnt;         // survivors per 128 candidates; null: write mu~ and E instead of verdicts
+  double *mu_out, *e_out; // [nsl][ld] indexed by m - m0 (cnt null)
+  int ld;
 };
 constexpr int SCREEN_NCONST = 2 + 32;
 // E = a^2 2^-24 (SCREEN_C_EVAL A1 + L2 k (|u - c|^2 A1 + A3))   (DESIGN.md 2.9), L2 = sup |d kappa / d(d2)|, and
@@ -113,7 +128,7 @@ struct SmallLoglikParams {
 
 // ---- host launchers: dispatch on (KID 0..4, dp in {2,4,6,8,12,16,32}); false = unsupported combination ----
 // KIDs: 0 SqExponential, 1 Matern32, 2 Matern52, 3 Matern12, 4 RationalQuadratic (kernel_fn.cuh).  The FP32 mean tier
-// (launch_xcov_mean_f32) exists for KIDs 0-2 only: its error bound needs sup |d kappa / d(d2)|, which is infinite for
+// (launch_screen_mean_bound) exists for KIDs 0-2 only: its error bound needs sup |d kappa / d(d2)|, which is infinite for
 // Matern12 and not derived for RQ's FP32 evaluation, so those kernels screen with FP64 means (DESIGN.md 2.14).
 constexpr int NUM_KID = 5;
 __host__ __device__ constexpr bool kid_has_f32_tier(int kid) { return kid >= 0 && kid <= 2; }
@@ -121,7 +136,8 @@ bool launch_build_k(int kid, int dp, const BuildKParams &p, dim3 grid, cudaStrea
 bool launch_loglik_grad_tile(int kid, int dp, const LlGradParams &p, dim3 grid, cudaStream_t st);
 bool launch_xcov(int kid, int dp, const XcovParams &p, dim3 grid, cudaStream_t st);
 bool launch_xcov_mean(int kid, int dp, const XcovParams &p, dim3 grid, cudaStream_t st);   // mu partials only (p.Ks unused)
-bool launch_xcov_mean_f32(int kid, int dp, const XcovF32Params &p, dim3 grid, cudaStream_t st);
+size_t screen_mean_bound_smem(int dp, int nsl);   // dynamic shared memory of one CTA
+bool launch_screen_mean_bound(int kid, int dp, const ScreenF32Params &p, int nblocks, cudaStream_t st);
 bool launch_kappa_f32_sweep(int kid, const double *r, int n, double *out, cudaStream_t st);
 bool launch_mma_d2(int dp, const float *u, const float *t, const float *nu, const float *nt, int mt, int nt_, float *d2,
                    cudaStream_t st);

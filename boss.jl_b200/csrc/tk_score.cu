@@ -68,108 +68,161 @@ __device__ __forceinline__ void mma_tf32(float (&d)[4], const unsigned (&a)[4], 
       : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
 
-// The FP32 mean tier of argmax screening (DESIGN.md 2.9): xcov_kernel<KID, DP, false>'s grid and partial layout, with
-// d2 = |u~|^2 + |t~_j|^2 - 2 u~.t~_j from centred FP32 points.  The cross term runs on the tensor cores (mma.sync TF32,
-// 3-term hi / lo split, accumulated in FP32); the norms are added and kappa_f32 evaluated on the accumulator fragments.
-// Warp w takes candidates 16w..16w+15 of the block against the 16 eight-point tiles of a 128-point training chunk,
-// tiles 0-7 into partial 2 (k0 / 128) and tiles 8-15 into partial 2 (k0 / 128) + 1.  A thread holds candidates g and
-// g + 8 (g = lane / 4) against training points 2t, 2t + 1 of each tile (t = lane % 4); each run of 4 tiles (8 points
-// per candidate) is summed in FP32 and added to an FP64 accumulator, and the four lanes of a candidate are combined
-// by a fixed butterfly, so the partials do not depend on scheduling.  Blocks of split 0 also write each candidate's
-// error bound E (tk_params.cuh).
+// 16-byte asynchronous copy global -> shared (L2 only), and the waits on its commit groups
+__device__ __forceinline__ void cp_async16(void *dst, const void *src) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
+// The FP32 mean tier of argmax screening (DESIGN.md 2.9), one CTA per 128 candidates over every training point of
+// every slice, then the bound verdicts of those candidates.
+//
+// Means: d2 = |u~|^2 + |t~_j|^2 - 2 u~.t~_j from centred FP32 points.  The cross term runs on the tensor cores
+// (mma.sync TF32, 3-term hi / lo split, accumulated in FP32); the norms are added and kappa_f32 evaluated on the
+// accumulator fragments.  Warp w takes candidates 16w..16w+15 against the 16 eight-point tiles of each 128-point stage of
+// training points.  A thread holds candidates g and g + 8 (g = lane / 4) against training points 2t, 2t + 1 of each tile
+// (t = lane % 4); each run of 4 tiles (8 points per candidate) is summed in FP32 and added to an FP64 accumulator, the
+// four lanes of a candidate are combined by a fixed butterfly, and the stage's two halves (tiles 0-7, 8-15) are scaled
+// by a^2 and added to mu~ in ascending (stage, half) order.  So mu~ does not depend on scheduling, and equals the
+// ordered sum of per-(stage, half) partials that reduce_rows_kernel forms on the FP64 tier.  A stage's B fragments and
+// (|t~|^2, alpha) are copied into a 2-deep ring while the previous stage computes.
+//
+// Verdicts, one thread per candidate: per slice mu~ +- E', E' = E with the sign of the slice's output coefficient (NaN
+// for both if mu~ or E is not finite), so that EI is at least as large at mu~ + E' as at the FP64 mean and no larger at
+// mu~ - E'; the EI bound at each (acq_candidate under p.hi and p.lo, into hi.acq and lo.acq); and the CTA's survivors,
+// !(hi < p.thr), to p.cnt[blockIdx.x].  With p.cnt null the CTA writes mu~ and E to p.mu_out / p.e_out instead.
 template <int KID, int DP>
-__global__ void __launch_bounds__(256) xcov_mean_mma_kernel(XcovF32Params q) {
-  constexpr int KS = (DP + 7) / 8, KP = 8 * KS;   // k-steps of the MMA, the padded dimension
-  const XcovParams &p = q.x;
-  // the candidates' -2 u~ (hi, lo; [128][KP] each) before the loop, the chunk's B fragments in it
-  __shared__ float4 sbuf[XCOV_KC / 8 * KS * 32];
-  __shared__ float4 snt[XCOV_KC / 2];   // (|t~|^2, alpha) of training points 2i, 2i + 1
+__global__ void __launch_bounds__(256) screen_mean_bound_kernel(ScreenF32Params p) {
+  constexpr int KS = (DP + 7) / 8, KP = 8 * KS;       // k-steps of the MMA, the padded dimension
+  constexpr int NF = XCOV_KC / 8 * KS * 32, NS = NF + XCOV_KC / 2;   // float4 of one stage: B fragments, (|t~|^2, alpha)
+  extern __shared__ float4 ring[];                     // [2][NS]; then mu~ and E, [nsl][128] each
+  double *smu = reinterpret_cast<double *>(ring + 2 * NS), *se = smu + p.nsl * 128;
   __shared__ float snu[128];
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5, g = lane >> 2, t = lane & 3;
-  const int cb = blockIdx.x;
-  if (tid < 128) {
-    const long long m = p.m0 + (long long)cb * 128 + tid;
-    double x64[DP];
-    load_scaled_point<DP>(x64, p.Xs + (size_t)(m - p.in_off) * p.d, p.d, p.invl, p.disc_bits, m < p.M);
-    double n2 = 0.0;
+  const long long mb = p.m0 + (long long)blockIdx.x * 128;   // the CTA's first candidate
+  for (int q = 0; q < p.nsl; ++q) {
+    const ScreenSlice &sl = p.sl[q];
+    const int nst = sl.n_pad / XCOV_KC;
+    auto stage = [&](int st) {   // stage st of the slice into ring slot st & 1, one commit group
+      float4 *dst = ring + (st & 1) * NS;
+      const float4 *tf = sl.tfrag + (size_t)st * NF, *ta = sl.tn_al + (size_t)st * (XCOV_KC / 2);
+      for (int e = tid; e < NS; e += 256) cp_async16(dst + e, e < NF ? tf + e : ta + (e - NF));
+      cp_async_commit();
+    };
+    stage(0);
+    if (tid < 128) {   // the candidates' -2 u~ (hi, lo; [128][KP] each) in slot 1, |u~|^2, E
+      const long long m = mb + tid;
+      double x64[DP];
+      load_scaled_point<DP>(x64, p.Xs + (size_t)(m - p.in_off) * p.d, p.d, sl.invl, sl.disc_bits, m < p.M);
+      double n2 = 0.0;
 #pragma unroll
-    for (int i = 0; i < DP; ++i) {
-      x64[i] -= q.A[2 + i];
-      n2 = fma(x64[i], x64[i], n2);
-    }
-    float *ua = reinterpret_cast<float *>(sbuf);
-#pragma unroll
-    for (int i = 0; i < KP; ++i) {
-      float hi, lo;
-      tf32_split(i < DP ? (float)x64[i] : 0.0f, hi, lo);
-      ua[tid * KP + i] = -2.0f * hi;
-      ua[128 * KP + tid * KP + i] = -2.0f * lo;
-    }
-    snu[tid] = (float)n2;
-    if (blockIdx.y == 0)
-      q.E[(size_t)cb * 128 + tid] =
-          p.a2 * 0x1p-24 * (SCREEN_C_EVAL * q.A[0] + screen_l2(KID) * screen_k_dot(DP) * fma(n2, q.A[0], q.A[1]));
-  }
-  __syncthreads();
-  unsigned ahi[KS][4], alo[KS][4];
-  {
-    const float *ua = reinterpret_cast<const float *>(sbuf);
-    const int r0 = 16 * w + g;
-#pragma unroll
-    for (int ks = 0; ks < KS; ++ks)
-#pragma unroll
-      for (int e = 0; e < 4; ++e) {   // a0: (g, t), a1: (g + 8, t), a2: (g, t + 4), a3: (g + 8, t + 4)
-        const int o = (r0 + 8 * (e & 1)) * KP + ks * 8 + t + 4 * (e >> 1);
-        ahi[ks][e] = __float_as_uint(ua[o]);
-        alo[ks][e] = __float_as_uint(ua[128 * KP + o]);
+      for (int i = 0; i < DP; ++i) {
+        x64[i] -= sl.A[2 + i];
+        n2 = fma(x64[i], x64[i], n2);
       }
-  }
-  const float nu0 = snu[16 * w + g], nu1 = snu[16 * w + g + 8];
-  for (int k0 = blockIdx.y * XCOV_KC; k0 < p.n_pad; k0 += gridDim.y * XCOV_KC) {
+      float *ua = reinterpret_cast<float *>(ring + NS);
+#pragma unroll
+      for (int i = 0; i < KP; ++i) {
+        float hi, lo;
+        tf32_split(i < DP ? (float)x64[i] : 0.0f, hi, lo);
+        ua[tid * KP + i] = -2.0f * hi;
+        ua[128 * KP + tid * KP + i] = -2.0f * lo;
+      }
+      snu[tid] = (float)n2;
+      se[q * 128 + tid] =
+          sl.a2 * 0x1p-24 * (SCREEN_C_EVAL * sl.A[0] + screen_l2(KID) * screen_k_dot(DP) * fma(n2, sl.A[0], sl.A[1]));
+    }
     __syncthreads();
-    for (int e = tid; e < XCOV_KC / 8 * KS * 32; e += 256) sbuf[e] = q.tfrag[(size_t)(k0 / 8) * KS * 32 + e];
-    if (tid < XCOV_KC / 2) snt[tid] = q.tn_al[k0 / 2 + tid];
-    __syncthreads();
+    unsigned ahi[KS][4], alo[KS][4];
+    {
+      const float *ua = reinterpret_cast<const float *>(ring + NS);
+      const int r0 = 16 * w + g;
 #pragma unroll
-    for (int kh = 0; kh < 2; ++kh) {
-      double acc0 = 0.0, acc1 = 0.0;   // candidates g and g + 8
+      for (int ks = 0; ks < KS; ++ks)
 #pragma unroll
-      for (int run = 0; run < 2; ++run) {
-        float s0 = 0.0f, s1 = 0.0f;
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          const int nt = kh * 8 + run * 4 + u;
-          float c[4] = {0.0f, 0.0f, 0.0f, 0.0f};
-#pragma unroll
-          for (int ks = 0; ks < KS; ++ks) {   // b = (b0 hi, b1 hi, b0 lo, b1 lo): B(t, g), B(t + 4, g)
-            const float4 b = sbuf[(nt * KS + ks) * 32 + lane];
-            mma_tf32(c, alo[ks], __float_as_uint(b.x), __float_as_uint(b.y));
-            mma_tf32(c, ahi[ks], __float_as_uint(b.z), __float_as_uint(b.w));
-            mma_tf32(c, ahi[ks], __float_as_uint(b.x), __float_as_uint(b.y));
-          }
-          const float4 na = snt[nt * 4 + t];   // points 2t, 2t + 1 of the tile
-          s0 = fmaf(na.y, kappa_f32<KID>(fmaxf(c[0] + nu0 + na.x, 0.0f)), s0);
-          s0 = fmaf(na.w, kappa_f32<KID>(fmaxf(c[1] + nu0 + na.z, 0.0f)), s0);
-          s1 = fmaf(na.y, kappa_f32<KID>(fmaxf(c[2] + nu1 + na.x, 0.0f)), s1);
-          s1 = fmaf(na.w, kappa_f32<KID>(fmaxf(c[3] + nu1 + na.z, 0.0f)), s1);
+        for (int e = 0; e < 4; ++e) {   // a0: (g, t), a1: (g + 8, t), a2: (g, t + 4), a3: (g + 8, t + 4)
+          const int o = (r0 + 8 * (e & 1)) * KP + ks * 8 + t + 4 * (e >> 1);
+          ahi[ks][e] = __float_as_uint(ua[o]);
+          alo[ks][e] = __float_as_uint(ua[128 * KP + o]);
         }
-        acc0 += (double)s0;
-        acc1 += (double)s1;
-      }
-      acc0 += __shfl_xor_sync(0xffffffffu, acc0, 1);
-      acc1 += __shfl_xor_sync(0xffffffffu, acc1, 1);
-      acc0 += __shfl_xor_sync(0xffffffffu, acc0, 2);
-      acc1 += __shfl_xor_sync(0xffffffffu, acc1, 2);
-      if (t == 0) {
-        double *dst = p.mu_part + (size_t)(2 * (k0 / XCOV_KC) + kh) * p.ld + (size_t)cb * 128 + 16 * w + g;
-        dst[0] = p.a2 * acc0;
-        dst[8] = p.a2 * acc1;
+    }
+    const float nu0 = snu[16 * w + g], nu1 = snu[16 * w + g + 8];
+    double mu0 = 0.0, mu1 = 0.0;   // candidates g and g + 8
+    for (int st = 0; st < nst; ++st) {
+      __syncthreads();   // slot (st + 1) & 1 is no longer read (stage st - 1, or the candidates' fragments)
+      if (st + 1 < nst) stage(st + 1);
+      else cp_async_commit();
+      cp_async_wait<1>();
+      __syncthreads();   // stage st has landed for every thread's copies
+      const float4 *sbuf = ring + (st & 1) * NS, *snt = sbuf + NF;
+#pragma unroll
+      for (int kh = 0; kh < 2; ++kh) {
+        double acc0 = 0.0, acc1 = 0.0;
+#pragma unroll
+        for (int run = 0; run < 2; ++run) {
+          float s0 = 0.0f, s1 = 0.0f;
+#pragma unroll
+          for (int u = 0; u < 4; ++u) {
+            const int nt = kh * 8 + run * 4 + u;
+            float c[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+#pragma unroll
+            for (int ks = 0; ks < KS; ++ks) {   // b = (b0 hi, b1 hi, b0 lo, b1 lo): B(t, g), B(t + 4, g)
+              const float4 b = sbuf[(nt * KS + ks) * 32 + lane];
+              mma_tf32(c, alo[ks], __float_as_uint(b.x), __float_as_uint(b.y));
+              mma_tf32(c, ahi[ks], __float_as_uint(b.z), __float_as_uint(b.w));
+              mma_tf32(c, ahi[ks], __float_as_uint(b.x), __float_as_uint(b.y));
+            }
+            const float4 na = snt[nt * 4 + t];   // points 2t, 2t + 1 of the tile
+            s0 = fmaf(na.y, kappa_f32<KID>(fmaxf(c[0] + nu0 + na.x, 0.0f)), s0);
+            s0 = fmaf(na.w, kappa_f32<KID>(fmaxf(c[1] + nu0 + na.z, 0.0f)), s0);
+            s1 = fmaf(na.y, kappa_f32<KID>(fmaxf(c[2] + nu1 + na.x, 0.0f)), s1);
+            s1 = fmaf(na.w, kappa_f32<KID>(fmaxf(c[3] + nu1 + na.z, 0.0f)), s1);
+          }
+          acc0 += (double)s0;
+          acc1 += (double)s1;
+        }
+        acc0 += __shfl_xor_sync(0xffffffffu, acc0, 1);
+        acc1 += __shfl_xor_sync(0xffffffffu, acc1, 1);
+        acc0 += __shfl_xor_sync(0xffffffffu, acc0, 2);
+        acc1 += __shfl_xor_sync(0xffffffffu, acc1, 2);
+        // the partial a^2 acc is rounded before it is added (no fused multiply-add), as in the ordered sum
+        mu0 = __dadd_rn(mu0, __dmul_rn(sl.a2, acc0));
+        mu1 = __dadd_rn(mu1, __dmul_rn(sl.a2, acc1));
       }
     }
+    if (t == 0) {
+      smu[q * 128 + 16 * w + g] = mu0;
+      smu[q * 128 + 16 * w + g + 8] = mu1;
+    }
+    __syncthreads();   // mu~ complete; the ring and snu are free for the next slice
   }
+  const long long m = mb + tid;
+  if (!p.cnt) {
+    if (tid < 128 && m < p.M)
+      for (int q = 0; q < p.nsl; ++q) {
+        p.mu_out[(size_t)q * p.ld + (m - p.m0)] = smu[q * 128 + tid];
+        p.e_out[(size_t)q * p.ld + (m - p.m0)] = se[q * 128 + tid];
+      }
+    return;
+  }
+  bool keep = false;
+  if (tid < 128 && m < p.M) {
+    for (int q = 0; q < p.nsl; ++q) {   // smu <- mu~ + E', se <- mu~ - E'
+      const double mq = smu[q * 128 + tid], E = p.hi.coefs[q % p.hi.y_dim] < 0.0 ? -se[q * 128 + tid] : se[q * 128 + tid];
+      const bool ok = isfinite(mq) && isfinite(E);
+      smu[q * 128 + tid] = ok ? mq + E : NAN;
+      se[q * 128 + tid] = ok ? mq - E : NAN;
+    }
+    keep = !(acq_candidate<true>(p.hi, 0, m, smu + tid, 128) < p.thr);
+    acq_candidate<true>(p.lo, 0, m, se + tid, 128);
+  }
+  const int k = __syncthreads_count(keep);
+  if (tid == 0) p.cnt[blockIdx.x] = k;
 }
 
-// The tensor-core d2 of xcov_mean_mma_kernel for given FP32 points, for the tests of its error model: u [16 gridDim.x]
+// The tensor-core d2 of screen_mean_bound_kernel for given FP32 points, for the tests of its error model: u [16 gridDim.x]
 // [8 KS] and t [8 gridDim.y][8 KS] row-major, nu / nt their norms; one warp per 16 x 8 tile, the same split, MMA chain
 // and assembly (without the clamp at 0), d2 [16 gridDim.x][8 gridDim.y] row-major.
 template <int KS>
@@ -328,8 +381,16 @@ bool launch_xcov_mean(int kid, int dp, const XcovParams &p, dim3 grid, cudaStrea
   BOSS_DISPATCH_KID_DP(CALL, kid, dp)
 #undef CALL
 }
-bool launch_xcov_mean_f32(int kid, int dp, const XcovF32Params &p, dim3 grid, cudaStream_t st) {
-#define CALL(K, D) xcov_mean_mma_kernel<K, D><<<grid, 256, 0, st>>>(p)
+size_t screen_mean_bound_smem(int dp, int nsl) {
+  return (size_t)2 * (XCOV_KC / 8 * ((dp + 7) / 8) * 32 + XCOV_KC / 2) * 16 + (size_t)nsl * 2 * 128 * 8;
+}
+bool launch_screen_mean_bound(int kid, int dp, const ScreenF32Params &p, int nblocks, cudaStream_t st) {
+  const size_t smem = screen_mean_bound_smem(dp, p.nsl);
+#define CALL(K, D)                                                                                                 \
+  do {                                                                                                             \
+    cudaFuncSetAttribute(screen_mean_bound_kernel<K, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+    screen_mean_bound_kernel<K, D><<<nblocks, 256, smem, st>>>(p);                                               \
+  } while (0)
   BOSS_DISPATCH_KID_DP_F32(CALL, kid, dp)
 #undef CALL
 }

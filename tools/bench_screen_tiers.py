@@ -25,7 +25,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CH0 = 75_776                 # the first chunk of the bench problem (FP64 tier), candidates
-SASS_INSTR_PER_PAIR = 14.0   # xcov_mean_mma_kernel<2, 8>: about 900 instructions per 64 pairs a thread (cuobjdump -sass)
+SASS_INSTR_PER_PAIR = 14.0   # the MMA mean loop at DP = 8: about 900 instructions per 64 pairs a thread (cuobjdump -sass)
 sys.path.insert(0, ROOT)
 sys.dont_write_bytecode = True
 
@@ -143,10 +143,10 @@ def main():
                     if us > 0:
                         ker[e.key] = {"us": us, "count": e.count}
             prof_out["tiers"][t] = dict(sorted(ker.items(), key=lambda kv: -kv[1]["us"])[:25])
-            mean_k = [(k, v) for k, v in ker.items() if "xcov_mean_mma_kernel" in k]
+            mean_k = [(k, v) for k, v in ker.items() if "screen_mean_bound_kernel" in k]
             if mean_k:
                 k, v = mean_k[0]
-                per_chunk = v["us"] / v["count"]
+                per_chunk = v["us"] / v["count"]   # one launch over every candidate after the first chunk
                 pairs = (M - CH0) * 2048                 # every candidate after the first chunk, n = 2048
                 clk = 1.965e9                            # the card's maximum SM clock (sm_max_clock)
                 prof_out["tiers"][t]["mean_tier"] = {
