@@ -110,7 +110,9 @@ def _ll_problem(n, d, S, seed):
 
 
 @pytest.mark.parametrize("kernel", KERNELS, ids=IDS)
-@pytest.mark.parametrize("n,path", [(20, "warp"), (300, "fused"), (300, "per_matrix"), (700, "blocked")])
+# n = 700 pads to 6 blocks, which still take the fused diagonal step (potrf_fused_kernel); n = 900 (8 blocks) runs the
+# separate SYRK -> potrf_tile_kernel -> chol_panel_kernel chain
+@pytest.mark.parametrize("n,path", [(20, "warp"), (300, "fused"), (300, "per_matrix"), (700, "fused"), (900, "blocked")])
 def test_loglik_paths(lib, kernel, n, path, monkeypatch):
     X, y, L, A, N = _ll_problem(n, 5, 12, seed=n)
     if path == "per_matrix":
