@@ -100,6 +100,7 @@ EXPORTS = {
     "boss_dbg_check_redzones": (C.c_int64, [_i64p]),
     "boss_dbg_redzone_selftest": (C.c_int64, []),
     "boss_dbg_screen_stats": (C.c_int, [_i64p]),
+    "boss_dbg_score_paths": (C.c_int, [_i64p]),
     "boss_dbg_screen_ambiguous": (C.c_int, [_i64p]),
     "boss_dbg_screen_mean": (C.c_int, [_vp, _vp, C.c_int64, _vp, _vp, _vp]),
     "boss_dbg_kappa_f32": (C.c_int, [C.c_int, _vp, C.c_int, _vp]),
@@ -770,6 +771,14 @@ def dbg_screen_stats():
     out = (C.c_int64 * 3)()
     _check(lib.boss_dbg_screen_stats(out), "boss_dbg_screen_stats")
     return int(out[0]), int(out[1]), int(out[2])
+
+
+def dbg_score_paths():
+    """The paths of the last scoring call on the current device, counted per (chunk, slice) pass: dict with keys
+    wide_fused, wide_split (wide without the fused epilogue), narrow, quarter, xgrad."""
+    out = (C.c_int64 * 5)()
+    _check(lib.boss_dbg_score_paths(out), "boss_dbg_score_paths")
+    return dict(zip(("wide_fused", "wide_split", "narrow", "quarter", "xgrad"), (int(v) for v in out)))
 
 
 def dbg_screen_ambiguous():

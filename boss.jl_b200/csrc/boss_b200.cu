@@ -140,6 +140,7 @@ struct Ctx {
   DevBuf topk;                       // top-k calls: running set, chunk scores, selection state, sorted result
   int64_t scr_stats[3] = {0, 0, 0};  // last scoring call: screened (1) or fell back (2), candidates bounded, pool size
   int64_t scr_amb[2] = {0, 0};       // last screened call: ambiguous candidates of the FP32 tier, pool before refinement and re-seed
+  int64_t score_paths[5] = {0, 0, 0, 0, 0};   // last scoring call's (chunk, slice) passes by path (boss_dbg_score_paths)
   // event pool for per-kernel-class timing
   cudaEvent_t ev_a[EV_POOL], ev_b[EV_POOL];
   int ev_class[EV_POOL];
@@ -1594,6 +1595,8 @@ bool score_slice(const ScoreCall &c, int q, const AcqParams &ap, const ChunkIO &
   // One CTA per candidate block walks all of W (large batches) and this is the chunk's last slice: the scoring
   // kernel finishes the candidates itself (fused epilogue) -- no reduce / acquisition / argmax launches.
   const bool fuse = nsp == 1 && !narrow && !quarter && q == c.nsl - 1 && getenv("BOSS_UNFUSED_SCORE") == nullptr;
+  ++C().score_paths[quarter ? 3 : narrow ? 2 : fuse ? 0 : 1];
+  if (a.xgrad()) ++C().score_paths[4];
   if (!fuse && !quarter)
     reduce_rows_kernel<<<(cnt + 255) / 256, 256, 0, C().stream>>>(C().part_mu.as<double>(), 2 * h->nblk, (size_t)CH,
                                                                C().muv.as<double>() + (size_t)q * CH, cnt);
@@ -2234,7 +2237,10 @@ int score_core(ScoreArgs &a) {
   }
   rc = c.setup();
   if (rc) return rc;
-  if (!a.internal) C().scr_stats[0] = C().scr_stats[1] = C().scr_stats[2] = C().scr_amb[0] = C().scr_amb[1] = 0;
+  if (!a.internal) {
+    C().scr_stats[0] = C().scr_stats[1] = C().scr_stats[2] = C().scr_amb[0] = C().scr_amb[1] = 0;
+    for (int64_t &p : C().score_paths) p = 0;
+  }
   const int ch0 = (int)std::min<long long>(c.CH, a.M);   // the first chunk
   Screen scr;
   if (Screen::eligible(a, ch0, c.d)) {
@@ -3756,6 +3762,17 @@ int boss_dbg_factors(const boss_gp *gp, double *L, double *W, double *alpha) {
 int boss_dbg_screen_stats(int64_t *out) {
   REQUIRE_INIT();
   for (int i = 0; i < 3; ++i) out[i] = C().scr_stats[i];
+  return 0;
+}
+
+// The paths score_slice took in the last scoring call on the current device, counted per (chunk, slice) pass: out[0] wide
+// with the fused epilogue, out[1] wide without it (row splits, a slice other than the last, or BOSS_UNFUSED_SCORE),
+// out[2] narrow, out[3] quarter; out[4] the passes that ran the x-gradient pipeline.  Nested calls of a screened or
+// multi-start call add to their caller's counts.  The counts are reset once the call has bound its slices and set up its
+// workspaces: a call that fails before that, or has M <= 0, leaves the previous call's counts (as scr_stats does).
+int boss_dbg_score_paths(int64_t *out) {
+  REQUIRE_INIT();
+  for (int i = 0; i < 5; ++i) out[i] = C().score_paths[i];
   return 0;
 }
 

@@ -393,6 +393,11 @@ int64_t boss_dbg_redzone_selftest(void);   /* negative control: writes 2 guard b
  * to the full path after the first chunk; out[1] = candidates bounded; out[2] = candidates that survived the bound and
  * the re-seeded threshold (the pool scored exactly) */
 int boss_dbg_screen_stats(int64_t *out);
+/* the scoring paths of the last scoring call on the current device, counted per (chunk, slice) pass: out[0] wide with
+ * the fused epilogue, out[1] wide without it, out[2] narrow (32-candidate CTAs), out[3] quarter; out[4] the passes that
+ * ran the x-gradient pipeline.  A call that fails before scoring, or has M <= 0, leaves the previous call's counts (as
+ * boss_dbg_screen_stats does) */
+int boss_dbg_score_paths(int64_t *out);
 /* the FP32 mean tier of the last screened call: out[0] = candidates in the ambiguous band (their means were recomputed in
  * FP64), out[1] = the pool as the chunks left it (definite keeps plus ambiguous candidates), before the FP64 refinement
  * and the re-seeded threshold */

@@ -36,6 +36,7 @@ import numpy as np
 import pytest
 
 from oracle import boss_oracle as O
+from tests.posterior_scale_oracle import floors, ratio as _ratio   # the rule, shared with the full-size tests
 
 pytestmark = pytest.mark.gpu
 
@@ -56,11 +57,6 @@ def _problem(n, d, dup_dist, seed):
     y = np.sin(3 * X).sum(0) + 0.05 * rng.standard_normal(n)
     Xs = np.concatenate([rng.random((d, 48)), X[:, :24], X[:, n - ndup:], 0.5 * (X[:, :ndup] + X[:, n - ndup:])], axis=1)
     return X, y, Xs
-
-
-def _ratio(got, ref, rel, floor):
-    got = np.asarray(got, dtype=np.float64); ref = np.asarray(ref, dtype=np.float64)
-    return float(np.max(np.abs(got - ref) / np.maximum(rel * np.abs(ref), floor)))
 
 
 CASES = []
@@ -123,8 +119,7 @@ def test_adversarial_posterior_and_loglik(lib, n, d, kid, ell, noise, dup):
              float(np.max(np.sum((Xs / (ls[:, None] + 1e-8)) ** 2, axis=0))))
     dk = 12 * EPS * a2 * x2
     c_var, c_mu = 4 * kappa * EPS * a2, 4 * kappa * EPS * float(np.max(np.abs(y)))
-    f_var = c_var + 2 * u1 * (1 + u1) * dk
-    f_mu = c_mu + float(np.sum(np.abs(alpha))) * (1 + u1) * dk
+    f_mu, f_var = floors(kappa, a2, float(np.max(np.abs(y))), float(np.sum(np.abs(alpha))), u1, x2)
     f_ll_abs = 0.5 * dk * (float(np.sum(np.abs(Kinv))) + float(np.sum(np.abs(alpha))) ** 2)
 
     def clip(v):   # the [-1e-8, 0) -> 0 branch of _clip_var (status 2 leaves the raw value on both sides)
