@@ -24,7 +24,6 @@
 
 #include "../../include/boss_b200.h"
 #include "cholesky.cuh"
-#include "chol_matrix.cuh"
 #include "score.cuh"
 #include "grad.cuh"
 #include "score_narrow.cuh"
@@ -364,11 +363,6 @@ int set_kernel_attrs() {
   CUDA_TRY(cudaFuncSetAttribute(score_quarter_kernel<1, 4, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, NQ_SMEM_BYTES));
   CUDA_TRY(cudaFuncSetAttribute(potrf_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PT_SMEM_BYTES));
   CUDA_TRY(cudaFuncSetAttribute(potrf_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PF_SMEM_BYTES));
-  CUDA_TRY(cudaFuncSetAttribute(chol_matrix_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, CM_SMEM_BYTES));
-  CUDA_TRY(cudaFuncSetAttribute(chol_matrix_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, CM_SMEM_BYTES));
-  CUDA_TRY(cudaFuncSetAttribute(chol_matrix_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, CM_SMEM_BYTES));
-  CUDA_TRY(cudaFuncSetAttribute(chol_matrix_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, CM_SMEM_BYTES));
-  CUDA_TRY(cudaFuncSetAttribute(chol_matrix_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, CM_SMEM_BYTES));
   C().attrs_done = true;
   return 0;
 }
@@ -389,10 +383,6 @@ struct FwdInline {
 };
 // gen non-null (left-looking only): the diagonal-block kernel forms its own input tile (potrf_fused_kernel: K_jj from
 // the hyper-parameters minus the SYRK of row block j) -- build_k must then have been launched with skip_diag.
-bool unfused_diag() {
-  static const bool v = getenv("BOSS_UNFUSED_DIAG") != nullptr;   // A/B knob: the round-1 three-kernel diagonal step
-  return v;
-}
 int run_cholesky(double *L, size_t L_stride, double *Winv, size_t Winv_stride, int nblk, int ktiles, int S,
                  double *logdet_blk, int *status, double *W, double *WT, double *TT, size_t W_stride = 0,
                  size_t TT_stride = 0, bool single_fit = false, const FwdInline *fwd = nullptr,
@@ -1576,7 +1566,7 @@ bool score_slice(const ScoreCall &c, int q, const AcqParams &ap, const ChunkIO &
   // takes ~0.3 of a wide one).  Same bits either way.
   const int ncb32 = (ch + NW_NB - 1) / NW_NB;
   const int nsp32 = pick_row_splits(ncb32, h->nblk, &cost_n);
-  bool narrow = 0.32 * cost_n < cost_w && getenv("BOSS_NO_NARROW") == nullptr;
+  bool narrow = 0.32 * cost_n < cost_w;
   // Tiny batches: quarter-row-block CTAs (4 nblk per 32 candidates, 4 to an SM).  Cost in the same unit: the
   // longest CTA's latency-bound walk over 8 nblk short stages, or the launch's tensor work spread over the SMs.
   const double cost_q = std::max(NQ_COST_CHAIN * h->nblk, NQ_COST_WORK * ncb32 * (h->nblk * (h->nblk + 1) / 2)) + NQ_COST_FIXED;
@@ -3201,55 +3191,7 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
   // factorisation, forward solve) and partially filled last waves overlap with another group's GEMM launches.
   cudaStream_t main_stream = C().stream;
   const size_t winv_stride = (size_t)nblk * TM * TM;
-  // n_pad <= 512, value only: one persistent CTA takes a whole matrix through the factorisation (chol_matrix.cuh)
-  // Measured (C3, 512 matrices): 2.2 ms vs 1.6 ms for the multi-kernel path -- 28 small jobs per matrix with cold rings and
-  // two-stage solve rings do not keep the tensor pipe fed -- so the path is opt-in (BOSS_PER_MATRIX=1) until it is tuned.
-  const bool per_matrix = !small && !need_w && nblk <= CM_MAX_NBLK && !unfused_diag() && getenv("BOSS_PER_MATRIX") != nullptr;
-  for (long long s0 = 0; s0 < S && per_matrix; s0 += Sb) {
-    const int sb = (int)std::min<long long>(Sb, S - s0);
-    CUDA_TRY(cudaMemsetAsync(status, 0, (size_t)sb * 4, C().stream));
-    CmParams cp{};
-    cp.S = sb;
-    PotrfParams &pp = cp.pp;
-    pp.L = C().chol_L.as<double>();
-    pp.L_stride = mat;
-    pp.nblk = nblk;
-    pp.ktiles = ktiles;
-    pp.logdet_blk = logdet_blk;
-    pp.status = status;
-    pp.fwd_ymm = dY + (ldy ? (size_t)s0 * ldy : 0);
-    pp.fwd_ldy = ldy;
-    pp.fwd_n = n;
-    pp.n_pad = n_pad;
-    pp.fwd_w = misc + owv;
-    pp.fwd_ssq = misc + ossq;
-    pp.gen_X = dX;
-    pp.gen_d = d;
-    pp.gen_dp = dp;
-    pp.gen_n = n;
-    pp.gen_kid = kernel_id;
-    pp.gen_rq_a = ks.rq_a;
-    pp.gen_ls = dls + (size_t)s0 * d;
-    pp.gen_amp = damp + s0;
-    pp.gen_noise = dnoise + s0;
-    pp.gen_disc = disc;
-    pp.store_L = 0;
-    {
-      Timed t(2);
-      const unsigned grid = (unsigned)std::min<long long>(sb, 2 * 148);
-      switch (kernel_id) {   // every KID explicitly (ids were decoded by loglik_impl)
-        case 0: chol_matrix_kernel<0><<<grid, 256, CM_SMEM_BYTES, C().stream>>>(cp); break;
-        case 1: chol_matrix_kernel<1><<<grid, 256, CM_SMEM_BYTES, C().stream>>>(cp); break;
-        case 2: chol_matrix_kernel<2><<<grid, 256, CM_SMEM_BYTES, C().stream>>>(cp); break;
-        case 3: chol_matrix_kernel<3><<<grid, 256, CM_SMEM_BYTES, C().stream>>>(cp); break;
-        case 4: chol_matrix_kernel<4><<<grid, 256, CM_SMEM_BYTES, C().stream>>>(cp); break;
-        default: return fail(BOSS_ERR_ARG, "boss_gp_loglik_batch: unknown kernel");
-      }
-    }
-    loglik_finish_kernel<<<(sb + 127) / 128, 128, 0, C().stream>>>(logdet_blk, pp.fwd_ssq, status, nblk, n, sb, dll + s0);
-    C().launches += 2;
-  }
-  for (long long s0 = 0; s0 < S && !small && !per_matrix; s0 += Sb) {
+  for (long long s0 = 0; s0 < S && !small; s0 += Sb) {
     const int sb = (int)std::min<long long>(Sb, S - s0);
     // 4 concurrent groups for long factorisations; 2 for small matrices, whose diagonal-block launches (one CTA per
     // matrix, two to an SM) then come closer to filling the GPU (C3, 512 matrices of n = 512: 1.57 vs 1.61 ms)
@@ -3294,7 +3236,7 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
       // three short launches and the tile's HBM trip dominate (C3, n = 512: 1.61 -> 1.55 ms); for long k-ranges the
       // dedicated SYRK kernel (5-stage ring, 218 registers) runs its DMMAs at 75 % of the SM's rate against 51 % for the
       // 128-register fused one (11.8 vs 17.5 us per 128-block of k at n = 2048), so larger matrices keep the separate steps.
-      const bool fuse_diag = !unfused_diag() && nblk <= 6;
+      const bool fuse_diag = nblk <= 6;
       bk.skip_diag = fuse_diag ? 1 : 0;     // the diagonal tiles are generated inside potrf_fused_kernel
       if (!(fuse_diag && nblk == 1)) {
         Timed t(1);

@@ -57,11 +57,11 @@ struct PotrfParams {
 constexpr int PT_TILES = 136;                        // 16*17/2 lower micro-tiles
 constexpr int PT_TMP_ELEMS = 64 * 64;                // scratch for the inverse products (one 64x64 block)
 constexpr int PT_SMEM_BYTES = (PT_TILES * 64 + PT_TMP_ELEMS + 128 + 128 + 8 + 128 + 8) * 8;   // 105 600 B -> 2 CTAs / SM
-// the fused kernel adds: 24 mbarrier slots, the exp table (32), 1/l (32), per-row forward-substitution sums (128)
+// the fused kernel adds: 12 mbarrier slots, the exp table (32), 1/l (32), per-row forward-substitution sums (128)
 constexpr int PF_RING_STAGES = 6;                    // 6 x 16 KB single-tile stages live in the (not yet used) T | tmp area
-constexpr int PF_BAR_SLOTS = 24;                     // mbarrier slots: [0,12) the SYRK ring here, [12,24) the rings of chol_matrix.cuh
+constexpr int PF_BAR_SLOTS = 2 * PF_RING_STAGES;     // mbarrier slots of the SYRK ring: full[6], empty[6]
 constexpr int PF_EXTRA_ELEMS = PF_BAR_SLOTS + EXPTAB_N + 32 + 128;
-constexpr int PF_SMEM_BYTES = PT_SMEM_BYTES + PF_EXTRA_ELEMS * 8;   // 107 264 B -> still 2 CTAs / SM
+constexpr int PF_SMEM_BYTES = PT_SMEM_BYTES + PF_EXTRA_ELEMS * 8;   // 107 168 B -> still 2 CTAs / SM
 
 // (I, J) of the t-th packed lower micro-tile
 struct PtIJ {
@@ -151,14 +151,9 @@ __device__ __forceinline__ void pf_syrk_batch(double (&acc)[17][2], const double
 // FUSED = false: the diagonal tile is read from global memory (posterior fit, right-looking steps).
 // FUSED = true : the CTA generates K_jj, subtracts the SYRK of row block j of L (streamed through a 6-stage TMA ring
 //                that lives in the tile store before it is needed) and carries the forward substitution's r_j.
-// s_mat: matrix of the batch; jc: block column (p.j for the stand-alone kernels).  LOCAL_ONLY (fused, persistent per-matrix kernel of chol_matrix.cuh): Winv_jj stays in
-// the tile store for the caller's panel solves and is not written to global memory; the function then returns with
-// the CTA synchronised.
-// ring_pos (LOCAL_ONLY): stages the SYRK ring has carried so far in this kernel; the barriers are initialised once per
-// kernel and their phases simply keep counting (re-initialising a used mbarrier did not take effect on B200, with or
-// without mbarrier.inval: the old arrival count survived).
-template <bool FUSED, bool LOCAL_ONLY = false>
-__device__ __forceinline__ void potrf_tile_body(const PotrfParams &p, const int s_mat, const int jc, int *ring_pos = nullptr) {
+// s_mat: matrix of the batch; jc: block column (p.j for the stand-alone kernels).
+template <bool FUSED>
+__device__ __forceinline__ void potrf_tile_body(const PotrfParams &p, const int s_mat, const int jc) {
   extern __shared__ __align__(16) double sm[];
   double *T = sm;                          // [136][64] packed lower tiles: A -> L -> W
   double *tmp = sm + PT_TILES * 64;        // [64][64] as 8x8 tiles (row-major tile grid, 8 tiles per row)
@@ -202,16 +197,12 @@ __device__ __forceinline__ void potrf_tile_body(const PotrfParams &p, const int 
     if (jc > 0) {
       // ---- SYRK of the diagonal tile: both operands are row block j of L, so a stage is ONE 16 KB macro-tile ----
       uint64_t *full = bars, *empty = bars + PF_RING_STAGES;
-      int pos0 = 0;   // absolute index of this job's first stage
-      if constexpr (LOCAL_ONLY) {
-        pos0 = *ring_pos;   // persistent kernel: barriers were initialised at kernel start, phases keep counting
-      } else {
-        if (tid < 2 * PF_RING_STAGES) {
-          mbar_init(smem_u32(&bars[tid]), tid < PF_RING_STAGES ? 1u : 8u);
-          mbar_fence_init();
-        }
-        __syncthreads();
+      int pos0 = 0;   // stage index the ring starts at (a variable: folding it away changes ptxas' register allocation)
+      if (tid < 2 * PF_RING_STAGES) {
+        mbar_init(smem_u32(&bars[tid]), tid < PF_RING_STAGES ? 1u : 8u);
+        mbar_fence_init();
       }
+      __syncthreads();
       const double *src = p.L + (size_t)s_mat * p.L_stride + (size_t)jc * p.ktiles * TILE_ELEMS;
       const int nk = jc * KT_PER_BLOCK;
       int issued = 0;
@@ -274,7 +265,6 @@ __device__ __forceinline__ void potrf_tile_body(const PotrfParams &p, const int 
           }
         }
       }
-      if constexpr (LOCAL_ONLY) *ring_pos = pos0 + nk;
       if (fwd) {
         r0 += __shfl_xor_sync(0xffffffffu, r0, 1);
         r0 += __shfl_xor_sync(0xffffffffu, r0, 2);
@@ -563,7 +553,6 @@ __device__ __forceinline__ void potrf_tile_body(const PotrfParams &p, const int 
   double *wi = p.Winv + (size_t)s_mat * p.Winv_stride + (size_t)jc * (TM * TM);
   double *wfull = p.W ? p.W + (size_t)s_mat * p.W_stride + ((size_t)jc * p.ktiles + (size_t)jc * KT_PER_BLOCK) * TILE_ELEMS : nullptr;
   double *wtfull = p.WT ? p.WT + (size_t)s_mat * p.W_stride + ((size_t)jc * p.ktiles + (size_t)jc * KT_PER_BLOCK) * TILE_ELEMS : nullptr;
-  if constexpr (!LOCAL_ONLY)
   for (int e = 2 * tid; e < TM * TM; e += 512) {   // 16 B per lane, a micro-tile per warp pass
     const int kt = e >> 11, micro = (e >> 6) & 31, w = e & 63;
     const int I = micro >> 1, J = (kt << 1) + (micro & 1);
@@ -622,7 +611,6 @@ __device__ __forceinline__ void potrf_tile_body(const PotrfParams &p, const int 
       p.fwd_ssq[(size_t)s_mat * p.nblk + jc] = t;
     }
   }
-  if constexpr (LOCAL_ONLY) __syncthreads();
 }
 
 __global__ void __launch_bounds__(256, 2) potrf_tile_kernel(PotrfParams p) { potrf_tile_body<false>(p, blockIdx.x, p.j); }

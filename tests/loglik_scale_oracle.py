@@ -20,11 +20,11 @@ import numpy as np
 from oracle import boss_oracle as OB
 from tests.kernels_more_oracle import KERNEL_MATERN12, RQ, O as OK
 
-TM = 128                                     # csrc/common.cuh:22, rows of a block
-LL_GROUPS = 16                               # csrc/boss_b200.cu:119, most stream groups a window runs as
-WORKSPACE_BYTES = 32 << 30                   # csrc/boss_b200.cu:3102-3104, the window's workspace budget
-MAX_WINDOW = 32768                           # csrc/boss_b200.cu:3105
-SMALL_N = 32                                 # csrc/tk_params.cuh:113, warp-register path (value mode only)
+TM = 128                                     # csrc/common.cuh `TM`, rows of a block
+LL_GROUPS = 16                               # csrc/boss_b200.cu `LL_GROUPS`, most stream groups a window runs as
+WORKSPACE_BYTES = 32 << 30                   # loglik_core's workspace budget for a window (`Sb`)
+MAX_WINDOW = 32768                           # loglik_core's cap on `Sb`
+SMALL_N = 32                                 # csrc/tk_params.cuh `SMALL_N`, warp-register path (value mode only)
 TOL_LL, TOL_GRAD, TOL_JAC, TOL_POST = 1e-8, 1e-8, 1e-9, 1e-9
 
 
@@ -192,35 +192,32 @@ def tile_contributions(X, y_minus_mean, lengthscales, amplitude, noise_std, kern
 # ---- windows and stream groups -------------------------------------------------------------------------------------
 
 def window_plan(n, d, S, mode, groups=None, timing=False):
-    """The windows and stream groups loglik_core runs a batch of S samples as.
+    """The windows and stream groups loglik_core runs a batch of S samples as (a name in a comment: the loglik_core
+    variable the line mirrors).
 
-    mode: "value" (boss_gp_loglik_batch), "per_matrix" (the same with BOSS_PER_MATRIX set), "grad" (the gradient
-    entry points) or "fit" (boss_gp_fit_batch).  groups: BOSS_LL_GROUPS, None when unset.  timing: boss_set_timing(1).
-    -> dict(Sb=..., small=..., windows=[dict(s0, sb, ngroups, gsz, groups=[(so, gs), ...]), ...]).  Per-matrix
-    windows run as one unit (ngroups 1)."""
+    mode: "value" (boss_gp_loglik_batch), "grad" (the gradient entry points) or "fit" (boss_gp_fit_batch).
+    groups: BOSS_LL_GROUPS, None when unset.  timing: boss_set_timing(1).
+    -> dict(Sb=..., small=..., windows=[dict(s0, sb, ngroups, gsz, groups=[(so, gs), ...]), ...])."""
     n_pad = (n + TM - 1) // TM * TM
     nblk = n_pad // TM
     mat = n_pad * n_pad
-    need_w = mode in ("grad", "fit")                                       # :3100
-    small = n <= SMALL_N and not need_w                                    # :3101
-    per = (3 if need_w else 1) * mat * 8 + (2 * nblk if need_w else nblk) * TM * TM * 8   # :3103
-    Sb = max(1, min(S, WORKSPACE_BYTES // per))                            # :3104
-    Sb = min(Sb, MAX_WINDOW)                                               # :3105
-    if small:                                                              # :3106, one launch for the whole batch
+    need_w = mode in ("grad", "fit")                                       # need_w
+    small = n <= SMALL_N and not need_w                                    # small
+    per = (3 if need_w else 1) * mat * 8 + (2 * nblk if need_w else nblk) * TM * TM * 8   # per
+    Sb = max(1, min(S, WORKSPACE_BYTES // per))                            # Sb
+    Sb = min(Sb, MAX_WINDOW)
+    if small:                                                              # one launch for the whole batch
         return dict(Sb=1, small=True, per=per, windows=[])
     windows = []
-    for s0 in range(0, S, Sb):                                             # :3202, :3246
+    for s0 in range(0, S, Sb):                                             # the window loop
         sb = min(Sb, S - s0)
-        if mode == "per_matrix":
-            windows.append(dict(s0=s0, sb=sb, ngroups=1, gsz=sb, groups=[(s0, sb)]))
-            continue
-        want = 2 if nblk <= 6 else 4                                       # :3250
-        if groups is not None:                                             # :3251
+        want = 2 if nblk <= 6 else 4                                       # want_groups
+        if groups is not None:
             want = max(1, min(LL_GROUPS, int(groups)))
-        ngroups = 1 if (timing or sb < 2 * want) else want                 # :3252
-        gsz = (sb + ngroups - 1) // ngroups                                # :3253
+        ngroups = 1 if (timing or sb < 2 * want) else want                 # ngroups
+        gsz = (sb + ngroups - 1) // ngroups                                # gsz
         gl = []
-        for gi in range(ngroups):                                          # :3256-3260
+        for gi in range(ngroups):                                          # the group loop: wo, gs
             wo = gi * gsz
             gs = min(gsz, sb - wo)
             if gs <= 0:

@@ -27,11 +27,11 @@ from tests.loglik_scale_oracle import _kappa_ld
 
 EPS = 2.0 ** -52
 TOL_POST, TOL_GRAD = 1e-9, 1e-8
-TM = 128                                     # csrc/common.cuh:22, rows of a block
-NW_NB = 32                                   # csrc/score_narrow.cuh:19, candidates of a narrow / quarter CTA
+TM = 128                                     # csrc/common.cuh `TM`, rows of a block
+NW_NB = 32                                   # csrc/score_narrow.cuh `NW_NB`, candidates of a narrow / quarter CTA
 NSM = 148                                    # SMs of the B200 the cost model counts waves over
-NQ_COST_CHAIN, NQ_COST_WORK, NQ_COST_FIXED = 0.085, 0.0019, 0.15   # csrc/boss_b200.cu:344
-PGRAD_SLOT_BYTES = 256 << 20                 # csrc/boss_b200.cu:1407
+NQ_COST_CHAIN, NQ_COST_WORK, NQ_COST_FIXED = 0.085, 0.0019, 0.15   # csrc/boss_b200.cu, same names
+PGRAD_SLOT_BYTES = 256 << 20                 # csrc/boss_b200.cu `PGRAD_SLOT_BYTES`
 PATHS = ("wide_fused", "wide_split", "narrow", "quarter")
 
 
@@ -251,12 +251,12 @@ def post_grad_ratios(got, ref, bounds):
 # ---- chunks and paths ----------------------------------------------------------------------------------------------
 
 def pick_row_splits(ncb, nblk):
-    """csrc/boss_b200.cu:313-338 -> (splits, cost in block-steps)."""
-    cost = ((ncb + NSM - 1) // NSM) * (nblk * (nblk + 1) // 2 + 1.0)            # :314
-    if ncb >= 4 * NSM or nblk < 2:                                               # :315
+    """pick_row_splits of csrc/boss_b200.cu -> (splits, cost in block-steps)."""
+    cost = ((ncb + NSM - 1) // NSM) * (nblk * (nblk + 1) // 2 + 1.0)
+    if ncb >= 4 * NSM or nblk < 2:
         return 1, cost
     best_t, best = 1e300, 1
-    for ns in range(1, nblk + 1):                                                # :318-335
+    for ns in range(1, nblk + 1):
         maxw = 0
         for y in range(ns):
             w, j = 0, 0
@@ -275,51 +275,50 @@ def pick_row_splits(ncb, nblk):
 
 
 def chunk_capacity(n_per_slice, M, d, xgrad, pgrad=False):
-    """ScoreCall::setup's chunk leading dimension CH and have_vt (csrc/boss_b200.cu:1442-1467)."""
+    """ScoreCall::setup's chunk leading dimension CH and have_vt (csrc/boss_b200.cu)."""
     max_npad = max((n + TM - 1) // TM * TM for n in n_per_slice)
     nsl = len(n_per_slice)
-    ncb_max = min((4 << 30) // (1024 * max_npad), 592)                          # :1446-1447
+    ncb_max = min((4 << 30) // (1024 * max_npad), 592)                          # ScoreCall::setup's ncb_max
     if ncb_max >= NSM:
-        ncb_max = ncb_max // NSM * NSM                                           # :1448
-    xgrad = xgrad or pgrad                                                       # :1164
+        ncb_max = ncb_max // NSM * NSM
+    xgrad = xgrad or pgrad                                                       # ScoreArgs::xgrad
     if xgrad:
-        ncb_max = max(1, min(ncb_max, 296))                                      # :1450
+        ncb_max = max(1, min(ncb_max, 296))                                      # a.xgrad() cap
     if pgrad:
-        per_block = 128 * nsl * (20 + 16 * d)                                    # :1452
-        ncb_max = max(1, min(ncb_max, PGRAD_SLOT_BYTES // per_block))           # :1453
-    CH = min(ncb_max, (M + 127) // 128) * 128                                    # :1455-1457
-    return CH, xgrad or CH <= 8192                                               # :1467
+        per_block = 128 * nsl * (20 + 16 * d)                                    # a.pgrad(): per_block
+        ncb_max = max(1, min(ncb_max, PGRAD_SLOT_BYTES // per_block))
+    CH = min(ncb_max, (M + 127) // 128) * 128                                    # need_cb, ncb_cap, CH
+    return CH, xgrad or CH <= 8192                                               # have_vt
 
 
 def score_plan(n_per_slice, M, d, xgrad, pgrad=False, nsl=1, path=None, unfused=False):
     """The (chunk, slice) passes of an unscreened scoring call: n_per_slice is one n for all nsl slices or a list of
     one n per slice (sample-major, as the call takes them); path / unfused: BOSS_SCORE_PATH / BOSS_UNFUSED_SCORE.
     xgrad: the call computes x-gradients (boss_ei_value_grad); pgrad: boss_gp_predict_grad, which implies xgrad.
-    BOSS_NO_NARROW (:1579) is not modelled: with it set the mirror does not describe the call.
     -> dict(CH, have_vt, xgrad, passes=[dict(chunk, m0, ch, slice, nblk, path, nsp, nsp32)])."""
     ns = list(n_per_slice) if np.ndim(n_per_slice) else [int(n_per_slice)] * nsl
     nsl = len(ns)
     CH, have_vt = chunk_capacity(ns, M, d, xgrad, pgrad)
     passes = []
-    for c, m0 in enumerate(range(0, M, CH)):                                     # :2263-2266
+    for c, m0 in enumerate(range(0, M, CH)):                                     # score_core's chunk loop
         ch = min(CH, M - m0)
-        ncb, ncb32 = (ch + 127) // 128, (ch + NW_NB - 1) // NW_NB               # :1566, :1577
+        ncb, ncb32 = (ch + 127) // 128, (ch + NW_NB - 1) // NW_NB               # score_slice's ncb, ncb32
         for q, n in enumerate(ns):
             nblk = (n + TM - 1) // TM
-            nsp, cost_w = pick_row_splits(ncb, nblk)                             # :1573
-            nsp32, cost_n = pick_row_splits(ncb32, nblk)                         # :1578
-            narrow = 0.32 * cost_n < cost_w                                      # :1579
-            cost_q = max(NQ_COST_CHAIN * nblk, NQ_COST_WORK * ncb32 * (nblk * (nblk + 1) // 2)) + NQ_COST_FIXED  # :1582
-            quarter = have_vt and cost_q < min(cost_w, 0.32 * cost_n if narrow else cost_w) and nblk >= 2   # :1583
-            if path == "wide":                                                   # :1584-1588
+            nsp, cost_w = pick_row_splits(ncb, nblk)                             # score_slice's nsp
+            nsp32, cost_n = pick_row_splits(ncb32, nblk)                         # score_slice's nsp32
+            narrow = 0.32 * cost_n < cost_w                                      # score_slice's narrow
+            cost_q = max(NQ_COST_CHAIN * nblk, NQ_COST_WORK * ncb32 * (nblk * (nblk + 1) // 2)) + NQ_COST_FIXED
+            quarter = have_vt and cost_q < min(cost_w, 0.32 * cost_n if narrow else cost_w) and nblk >= 2   # score_slice's quarter
+            if path == "wide":                                                   # score_slice's BOSS_SCORE_PATH switch
                 narrow = quarter = False
             elif path == "narrow":
                 narrow, quarter = True, False
             elif path == "quarter" and have_vt:
                 quarter = True
-            if quarter:                                                          # :1589
+            if quarter:
                 narrow = False
-            fuse = nsp == 1 and not narrow and not quarter and q == nsl - 1 and not unfused   # :1597
+            fuse = nsp == 1 and not narrow and not quarter and q == nsl - 1 and not unfused   # score_slice's fuse
             p = "quarter" if quarter else "narrow" if narrow else "wide_fused" if fuse else "wide_split"
             passes.append(dict(chunk=c, m0=m0, ch=ch, slice=q, nblk=nblk, path=p, nsp=nsp, nsp32=nsp32))
     return dict(CH=CH, have_vt=have_vt, xgrad=xgrad or pgrad, passes=passes)

@@ -112,45 +112,13 @@ def _ll_problem(n, d, S, seed):
 @pytest.mark.parametrize("kernel", KERNELS, ids=IDS)
 # n = 700 pads to 6 blocks, which still take the fused diagonal step (potrf_fused_kernel); n = 900 (8 blocks) runs the
 # separate SYRK -> potrf_tile_kernel -> chol_panel_kernel chain
-@pytest.mark.parametrize("n,path", [(20, "warp"), (300, "fused"), (300, "per_matrix"), (700, "fused"), (900, "blocked")])
-def test_loglik_paths(lib, kernel, n, path, monkeypatch):
+@pytest.mark.parametrize("n,path", [(20, "warp"), (300, "fused"), (700, "fused"), (900, "blocked")])
+def test_loglik_paths(lib, kernel, n, path):
     X, y, L, A, N = _ll_problem(n, 5, 12, seed=n)
-    if path == "per_matrix":
-        monkeypatch.setenv("BOSS_PER_MATRIX", "1")   # read per call
     ll = lib.loglik_batch(X, y, L, A, N, kid_of(lib, kernel))
     ref = O.gp_loglik_batch(X, y, L, A, N, kernel)
     assert np.all(np.isfinite(ref))
     assert np.max(np.abs(ll - ref) / np.abs(ref)) <= TOL_LL
-
-
-_UNFUSED = r'''
-import sys, json
-import numpy as np
-sys.path.insert(0, sys.argv[1])
-import boss_b200
-from boss_b200 import _lib as lib
-from tests.kernels_more_oracle import O, RQ
-from tests.util_problems import make_problem, make_hyper_samples
-lib.init(0)
-X, Y, _, _, _ = make_problem(300, 5, seed=300)
-L, A, N = make_hyper_samples(12, 5, seed=301)
-worst = 0.0
-for k in (3, RQ(0.5), RQ(2.0), RQ(50.0)):
-    kid = lib.kernel_rational_quadratic(k.a) if isinstance(k, RQ) else k
-    ll = lib.loglik_batch(X, Y[0], L, A, N, kid)
-    ref = O.gp_loglik_batch(X, Y[0], L, A, N, k)
-    worst = max(worst, float(np.max(np.abs(ll - ref) / np.abs(ref))))
-print(json.dumps({"worst": worst}))
-'''
-
-
-def test_loglik_unfused_diagonal_path():
-    """BOSS_UNFUSED_DIAG is read once per process: its own process."""
-    import json
-    r = subprocess.run([sys.executable, "-c", _UNFUSED, ROOT], env=dict(os.environ, BOSS_UNFUSED_DIAG="1"),
-                       capture_output=True, text=True, cwd=ROOT, timeout=600)
-    assert r.returncode == 0, r.stderr[-2000:]
-    assert json.loads(r.stdout.strip().splitlines()[-1])["worst"] <= TOL_LL
 
 
 @pytest.mark.parametrize("kernel", KERNELS, ids=IDS)

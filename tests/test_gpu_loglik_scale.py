@@ -247,13 +247,9 @@ def _chunks(S, step):
     return [(a, min(S, a + step)) for a in range(0, S, step)]
 
 
-@pytest.mark.parametrize("per_matrix", [False, True], ids=["default", "per_matrix"])
-def test_value_across_a_window(lib, per_matrix, monkeypatch):
+def test_value_across_a_window(lib):
     n, d, S = 100, 3, 32768 + 5
-    mode = "per_matrix" if per_matrix else "value"
-    if per_matrix:
-        monkeypatch.setenv("BOSS_PER_MATRIX", "1")
-    plan = LS.window_plan(n, d, S, mode)
+    plan = LS.window_plan(n, d, S, "value")
     Sb = plan["Sb"]
     assert Sb == 32768 and len(plan["windows"]) == 2
     X, Yp, L, A, N = _window_problem(n, d, S, seed=100)
@@ -266,7 +262,7 @@ def test_value_across_a_window(lib, per_matrix, monkeypatch):
     for a, b in _chunks(S, 10000):                      # chunks that do not line up with the window
         assert _same(ll[a:b], f(a, b)), (a, b)
     for s in _oracle_samples(S, Sb, 60, 7):
-        _note(f"window ({mode}): value", LS.rel_ratio(ll[s], OB.gp_loglik(X, Yp[s], L[s], A[s], N[s], kid)))
+        _note("window: value", LS.rel_ratio(ll[s], OB.gp_loglik(X, Yp[s], L[s], A[s], N[s], kid)))
 
 
 def test_gradients_across_a_window(lib):

@@ -449,7 +449,7 @@ def test_loglik_grad_batch(lib, n, d, kid, S):
     ll_ref, g_ref = O.gp_loglik_grad_batch(X, Y[0], L, A, N, kid)
     ll, g = lib.loglik_grad_batch(X, Y[0], L, A, N, kid)
     assert relerr(ll, ll_ref) <= TOL_LL
-    # same factorisation kernels (n > 32) unless the opt-in per-matrix path (BOSS_PER_MATRIX) evaluates the value-only batch
+    # same factorisation kernels as the value-only batch for n > 32; at n <= 32 that batch takes the warp-register path
     assert relerr(ll, lib.loglik_batch(X, Y[0], L, A, N, kid)) <= 1e-12
     scale = np.maximum(np.max(np.abs(g_ref), axis=1, keepdims=True), 1e-300)
     assert np.max(np.abs(g - g_ref) / scale) <= 1e-8, np.max(np.abs(g - g_ref) / scale)

@@ -76,7 +76,7 @@ def test_gradient_check_rejects_a_missing_tile_and_a_wrong_lengthscale(n, d, ker
 
 
 def test_window_plan_counts_windows():
-    for mode in ("value", "per_matrix", "grad", "fit"):
+    for mode in ("value", "grad", "fit"):
         Sb = LS.window_plan(100, 3, 10 ** 6, mode)["Sb"]
         assert Sb == 32768                                   # n_pad = 128: the 32768 cap, not the workspace, binds
         assert len(LS.window_plan(100, 3, Sb, mode)["windows"]) == 1
