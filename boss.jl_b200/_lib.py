@@ -102,6 +102,7 @@ EXPORTS = {
     "boss_dbg_screen_stats": (C.c_int, [_i64p]),
     "boss_dbg_score_paths": (C.c_int, [_i64p]),
     "boss_dbg_screen_ambiguous": (C.c_int, [_i64p]),
+    "boss_dbg_screen_var": (C.c_int, [_i64p]),
     "boss_dbg_screen_mean": (C.c_int, [_vp, _vp, C.c_int64, _vp, _vp, _vp]),
     "boss_dbg_kappa_f32": (C.c_int, [C.c_int, _vp, C.c_int, _vp]),
     "boss_dbg_mma_d2": (C.c_int, [C.c_int, _vp, _vp, _vp, _vp, C.c_int, C.c_int, _vp]),
@@ -786,6 +787,14 @@ def dbg_screen_ambiguous():
     definite keeps plus ambiguous candidates -- before the FP64 refinement and the re-seed)."""
     out = (C.c_int64 * 2)()
     _check(lib.boss_dbg_screen_ambiguous(out), "boss_dbg_screen_ambiguous")
+    return int(out[0]), int(out[1])
+
+
+def dbg_screen_var():
+    """The variance tier of the last screened call (W's first row block, DESIGN.md 2.9): (pool rows it bounded, rows it
+    kept for the exact pass); (0, 0) when it did not run."""
+    out = (C.c_int64 * 2)()
+    _check(lib.boss_dbg_screen_var(out), "boss_dbg_screen_var")
     return int(out[0]), int(out[1])
 
 

@@ -139,6 +139,7 @@ struct Ctx {
   DevBuf topk;                       // top-k calls: running set, chunk scores, selection state, sorted result
   int64_t scr_stats[3] = {0, 0, 0};  // last scoring call: screened (1) or fell back (2), candidates bounded, pool size
   int64_t scr_amb[2] = {0, 0};       // last screened call: ambiguous candidates of the FP32 tier, pool before refinement and re-seed
+  int64_t scr_var[2] = {0, 0};       // last screened call: pool rows into and out of the variance tier (0, 0: not run)
   int64_t score_paths[5] = {0, 0, 0, 0, 0};   // last scoring call's (chunk, slice) passes by path (boss_dbg_score_paths)
   // event pool for per-kernel-class timing
   cudaEvent_t ev_a[EV_POOL], ev_b[EV_POOL];
@@ -160,6 +161,10 @@ struct Ctx {
   void *pinned = nullptr;            // pinned slots for chunks of host arrays (see HostStaging)
   size_t pinned_cap = 0;
   cudaEvent_t pin_ev[2] = {nullptr, nullptr};
+  // the FP32 screening pass of device-resident calls runs here beside the first chunk's chain (Screen): the lowest
+  // priority, the library stream the highest, so that the chain's kernels take SMs as the pass's CTAs retire
+  cudaStream_t side = nullptr;
+  cudaEvent_t side_fork = nullptr, side_join = nullptr;
 };
 
 Ctx *g_ctx[MAX_DEV] = {};            // created by boss_init / boss_init_multi, emptied by boss_shutdown
@@ -250,18 +255,19 @@ int fail(int code, const std::string &msg) {
                                      std::to_string(__LINE__) + ")");                                  \
   } while (0)
 
-// timing helpers: bracket one launch with a pooled event pair
+// timing helpers: bracket one launch with a pooled event pair, recorded on the stream the launch goes to
 struct Timed {
   int slot = -1;
-  Timed(int cls) {
+  cudaStream_t st;
+  Timed(int cls, cudaStream_t s = nullptr) : st(s ? s : C().stream) {
     if (C().timing && C().ev_used < EV_POOL) {
       slot = C().ev_used++;
       C().ev_class[slot] = cls;
-      cudaEventRecord(C().ev_a[slot], C().stream);
+      cudaEventRecord(C().ev_a[slot], st);
     }
   }
   ~Timed() {
-    if (slot >= 0) cudaEventRecord(C().ev_b[slot], C().stream);
+    if (slot >= 0) cudaEventRecord(C().ev_b[slot], st);
   }
 };
 
@@ -541,7 +547,12 @@ int init_device(int device) {   // g_reg_mu held
   cudaDeviceProp prop;
   CUDA_TRY(cudaGetDeviceProperties(&prop, device));
   if (prop.major != 10) return fail(BOSS_ERR_STATE, std::string("boss_init: built for sm_100a, device is ") + prop.name);
-  CUDA_TRY(cudaStreamCreateWithFlags(&cx->stream, cudaStreamNonBlocking));
+  int prio_lo = 0, prio_hi = 0;
+  CUDA_TRY(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
+  CUDA_TRY(cudaStreamCreateWithPriority(&cx->stream, cudaStreamNonBlocking, prio_hi));
+  CUDA_TRY(cudaStreamCreateWithPriority(&cx->side, cudaStreamNonBlocking, prio_lo));
+  CUDA_TRY(cudaEventCreateWithFlags(&cx->side_fork, cudaEventDisableTiming));
+  CUDA_TRY(cudaEventCreateWithFlags(&cx->side_join, cudaEventDisableTiming));
   for (int i = 0; i < EV_POOL; ++i) {
     CUDA_TRY(cudaEventCreate(&cx->ev_a[i]));
     CUDA_TRY(cudaEventCreate(&cx->ev_b[i]));
@@ -596,6 +607,12 @@ void shutdown_device(Ctx *cx) {   // g_reg_mu held
     }
     cx->ev_ready = false;
   }
+  cudaStreamSynchronize(cx->side);
+  cudaStreamDestroy(cx->side);
+  cudaEventDestroy(cx->side_fork);
+  cudaEventDestroy(cx->side_join);
+  cx->side = nullptr;
+  cx->side_fork = cx->side_join = nullptr;
   cudaStreamDestroy(cx->stream);
   cx->stream = nullptr;
   cx->attrs_done = false;
@@ -1815,12 +1832,16 @@ struct Screen {
   // FP32 mean tier from the second chunk on (BOSS_SCREEN_F64=1: the FP64 tier throughout); the threshold re-seeded
   // from the whole pool before it is scored (BOSS_SCREEN_NO_RESEED=1: not)
   bool f32 = false, reseed = false;
+  // device-resident FP32 tier: one launch over every candidate after the first chunk, on the context's side stream
+  // beside the first chunk's chain; `pending` until the library stream waits for it
+  bool side = false, pending = false;
   long long n0 = 0, n_amb = 0;   // pool rows of the first chunk; ambiguous candidates of the call
   // device buffers: the bounds of one chunk (hi in the FP32 tier) and lo, per-256 survivor counts, the pool sizes (two
   // slots for the chunks, two for the re-compaction), the seed selection (two ping-pong rounds), the seed batch, the
   // refinement batch, the survivor pool with each row's bound and verdict, and the re-compacted pool
   double *bound = nullptr, *lo = nullptr, *seed_x = nullptr, *seed_pm = nullptr, *pool_x = nullptr, *pool_pm = nullptr;
-  double *pool_bound = nullptr, *ref_x = nullptr, *ref_pm = nullptr, *consts = nullptr;
+  double *pool_bound = nullptr, *ref_x = nullptr, *ref_pm = nullptr, *consts = nullptr, *a2s = nullptr;
+  int *fail_flag = nullptr;   // [2]: the side pass's and the variance tier's failed-variance flags
   int *ti[2] = {}, *ref_row = nullptr, *ref_cnt = nullptr;
   unsigned long long *tk[2] = {};
   long long *cnt = nullptr, *base = nullptr, *pool_idx = nullptr;   // cnt: survivors per 128 candidates, then offsets
@@ -1828,6 +1849,13 @@ struct Screen {
   std::vector<float *> xt32, al32;   // per slice: the MMA tier's B fragments of the centred training inputs, |t~|^2 and alpha
 
   bool on() const { return state == SCREENING; }
+
+  // every exit of the call orders the library stream after the side stream's pass (it reads the caller's candidates)
+  ~Screen() { join(); }
+  void join() {
+    if (pending) cudaStreamWaitEvent(C().stream, C().side_join, 0);
+    pending = false;
+  }
 
   // bytes of one pool row: candidate, index, bound, verdict, prior means, constraint-mask entry
   static size_t pool_row(const ScoreArgs &a, int d) {
@@ -1857,12 +1885,13 @@ struct Screen {
     // bounds and counts for one chunk, or for all candidates after the first when they are on the device (FP32 tier)
     const size_t span = a.dev && f32 ? std::max<long long>(CH, M) : CH;
     const size_t o_bound = take(tot, span * 8), o_lo = take(tot, span * 8);
-    const size_t o_cnt = take(tot, (span + 127) / 128 * 8), o_base = take(tot, 32);
+    const size_t o_cnt = take(tot, (span + 127) / 128 * 8), o_base = take(tot, 48);
     const size_t o_tk0 = take(tot, ntk * 8), o_tk1 = take(tot, ntk * 8), o_ti0 = take(tot, ntk * 4), o_ti1 = take(tot, ntk * 4);
     const size_t o_sx = take(tot, (size_t)ns_max * d * 8), o_spm = take(tot, (size_t)ns_max * y_dim * 8), o_scm = take(tot, ns_max);
     const size_t o_rx = take(tot, (size_t)CH * d * 8), o_rpm = take(tot, pm ? (size_t)CH * y_dim * 8 : 0);
     const size_t o_rrow = take(tot, (size_t)CH * 4), o_rcnt = take(tot, 8);
-    const size_t o_consts = take(tot, (size_t)c.nsl * SCREEN_NCONST * 8);
+    const size_t o_consts = take(tot, (size_t)c.nsl * SCREEN_NCONST * 8), o_a2s = take(tot, (size_t)c.nsl * 8),
+                 o_fail = take(tot, 8);
     std::vector<size_t> o_xt(c.nsl), o_al(c.nsl);
     for (int q = 0; q < c.nsl; ++q) {
       o_xt[q] = take(tot, f32 ? (size_t)c.sl[q]->n_pad * ((c.sl[q]->dp + 7) / 8 * 8) * 8 : 0);
@@ -1886,14 +1915,28 @@ struct Screen {
     ref_row = reinterpret_cast<int *>(b + o_rrow);
     ref_cnt = reinterpret_cast<int *>(b + o_rcnt);
     consts = reinterpret_cast<double *>(b + o_consts);
+    a2s = reinterpret_cast<double *>(b + o_a2s);
+    fail_flag = reinterpret_cast<int *>(b + o_fail);
     xt32.assign(c.nsl, nullptr);
     al32.assign(c.nsl, nullptr);
+    // Device-resident candidates: the constants and the FP32 pass over [ch0, M) go to the side stream, forked here
+    // (after the wait for the caller's stream).  Nested calls of the first chunk rewrite the small block, so the pass
+    // reads its own copy of the prior variances.
+    side = f32 && a.dev && M > ch0;
+    cudaStream_t cs = C().stream;
+    if (side) {
+      CUDA_TRY(cudaMemcpyAsync(a2s, c.small, (size_t)c.nsl * 8, cudaMemcpyDeviceToDevice, C().stream));
+      CUDA_TRY(cudaEventRecord(C().side_fork, C().stream));
+      CUDA_TRY(cudaStreamWaitEvent(C().side, C().side_fork, 0));
+      cs = C().side;
+      pending = true;
+    }
     for (int q = 0; q < c.nsl && f32; ++q) {   // per call, so that an appended point or a refit is never missed
       const boss_gp *h = c.sl[q];
       xt32[q] = reinterpret_cast<float *>(b + o_xt[q]);
       al32[q] = reinterpret_cast<float *>(b + o_al[q]);
-      screen_consts_kernel<<<1, 1024, 0, C().stream>>>(h->Xt, h->alpha, h->n, h->n_pad, h->dp, xt32[q], al32[q],
-                                                       consts + (size_t)SCREEN_NCONST * q);
+      screen_consts_kernel<<<1, 1024, 0, cs>>>(h->Xt, h->alpha, h->n, h->n_pad, h->dp, xt32[q], al32[q],
+                                               consts + (size_t)SCREEN_NCONST * q);
       ++C().launches;
     }
     tot = 0;
@@ -1908,9 +1951,61 @@ struct Screen {
     pool_ver = b + o_pv;
     pool_pm = pm ? reinterpret_cast<double *>(b + o_ppm) : nullptr;
     pool_cm = cm ? b + o_pcm : nullptr;
-    CUDA_TRY(cudaMemsetAsync(base, 0, 32, C().stream));
+    CUDA_TRY(cudaMemsetAsync(base, 0, 48, C().stream));
     state = SCREENING;
     return 0;
+  }
+
+  // EI at the prior variance, PoF = 1, no guards: the bound pass's parameters, bound[m - out_off]
+  static AcqParams bound_params(const AcqParams &ap, double *bound, long long out_off) {
+    AcqParams bp = ap;
+    bp.sumsq = nullptr;
+    bp.has_ymax = 0;
+    bp.lb = bp.ub = nullptr;
+    bp.cons_mask = nullptr;
+    bp.acq = bound;
+    bp.out_off = out_off;
+    bp.blk_val = nullptr;
+    bp.blk_idx = nullptr;
+    return bp;
+  }
+
+  // The FP32 tier over the chunk of ap: hi and lo of candidate m at [m - out_off], and with cnt the survivors
+  // !(hi < thr (1 - 2^-32)) per 128 candidates
+  void launch_f32(const ScoreCall &c, const AcqParams &ap, const ChunkIO &io, long long out_off, long long *cnt_out,
+                  cudaStream_t st) {
+    ScreenF32Params sp{};
+    sp.Xs = io.xs;
+    sp.m0 = ap.m0;
+    sp.M = ap.m0 + ap.chunk;
+    sp.in_off = io.off;
+    sp.d = c.d;
+    sp.nsl = c.nsl;
+    for (int q = 0; q < c.nsl; ++q) {
+      const boss_gp *h = c.sl[q];
+      sp.sl[q] = ScreenSlice{reinterpret_cast<const float4 *>(xt32[q]), reinterpret_cast<const float4 *>(al32[q]),
+                             consts + (size_t)SCREEN_NCONST * q, h->invl, h->disc, h->a2, h->n_pad};
+    }
+    sp.hi = bound_params(ap, bound, out_off);
+    sp.lo = sp.hi;
+    sp.lo.acq = lo;
+    sp.thr = thr * (1.0 - 0x1p-32);
+    sp.cnt = cnt_out;
+    {
+      Timed t(1, st);
+      launch_screen_mean_bound(c.sl[0]->kernel_id, c.sl[0]->dp, sp, (ap.chunk + 127) / 128, st);
+    }
+    ++C().launches;
+  }
+
+  // Device-resident FP32 tier: the bounds of every candidate after the first chunk (ap's chunk) on the side stream,
+  // at bound[m] and lo[m], beside the first chunk on the library stream.  No threshold exists yet: the counts come
+  // after the join (chunk()), with the fused kernel's rule.
+  void launch_side(const ScoreCall &c, AcqParams ap, const ChunkIO &io) {
+    ap.a2 = a2s;
+    ap.any_fail = fail_flag;   // never set (the prior variance a^2 + 1e-18 passes _clip_var), and never read
+    launch_f32(c, ap, io, 0, nullptr, C().side);
+    cudaEventRecord(C().side_join, C().side);
   }
 
   // One chunk: the means of every slice (xcov without K*^T), the bounds, the survivors appended to the pool.  The first
@@ -1919,46 +2014,22 @@ struct Screen {
   // surviving.  The first chunk takes the FP64 means, so the seed batch, T and that decision are those of the FP64
   // tier; later chunks of the FP32 tier bound EI from mu~ +- E' in one launch of screen_mean_bound_kernel and leave the
   // ambiguous ones to Screen::finish.  With device-resident candidates, the FP32 tier's "chunk" is everything after the
-  // first chunk (see score_core).
+  // first chunk (see score_core), bounded on the side stream while the first chunk runs (launch_side).
   int chunk(const ScoreCall &c, const AcqParams &ap, const ChunkIO &io, int cidx, TopkBufs &tb) {
     const ScoreArgs &a = c.a;
     const long long m0 = ap.m0;
     const int ch = ap.chunk, ncb = (ch + 127) / 128, nb = (ch + 255) / 256;
     const bool t32 = f32 && cidx > 0;
-    AcqParams bp = ap;   // EI at the prior variance, PoF = 1, no guards -> bound[c]
-    bp.sumsq = nullptr;
-    bp.has_ymax = 0;
-    bp.lb = bp.ub = nullptr;
-    bp.cons_mask = nullptr;
-    bp.acq = bound;
-    bp.out_off = m0;
-    bp.blk_val = nullptr;
-    bp.blk_idx = nullptr;
+    const AcqParams bp = bound_params(ap, bound, m0);
+    const double *bnd = bound, *blo = lo;   // the chunk's bounds, candidate m0 first
     // FP32 tier: hi < thr (1 - 2^-32) drops, lo >= thr (1 + 2^-32) keeps, anything else (NaN too) is ambiguous.  The
     // first chunk (FP64 tier) sets thr in seed().
-    if (t32) {
-      ScreenF32Params sp{};
-      sp.Xs = io.xs;
-      sp.m0 = m0;
-      sp.M = m0 + ch;
-      sp.in_off = io.off;
-      sp.d = c.d;
-      sp.nsl = c.nsl;
-      for (int q = 0; q < c.nsl; ++q) {
-        const boss_gp *h = c.sl[q];
-        sp.sl[q] = ScreenSlice{reinterpret_cast<const float4 *>(xt32[q]), reinterpret_cast<const float4 *>(al32[q]),
-                               consts + (size_t)SCREEN_NCONST * q, h->invl, h->disc, h->a2, h->n_pad};
-      }
-      sp.hi = bp;
-      sp.lo = bp;
-      sp.lo.acq = lo;
-      sp.thr = thr * (1.0 - 0x1p-32);
-      sp.cnt = cnt;
-      {
-        Timed t(1);
-        launch_screen_mean_bound(c.sl[0]->kernel_id, c.sl[0]->dp, sp, ncb, C().stream);
-      }
-      ++C().launches;
+    if (t32 && side) {   // the side stream's pass (launch_side) has the bounds
+      join();
+      bnd = bound + m0;
+      blo = lo + m0;
+    } else if (t32) {
+      launch_f32(c, ap, io, m0, cnt, C().stream);
     } else {
       for (int q = 0; q < c.nsl; ++q) {
         const boss_gp *h = c.sl[q];
@@ -1983,12 +2054,12 @@ struct Screen {
       if (rc || !on()) return rc;
     }
     const double thr_drop = t32 ? thr * (1.0 - 0x1p-32) : thr;
-    if (!t32) {
-      screen_count_kernel<<<ncb, 128, 0, C().stream>>>(bound, nullptr, ch, thr_drop, cnt);
+    if (!t32 || side) {
+      screen_count_kernel<<<ncb, 128, 0, C().stream>>>(bnd, nullptr, ch, thr_drop, cnt);
       ++C().launches;
     }
     screen_scan_kernel<<<1, 1024, 0, C().stream>>>(cnt, ncb, base, cidx & 1);
-    CompactParams cpar{bound, nullptr, ch, thr_drop, t32 ? lo : nullptr, thr * (1.0 + 0x1p-32), cnt, m0, xs_c, pm_c, cm_c,
+    CompactParams cpar{bnd, nullptr, ch, thr_drop, t32 ? blo : nullptr, thr * (1.0 + 0x1p-32), cnt, m0, xs_c, pm_c, cm_c,
                        c.d, a.y_dim, pool_x, pool_pm, pool_cm, pool_idx, nullptr, pool_bound, pool_ver};
     screen_compact_kernel<<<ncb, 128, 0, C().stream>>>(cpar);
     C().launches += 2;
@@ -2044,6 +2115,12 @@ struct Screen {
     C().scr_amb[1] = npool;
     if (nfin < 1) return fail(BOSS_ERR_STATE, "score: argmax screening kept no candidate");   // the seed's winner always survives
     if (nfin < a.topk) return fail(BOSS_ERR_STATE, "score: top-k screening kept fewer than k candidates");   // the seed's k best survive
+    const bool multi_blk = std::all_of(c.sl.begin(), c.sl.begin() + c.nsl, [](const boss_gp *h) { return h->nblk >= 2; });
+    if (multi_blk && nfin > SEED_N) {
+      rc = var_tier(c, thr2, px, ppm, pcm, pidx, nfin);
+      if (rc) return rc;
+      if (nfin < std::max<long long>(1, a.topk)) return fail(BOSS_ERR_STATE, "score: the variance tier kept too few candidates");
+    }
     SubsetResult r;
     rc = score_subset(c, px, ppm, pcm, nfin, a.top_val, a.top_idx, pidx, false, r);
     if (rc) return rc;
@@ -2062,9 +2139,10 @@ struct Screen {
  private:
   size_t p2_off[3] = {0, 0, 0};   // re-compacted pool: offsets of the indices, prior means, mask entries
 
-  void fall_back() {
+  void fall_back() {   // the full path goes on behind the side stream's (wasted) pass
     C().scr_stats[0] = 2;
     state = FELL_BACK;
+    join();
   }
 
   // The seed batch of the first chunk: the exact scores of its highest bounds.  Their best (argmax) or k-th best
@@ -2182,15 +2260,22 @@ struct Screen {
   }
 
   // pool rows with verdict 1 and bound >= thr2 (or NaN), in order, into the second pool buffer; their count -> nfin
-  int recompact(const ScoreCall &c, long long npool, double thr2, long long &nfin) {
-    const ScoreArgs &a = c.a;
+  // the second pool buffer for n rows: candidates first, then the offsets in p2_off
+  int size_pool2(const ScoreCall &c, long long n) {
     size_t tot = 0;
-    const size_t o_x = take(tot, (size_t)npool * c.d * 8);
-    p2_off[0] = take(tot, (size_t)npool * 8);
-    p2_off[1] = take(tot, pool_pm ? (size_t)npool * a.y_dim * 8 : 0);
-    p2_off[2] = take(tot, pool_cm ? (size_t)npool : 0);
+    const size_t o_x = take(tot, (size_t)n * c.d * 8);
+    p2_off[0] = take(tot, (size_t)n * 8);
+    p2_off[1] = take(tot, pool_pm ? (size_t)n * c.a.y_dim * 8 : 0);
+    p2_off[2] = take(tot, pool_cm ? (size_t)n : 0);
     (void)o_x;
     CUDA_TRY(C().scr_pool2.ensure(tot));
+    return 0;
+  }
+
+  int recompact(const ScoreCall &c, long long npool, double thr2, long long &nfin) {
+    const ScoreArgs &a = c.a;
+    int rc = size_pool2(c, npool);
+    if (rc) return rc;
     unsigned char *b = C().scr_pool2.as<unsigned char>();
     int par = 0;
     for (long long r0 = 0; r0 < npool; r0 += c.CH, par ^= 1) {
@@ -2208,6 +2293,91 @@ struct Screen {
     }
     CUDA_TRY(cudaMemcpyAsync(&nfin, base + 2 + par, 8, cudaMemcpyDeviceToHost, C().stream));
     CUDA_TRY(cudaStreamSynchronize(C().stream));
+    return 0;
+  }
+
+  // The variance tier (DESIGN.md 2.9): W = L^-1 is lower triangular, so the first row block of V = W K* involves the
+  // first 128 training points only, and its column sum of squares S1 is at most the full S.  Per piece of pool rows:
+  // K* and the mean partials (xcov_kernel<.., true>), mu reduced as on the exact path, the first row block of V by
+  // score_quarter_kernel with nblk = 1 (the same k order and DMMA chain as that block in the full pass; nblk >= 2 in
+  // score_slice is its cost model, not a kernel condition), quarter_sumsq_kernel's partials of that block and the
+  // fixed-order reduction with the other row blocks' partials taken as +0.  FP addition is monotone and every partial
+  // is >= 0, so the computed S1 <= the computed S, and EI at a^2 - S1 with the exact mu, PoF 1 and no guards bounds
+  // each row's exact score.  Rows with bound >= thr2 (or NaN) are kept in order, the index map composed; the rows
+  // move between the two pool buffers.  A failed variance (a -inf bound) keeps the whole pool, so the exact pass still
+  // sees the failure.
+  int var_tier(const ScoreCall &c, double thr2, const double *&px, const double *&ppm, const unsigned char *&pcm,
+               const long long *&pidx, long long &nfin) {
+    const ScoreArgs &a = c.a;
+    constexpr int PIECE = 8192;   // rows per pass: V^T scratch of PIECE x n_pad, what the exact pass on PIECE rows takes
+    const int piece = std::min(c.CH, PIECE);
+    int max_npad = 0;
+    for (int q = 0; q < c.nsl; ++q) max_npad = std::max(max_npad, c.sl[q]->n_pad);
+    CUDA_TRY(C().vt.ensure((size_t)piece * max_npad * 8));
+    const bool to_pool = px != pool_x;   // the rows are in the second buffer: write the first
+    if (!to_pool) {
+      int rc = size_pool2(c, nfin);
+      if (rc) return rc;
+    }
+    unsigned char *b2 = C().scr_pool2.as<unsigned char>();
+    double *ox = to_pool ? pool_x : reinterpret_cast<double *>(b2);
+    long long *oidx = to_pool ? pool_idx : reinterpret_cast<long long *>(b2 + p2_off[0]);
+    double *opm = !pool_pm ? nullptr : to_pool ? pool_pm : reinterpret_cast<double *>(b2 + p2_off[1]);
+    unsigned char *ocm = !pool_cm ? nullptr : to_pool ? pool_cm : b2 + p2_off[2];
+    CUDA_TRY(cudaMemsetAsync(fail_flag + 1, 0, 4, C().stream));
+    int par = 0;
+    for (long long r0 = 0; r0 < nfin; r0 += piece, par ^= 1) {
+      const int n = (int)std::min<long long>(piece, nfin - r0), ncb = (n + 127) / 128, ncb32 = (n + NW_NB - 1) / NW_NB;
+      const double *xs = px + (size_t)r0 * c.d;
+      for (int q = 0; q < c.nsl; ++q) {
+        const boss_gp *h = c.sl[q];
+        const int nks = std::max(1, std::min(h->nblk, (16 * 148 + ncb - 1) / ncb));
+        launch_xcov(h->kernel_id, h->dp, xcov_params(h, xs, n, 0, 0, c.d, c.CH), dim3(ncb, nks), C().stream);
+        reduce_rows_kernel<<<(ncb * 128 + 255) / 256, 256, 0, C().stream>>>(C().part_mu.as<double>(), 2 * h->nblk,
+                                                                          (size_t)c.CH, C().muv.as<double>() + (size_t)q * c.CH,
+                                                                          ncb * 128);
+        NarrowParams np{h->W, C().ks.as<double>(), 1, h->ktiles, nullptr, c.CH, C().vt.as<double>()};
+        score_quarter_kernel<0, 4, 1><<<dim3(ncb32, 4), NQ_THREADS, NQ_SMEM_BYTES, C().stream>>>(np);
+        quarter_sumsq_kernel<<<dim3(ncb32, 1), 256, 0, C().stream>>>(C().vt.as<double>(), h->ktiles,
+                                                                    C().part_ss.as<double>(), c.CH);
+        reduce_rows2_kernel<<<(ncb * 128 + 255) / 256, 256, 0, C().stream>>>(C().part_ss.as<double>(), 2, (size_t)c.CH,
+                                                                           C().sumsq.as<double>() + (size_t)q * c.CH,
+                                                                           ncb * 128);
+      }
+      ChunkIO io;
+      io.xs = xs;
+      io.pm = ppm ? ppm + (size_t)r0 * a.y_dim : nullptr;
+      AcqParams bp = c.acq_params(0, n, io);
+      bp.M = n;
+      bp.has_ymax = 0;
+      bp.lb = bp.ub = nullptr;
+      bp.cons_mask = nullptr;
+      bp.acq = bound;
+      bp.out_off = 0;
+      bp.blk_val = nullptr;
+      bp.blk_idx = nullptr;
+      bp.any_fail = fail_flag + 1;
+      acq_kernel<<<(n + 255) / 256, 256, 0, C().stream>>>(bp);
+      screen_count_kernel<<<ncb, 128, 0, C().stream>>>(bound, nullptr, n, thr2, cnt);
+      screen_scan_kernel<<<1, 1024, 0, C().stream>>>(cnt, ncb, base + 4, par);
+      CompactParams cp{bound, nullptr, n, thr2, nullptr, 0.0, cnt, 0, xs, io.pm, pcm ? pcm + r0 : nullptr, c.d, a.y_dim,
+                       ox, opm, ocm, oidx, pidx + r0, nullptr, nullptr};
+      screen_compact_kernel<<<ncb, 128, 0, C().stream>>>(cp);
+      C().launches += 5 * c.nsl + 4;
+    }
+    long long kept = 0;
+    int failed = 0;
+    CUDA_TRY(cudaMemcpyAsync(&kept, base + 4 + par, 8, cudaMemcpyDeviceToHost, C().stream));
+    CUDA_TRY(cudaMemcpyAsync(&failed, fail_flag + 1, 4, cudaMemcpyDeviceToHost, C().stream));
+    CUDA_TRY(cudaStreamSynchronize(C().stream));
+    if (failed) return 0;
+    C().scr_var[0] = nfin;
+    C().scr_var[1] = kept;
+    px = ox;
+    ppm = opm;
+    pcm = ocm;
+    pidx = oidx;
+    nfin = kept;
     return 0;
   }
 };
@@ -2228,7 +2398,7 @@ int score_core(ScoreArgs &a) {
   rc = c.setup();
   if (rc) return rc;
   if (!a.internal) {
-    C().scr_stats[0] = C().scr_stats[1] = C().scr_stats[2] = C().scr_amb[0] = C().scr_amb[1] = 0;
+    C().scr_stats[0] = C().scr_stats[1] = C().scr_stats[2] = C().scr_amb[0] = C().scr_amb[1] = C().scr_var[0] = C().scr_var[1] = 0;
     for (int64_t &p : C().score_paths) p = 0;
   }
   const int ch0 = (int)std::min<long long>(c.CH, a.M);   // the first chunk
@@ -2270,6 +2440,7 @@ int score_core(ScoreArgs &a) {
       ap.out_off = m0;
     }
     if (scr.on()) {
+      if (cidx == 0 && scr.side) scr.launch_side(c, c.acq_params(ch, (int)(a.M - ch), io), io);
       rc = scr.chunk(c, ap, io, cidx, tb);
       if (rc) return rc;
     }
@@ -3724,6 +3895,12 @@ int boss_dbg_screen_ambiguous(int64_t *out) {
   REQUIRE_INIT();
   out[0] = C().scr_amb[0];
   out[1] = C().scr_amb[1];
+  return 0;
+}
+int boss_dbg_screen_var(int64_t *out) {
+  REQUIRE_INIT();
+  out[0] = C().scr_var[0];
+  out[1] = C().scr_var[1];
   return 0;
 }
 

@@ -72,8 +72,8 @@ struct ScreenF32Params {
   ScreenSlice sl[SCREEN_F32_MAX_SL];
   AcqParams hi, lo;       // the bound pass at mu~ + E' and at mu~ - E' (mu / sumsq unused; hi.acq, lo.acq get the bounds)
   double thr;             // a candidate survives unless its hi bound is below thr
-  long long *cnt;         // survivors per 128 candidates; null: write mu~ and E instead of verdicts
-  double *mu_out, *e_out; // [nsl][ld] indexed by m - m0 (cnt null)
+  long long *cnt;         // survivors per 128 candidates, or null: the bounds only
+  double *mu_out, *e_out; // or [nsl][ld] indexed by m - m0: mu~ and E instead of the bounds
   int ld;
 };
 constexpr int SCREEN_NCONST = 2 + 32;

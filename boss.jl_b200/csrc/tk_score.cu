@@ -91,8 +91,9 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 //
 // Verdicts, one thread per candidate: per slice mu~ +- E', E' = E with the sign of the slice's output coefficient (NaN
 // for both if mu~ or E is not finite), so that EI is at least as large at mu~ + E' as at the FP64 mean and no larger at
-// mu~ - E'; the EI bound at each (acq_candidate under p.hi and p.lo, into hi.acq and lo.acq); and the CTA's survivors,
-// !(hi < p.thr), to p.cnt[blockIdx.x].  With p.cnt null the CTA writes mu~ and E to p.mu_out / p.e_out instead.
+// mu~ - E'; the EI bound at each (acq_candidate under p.hi and p.lo, into hi.acq and lo.acq); and, unless p.cnt is
+// null, the CTA's survivors, !(hi < p.thr), to p.cnt[blockIdx.x].  With p.mu_out set the CTA writes mu~ and E to
+// p.mu_out / p.e_out instead.
 template <int KID, int DP>
 __global__ void __launch_bounds__(256) screen_mean_bound_kernel(ScreenF32Params p) {
   constexpr int KS = (DP + 7) / 8, KP = 8 * KS;       // k-steps of the MMA, the padded dimension
@@ -199,7 +200,7 @@ __global__ void __launch_bounds__(256) screen_mean_bound_kernel(ScreenF32Params 
     __syncthreads();   // mu~ complete; the ring and snu are free for the next slice
   }
   const long long m = mb + tid;
-  if (!p.cnt) {
+  if (p.mu_out) {
     if (tid < 128 && m < p.M)
       for (int q = 0; q < p.nsl; ++q) {
         p.mu_out[(size_t)q * p.ld + (m - p.m0)] = smu[q * 128 + tid];
@@ -218,6 +219,7 @@ __global__ void __launch_bounds__(256) screen_mean_bound_kernel(ScreenF32Params 
     keep = !(acq_candidate<true>(p.hi, 0, m, smu + tid, 128) < p.thr);
     acq_candidate<true>(p.lo, 0, m, se + tid, 128);
   }
+  if (!p.cnt) return;
   const int k = __syncthreads_count(keep);
   if (tid == 0) p.cnt[blockIdx.x] = k;
 }

@@ -402,6 +402,10 @@ int boss_dbg_score_paths(int64_t *out);
  * FP64), out[1] = the pool as the chunks left it (definite keeps plus ambiguous candidates), before the FP64 refinement
  * and the re-seeded threshold */
 int boss_dbg_screen_ambiguous(int64_t *out);
+/* the variance tier of the last screened call: out[0] = pool rows it bounded (the pool after the re-seed), out[1] = the
+ * rows it kept for the exact pass; both 0 when the tier did not run (one row block of W, at most SEED_N pool rows, or a
+ * bound with a failed variance) */
+int boss_dbg_screen_var(int64_t *out);
 /* the FP32 tier's mean mu~ and error bound E, and the FP64 mean, of M candidates (d x M column-major) under gp
  * (K*^T alpha, no prior mean) */
 int boss_dbg_screen_mean(const boss_gp *gp, const double *Xs, int64_t M, double *mu32, double *E, double *mu64);

@@ -13,7 +13,9 @@ whether the (value, index) pairs are bit-identical to the f64 tier's.  One JSON 
 it was measured at.
 --profile FILE: afterwards, one resident bench call per tier under torch.profiler (a run of its own, after the timed
 rounds); the CUDA time per kernel name and tier goes to FILE as JSON, with the FP32 tier's mean kernel per chunk and
-its (candidate, training point) pairs per second beside two bounds whose rates are assumptions, not measurements."""
+its (candidate, training point) pairs per second beside two bounds whose rates are assumptions, not measurements, the
+call's kernel timeline with streams, the kernels that start inside the FP32 pass's span, and the variance tier's rows
+in and out."""
 import argparse
 import json
 import os
@@ -106,11 +108,11 @@ def main():
                     os.environ[k] = "1"
                 ms_t, r = timed(fn, args.steps)
                 ms[t].append(ms_t)
-                st, amb = _lib.dbg_screen_stats(), _lib.dbg_screen_ambiguous()
+                st, amb, var = _lib.dbg_screen_stats(), _lib.dbg_screen_ambiguous(), _lib.dbg_screen_var()
                 l0 = _lib.launch_count()
                 fn()
                 info[t] = {"screen_state": st[0], "bounded": st[1], "pool": st[2], "ambiguous": amb[0],
-                           "launches_per_call": _lib.launch_count() - l0}
+                           "var_tier_rows_in_out": list(var), "launches_per_call": _lib.launch_count() - l0}
                 key = (np.float64(r[0]).view(np.int64), r[1])
                 ref = key if ref is None else ref
                 same = same and key == ref
@@ -137,6 +139,22 @@ def main():
                 fn()
                 torch.cuda.synchronize()
             ker = {}
+            # the call's kernels in start order (device clock, us from the first), with the stream they ran on: the
+            # device-resident FP32 pass runs on a side stream beside the first chunk's kernels
+            evs = sorted((e for e in pr.events() if e.device_type.name == "CUDA"), key=lambda e: e.time_range.start)
+            t0 = evs[0].time_range.start if evs else 0
+            tl = [{"name": e.name[:80], "start_us": e.time_range.start - t0, "dur_us": e.time_range.end - e.time_range.start,
+                   "stream": getattr(e, "device_resource_id", None)} for e in evs]
+            prof_out.setdefault("timeline", {})[t] = tl
+            span = [(x["start_us"], x["start_us"] + x["dur_us"]) for x in tl if "screen_mean_bound_kernel" in x["name"]]
+            if span:
+                a0, a1 = span[0]
+                inside = [x for x in tl if "screen_mean_bound_kernel" not in x["name"] and a0 <= x["start_us"] < a1]
+                prof_out.setdefault("inside_fp32_pass", {})[t] = {
+                    "pass_us": [a0, a1], "kernels_started_inside": len(inside),
+                    "kernel_us_inside": sum(min(x["dur_us"], a1 - x["start_us"]) for x in inside),
+                    "names": sorted({x["name"] for x in inside})}
+            prof_out.setdefault("var_tier_rows_in_out", {})[t] = list(_lib.dbg_screen_var())
             for e in pr.key_averages():
                 if e.device_type.name == "CUDA" or getattr(e, "cuda_time_total", 0) > 0:
                     us = getattr(e, "device_time_total", None) or getattr(e, "cuda_time_total", 0)
