@@ -88,6 +88,8 @@ EXPORTS = {
                                                  _vp, C.c_int, _vp, C.c_int64, _vp, _vp, _vp]),
     "boss_gp_loglik_grad_batch_mean_dev": (C.c_int, [_vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, C.c_int, C.c_int64, _vp,
                                                      _vp, _vp, C.c_int, _vp, C.c_int64, _vp, _vp, _vp, _vp]),
+    "boss_gp_map_multistart": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int64,
+                                         C.c_int, C.c_int, _vp, _vp, _vp, _vp, _vp, C.POINTER(C.c_int)]),
     "boss_set_timing": (None, [C.c_int]),
     "boss_last_kernel_ms": (C.c_double, [C.c_int]),
     "boss_last_kernel_count": (C.c_int, [C.c_int]),
@@ -710,6 +712,34 @@ def loglik_batch_dev(X_ptr, d, n, Y_ptr, ldy, ls_ptr, amp_ptr, noise_ptr, kernel
     _check(lib.boss_gp_loglik_batch_dev(_vp(X_ptr), d, n, _vp(Y_ptr), ldy, _vp(ls_ptr), _vp(amp_ptr), _vp(noise_ptr),
                                         int(kernel_id), _ptr(dm), int(S), _vp(out_ptr), _vp(stream) if stream else None),
            "boss_gp_loglik_batch_dev")
+
+
+def gp_map_multistart(X, Y_minus_mean, prior_kind, prior_par, starts, kernel_id=KERNEL_MATERN52, discrete_mask=None,
+                      iters=40, history=8):
+    """Device-resident MAP fit of the hyper-parameters (boss_gp_map_multistart): every output slice on its own, all
+    (slice, start) pairs in lock-step.  X (d, n); Y_minus_mean (y_dim, n); prior_kind (y_dim, P) int, prior_par
+    (y_dim, P, 2) with P = d + 2 entries [lambda_1..lambda_d, alpha, sigma]; starts (y_dim, M, P) raw values.
+    -> params (y_dim, M, P), f (y_dim, M), best_params (y_dim, P), best_val (y_dim,), best_idx (y_dim,), evals."""
+    Xc = _cols(X)
+    n, d = Xc.shape
+    P = d + 2
+    Y = _f64(np.atleast_2d(Y_minus_mean))
+    y_dim = Y.shape[0]
+    assert Y.shape == (y_dim, n)
+    kind = np.ascontiguousarray(prior_kind, dtype=np.int32)
+    assert kind.shape == (y_dim, P), kind.shape
+    par = _f64(prior_par, (y_dim, P, 2))
+    st = _f64(starts)
+    assert st.ndim == 3 and st.shape[0] == y_dim and st.shape[2] == P, st.shape
+    M = st.shape[1]
+    dm = _opt(discrete_mask, np.uint8)
+    po = np.empty((y_dim, M, P)); fo = np.empty((y_dim, M)); bp = np.empty((y_dim, P))
+    bv = np.empty(y_dim); bi = np.empty(y_dim, dtype=np.int64)
+    ev = C.c_int()
+    _check(lib.boss_gp_map_multistart(_ptr(Xc), d, n, y_dim, _ptr(Y), int(kernel_id), _ptr(dm), _ptr(kind), _ptr(par),
+                                      _ptr(st), M, int(iters), int(history), _ptr(po), _ptr(fo), _ptr(bp), _ptr(bv),
+                                      _ptr(bi), C.byref(ev)), "boss_gp_map_multistart")
+    return po, fo, bp, bv, bi, ev.value
 
 
 def set_timing(on: bool):

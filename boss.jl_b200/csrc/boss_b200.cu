@@ -3249,13 +3249,15 @@ struct MeanJac {
 };
 
 // one batch inside the current context
+// internal: a call from inside another entry point on device inputs already ordered on the library stream (the
+// hyper-parameter driver, boss_gp_map_multistart): no caller-stream wait, and the call returns without synchronising
 static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t ldy, const double *ls,
                        const double *amp, const double *noise, KernelSpec ks, const uint8_t *discrete_mask, int64_t S,
                        double *loglik, bool dev, double *grad, boss_gp **fit_out, void *caller_stream,
-                       const MeanJac *mj = nullptr) {
+                       const MeanJac *mj = nullptr, bool internal = false) {
   const int dp = pick_dp(d), kernel_id = ks.kid;
   if (S == 0) return 0;
-  if (dev) {
+  if (dev && !internal) {
     int rc = wait_for_caller(caller_stream);
     if (rc) return rc;
   }
@@ -3338,7 +3340,7 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
   double *logdet_blk = misc + old_;
   int *status = reinterpret_cast<int *>(misc + ost);
 
-  timing_begin();
+  if (!internal) timing_begin();
   if (small) {
     SmallLoglikParams sp{};
     sp.X = dX;
@@ -3534,6 +3536,7 @@ static int loglik_core(const double *X, int d, int n, const double *Ymm, int64_t
   if (!dev && grad) CUDA_TRY(cudaMemcpyAsync(grad, dgrad, (size_t)S * (d + 2) * 8, cudaMemcpyDeviceToHost, C().stream));
   if (!dev && mj)
     CUDA_TRY(cudaMemcpyAsync(mj->grad_mean, dgm, (size_t)S * mj->k * 8, cudaMemcpyDeviceToHost, C().stream));
+  if (internal) return 0;
   CUDA_TRY(cudaStreamSynchronize(C().stream));
   timing_end();
   if (!dev) {
@@ -3666,6 +3669,248 @@ int boss_gp_loglik_grad_batch_dev(const double *X_dev, int d, int n, const doubl
   if (!grad_dev) return fail(BOSS_ERR_ARG, "boss_gp_loglik_grad_batch_dev: grad is NULL");
   return loglik_impl(X_dev, d, n, Y_minus_mean_dev, ldy, lengthscales_dev, amplitude_dev, noise_std_dev, kernel_id,
                      discrete_mask, S, loglik_dev, true, grad_dev, nullptr, stream);
+}
+
+// ---------------------------------------------------------------------------------------------
+// device-resident MAP fit of the hyper-parameters (OptimizationMAP, DESIGN.md 2.15)
+// ---------------------------------------------------------------------------------------------
+// The (slice, start) pairs [pair0, pair0 + Mloc) inside the current context: the acquisition driver's projected L-BFGS
+// state machine (multistart.cuh) at capacity MS_MAP_MAXD, every round's trial points evaluated by one internal
+// loglik_core call between map_prep_kernel and map_prior_kernel.  Returns each pair's final value and raw parameters
+// (raw_out [Mloc][P], as evaluated on the device) and the number of evaluations made.
+static int map_multistart_single(const double *X, int d, int n, int y_dim, const double *Y, KernelSpec ks,
+                                 const uint8_t *discrete_mask, const int32_t *kind, const double *par,
+                                 const double *starts_z, int64_t pair0, int64_t Mslice, int64_t Mloc, int iters,
+                                 int history, double *raw_out, double *f_out, long long *evals) {
+  const int P = d + 2;
+  const int H = std::max(1, std::min(history, MS_MAXH - 1));
+  const int RC = H + 1;
+  if (iters < 0) iters = 0;
+  const long long M = Mloc;
+  const size_t MP = (size_t)M * P, cap = (size_t)M;   // step-size fan 1: a round's batch holds at most M points
+  // one workspace: X g dirn | Sh Yh | f t | Xc gc fc | ls amp noise ybuf ll graw | X Y par | counters, per-start ints,
+  // idx, kinds
+  const size_t n_dbl = 3 * MP + 2 * (size_t)RC * MP + 2 * (size_t)M + 2 * cap * P + cap +
+                       cap * d + 2 * cap + cap * n + cap + cap * P + (size_t)n * d + (size_t)y_dim * n +
+                       (size_t)y_dim * P * 2;
+  CUDA_TRY(C().ms_buf.ensure(n_dbl * 8 + (size_t)M * 24 + cap * 4 + (size_t)y_dim * P * 4 + 64));
+  double *base = C().ms_buf.as<double>();
+  MsStateT<MS_MAP_MAXD> st{};
+  st.d = P;
+  st.H = RC;
+  st.iters = iters;
+  st.M = M;
+  st.X = base;
+  st.g = st.X + MP;
+  st.dirn = st.g + MP;
+  st.Sh = st.dirn + MP;
+  st.Yh = st.Sh + (size_t)RC * MP;
+  st.f = st.Yh + (size_t)RC * MP;
+  st.t = st.f + M;
+  st.Xc = st.t + M;
+  st.gc = st.Xc + cap * P;
+  st.fc = st.gc + cap * P;
+  double *ls = st.fc + cap, *amp = ls + cap * d, *noise = amp + cap, *ybuf = noise + cap, *ll = ybuf + cap * n,
+         *graw = ll + cap, *dX = graw + cap * P, *dY = dX + (size_t)n * d, *dpar = dY + (size_t)y_dim * n;
+  st.counters = reinterpret_cast<int *>(dpar + (size_t)y_dim * P * 2);
+  st.hist_len = st.counters + 4;
+  st.hist_start = st.hist_len + M;
+  st.trials = st.hist_start + M;
+  st.steps = st.trials + M;
+  st.state = st.steps + M;
+  st.nev = st.state + M;
+  st.idx = st.nev + M;      // [cap]
+  int *dkind = st.idx + cap;
+  st.fan = 1;
+  for (int j = 0; j < P; ++j) {
+    st.lb[j] = -30.0;
+    st.ub[j] = 30.0;
+  }
+  st.step0 = 0.1 * 60.0;
+  const unsigned nbm = (unsigned)((M + 127) / 128);
+
+  // X, the Y rows, the prior tables and the starts go to the device once per solve (pageable sources: synchronous
+  // staging, the workspace is idle here)
+  CUDA_TRY(cudaMemcpyAsync(dX, X, (size_t)n * d * 8, cudaMemcpyHostToDevice, C().stream));
+  CUDA_TRY(cudaMemcpyAsync(dY, Y, (size_t)y_dim * n * 8, cudaMemcpyHostToDevice, C().stream));
+  CUDA_TRY(cudaMemcpyAsync(dpar, par, (size_t)y_dim * P * 2 * 8, cudaMemcpyHostToDevice, C().stream));
+  CUDA_TRY(cudaMemcpyAsync(dkind, kind, (size_t)y_dim * P * 4, cudaMemcpyHostToDevice, C().stream));
+  CUDA_TRY(cudaMemcpyAsync(st.Xc, starts_z, MP * 8, cudaMemcpyHostToDevice, C().stream));
+  CUDA_TRY(cudaStreamSynchronize(C().stream));
+
+  long long evaluated = 0;
+  auto eval = [&](const double *Zp, const int *idxp, long long cnt, double *fp, double *gp) -> int {
+    MapEvalParams ep{};
+    ep.Z = Zp;
+    ep.idx = idxp;
+    ep.count = cnt;
+    ep.pair0 = pair0;
+    ep.M = Mslice;
+    ep.d = d;
+    ep.n = n;
+    ep.kind = dkind;
+    ep.par = dpar;
+    ep.Y = dY;
+    ep.ls = ls;
+    ep.amp = amp;
+    ep.noise = noise;
+    ep.ybuf = ybuf;
+    ep.ll = ll;
+    ep.graw = graw;
+    ep.f = fp;
+    ep.g = gp;
+    evaluated += cnt;
+    map_prep_kernel<<<(unsigned)cnt, 128, 0, C().stream>>>(ep);
+    ++C().launches;
+    int rc = loglik_core(dX, d, n, ybuf, n, ls, amp, noise, ks, discrete_mask, cnt, ll, true, graw, nullptr, nullptr,
+                         nullptr, true);
+    if (rc) return rc;
+    map_prior_kernel<<<(unsigned)((cnt + 127) / 128), 128, 0, C().stream>>>(ep);
+    ++C().launches;
+    return 0;
+  };
+
+  ms_init_kernel<<<nbm, 128, 0, C().stream>>>(st, st.Xc);
+  ++C().launches;
+  int rc = eval(st.X, nullptr, M, st.f, st.g);
+  if (rc) return rc;
+  const int max_rounds = iters > 0 ? 2 * iters + MS_MAX_TRIALS : 0;
+  st.budget = max_rounds;
+  int active = iters > 0 ? (int)M : 0;
+  const bool trace = getenv("BOSS_MS_TRACE") != nullptr;   // one line per round on stderr: round, batch size
+  CUDA_TRY(cudaMemsetAsync(st.counters, 0, 16, C().stream));
+  int hc[3] = {0, 0, 0};
+  int rounds = 0;
+  double t_prev = 0.0;
+  for (int round = 0; round < max_rounds && active > 0; ++round, ++rounds) {
+    if (trace) {
+      timespec ts;
+      clock_gettime(CLOCK_MONOTONIC, &ts);
+      const double t_now = ts.tv_sec * 1e6 + ts.tv_nsec * 1e-3;
+      fprintf(stderr, "boss map multistart: round %d active %d prev_round_us %.0f\n", round, active,
+              round ? t_now - t_prev : 0.0);
+      t_prev = t_now;
+    }
+    CUDA_TRY(cudaMemsetAsync(st.counters, 0, 8, C().stream));
+    ms_propose_kernel<<<nbm, 128, 0, C().stream>>>(st);
+    ++C().launches;
+    rc = eval(st.Xc, st.idx, active, st.fc, st.gc);
+    if (rc) return rc;
+    ms_advance_kernel<<<(active + 127) / 128, 128, 0, C().stream>>>(st, active);
+    ++C().launches;
+    CUDA_TRY(cudaMemcpyAsync(hc, st.counters, 12, cudaMemcpyDeviceToHost, C().stream));
+    CUDA_TRY(cudaStreamSynchronize(C().stream));
+    if (hc[0] != active) return fail(BOSS_ERR_STATE, "boss_gp_map_multistart: internal batch-length mismatch");
+    active = hc[1];
+  }
+  // raw values of the final points, exactly as the evaluations saw them
+  MapEvalParams ep{};
+  ep.Z = st.X;
+  ep.count = M;
+  ep.pair0 = pair0;
+  ep.M = Mslice;
+  ep.d = d;
+  ep.n = n;
+  ep.kind = dkind;
+  ep.par = dpar;
+  ep.ls = ls;
+  ep.amp = amp;
+  ep.noise = noise;
+  map_prep_kernel<<<(unsigned)M, 128, 0, C().stream>>>(ep);
+  ++C().launches;
+  CUDA_TRY(cudaGetLastError());
+  std::vector<double> hls((size_t)M * d), hamp(M), hnoise(M);
+  CUDA_TRY(cudaMemcpyAsync(hls.data(), ls, (size_t)M * d * 8, cudaMemcpyDeviceToHost, C().stream));
+  CUDA_TRY(cudaMemcpyAsync(hamp.data(), amp, (size_t)M * 8, cudaMemcpyDeviceToHost, C().stream));
+  CUDA_TRY(cudaMemcpyAsync(hnoise.data(), noise, (size_t)M * 8, cudaMemcpyDeviceToHost, C().stream));
+  CUDA_TRY(cudaMemcpyAsync(f_out, st.f, (size_t)M * 8, cudaMemcpyDeviceToHost, C().stream));
+  CUDA_TRY(cudaStreamSynchronize(C().stream));
+  for (long long m = 0; m < M; ++m) {
+    for (int j = 0; j < d; ++j) raw_out[m * P + j] = hls[m * d + j];
+    raw_out[m * P + d] = hamp[m];
+    raw_out[m * P + d + 1] = hnoise[m];
+  }
+  if (trace)
+    fprintf(stderr, "boss map multistart: rounds %d evaluations %lld (pairs %lld)\n", rounds, evaluated, M);
+  *evals = evaluated;
+  return 0;
+}
+
+int boss_gp_map_multistart(const double *X, int d, int n, int y_dim, const double *Y_minus_mean, int kernel_id,
+                           const uint8_t *discrete_mask, const int32_t *prior_kind, const double *prior_par,
+                           const double *starts, int64_t M, int iters, int history, double *params_out, double *f_out,
+                           double *best_params, double *best_val, int64_t *best_idx, int *evals_out) {
+  if (!X || !Y_minus_mean || !prior_kind || !prior_par || !starts || d < 1 || n < 1 || M < 1 || y_dim < 1 ||
+      y_dim > 16)
+    return fail(BOSS_ERR_ARG, "boss_gp_map_multistart: bad arguments");
+  if (d > 32) return fail(BOSS_ERR_ARG, "boss_gp_map_multistart: x_dim > 32 is not supported");
+  KernelSpec ks;
+  if (!decode_kernel(kernel_id, &ks)) return fail(BOSS_ERR_ARG, "boss_gp_map_multistart: unknown kernel_id");
+  const int P = d + 2;
+  const int64_t total = (int64_t)y_dim * M;
+  for (int e = 0; e < y_dim * P; ++e)
+    if (prior_kind[e] < 0 || prior_kind[e] > 3)
+      return fail(BOSS_ERR_ARG, "boss_gp_map_multistart: unknown prior kind");
+  // the search runs in z = log(raw) for the free entries; a pinned (Dirac) entry stays at z = 0
+  std::vector<double> z((size_t)total * P);
+  for (int64_t q = 0; q < total; ++q) {
+    const int sl = (int)(q / M);
+    for (int j = 0; j < P; ++j) {
+      const double v = starts[(size_t)q * P + j];
+      if (prior_kind[sl * P + j] == 0) {
+        z[(size_t)q * P + j] = 0.0;
+        continue;
+      }
+      if (!(std::isfinite(v) && v > 0.0))
+        return fail(BOSS_ERR_ARG, "boss_gp_map_multistart: a free start entry is not finite and > 0");
+      z[(size_t)q * P + j] = std::log(v);
+    }
+  }
+  std::vector<double> raw((size_t)total * P), f((size_t)total);
+  // multi-device: contiguous ranges of (slice, start) pairs; a pair's trajectory does not depend on the others
+  const int nd = (g_ndev > 1 && tl_dev < 0 && total >= 2LL * g_ndev) ? g_ndev : 1;
+  std::vector<long long> ev(nd, 0);
+  int rc;
+  if (nd <= 1) {
+    REQUIRE_INIT();
+    rc = map_multistart_single(X, d, n, y_dim, Y_minus_mean, ks, discrete_mask, prior_kind, prior_par, z.data(), 0, M,
+                               total, iters, history, raw.data(), f.data(), &ev[0]);
+  } else {
+    const int64_t per = (total + nd - 1) / nd;
+    rc = for_each_device(nd, [&](int k, Ctx *) {
+      const int64_t first = std::min<int64_t>(total, (int64_t)k * per), cnt = std::min<int64_t>(per, total - first);
+      if (cnt <= 0) return 0;
+      return map_multistart_single(X, d, n, y_dim, Y_minus_mean, ks, discrete_mask, prior_kind, prior_par,
+                                   z.data() + (size_t)first * P, first, M, cnt, iters, history,
+                                   raw.data() + (size_t)first * P, f.data() + first, &ev[k]);
+    });
+  }
+  if (rc) return rc;
+  // per slice: Julia's first maximal index over the starts; -1 / -Inf when every start failed
+  for (int i = 0; i < y_dim; ++i) {
+    double bv = -std::numeric_limits<double>::infinity();
+    int64_t bi = -1;
+    for (int64_t s = 0; s < M; ++s) {
+      const double v = f[(size_t)i * M + s];
+      if (v > bv) {
+        bv = v;
+        bi = s;
+      }
+    }
+    if (best_val) best_val[i] = bv;
+    if (best_idx) best_idx[i] = bi;
+    if (best_params)
+      for (int j = 0; j < P; ++j)
+        best_params[(size_t)i * P + j] = bi >= 0 ? raw[((size_t)i * M + bi) * P + j] : std::nan("");
+  }
+  if (params_out) std::memcpy(params_out, raw.data(), raw.size() * 8);
+  if (f_out) std::memcpy(f_out, f.data(), f.size() * 8);
+  if (evals_out) {
+    long long tot = 0;
+    for (long long e : ev) tot += e;
+    *evals_out = (int)((tot + total - 1) / total);
+  }
+  return 0;
 }
 
 static int check_mean_jac(const char *who, int n, const double *grad, const double *mean_jac, int k, int64_t ldj,

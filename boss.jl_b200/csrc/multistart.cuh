@@ -13,15 +13,21 @@
 // ring, step counter and termination are per start - so a start's trajectory does not depend on which other
 // starts are in the batch, and therefore not on how the starts are sharded over GPUs.
 #pragma once
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace boss {
 
-constexpr int MS_MAXD = 32;
+constexpr int MS_MAXD = 32;            // acquisition driver: x_dim <= 32
+constexpr int MS_MAP_MAXD = 34;        // hyper-parameter driver (boss_gp_map_multistart): d + 2 <= 34 entries
 constexpr int MS_MAXH = 16;
 constexpr int MS_MAX_TRIALS = 12;     // step sizes 1, 1/2, ..., 2^-11 per line search
 
-struct MsState {
+// MAXD: the dimension capacity (per-thread arrays of the two-loop recursion, the box); a driver instantiates the
+// kernels below at its own capacity
+template <int MAXD>
+struct MsStateT {
   int d, H, iters;           // H = ring capacity; iters = accepted steps after which a start is finished
   long long M;
   double *X, *f, *g;         // [M][d], [M], [M][d]  current (accepted) point, value, gradient
@@ -34,15 +40,17 @@ struct MsState {
   int *state;                // [M] 0 = needs a direction, 1 = in a line search, 2 = finished
   int *idx;                  // [cap] compact list: idx[slot] = start
   int fan;                   // trial points per unfinished start in this round (speculative step-size fan, see below)
-  double lb[MS_MAXD], ub[MS_MAXD];
+  double lb[MAXD], ub[MAXD];
   double step0;
   int *counters;             // [0] length of this round's compact list, [1] starts still unfinished after the round,
                              // [2] running total of the evaluations a one-trial-per-round search would have made
 };
+using MsState = MsStateT<MS_MAXD>;
 
 __device__ __forceinline__ double ms_clip(double v, double lo, double hi) { return v < lo ? lo : (v > hi ? hi : v); }
 
-__global__ void ms_init_kernel(MsState st, const double *starts) {
+template <int MAXD>
+__global__ void ms_init_kernel(MsStateT<MAXD> st, const double *starts) {
   const long long m = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (m >= st.M) return;
   for (int j = 0; j < st.d; ++j) st.X[m * st.d + j] = ms_clip(starts[m * st.d + j], st.lb[j], st.ub[j]);
@@ -63,19 +71,21 @@ __global__ void ms_sanitize_kernel(double *f, long long M) {
 // trials are examined in order and the first acceptable one wins, so the trajectory is exactly the sequential one.
 // A start that has just accepted a step (or has not moved yet) first gets its L-BFGS ascent direction from its own
 // history (two-loop recursion).
-__global__ void ms_propose_kernel(MsState st) {
+template <int MAXD>
+__global__ void ms_propose_kernel(MsStateT<MAXD> st) {
   const long long m = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (m >= st.M || st.state[m] == 2) return;
   const int d = st.d;
   if (st.state[m] == 0) {
     const int hist_len = st.hist_len[m], hist_start = st.hist_start[m];
-    double q[MS_MAXD], gl[MS_MAXD], al[MS_MAXH], rh[MS_MAXH];
+    double q[MAXD], gl[MAXD], al[MS_MAXH], rh[MS_MAXH];
     double gnorm2 = 0.0;
-    unsigned bound = 0;   // coordinates that sit on a bound with the gradient pointing out of the box
+    using Mask = typename std::conditional<(MAXD > 32), unsigned long long, unsigned>::type;
+    Mask bound = 0;   // coordinates that sit on a bound with the gradient pointing out of the box
     for (int j = 0; j < d; ++j) {
       const double x = st.X[m * d + j], gj = st.g[m * d + j];
       const bool out = (x <= st.lb[j] && gj < 0.0) || (x >= st.ub[j] && gj > 0.0);
-      bound |= out ? (1u << j) : 0u;
+      bound |= out ? (Mask(1) << j) : Mask(0);
       gl[j] = out ? 0.0 : gj;            // projected gradient
       q[j] = gl[j];
       gnorm2 = fma(gl[j], gl[j], gnorm2);
@@ -114,7 +124,7 @@ __global__ void ms_propose_kernel(MsState st) {
     }
     double dg = 0.0;
     for (int j = 0; j < d; ++j) {
-      if ((bound >> j) & 1u) q[j] = 0.0;             // stay on the active bounds
+      if ((bound >> j) & Mask(1)) q[j] = 0.0;             // stay on the active bounds
       dg = fma(q[j], gl[j], dg);
     }
     const bool bad = !(dg > 0.0);                    // not an ascent direction -> steepest ascent
@@ -136,7 +146,8 @@ __global__ void ms_propose_kernel(MsState st) {
 // step; finished after `iters` steps or when the step no longer moves the point.  Rejected: halve the step; after
 // MS_MAX_TRIALS step sizes the history is dropped and the search restarts along the projected gradient, and a start
 // whose projected-gradient search fails as well is finished (no acceptable step exists any more).
-__global__ void ms_advance_kernel(MsState st, int count) {
+template <int MAXD>
+__global__ void ms_advance_kernel(MsStateT<MAXD> st, int count) {
   const int grp = blockIdx.x * blockDim.x + threadIdx.x;   // one thread per start of the round = per group of `fan` slots
   if (grp >= count) return;
   const long long m = st.idx[grp * st.fan];
@@ -220,6 +231,84 @@ __global__ void ms_round_kernel(double *X, long long M, int d, unsigned long lon
   const long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (e >= M * d) return;
   if ((disc_bits >> (e % d)) & 1ull) X[e] = rint(X[e]);
+}
+
+// ---- hyper-parameter fit (boss_gp_map_multistart, DESIGN.md 2.15) -------------------------------------------------
+// A start is one (output slice, start) pair; its P = d + 2 entries [lambda_1..lambda_d, alpha, sigma] are searched in
+// z = log(raw).  Prior kinds per entry: 0 Dirac(v) (pinned: raw = v, z stays 0), 1 Normal(mu, s), 2 LogNormal(mu, s),
+// 3 Uniform(lo, hi) (inclusive), with the log-densities of boss.jl_b200/types.py.
+struct MapEvalParams {
+  const double *Z;          // [count][P] points of this batch in z
+  const int *idx;           // slot -> local start (the round's compact list), or null: slot k is start k
+  long long count;          // slots in the batch
+  long long pair0;          // global (slice, start) index of local start 0: slice = (pair0 + start) / M
+  long long M;              // starts per slice
+  int d, n;
+  const int *kind;          // [y_dim][P]
+  const double *par;        // [y_dim][P][2]
+  const double *Y;          // [y_dim][n] data minus prior mean
+  double *ls, *amp, *noise; // [count][d], [count], [count] raw hyper-parameters of the slots
+  double *ybuf;             // [count][n] the slot's slice row of Y (null: not gathered)
+  const double *ll, *graw;  // log-likelihood and its raw gradient of the slots ([count], [count][P])
+  double *f, *g;            // [count], [count][P] value and z-gradient of the slots
+};
+
+// one block per slot: raw hyper-parameters (exp(z), or the pinned value) and the slot's Y row
+__global__ void map_prep_kernel(MapEvalParams p) {
+  const long long k = blockIdx.x;
+  const long long m = p.idx ? p.idx[k] : k;
+  const int sl = (int)((p.pair0 + m) / p.M), P = p.d + 2;
+  for (int j = threadIdx.x; j < P; j += blockDim.x) {
+    const int e = sl * P + j;
+    const double raw = p.kind[e] == 0 ? p.par[2 * e] : exp(p.Z[k * P + j]);
+    if (j < p.d)
+      p.ls[k * p.d + j] = raw;
+    else if (j == p.d)
+      p.amp[k] = raw;
+    else
+      p.noise[k] = raw;
+  }
+  if (p.ybuf)
+    for (int i = threadIdx.x; i < p.n; i += blockDim.x) p.ybuf[k * p.n + i] = p.Y[(size_t)sl * p.n + i];
+}
+
+// one thread per slot: value = log-likelihood + log-prior at the raw values, gradient in z = raw * dll/draw +
+// dlogprior/dz (0 for a pinned entry); a non-finite value (K not positive definite, a Uniform support left) is -Inf
+// with a zero gradient
+__global__ void map_prior_kernel(MapEvalParams p) {
+  const long long k = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (k >= p.count) return;
+  const long long m = p.idx ? p.idx[k] : k;
+  const int sl = (int)((p.pair0 + m) / p.M), P = p.d + 2;
+  const double ln_sqrt2pi = 0.91893853320467274178;   // log(sqrt(2 pi))
+  double v = p.ll[k];
+  for (int j = 0; j < P; ++j) {
+    const int e = sl * P + j, kind = p.kind[e];
+    double dz = 0.0;
+    if (kind != 0) {
+      const double x = j < p.d ? p.ls[k * p.d + j] : j == p.d ? p.amp[k] : p.noise[k];
+      const double a = p.par[2 * e], b = p.par[2 * e + 1];
+      double lp = 0.0, dlp = 0.0;
+      if (kind == 1) {          // Normal: -r^2/2 - log(s sqrt(2 pi)), r = (x - mu)/s;  d/dz = x d/dx
+        const double r = (x - a) / b;
+        lp = -0.5 * r * r - (log(b) + ln_sqrt2pi);
+        dlp = -r / b * x;
+      } else if (kind == 2) {   // LogNormal: -r^2/2 - log(x s sqrt(2 pi)), r = (log x - mu)/s
+        const double r = (log(x) - a) / b;
+        lp = -0.5 * r * r - log(x * b * 2.50662827463100050242);
+        dlp = -r / b - 1.0;
+      } else {                  // Uniform(lo, hi), inclusive
+        lp = (a <= x && x <= b) ? -log(b - a) : -INFINITY;
+      }
+      v += lp;
+      dz = fma(x, p.graw[k * P + j], dlp);
+    }
+    p.g[k * P + j] = dz;
+  }
+  const bool ok = isfinite(v);
+  p.f[k] = ok ? v : -INFINITY;
+  if (!ok)
+    for (int j = 0; j < P; ++j) p.g[k * P + j] = 0.0;
 }
 
 }  // namespace boss

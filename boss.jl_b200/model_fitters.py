@@ -7,6 +7,7 @@ import numpy as np
 
 from .gaussian_process import (GaussianProcessParams, Semiparametric, SemiparametricParams, data_loglike,
                                data_loglike_and_grad)
+from . import _lib
 from .types import BossOptions, BossProblem, MAPParams
 
 
@@ -28,7 +29,11 @@ class OptimizationMAP:
                  GaussianProcess models, and Semiparametric models whose Parametric has a `jacobian` (theta enters raw,
                  its gradient from boss_gp_loglik_grad_batch_mean); a Semiparametric model without one falls back to
                  "compass".
-      "compass"  derivative-free compass search in log space (what NEWUOA / BOBYQA are used for in the examples)."""
+      "compass"  derivative-free compass search in log space (what NEWUOA / BOBYQA are used for in the examples).
+      "device"   the whole multi-start L-BFGS on the device (boss_gp_map_multistart): each output slice fitted on its
+                 own as the reference does for sliceable models (optimization.jl:76-84), the log-prior and its gradient
+                 evaluated there too.  GaussianProcess models whose priors are Dirac / Normal / LogNormal / Uniform
+                 (a lengthscale Product decomposes into its parts); any other model or prior runs "lbfgs" unchanged."""
 
     def __init__(self, multistart=20, iters: int = 40, step0: float = 0.5, seed: Optional[int] = None,
                  algorithm: str = "lbfgs"):
@@ -139,6 +144,10 @@ def estimate_parameters(fitter, problem: BossProblem, options: BossOptions = Bos
         return estimate_parameters(om, problem, options, return_all=return_all)
     if isinstance(fitter, OptimizationMAP):
         starts = list(fitter.multistart) if not isinstance(fitter.multistart, int) else [sampler() for _ in range(fitter.multistart)]
+        if fitter.algorithm == "device":
+            tables = gp_prior_tables(model, data.x_dim, data.y_dim)
+            if tables is not None:
+                return _device_map(fitter, model, data, starts, tables, return_all)
         tmpl = starts[0]
         fixed = _dirac_mask(model, tmpl)
         V0 = np.stack([_vectorize(p) for p in starts])             # S x P_all
@@ -163,7 +172,8 @@ def estimate_parameters(fitter, problem: BossProblem, options: BossOptions = Bos
             b = int(np.argmax(f0))
             return MAPParams(starts[b], float(f0[b]))
         _devectorize_rows = lambda rows, owners: [_devec_free(o, v) for v, o in zip(rows, owners)]
-        if fitter.algorithm == "lbfgs" and (not isinstance(model, Semiparametric) or model.parametric.jacobian is not None):
+        if fitter.algorithm in ("lbfgs", "device") and (not isinstance(model, Semiparametric) or
+                                                        model.parametric.jacobian is not None):
             lo, hi = _search_box(model, V0)
             return _lbfgs_map(fitter, model, data, V, free, tmpl, _devec_free, return_all, lo[free], hi[free])
         f = ll(_devectorize_rows(V, range(S)))
@@ -265,3 +275,71 @@ def _lbfgs_map(fitter, model, data, V, free, tmpl, devec_free, return_all, lo, h
         return [MAPParams(devec_free(i, X[:, i]), float(f[i])) for i in range(S) if np.isfinite(f[i])]
     b = int(np.argmax(f))
     return MAPParams(devec_free(b, X[:, b]), float(f[b]))
+
+
+def _prior_entry(pr):
+    """One prior -> (kind, (p0, p1)) of boss_gp_map_multistart's tables, or None for a prior the device lacks."""
+    from .types import Dirac, LogNormal, Normal, Uniform
+    if isinstance(pr, Dirac):
+        return 0, (float(pr.value), 0.0)
+    if isinstance(pr, Normal):
+        return 1, (float(pr.mu), float(pr.sigma))
+    if isinstance(pr, LogNormal):
+        return 2, (float(pr.mu), float(pr.sigma))
+    if isinstance(pr, Uniform):
+        return 3, (float(pr.lo), float(pr.hi))
+    return None
+
+
+def gp_prior_tables(model, d, y_dim):
+    """A GaussianProcess's priors as boss_gp_map_multistart's tables: kind (y_dim, d + 2) int32 and par (y_dim, d + 2, 2),
+    entries [lambda_1..lambda_d, alpha, sigma] per slice.  A lengthscale Product decomposes into its d parts (a single
+    univariate prior stands for the one lengthscale when d == 1).  None when the model is not a GaussianProcess or a
+    prior is not one of Dirac, Normal, LogNormal, Uniform: the caller then runs the host fitter."""
+    from .gaussian_process import GaussianProcess
+    from .types import Product
+    if not isinstance(model, GaussianProcess):
+        return None
+    kind = np.zeros((y_dim, d + 2), dtype=np.int32)
+    par = np.zeros((y_dim, d + 2, 2))
+    for i in range(y_dim):
+        lp = model.lengthscale_priors[i]
+        parts = list(lp.parts) if isinstance(lp, Product) else ([lp] if d == 1 else None)
+        if parts is None or len(parts) != d:
+            return None
+        for j, pr in enumerate(parts + [model.amplitude_priors[i], model.noise_std_priors[i]]):
+            e = _prior_entry(pr)
+            if e is None:
+                return None
+            kind[i, j], par[i, j] = e
+    return kind, par
+
+
+def _device_map(fitter, model, data, starts, tables, return_all):
+    """OptimizationMAP(algorithm="device"): one boss_gp_map_multistart call.  Start s of slice i is starts[s]'s slice-i
+    component; the result combines every slice's best point, its loglike the sum of the slices' best values (= the model
+    log-likelihood at those parameters).  return_all: entry s combines start s of every slice (failed ones dropped)."""
+    from .gaussian_process import _kernel_parts
+    kind, par = tables
+    d, y_dim = data.x_dim, data.y_dim
+    S = len(starts)
+    st = np.empty((y_dim, S, d + 2))
+    for s, p in enumerate(starts):
+        st[:, s, :d] = np.asarray(p.lengthscales, dtype=np.float64).T
+        st[:, s, d] = p.amplitudes
+        st[:, s, d + 1] = p.noise_std
+    Ymm = np.empty((y_dim, data.X.shape[1]))
+    for i in range(y_dim):
+        m = model.mean_at(i, data.X)
+        Ymm[i] = data.Y[i] if m is None else data.Y[i] - m
+    kid, mask = _kernel_parts(model.kernel)
+    po, fo, bp, bv, bi, _ = _lib.gp_map_multistart(data.X, Ymm, kind, par, st, kid, mask, iters=fitter.iters)
+    if np.any(bi < 0):
+        raise RuntimeError("All optimization runs failed!")                          # optim_multistart.jl:34
+
+    def params_of(rows):                                                            # (y_dim, d + 2) -> params
+        return GaussianProcessParams(rows[:, :d].T.copy(), rows[:, d].copy(), rows[:, d + 1].copy())
+    if return_all:
+        tot = fo.sum(axis=0)
+        return [MAPParams(params_of(po[:, s]), float(tot[s])) for s in range(S) if np.isfinite(tot[s])]
+    return MAPParams(params_of(bp), float(bv.sum()))

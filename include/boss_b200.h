@@ -365,6 +365,34 @@ int boss_gp_loglik_grad_batch_mean_dev(const double *X_dev, int d, int n, const 
                                        int64_t S, double *loglik_dev, double *grad_dev, double *grad_mean_dev,
                                        void *stream);
 
+/* OptimizationMAP (src/model_fitters/optimization.jl:75-164) for a GaussianProcess, every output slice fitted on its
+ * own as the reference does for sliceable models (:76-84), all M starts of all slices advancing in lock-step on the
+ * device (projected L-BFGS + Armijo, the state machine of boss_ei_maximize_multistart, one trial point per start and
+ * round).  Every round is one batched log-likelihood + gradient pass over the unfinished (slice, start) pairs; the
+ * points, values and gradients stay in HBM, X and Y go to the device once per call (DESIGN.md 2.15).
+ *   X             d x n;  Y_minus_mean  n per slice, slice i at Y_minus_mean + i*n;  1 <= y_dim <= 16, d <= 32
+ *   entries       P = d + 2 per slice: [lambda_1..lambda_d, alpha, sigma] (boss_gp_loglik_grad_batch's gradient order),
+ *                 raw values as the other entry points take them (the library adds MIN_PARAM_VALUE)
+ *   prior_kind    [y_dim][P]: 0 Dirac(v) pinned (raw value exactly v everywhere, log-prior 0, its start is ignored),
+ *                 1 Normal(mu, s), 2 LogNormal(mu, s), 3 Uniform(lo, hi) inclusive (-Inf outside: the trial is
+ *                 rejected); any other kind is BOSS_ERR_ARG.  prior_par [y_dim][P][2] = (v, -), (mu, s), (mu, s), (lo, hi)
+ *   starts, params_out  [y_dim][M][P] raw;  f_out [y_dim][M];  best_params [y_dim][P];  best_val, best_idx [y_dim]
+ *                 (any output may be NULL).  A free start entry must be finite and > 0 (BOSS_ERR_ARG otherwise).
+ * Search space: z = log(raw) for every free entry inside the box [-30, 30] (boss.jl_b200's _vectorize and _search_box);
+ * a pinned entry keeps z = 0 and gradient 0.  The reference's Bijectors use other maps (the identity for a Normal
+ * prior, for instance), so trajectories differ from Optim's; the objective is the same.
+ * Value of a pair: the slice's data log-likelihood plus its log-prior at the raw values (no Jacobian of the map);
+ * gradient in z: raw * dll/draw + dlogprior/dz, analytic on the device.  K not positive definite or a non-finite value:
+ * -Inf (SafeFunction).  best_idx[i]: first maximal start of slice i; -1 with best_val = -Inf (best_params NaN) when
+ * every start of the slice failed -- the call still returns 0 and the caller raises "All optimization runs failed!"
+ * (optim_multistart.jl:34).  evals_out: evaluations made / (y_dim M), rounded up.
+ * A pair's trajectory does not depend on the other pairs: under boss_init_multi contiguous ranges of pairs go to the
+ * devices and the result is bit-identical to the single-device call.  BOSS_MS_TRACE=1 traces the rounds on stderr. */
+int boss_gp_map_multistart(const double *X, int d, int n, int y_dim, const double *Y_minus_mean, int kernel_id,
+                           const uint8_t *discrete_mask, const int32_t *prior_kind, const double *prior_par,
+                           const double *starts, int64_t M, int iters, int history, double *params_out, double *f_out,
+                           double *best_params, double *best_val, int64_t *best_idx, int *evals_out);
+
 /* ---- instrumentation ---------------------------------------------------------------------
  * CUDA-event time (ms) of the dominant kernel class inside the last scoring / loglik call, and the
  * number of kernel launches the library has issued since boss_init (bench.py's gpu_launches). */

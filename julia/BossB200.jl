@@ -31,18 +31,22 @@
 #     (Semiparametric: θ through ForwardDiff.jacobian of the parametric mean)             -> boss_gp_loglik_grad_batch_mean
 #   acq(x::Vector{<:ForwardDiff.Dual})    (acquisition_maximizers/optimization.jl:36)   -> boss_ei_value_grad /
 #                                                                                          boss_mcei_value_grad
+#   estimate_parameters(::OptimizationMAP) (model_fitters/optimization.jl:75-164)        -> boss_gp_map_multistart
+#   estimate_parameters(::SampleOptMAP)    (model_fitters/sample_opt.jl:37-48)          -> SamplingMAP batch + the above
 module BossB200
 
 using BOSS
 using BOSS: GaussianProcess, GaussianProcessParams, Semiparametric, SemiparametricParams, ExperimentData,
             ModelPosteriorSlice, DefaultModelPosterior, BossProblem, BossOptions, AcquisitionMaximizer, ModelFitter,
-            GridAM, SamplingAM, OptimizationAM, SampleOptAM, SequentialBatchAM, SamplingMAP, ExpectedImprovement,
+            GridAM, SamplingAM, OptimizationAM, SampleOptAM, SequentialBatchAM, SamplingMAP, OptimizationMAP,
+            SampleOptMAP, ExpectedImprovement,
             LinFitness, NonlinFitness, MAPParams, BIParams, Infinity, mean_getindex, best_so_far, get_params, y_dim
 using KernelFunctions: SqExponentialKernel, Matern32Kernel, Matern52Kernel, ExponentialKernel, RationalQuadraticKernel
 using Distances: Euclidean
 using LinearAlgebra: diag, PosDefException
 using Random: shuffle
 using ForwardDiff
+import Distributions
 import Statistics: mean, var, cov
 import StatsBase: mean_and_var, mean_and_cov
 
@@ -583,6 +587,92 @@ function BOSS.estimate_parameters(f::B200Fitter{<:SamplingMAP}, problem::BossPro
     return_all && return [MAPParams(p, l) for (p, l) in zip(ps, lls)]
     b = argmax(lls)                                           # first maximum == the reference's strict `v > best_v`
     return MAPParams(ps[b], lls[b])
+end
+# ---- OptimizationMAP / SampleOptMAP on the device (boss_gp_map_multistart, DESIGN.md 2.15) ---------------------------
+# One prior -> (kind, p0, p1) of the C tables, or nothing for a prior the device lacks
+prior_entry(p::Distributions.Dirac) = (0, Float64(p.value), 0.0)
+prior_entry(p::Distributions.Normal) = (1, Float64(p.μ), Float64(p.σ))
+prior_entry(p::Distributions.LogNormal) = (2, Float64(p.μ), Float64(p.σ))
+prior_entry(p::Distributions.Uniform) = (3, Float64(p.a), Float64(p.b))
+prior_entry(p) = nothing
+# the univariate parts of a lengthscale prior (product_distribution of independent components), or nothing
+prior_parts(p::Distributions.Product, d) = length(p.v) == d ? collect(p.v) : nothing
+prior_parts(p::Distributions.UnivariateDistribution, d) = d == 1 ? [p] : nothing
+prior_parts(p, d) = (hasproperty(p, :dists) && length(p.dists) == d) ? collect(p.dists) : nothing
+
+"(kind (d+2) × y_dim Int32, par 2 × (d+2) × y_dim) of a GaussianProcess, or nothing when a prior does not decompose into
+Dirac / Normal / LogNormal / Uniform entries."
+function map_prior_tables(model::GaussianProcess, d::Int, yd::Int)
+    kind = zeros(Int32, d + 2, yd); par = zeros(2, d + 2, yd)
+    for i in 1:yd
+        parts = prior_parts(model.lengthscale_priors[i], d)
+        isnothing(parts) && return nothing
+        for (j, p) in enumerate(vcat(parts, [model.amplitude_priors[i], model.noise_std_priors[i]]))
+            e = prior_entry(p)
+            isnothing(e) && return nothing
+            kind[j, i] = e[1]; par[1, j, i] = e[2]; par[2, j, i] = e[3]
+        end
+    end
+    return kind, par
+end
+
+"All starts of all output slices in one boss_gp_map_multistart call; start s of slice i is ps[s]'s slice-i part.
+The search runs in log(raw) inside [-30, 30] (not the reference's Bijectors), every slice on its own
+(optimization.jl:76-84).  Returns the combined best params and their model log-likelihood (return_all: per start s)."
+function map_multistart(model::GaussianProcess, data::ExperimentData, tables, ps, iters::Int; return_all::Bool=false)
+    kind, par = tables
+    X = Matrix{Float64}(data.X)
+    d, n = size(X)
+    yd = y_dim(data); M = length(ps); P = d + 2
+    Y = Matrix{Float64}(undef, n, yd)
+    for i in 1:yd
+        mX = eval_mean(mean_getindex(model.mean, i), X)
+        Y[:, i] .= isnothing(mX) ? data.Y[i, :] : data.Y[i, :] .- mX
+    end
+    S = Array{Float64}(undef, P, M, yd)                   # C layout [y_dim][M][P]
+    for (s, p) in enumerate(ps), i in 1:yd
+        S[1:d, s, i] .= p.λ[:, i]; S[d + 1, s, i] = p.α[i]; S[d + 2, s, i] = p.σ[i]
+    end
+    mask = discrete_mask(model.kernel)
+    po = Array{Float64}(undef, P, M, yd); fo = Matrix{Float64}(undef, M, yd); bp = Matrix{Float64}(undef, P, yd)
+    bv = Vector{Float64}(undef, yd); bi = Vector{Int64}(undef, yd); ev = Ref{Cint}(0)
+    GC.@preserve X Y kind par S mask po fo bp bv bi check(ccall((:boss_gp_map_multistart, LIB), Cint,
+        (Ptr{Cdouble}, Cint, Cint, Cint, Ptr{Cdouble}, Cint, Ptr{UInt8}, Ptr{Int32}, Ptr{Cdouble}, Ptr{Cdouble}, Int64, Cint,
+         Cint, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Int64}, Ref{Cint}),
+        X, d, n, yd, Y, kernel_id(model.kernel), cptr(mask), kind, par, S, M, iters, 8, po, fo, bp, bv, bi, ev))
+    any(<(0), bi) && error("All optimization runs failed!")              # optim_multistart.jl:34
+    mk(rows) = GaussianProcessParams(rows[1:d, :], rows[d + 1, :], rows[d + 2, :])
+    if return_all
+        tot = vec(sum(fo; dims=2))
+        return [MAPParams(mk(po[:, s, :]), tot[s]) for s in 1:M if isfinite(tot[s])]
+    end
+    return MAPParams(mk(bp), sum(bv))
+end
+
+map_tables(problem) = problem.model isa GaussianProcess && supported(problem.model) ?
+    map_prior_tables(problem.model, size(problem.data.X, 1), y_dim(problem.data)) : nothing
+
+# OptimizationMAP (optimization.jl:75-164): starts from the model's params_sampler as optimization.jl:116,131-141 draws
+# them; models or priors the device lacks run the stock method.  Reviewed, not run (no Julia installation was available).
+function BOSS.estimate_parameters(f::B200Fitter{<:OptimizationMAP}, problem::BossProblem, options::BossOptions;
+                                  return_all::Bool=false)
+    tables = map_tables(problem)
+    isnothing(tables) && return BOSS.estimate_parameters(f.inner, problem, options; return_all)
+    sampler = BOSS.params_sampler(problem.model, problem.data)
+    ps = [sampler() for _ in 1:f.inner.multistart]
+    iters = get(f.inner.kwargs, :iterations, 40)
+    return map_multistart(problem.model, problem.data, tables, ps, iters; return_all)
+end
+# SampleOptMAP (sample_opt.jl:37-48): the SamplingMAP batch on the device, its `multistart` best samples as the starts
+function BOSS.estimate_parameters(f::B200Fitter{<:SampleOptMAP}, problem::BossProblem, options::BossOptions;
+                                  return_all::Bool=false)
+    tables = map_tables(problem)
+    isnothing(tables) && return BOSS.estimate_parameters(f.inner, problem, options; return_all)
+    all_ = BOSS.estimate_parameters(B200Fitter(f.inner.sampler), problem, options; return_all=true)
+    order = sortperm([p.loglike for p in all_]; rev=true)[1:f.inner.optimizer.multistart]
+    ps = [all_[k].params for k in order]
+    iters = get(f.inner.optimizer.kwargs, :iterations, 40)
+    return map_multistart(problem.model, problem.data, tables, ps, iters; return_all)
 end
 # every other fitter runs its own BOSS.jl method (the accelerated batch API above is available to custom fitters)
 BOSS.estimate_parameters(f::B200Fitter, problem::BossProblem, options::BossOptions; kwargs...) =
