@@ -189,28 +189,37 @@ __device__ __forceinline__ double kappa(double d2, double rq_a) {
   }
 }
 
-// FP32 kappa for the FP32 mean tier of argmax screening (DESIGN.md 2.9): one MUFU.RSQ (Matern only) and one MUFU.EX2.
-// r = d2 rsqrt(max(d2, 1e-30)) is 0 at d2 = 0 (|r~ - r| <= 1e-15 below the floor); t >= ~87 flushes exp to 0.
-// Absolute error against kappa at the same d2, measured over r in [0, 40]: tests/test_gpu_screen_f32.py.
-template <int KID>
-__device__ __forceinline__ float kappa_f32(float d2) {
+// The FP32 mean tier of argmax screening (DESIGN.md 2.9) evaluates kappa two lanes at a time with the packed FP32
+// instructions of sm_100 (FADD2 / FMUL2 / FFMA2: one issue slot for two results).
+__device__ __forceinline__ float2 f2(float a) { return make_float2(a, a); }
+__device__ __forceinline__ float ex2_mufu(float x) {
   float e;
-  if (KID == 0) {
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(d2 * -0.72134752044448170f /* -log2(e)/2 */));
-    return e;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(x));
+  return e;
+}
+
+// FP32 kappa of two squared distances d2 >= 1e-30 (the tier clamps d2 at 1e-30 once, which is also the rsqrt's
+// floor: r~ = d2 rsqrt(d2) is below 1e-15 there): one MUFU.RSQ (Matern only) and one MUFU.EX2 per lane, the rest
+// packed.  exp(-t) flushes to 0 for t >= ~87.  Absolute error against kappa at the same d2, measured over r in
+// [0, 40]: tests/test_gpu_screen_f32.py.
+template <int KID>
+__device__ __forceinline__ float2 kappa_f32x2(float2 d2) {
+  constexpr float C = KID == 0 ? -0.72134752044448170f    /* -log2(e)/2 */
+                    : KID == 1 ? -2.4988211106473432f     /* -sqrt3 log2(e) */
+                               : -3.2259641822295610f;    /* -sqrt5 log2(e) */
+  float2 r = d2;   // SE: the exponent is C d2
+  if (KID != 0) {
+    float y0, y1;
+    asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(y0) : "f"(d2.x));
+    asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(y1) : "f"(d2.y));
+    r = __fmul2_rn(d2, make_float2(y0, y1));
   }
-  float y;
-  asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(fmaxf(d2, 1e-30f)));
-  const float r = d2 * y;
-  if (KID == 1) {
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(r * -2.4988211106473432f /* -sqrt3 log2(e) */));
-    const float t = 1.7320508075688772f * r;
-    return fmaf(t, e, e);
-  } else {
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(r * -3.2259641822295610f /* -sqrt5 log2(e) */));
-    const float t = 2.2360679774997896f * r;
-    return fmaf(fmaf(1.6666666666666667f, d2, t), e, e);
-  }
+  const float2 x = __fmul2_rn(r, f2(C));
+  const float2 e = make_float2(ex2_mufu(x.x), ex2_mufu(x.y));
+  if (KID == 0) return e;
+  if (KID == 1) return __ffma2_rn(__fmul2_rn(f2(1.7320508075688772f), r), e, e);
+  const float2 t = __fmul2_rn(f2(2.2360679774997896f), r);
+  return __ffma2_rn(__ffma2_rn(f2(1.6666666666666667f), d2, t), e, e);
 }
 
 // x = hi + lo + r with hi, lo TF32 (round to nearest, ties away): |x - hi| <= 2^-11 |x|, |r| <= 2^-22 |x|.  x - hi is

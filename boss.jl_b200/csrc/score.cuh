@@ -273,8 +273,8 @@ __global__ void __launch_bounds__(1024) screen_consts_kernel(const double *Xt, c
       tfrag[f] = hi;
       tfrag[f + 2] = lo;
     }
-    tn_al[2 * j] = (float)n2;
-    tn_al[2 * j + 1] = (float)alpha[j];
+    tn_al[4 * (j >> 1) + (j & 1)] = (float)n2;   // the norms and the alphas of points 2i, 2i + 1 as FP32 pairs
+    tn_al[4 * (j >> 1) + 2 + (j & 1)] = (float)alpha[j];
     a1 += aj;
     a2 = fma(aj, n2, a2);
   }

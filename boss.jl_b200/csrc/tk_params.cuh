@@ -57,7 +57,7 @@ constexpr int XCOV_KC = 128;  // training points staged per shared-memory pass
 struct ScreenSlice {
   const float4 *tfrag;   // [n_pad / 8][KP / 8][32] per eight-point tile, k-step and lane: the MMA's B fragments of the
                          // centred training inputs t~ = fp32(ut - c), TF32-split: (b0 hi, b1 hi, b0 lo, b1 lo)
-  const float4 *tn_al;   // [n_pad / 2] (|t~_j|^2, alpha_j, |t~_j+1|^2, alpha_j+1) rounded to FP32
+  const float4 *tn_al;   // [n_pad / 2] (|t~_j|^2, |t~_j+1|^2, alpha_j, alpha_j+1) rounded to FP32, j even
   const double *A;       // [SCREEN_NCONST] A1 = sum |alpha_j|, A3 = sum |alpha_j| |ut_j - c|^2, the centre c (DP)
   const double *invl;    // [DP]
   unsigned long long disc_bits;

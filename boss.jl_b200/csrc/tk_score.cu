@@ -80,8 +80,8 @@ __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_gr
 // every slice, then the bound verdicts of those candidates.
 //
 // Means: d2 = |u~|^2 + |t~_j|^2 - 2 u~.t~_j from centred FP32 points.  The cross term runs on the tensor cores
-// (mma.sync TF32, 3-term hi / lo split, accumulated in FP32); the norms are added and kappa_f32 evaluated on the
-// accumulator fragments.  Warp w takes candidates 16w..16w+15 against the 16 eight-point tiles of each 128-point stage of
+// (mma.sync TF32, 3-term hi / lo split, accumulated in FP32); the norms are added and kappa_f32x2 evaluated on the
+// accumulator fragments, training points 2t and 2t + 1 as the two lanes of the packed FP32 instructions.  Warp w takes candidates 16w..16w+15 against the 16 eight-point tiles of each 128-point stage of
 // training points.  A thread holds candidates g and g + 8 (g = lane / 4) against training points 2t, 2t + 1 of each tile
 // (t = lane % 4); each run of 4 tiles (8 points per candidate) is summed in FP32 and added to an FP64 accumulator, the
 // four lanes of a candidate are combined by a fixed butterfly, and the stage's two halves (tiles 0-7, 8-15) are scaled
@@ -149,7 +149,7 @@ __global__ void __launch_bounds__(256) screen_mean_bound_kernel(ScreenF32Params 
           alo[ks][e] = __float_as_uint(ua[128 * KP + o]);
         }
     }
-    const float nu0 = snu[16 * w + g], nu1 = snu[16 * w + g + 8];
+    const float2 nu0 = f2(snu[16 * w + g]), nu1 = f2(snu[16 * w + g + 8]);
     double mu0 = 0.0, mu1 = 0.0;   // candidates g and g + 8
     for (int st = 0; st < nst; ++st) {
       __syncthreads();   // slot (st + 1) & 1 is no longer read (stage st - 1, or the candidates' fragments)
@@ -163,7 +163,7 @@ __global__ void __launch_bounds__(256) screen_mean_bound_kernel(ScreenF32Params 
         double acc0 = 0.0, acc1 = 0.0;
 #pragma unroll
         for (int run = 0; run < 2; ++run) {
-          float s0 = 0.0f, s1 = 0.0f;
+          float2 s0 = f2(0.0f), s1 = f2(0.0f);   // points 2t and 2t + 1 of the run's tiles, summed apart
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
             const int nt = kh * 8 + run * 4 + u;
@@ -176,13 +176,16 @@ __global__ void __launch_bounds__(256) screen_mean_bound_kernel(ScreenF32Params 
               mma_tf32(c, ahi[ks], __float_as_uint(b.x), __float_as_uint(b.y));
             }
             const float4 na = snt[nt * 4 + t];   // points 2t, 2t + 1 of the tile
-            s0 = fmaf(na.y, kappa_f32<KID>(fmaxf(c[0] + nu0 + na.x, 0.0f)), s0);
-            s0 = fmaf(na.w, kappa_f32<KID>(fmaxf(c[1] + nu0 + na.z, 0.0f)), s0);
-            s1 = fmaf(na.y, kappa_f32<KID>(fmaxf(c[2] + nu1 + na.x, 0.0f)), s1);
-            s1 = fmaf(na.w, kappa_f32<KID>(fmaxf(c[3] + nu1 + na.z, 0.0f)), s1);
+            const float2 tn = make_float2(na.x, na.y), al = make_float2(na.z, na.w);
+            float2 d0 = __fadd2_rn(__fadd2_rn(make_float2(c[0], c[1]), nu0), tn);
+            float2 d1 = __fadd2_rn(__fadd2_rn(make_float2(c[2], c[3]), nu1), tn);
+            d0 = make_float2(fmaxf(d0.x, 1e-30f), fmaxf(d0.y, 1e-30f));
+            d1 = make_float2(fmaxf(d1.x, 1e-30f), fmaxf(d1.y, 1e-30f));
+            s0 = __ffma2_rn(al, kappa_f32x2<KID>(d0), s0);
+            s1 = __ffma2_rn(al, kappa_f32x2<KID>(d1), s1);
           }
-          acc0 += (double)s0;
-          acc1 += (double)s1;
+          acc0 += (double)(s0.x + s0.y);
+          acc1 += (double)(s1.x + s1.y);
         }
         acc0 += __shfl_xor_sync(0xffffffffu, acc0, 1);
         acc1 += __shfl_xor_sync(0xffffffffu, acc1, 1);
@@ -268,11 +271,16 @@ bool launch_mma_d2(int dp, const float *u, const float *t, const float *nu, cons
   }
 }
 
-// FP32 kappa at d2 = r^2 (rounded to FP32) for the error-bound sweep of the tests
+// The FP32 tier's kappa_f32x2 at d2 = max(fp32(r^2), 1e-30), as the tier clamps it, for the error-bound sweep of the
+// tests: thread i evaluates distances 2i and 2i + 1 as the two lanes
 template <int KID>
 __global__ void kappa_f32_sweep_kernel(const double *r, int n, double *out) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) out[i] = (double)kappa_f32<KID>((float)(r[i] * r[i]));
+  const int i = 2 * (blockIdx.x * blockDim.x + threadIdx.x);
+  if (i >= n) return;
+  const double r1 = i + 1 < n ? r[i + 1] : 0.0;
+  const float2 k = kappa_f32x2<KID>(make_float2(fmaxf((float)(r[i] * r[i]), 1e-30f), fmaxf((float)(r1 * r1), 1e-30f)));
+  out[i] = (double)k.x;
+  if (i + 1 < n) out[i + 1] = (double)k.y;
 }
 
 // full posterior covariance of a small candidate batch (cov / mean_and_cov, gaussian_process.jl:163-167,180-184)
@@ -397,7 +405,7 @@ bool launch_screen_mean_bound(int kid, int dp, const ScreenF32Params &p, int nbl
 #undef CALL
 }
 bool launch_kappa_f32_sweep(int kid, const double *r, int n, double *out, cudaStream_t st) {
-  const int nb = (n + 255) / 256;
+  const int nb = (n + 511) / 512;
   if (n < 1) return true;
   if (kid == 0) kappa_f32_sweep_kernel<0><<<nb, 256, 0, st>>>(r, n, out);
   else if (kid == 1) kappa_f32_sweep_kernel<1><<<nb, 256, 0, st>>>(r, n, out);

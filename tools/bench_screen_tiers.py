@@ -27,7 +27,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CH0 = 75_776                 # the first chunk of the bench problem (FP64 tier), candidates
-SASS_INSTR_PER_PAIR = 14.0   # the MMA mean loop at DP = 8: about 900 instructions per 64 pairs a thread (cuobjdump -sass)
+SASS_INSTR_PER_PAIR = 10.6   # the MMA mean loop at DP = 8: 676 instructions per 64 pairs a thread (cuobjdump -sass)
+MUFU_PER_PAIR = 2            # rsqrt and ex2 (Matern52)
 sys.path.insert(0, ROOT)
 sys.dont_write_bytecode = True
 
@@ -172,7 +173,8 @@ def main():
                     "pairs_per_s": pairs / (v["us"] * 1e-6),
                     "bound_issue_pairs_per_s (assumed: 1 warp instruction / clock / SM sub-partition, "
                     "SASS_INSTR_PER_PAIR from cuobjdump)": 4 * 148 * clk * 32 / SASS_INSTR_PER_PAIR,
-                    "bound_mufu_pairs_per_s (assumed: 16 MUFU results / clock / SM, 2 per pair)": 16 * 148 * clk / 2}
+                    f"bound_mufu_pairs_per_s (assumed: 16 MUFU results / clock / SM, {MUFU_PER_PAIR} per pair)":
+                        16 * 148 * clk / MUFU_PER_PAIR}
         for k in ("BOSS_SCREEN_F64", "BOSS_SCREEN_NO_RESEED"):
             os.environ.pop(k, None)
         with open(args.profile, "w") as f:
